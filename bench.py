@@ -2,7 +2,7 @@
 """bench.py — BM4D denoise voxels/s on a synthetic uint16 1024^3 ExaSPIM-like
 volume, z-slab sharded over N B200s (BASELINE.json metric, configs[3]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--size S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--size S] [--dump-outputs DIR]
 
 One step = one full two-stage BM4D denoise (hard threshold + Wiener) of the
 whole volume: every rank denoises its z-slab (+ halos on the global grid, no
@@ -21,6 +21,13 @@ per-slab uint16 histograms for the global offset / sigma statistics.
 --impl reference times the reference arm: the reference's BM4D is the closed
 third-party wheel bm4d==4.2.5 (absent from this image and un-installable, no
 network), so the arm runs this repo's CPU restatement (oracle/) — labelled as such.
+
+--dump-outputs DIR writes what the last timed step returned, so that two builds
+can be compared output for output on the same seeded input:
+  denoised.npy    float32, the denoised volume at DUMP_VOXELS seeded flat
+                  positions (every voxel when the volume is smaller), ascending
+  tile_stats.npy  float64, the step's tile statistics in b4d_stats field order
+                  (n, n_nonzero, offset, median, mad, sigma, vmin, vmax)
 """
 import argparse
 import json
@@ -46,6 +53,7 @@ import numpy as np  # noqa: E402
 SIGMA = 24.0  # scripts/precompute.py:284
 SEED = 4  # SURVEY §8d config 4
 NS, LBLK, K_HT, K_WIE = 11, 4, 16, 32
+DUMP_VOXELS = 1 << 22  # --dump-outputs: 16 MiB of float32 at most
 
 
 def log(*a):
@@ -82,6 +90,39 @@ def make_sample_host(shape):
     from b4d import synth
 
     return synth.vol(shape[0], shape[1], shape[2], seed=SEED, sigma=SIGMA)
+
+
+def dump_sample_index(size):
+    """Ascending flat indices into the size^3 volume of the voxels --dump-outputs writes: all of them up to
+    DUMP_VOXELS, else a draw seeded by SEED, so that it depends on the size alone (not on the run or the world size)."""
+    n = size ** 3
+    if n <= DUMP_VOXELS:
+        return np.arange(n, dtype=np.int64)
+    return np.unique(np.random.default_rng(SEED).integers(0, n, DUMP_VOXELS, dtype=np.int64))
+
+
+def dump_outputs(path, y, stats, size, own_b, own_e, world, rank, device):
+    """Write the sampled denoised volume and the tile statistics of one step to path (rank 0).  Each rank fills
+    the sampled voxels of its owned planes [own_b, own_e); the others stay 0, so an integer sum over the ranks
+    assembles the float32 bit patterns unchanged."""
+    import torch
+    import torch.distributed as dist
+
+    from b4d import _lib
+
+    idx = dump_sample_index(size)
+    plane = size * size
+    lo, hi = (int(i) for i in np.searchsorted(idx, (own_b * plane, own_e * plane)))
+    bits = torch.zeros(idx.size, dtype=torch.int32, device=device)
+    mine = torch.from_numpy(idx[lo:hi] - own_b * plane).to(device)
+    bits[lo:hi] = y.reshape(-1)[mine].view(torch.int32)
+    if world > 1:
+        dist.all_reduce(bits)
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+        np.save(os.path.join(path, "denoised.npy"), bits.cpu().numpy().view(np.float32))
+        np.save(os.path.join(path, "tile_stats.npy"), np.array([stats[k] for k, _ in _lib.Stats._fields_], np.float64))
+        log("outputs of the last timed step written to %s (%d sampled voxels)" % (path, idx.size))
 
 
 # --------------------------------------------------------------- clocks ------
@@ -284,7 +325,13 @@ def main():
     ap.add_argument("--no-exchange", action="store_true",
                     help="N > 1: 26-plane halos and no data-path exchange instead of 13-plane halos + one "
                          "neighbour exchange of basic-estimate planes between the stages")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned to DIR/*.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs dumps the GPU path; --impl reference has no such output")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -396,9 +443,10 @@ def main():
     launches = 0
     barrier()
     ev0.record(ext)
-    for _ in range(args.steps):
+    for i in range(args.steps):
         stats, y = step_resident()
-        del y
+        if i + 1 < args.steps:  # the last step's output stays for --dump-outputs
+            del y
         tm = dn.last_timings()
         for k, (ms, nl) in tm.items():
             fam[k] = fam.get(k, 0.0) + ms
@@ -410,6 +458,9 @@ def main():
     log("rank %d host ms per step (warm-up included): %s" % (rank, {k: round(v / (args.steps + max(args.warmup, 3)), 2) for k, v in host_ms.items()}))
     clocks = sampler.stop() if rank == 0 else None
     mstats = dn.last_match_stats()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, y, stats, S, own_b, own_e, world, rank, dev)
+    del y
 
     # ---- the HBM-bound tail of the path: fused offset-subtract + noise-scaled quantize (K7) on the
     # denoised slab, device in / device out, timed alone (burst) with CUDA events

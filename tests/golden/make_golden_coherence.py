@@ -1,28 +1,31 @@
-"""Golden vectors for the spatial-coherence gate, made by RUNNING THE REFERENCE (this container only).
+"""Golden vectors for the spatial-coherence gate, made by RUNNING THE REFERENCE.
 
-    python tests/golden/make_golden_coherence.py
+    python tests/golden/make_golden_coherence.py REFERENCE_CHECKOUT
 
-Imports machine_learning/metrics.py straight from /root/reference/src (read-only, nothing copied) and records, for
+Imports machine_learning/metrics.py straight from REFERENCE_CHECKOUT/src (read-only, nothing copied) and records, for
 seeded patches (labels uint64, raw float32 counts): patch_has_incoherent_segment(labels, raw, ...)
 (metrics.py:189-260) and, per segment, local_autocorr(raw, labels == id, lag) (:64-112) and
 highfreq_energy_fraction(raw, labels == id, smooth = gaussian_filter(raw, sigma)) (:115-155).  Cases, in the spirit
 of tests/test_metrics.py:24-40: a smooth PSF-like blob (coherent), a salt-and-pepper block (the artifact), both in
 one patch, a thin faint neurite, a segment below the voxel minimum, a constant segment (degenerate variance), a
-ragged shape, other lags / sigmas / thresholds.  /root/reference does not exist on the GPU box: the vectors travel
-as tests/golden/reference_coherence.npz.
+ragged shape, other lags / sigmas / thresholds.  The inputs are not stored (the seeded noise does not compress): the
+tests rebuild them with cases() and check them against the SHA-256 digest kept in tests/golden/reference_coherence.npz
+next to the reference's outputs.
 """
+import hashlib
 import importlib.util
 import os
+import sys
 
 import numpy as np
 from scipy import ndimage
 
-REF = "/root/reference/src/aind_exaspim_image_compression/machine_learning"
+REF_SUBDIR = os.path.join("src", "aind_exaspim_image_compression", "machine_learning")
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def _load(name):
-    spec = importlib.util.spec_from_file_location("ref_" + name, os.path.join(REF, name + ".py"))
+def _load(ref, name):
+    spec = importlib.util.spec_from_file_location("ref_" + name, os.path.join(ref, REF_SUBDIR, name + ".py"))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     return mod
@@ -40,6 +43,14 @@ def salt_pepper(shape, lo, hi, amp, rate, rng):
     region[lo[0]:hi[0], lo[1]:hi[1], lo[2]:hi[2]] = True
     v[(rng.random(shape) < rate) & region] = amp
     return v, region
+
+
+def digest(labels, raw):
+    """SHA-256 of one case's inputs (shape, uint64 labels, float32 raw) as 32 uint8."""
+    h = hashlib.sha256(repr(labels.shape).encode())
+    h.update(np.ascontiguousarray(labels, np.uint64).tobytes())
+    h.update(np.ascontiguousarray(raw, np.float32).tobytes())
+    return np.frombuffer(h.digest(), np.uint8)
 
 
 def cases():
@@ -91,8 +102,8 @@ def cases():
     return out
 
 
-def main():
-    me = _load("metrics")
+def main(ref):
+    me = _load(ref, "metrics")
     data = {}
     cs = cases()
     for i, (lab, raw, kw) in enumerate(cs):
@@ -102,8 +113,7 @@ def main():
         ids = np.unique(lab[lab > 0])
         sc = np.array([[float((lab == l).sum()), me.local_autocorr(raw, lab == l, lag=lag),
                         me.highfreq_energy_fraction(raw, lab == l, smooth=smooth)] for l in ids], dtype=np.float64).reshape(-1, 3)
-        data["labels%d" % i] = lab
-        data["raw%d" % i] = raw.astype(np.float32)
+        data["digest%d" % i] = digest(lab, raw)
         data["ids%d" % i] = ids.astype(np.uint64)
         data["scores%d" % i] = sc
         data["verdict%d" % i] = np.array(verdict)
@@ -115,4 +125,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

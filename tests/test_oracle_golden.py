@@ -97,14 +97,20 @@ def test_truncating_variant(oracle_lib):
 
 
 def _coherence_cases():
-    import os
+    """The reference's outputs with their inputs, rebuilt from the seeded recipe of
+    tests/golden/make_golden_coherence.py and checked byte for byte against the digests stored with the outputs."""
+    from golden import make_golden_coherence
 
     g = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_coherence.npz"))
-    for i in range(int(g["n"])):
+    inputs = make_golden_coherence.cases()
+    assert len(inputs) == int(g["n"])
+    for i, (lab, raw, _) in enumerate(inputs):
+        assert np.array_equal(make_golden_coherence.digest(lab, raw), g["digest%d" % i]), \
+            "case %d: the rebuilt inputs are not the ones the reference was run on" % i
         p = g["params%d" % i]
         kw = dict(min_autocorr=float(p[0]), max_highfreq_frac=float(p[1]), min_segment_voxels=int(p[2]),
                   smooth_sigma=float(p[3]), coherence_lag=int(p[4]))
-        yield g["labels%d" % i], g["raw%d" % i], kw, g["ids%d" % i], g["scores%d" % i], bool(g["verdict%d" % i])
+        yield lab, raw, kw, g["ids%d" % i], g["scores%d" % i], bool(g["verdict%d" % i])
 
 
 def test_coherence_gate_restatement_matches_the_reference(oracle_lib):
