@@ -63,6 +63,27 @@ struct DevBuf {
     }
 };
 
+// u = clamp(int(rint((z + cf) * scale)) + ishift, 0, 65535); see oracle MatchMap.
+struct MatchMap {
+    float cf = 0.0f, scale = 1.0f;
+    int ishift = 0;
+    int integral = 1;
+};
+
+// Geometry of one pass: `nvol` volumes of D x H x W and the reference-block origins of each stage along z.
+struct Plan {
+    int D, H, W, nvol;
+    std::vector<int> rz1, rz2, ry, rx;
+};
+
+// Two-call slab form: what b4d_slab_stage2_begin already launched of the stage-2 front end (planes [o0, o1) of
+// the matching image, cell planes [cz0, cz1), tile layers [tz0, tz1) classified and matched).
+struct OwnedFront {
+    bool done = false;
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // device time of part 1, added to the stage-2 matching slot
+    int o0 = 0, o1 = 0, cz0 = 0, cz1 = 0, tz0 = 0, tz1 = 0;
+};
+
 }  // namespace
 
 struct b4d_handle {
@@ -79,21 +100,16 @@ struct b4d_handle {
     long long pass_voxels = CHUNK_VOXELS;  // voxels per pass (b4d_set_pass_voxels)
     long long pipeline_min_voxels = 1ll << 26;  // host transfers are pipelined from this volume size up
     HostMover mover;  // pageable host arrays <-> device (pinned ring + copy threads)
-    // state between b4d_slab_stage1_u16 and b4d_slab_stage2
     // coloured noise (b4d_set_noise_model): relative coefficient variances of both transforms, or white
     bool psd = false;
     float nu_ht[64], nu_wie[64];
+    // state between b4d_slab_stage1_u16 and b4d_slab_stage2: the slab (planes from slab_z_begin on) and its map
     bool slab_open = false;
-    // two-call slab form: what b4d_slab_stage2_begin already launched (planes [pre_o0, pre_o1) of the matching image,
-    // cell planes [pre_cz0, pre_cz1), tile layers [pre_tz0, pre_tz1) classified and matched)
-    bool pre_done = false;
-    cudaEvent_t pre_ev0 = nullptr, pre_ev1 = nullptr;  // device time of part 1, added to the stage-2 matching slot
-    int pre_o0 = 0, pre_o1 = 0, pre_cz0 = 0, pre_cz1 = 0, pre_tz0 = 0, pre_tz1 = 0;
-    int64_t slab_shape[3] = {0, 0, 0};
-    int64_t slab_z_begin = 0, slab_z_total = 0;
+    Plan slab;
+    int64_t slab_z_begin = 0;
     float slab_sigma = 0.f;
-    float slab_cf = 0.f, slab_scale = 1.f;
-    int slab_ishift = 0;
+    MatchMap slab_mm;
+    OwnedFront pre;
 };
 
 namespace {
@@ -224,12 +240,6 @@ B4dTables make_tables(const b4d_profile &p, float sigma, const float *nu_ht = nu
     return t;
 }
 
-// u = clamp(int(rint((z + cf) * scale)) + ishift, 0, 65535); see oracle MatchMap.
-struct MatchMap {
-    float cf = 0.0f, scale = 1.0f;
-    int ishift = 0;
-    int integral = 1;
-};
 int centre_shift(double lo, double hi) { return (int)(std::floor((65535.0 - (hi - lo)) * 0.5) - lo); }
 
 int tau_for(float tau, float sigma, float scale, int Ns, uint32_t *out) {
@@ -245,10 +255,20 @@ int tau_for(float tau, float sigma, float scale, int Ns, uint32_t *out) {
     return 0;
 }
 
-struct Plan {
-    int D, H, W, nvol;
-    std::vector<int> rz1, rz2, ry, rx;
-};
+// Planes [z_begin, z_begin + shape[0]) of a z_total-plane volume: the reference origins along z of each stage are
+// those of the whole volume whose search window lies inside the slab (a whole volume: z_begin = 0, z_total = D).
+Plan make_plan(const int64_t shape[3], int64_t z_begin, int64_t z_total, int nvol, const b4d_profile &p) {
+    Plan pl;
+    pl.D = (int)shape[0];
+    pl.H = (int)shape[1];
+    pl.W = (int)shape[2];
+    pl.nvol = nvol;
+    pl.rz1 = slab_origins(z_total, z_begin, shape[0], p.search_ht / 2);
+    pl.rz2 = slab_origins(z_total, z_begin, shape[0], p.search_wie / 2);
+    pl.ry = ref_origins(shape[1]);
+    pl.rx = ref_origins(shape[2]);
+    return pl;
+}
 
 void fill_geom(const Plan &pl, const std::vector<int> &rz, const int *d_refs, B4dGeom *g) {
     g->D = pl.D;
@@ -266,6 +286,28 @@ void fill_geom(const Plan &pl, const std::vector<int> &rz, const int *d_refs, B4
     g->refx = d_refs + rz.size() + pl.ry.size();
     g->vol_stride = (long long)pl.D * pl.H * pl.W;
     g->refs_per_vol = (long long)g->nrz * g->nry * g->nrx;
+}
+
+// The reference-origin lists of both stages on the device, [rz1 | ry | rx | rz2 | ry | rx], and their geometry.
+int upload_geometry(b4d_handle *h, const Plan &pl, B4dGeom *g1, B4dGeom *g2) {
+    std::vector<int> refs;
+    refs.insert(refs.end(), pl.rz1.begin(), pl.rz1.end());
+    refs.insert(refs.end(), pl.ry.begin(), pl.ry.end());
+    refs.insert(refs.end(), pl.rx.begin(), pl.rx.end());
+    const size_t off2 = refs.size();
+    refs.insert(refs.end(), pl.rz2.begin(), pl.rz2.end());
+    refs.insert(refs.end(), pl.ry.begin(), pl.ry.end());
+    refs.insert(refs.end(), pl.rx.begin(), pl.rx.end());
+    B4D_TRY(h->refs.ensure(refs.size() * sizeof(int)));
+    CU_TRY(cudaMemcpyAsync(h->refs.p, refs.data(), refs.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    CU_TRY(cudaStreamSynchronize(h->stream));  // `refs` is a stack vector
+    fill_geom(pl, pl.rz1, h->refs.as<int>(), g1);
+    fill_geom(pl, pl.rz2, h->refs.as<int>() + off2, g2);
+    const long long R1 = g1->refs_per_vol * pl.nvol, R2 = g2->refs_per_vol * pl.nvol;
+    if ((long long)pl.nvol * g1->tz * g1->ty * g1->tx > 2147483647ll || (R1 + 3) / 4 > 2147483647ll ||
+        (R2 + 3) / 4 > 2147483647ll)
+        return fail(B4D_ERR_TOO_LARGE, "too many reference blocks for one launch");
+    return 0;
 }
 
 // Ordering events owned for the duration of one call: destroyed on every exit path.
@@ -319,124 +361,109 @@ struct StageClock {
     }
 };
 
-// The two-stage pipeline on device-resident inputs.
-//   d_zf   float32 noisy volumes            [nvol*V]
-//   d_u    uint16 matching image (stage 1)  [nvol*V]   (overwritten by stage 2)
-//   d_out  float32 result                   [nvol*V]
-// Where the result goes when it is wanted in HOST memory: planes [p0, p1) of the (single)
-// volume, to `host` (p1 - p0 planes).  Stage 2 then runs in z chunks and every chunk of
-// finished planes is normalised and copied out on a second stream while the next chunks
-// still compute — the device-to-host copy (4 B/voxel over PCIe) hides behind the filter.
+// Where the result goes when it is wanted in HOST memory: planes [p0, p1) of the (single) volume, to `host`
+// (p1 - p0 planes).  stage2_back then runs the filter in z chunks and every chunk of finished planes is
+// normalised and copied out on a second stream while the next chunks still compute — the device-to-host copy
+// (4 B/voxel over PCIe) hides behind the filter.
 struct HostSink {
     void *host = nullptr;  // float32, or uint16 with a QuantSpec
     long long p0 = 0, p1 = 0;
-    bool done = false;  // set when run_pipeline delivered the result itself
+    bool done = false;  // set when stage2_back delivered the result itself
 };
 // Fused K6 + K7: the last normalise writes q = quantize(result) as uint16 instead of the float32 result
-// (d_out of run_pipeline then points at uint16 storage; 2 B/voxel leave the device instead of 4).
+// (the pass's `out` then points at uint16 storage; 2 B/voxel leave the device instead of 4).
 struct QuantSpec {
     float sub = 0.f, add = 0.f, step = 1.f;
     int trunc = 0;
 };
 
-// Where the input comes from when it is a uint16 volume in HOST memory: it is uploaded in z
-// chunks on the copy stream and the stage-1 front end (float conversion, block energies, tile
-// classification, matching) follows chunk by chunk, so that the host-to-device copy (2 B/voxel
-// over PCIe) hides behind the stage-1 matcher.  d_u / d_zf of run_pipeline are the destinations.
-struct HostSource {
-    const uint16_t *host = nullptr;
-    bool used = false;       // set when run_pipeline did the upload itself
-    int ishift = 0;          // centre shift of the stage-2 matching image (from the data range)
-};
 constexpr int UPLOAD_CHUNKS = 8;
 // Chunked launches under-fill the GPU on small volumes (a 128^3 patch ran 1.5x slower in 8 chunks and its
 // whole upload takes 0.1 ms), so the transfers are pipelined only from `pipeline_min_voxels` up.
 bool can_stream_upload(const b4d_handle *h, const Plan &pl) {
     return pl.nvol == 1 && ((long long)pl.H * pl.W) % 8 == 0 && pl.D >= 16 * UPLOAD_CHUNKS &&
-           (long long)pl.D * pl.H * pl.W >= h->pipeline_min_voxels;
+           (long long)pl.D * pl.H * pl.W >= h->pipeline_min_voxels && !pl.rz1.empty();
 }
 
-// phase 0 = both stages; 1 = stage 1 only (basic estimate left in h->basic); 2 = stage 2 only
-// (h->basic holds the basic estimate, possibly completed by a neighbour exchange).
-int run_pipeline(b4d_handle *h, const Plan &pl, const float *d_zf, uint16_t *d_u, const MatchMap &mm_in, float sigma,
-                 float *d_out, StageClock &clk, int phase = 0, HostSink *sink = nullptr, HostSource *src = nullptr,
-                 const QuantSpec *q = nullptr) {
-    const b4d_profile &p = h->prof;
-    MatchMap mm = mm_in;
-    const long long V = (long long)pl.D * pl.H * pl.W, TV = V * pl.nvol;
-    cudaStream_t s = h->stream;
+// The two-word min / max sink of the uint16 conversion kernels: reset before the launch, read back after it
+// (this synchronises `s`).
+int range_reset(DevBuf &sink, cudaStream_t s) {
+    B4D_TRY(sink.ensure(64));
+    const unsigned init[2] = {0xFFFFu, 0u};
+    CU_TRY(cudaMemcpyAsync(sink.p, init, sizeof(init), cudaMemcpyHostToDevice, s));
+    return 0;
+}
+int range_read(const DevBuf &sink, cudaStream_t s, double *lo, double *hi) {
+    unsigned got[2] = {0, 0};
+    CU_TRY(cudaMemcpyAsync(got, sink.p, sizeof(got), cudaMemcpyDeviceToHost, s));
+    CU_TRY(cudaStreamSynchronize(s));
+    *lo = got[0];
+    *hi = got[1];
+    return 0;
+}
 
+// One pass of the two-stage pipeline over device-resident volumes, set up once per call by make_pass:
+//   zf     float32 noisy volumes            [nvol*V]
+//   u      uint16 matching image of stage 1 [nvol*V]   (overwritten by that of stage 2)
+//   basic  float32 basic estimate           [nvol*V]   (h->basic, or `out` when profile.stages = 1)
+//   out    result                           [nvol*V]   (float32, or uint16 with a QuantSpec)
+struct Pass {
+    b4d_handle *h;
+    const Plan *pl;
+    StageClock *clk;
+    MatchMap mm;  // a streamed stage-1 upload sets ishift from the data range
+    float *zf;
+    uint16_t *u;
+    float *basic, *out;
+    long long TV, R1, R2;  // voxels and reference blocks of each stage, all volumes
+    B4dGeom g1, g2;
+    B4dTables tab;
+    MatchParams mp1, mp2;
+    FilterParams fp1, fp2;
+};
+
+int make_pass(b4d_handle *h, const Plan &pl, float sigma, const MatchMap &mm, float *zf, uint16_t *u, float *out,
+              StageClock &clk, Pass &ps) {
+    const b4d_profile &p = h->prof;
     uint32_t tau1 = 0, tau2 = 0;
     B4D_TRY(tau_for(p.tau_ht, sigma, mm.scale, p.search_ht, &tau1));
     if (p.stages == 2) B4D_TRY(tau_for(p.tau_wie, sigma, mm.scale, p.search_wie, &tau2));
-
-    // reference-origin lists: [rz1 | ry | rx | rz2 | ry | rx]
-    std::vector<int> refs;
-    refs.insert(refs.end(), pl.rz1.begin(), pl.rz1.end());
-    refs.insert(refs.end(), pl.ry.begin(), pl.ry.end());
-    refs.insert(refs.end(), pl.rx.begin(), pl.rx.end());
-    const size_t off2 = refs.size();
-    refs.insert(refs.end(), pl.rz2.begin(), pl.rz2.end());
-    refs.insert(refs.end(), pl.ry.begin(), pl.ry.end());
-    refs.insert(refs.end(), pl.rx.begin(), pl.rx.end());
-    B4D_TRY(h->refs.ensure(refs.size() * sizeof(int)));
-    CU_TRY(cudaMemcpyAsync(h->refs.p, refs.data(), refs.size() * sizeof(int), cudaMemcpyHostToDevice, s));
-    CU_TRY(cudaStreamSynchronize(s));  // `refs` is a stack vector
-
-    B4dGeom g1, g2;
-    fill_geom(pl, pl.rz1, h->refs.as<int>(), &g1);
-    fill_geom(pl, pl.rz2, h->refs.as<int>() + off2, &g2);
-    const long long R1 = g1.refs_per_vol * pl.nvol, R2 = g2.refs_per_vol * pl.nvol;
-    if ((long long)pl.nvol * g1.tz * g1.ty * g1.tx > 2147483647ll || (R1 + 3) / 4 > 2147483647ll ||
-        (R2 + 3) / 4 > 2147483647ll)
-        return fail(B4D_ERR_TOO_LARGE, "too many reference blocks for one launch");
-    const int Kmax = std::max(p.k_ht, p.k_wie);
-    B4D_TRY(h->widx.ensure((size_t)std::max(R1, R2) * Kmax * sizeof(uint16_t)));
-    B4D_TRY(h->cnt.ensure((size_t)std::max(R1, R2)));
-    B4D_TRY(h->basic.ensure((size_t)TV * sizeof(float)));
-    B4D_TRY(h->s2.ensure((size_t)TV * sizeof(uint2)));
-    {
-        const size_t ncell = (size_t)pl.nvol * pl.D * g1.ty * g1.tx;  // per-plane window ranges of every tile
-        const size_t ntile = (size_t)pl.nvol * std::max(g1.tz, g2.tz) * g1.ty * g1.tx;
-        B4D_TRY(h->cells.ensure(ncell * sizeof(uint32_t)));
-        B4D_TRY(h->tcls.ensure(ntile * sizeof(uint32_t)));
-    }
+    B4D_TRY(upload_geometry(h, pl, &ps.g1, &ps.g2));
+    ps.h = h;
+    ps.pl = &pl;
+    ps.clk = &clk;
+    ps.mm = mm;
+    ps.zf = zf;
+    ps.u = u;
+    ps.out = out;
+    ps.TV = (long long)pl.D * pl.H * pl.W * pl.nvol;
+    ps.R1 = ps.g1.refs_per_vol * pl.nvol;
+    ps.R2 = ps.g2.refs_per_vol * pl.nvol;
+    const long long Rmax = std::max(ps.R1, ps.R2);
+    B4D_TRY(h->widx.ensure((size_t)Rmax * std::max(p.k_ht, p.k_wie) * sizeof(uint16_t)));
+    B4D_TRY(h->cnt.ensure((size_t)Rmax));
+    B4D_TRY(h->basic.ensure((size_t)ps.TV * sizeof(float)));
+    B4D_TRY(h->s2.ensure((size_t)ps.TV * sizeof(uint2)));
+    const size_t ncell = (size_t)pl.nvol * pl.D * ps.g1.ty * ps.g1.tx;  // per-plane window ranges of every tile
+    const size_t ntile = (size_t)pl.nvol * std::max(ps.g1.tz, ps.g2.tz) * ps.g1.ty * ps.g1.tx;
+    B4D_TRY(h->cells.ensure(ncell * sizeof(uint32_t)));
+    B4D_TRY(h->tcls.ensure(ntile * sizeof(uint32_t)));
     B4D_TRY(h->stats.ensure(4 * sizeof(unsigned long long)));
     // Both stages aggregate in order-independent fixed point (int64): the result does not
     // depend on scheduling, a slab equals the whole volume bit for bit, and the basic estimate
     // that feeds the stage-2 matching (a discontinuous decision) is reproducible.
     // profile.deterministic is kept in the ABI and is always honoured.
-    B4D_TRY(h->numq.ensure((size_t)TV * sizeof(long long)));
-    B4D_TRY(h->gmap.ensure((size_t)TV * sizeof(uint32_t)));
-    const B4dTables tab = make_tables(p, sigma, h->psd ? h->nu_ht : nullptr, h->psd ? h->nu_wie : nullptr);
+    B4D_TRY(h->numq.ensure((size_t)ps.TV * sizeof(long long)));
+    B4D_TRY(h->gmap.ensure((size_t)ps.TV * sizeof(uint32_t)));
+    ps.tab = make_tables(p, sigma, h->psd ? h->nu_ht : nullptr, h->psd ? h->nu_wie : nullptr);
     if (h->psd && (p.search_ht > 11 || p.search_wie > 11))
         return fail(B4D_ERR_UNSUPPORTED, "a coloured-noise model needs search windows of at most 11");
-    b4d_upload_tables(tab, s);
-    if (phase < 2) CU_TRY(cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), s));
+    b4d_upload_tables(ps.tab, h->stream);  // on every call: the tables are shared by all handles
+    ps.basic = p.stages == 1 ? out : h->basic.as<float>();
 
-    auto zero_acc = [&]() -> int {
-        CU_TRY(cudaMemsetAsync(h->numq.p, 0, (size_t)TV * sizeof(long long), s));
-        CU_TRY(cudaMemsetAsync(h->gmap.p, 0, (size_t)TV * sizeof(uint32_t), s));
-        return 0;
-    };
-    auto normalise = [&](const float *fb, float *dst) {
-        b4d_launch_normalise_wm(h->numq.as<long long>(), h->gmap.as<uint32_t>(), fb, dst, pl.D, pl.H, pl.W, pl.nvol,
-                                0, pl.D, 1.0f / mm.scale, tab.kf, s);
-    };
-
-    float *d_basic = (p.stages == 1 && phase == 0) ? d_out : h->basic.as<float>();
-    bool fused_match = false;
-    MatchParams mp;
-    FilterParams fp;
-    if (phase < 2) {
-    // ---- stage 1: hard thresholding
-    B4D_TRY(zero_acc());
-    const bool streamed = src && src->host && can_stream_upload(h, pl) && R1 > 0;
-    clk.mark(B4D_T_PREP, 1);
-    if (!streamed) b4d_launch_block_energy(d_u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, pl.nvol, s);
-    clk.mark(B4D_T_K0, 1);
-    mp.g = g1;
-    mp.u = d_u;
+    MatchParams &mp = ps.mp1;
+    mp.g = ps.g1;
+    mp.u = u;
     mp.s21 = h->s2.as<uint2>();
     mp.cells = h->cells.as<uint32_t>();
     mp.tcls = h->tcls.as<uint32_t>();
@@ -446,50 +473,14 @@ int run_pipeline(b4d_handle *h, const Plan &pl, const float *d_zf, uint16_t *d_u
     mp.cnt = h->cnt.as<uint8_t>();
     mp.ssd_out = nullptr;
     mp.stats = h->stats.as<unsigned long long>();
-    if (streamed) {
-        const long long P = (long long)pl.H * pl.W;
-        const int E = p.search_ht + 12, cd = (pl.D + 3) / 4;
-        B4D_TRY(h->sink.ensure(64));
-        const unsigned init[2] = {0xFFFFu, 0u};
-        CU_TRY(cudaMemcpyAsync(h->sink.p, init, sizeof(init), cudaMemcpyHostToDevice, s));
-        EventSet owned;
-        cudaEvent_t evs[UPLOAD_CHUNKS];
-        int zprev = 0, odone = 0, cdone = 0, tdone = 0;
-        for (int k = 0; k < UPLOAD_CHUNKS; ++k) {
-            int zu = (k + 1 == UPLOAD_CHUNKS) ? pl.D : (int)(((long long)(k + 1) * pl.D / UPLOAD_CHUNKS + 3) & ~3ll);
-            zu = std::min(zu, pl.D);
-            CU_TRY(copy_in(h, d_u + zprev * P, src->host + zprev * P, (size_t)(zu - zprev) * P * sizeof(uint16_t), 0,
-                           h->copy_stream));
-            CU_TRY(owned.make(&evs[k]));
-            CU_TRY(cudaEventRecord(evs[k], h->copy_stream));
-            CU_TRY(cudaStreamWaitEvent(s, evs[k], 0));
-            // planes [0, zu) are on the device: everything that needs no plane beyond zu - 1
-            b4d_launch_u16_to_f32(d_u + zprev * P, const_cast<float *>(d_zf) + zprev * P, (long long)(zu - zprev) * P,
-                                  h->sink.as<unsigned>(), s);
-            const int o1 = (zu == pl.D) ? pl.D - 3 : zu - 3;            // block origins with all 4 planes present
-            b4d_launch_block_energy_range(d_u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, 1, odone, o1, s);
-            odone = std::max(odone, o1);
-            const int c1 = (zu == pl.D) ? cd : zu / 4;                   // complete 4-plane cells
-            int t1 = tdone;                                              // tile layers whose neighbourhood is complete
-            while (t1 < g1.tz && std::min(pl.rz1[4 * t1] - p.search_ht / 2 + E - 1, pl.D - 1) < zu) ++t1;
-            b4d_launch_match_range(mp, p.search_ht, cdone, c1, (long long)tdone * g1.ty * g1.tx,
-                                   (long long)t1 * g1.ty * g1.tx, s);
-            cdone = c1;
-            tdone = t1;
-            zprev = zu;
-        }
-        unsigned got[2] = {0, 0};
-        CU_TRY(cudaMemcpyAsync(got, h->sink.p, sizeof(got), cudaMemcpyDeviceToHost, s));
-        CU_TRY(cudaStreamSynchronize(s));
-        mm.ishift = centre_shift((double)got[0], (double)got[1]);
-        src->ishift = mm.ishift;
-        src->used = true;
-    } else if (R1 > 0) {
-        b4d_launch_match(mp, p.search_ht, s);
-    }
-    clk.mark(B4D_T_MATCH1, 4);
-    fp.g = g1;
-    fp.zf = d_zf;
+    ps.mp2 = mp;
+    ps.mp2.g = ps.g2;
+    ps.mp2.tau = tau2;
+    ps.mp2.K = p.k_wie;
+
+    FilterParams &fp = ps.fp1;
+    fp.g = ps.g1;
+    fp.zf = zf;
     fp.basic = nullptr;
     fp.widx = mp.widx;
     fp.cnt = mp.cnt;
@@ -500,148 +491,230 @@ int run_pipeline(b4d_handle *h, const Plan &pl, const float *d_zf, uint16_t *d_u
     fp.qscale = mm.scale;  // data * scale spans at most the 16-bit matching range: terms stay below 2^39
     fp.numq = h->numq.as<long long>();
     fp.gmap = h->gmap.as<uint32_t>();
-    if (R1 > 0) b4d_launch_filter(fp, false, s);
-    clk.mark(B4D_T_FILTER1, 1);
-    if (phase == 0 && p.stages == 2) {
-        // the normalise kernel also writes the matching image of stage 2 (rint(basic * scale) + shift): the
-        // separate conversion pass (4 B read + 2 B write per voxel) is not needed
-        b4d_launch_normalise_match(h->numq.as<long long>(), h->gmap.as<uint32_t>(), d_zf, d_basic, d_u, mm.scale,
-                                   mm.ishift, pl.D, pl.H, pl.W, pl.nvol, 1.0f / mm.scale, tab.kf, s);
-        fused_match = true;
-    } else {
-        normalise(d_zf, d_basic);
+    ps.fp2 = fp;
+    ps.fp2.g = ps.g2;
+    ps.fp2.basic = ps.basic;
+    ps.fp2.K = p.k_wie;
+    ps.fp2.Ns = p.search_wie;
+    return 0;
+}
+
+int zero_acc(const Pass &ps) {
+    CU_TRY(cudaMemsetAsync(ps.h->numq.p, 0, (size_t)ps.TV * sizeof(long long), ps.h->stream));
+    CU_TRY(cudaMemsetAsync(ps.h->gmap.p, 0, (size_t)ps.TV * sizeof(uint32_t), ps.h->stream));
+    return 0;
+}
+
+// Planes [z0, z1) of every volume of the accumulators divided out: num / den from `fallback` into `dst`, or
+// quantized into `dst` as uint16 with `q`.
+void normalise(const Pass &ps, const float *fallback, float *dst, int z0, int z1, const QuantSpec *q, cudaStream_t s) {
+    const Plan &pl = *ps.pl;
+    const long long *numq = ps.h->numq.as<long long>();
+    const uint32_t *gmap = ps.h->gmap.as<uint32_t>();
+    if (q)
+        b4d_launch_normalise_q16(numq, gmap, fallback, reinterpret_cast<uint16_t *>(dst), pl.D, pl.H, pl.W, pl.nvol,
+                                 z0, z1, 1.0f / ps.mm.scale, ps.tab.kf, q->sub, q->add, q->step, q->trunc, s);
+    else
+        b4d_launch_normalise_wm(numq, gmap, fallback, dst, pl.D, pl.H, pl.W, pl.nvol, z0, z1, 1.0f / ps.mm.scale,
+                                ps.tab.kf, s);
+}
+
+// Stage-1 front end of one uint16 volume in host memory: it is uploaded in z chunks on the copy stream and the
+// float conversion, block energies, tile classification and matching follow chunk by chunk, so that the
+// host-to-device copy (2 B/voxel over PCIe) hides behind the stage-1 matcher.  The data range sets the centre
+// shift of the stage-2 matching image.
+int stage1_streamed_front(Pass &ps, const uint16_t *host_src) {
+    b4d_handle *h = ps.h;
+    const Plan &pl = *ps.pl;
+    const b4d_profile &p = h->prof;
+    cudaStream_t s = h->stream;
+    const long long P = (long long)pl.H * pl.W;
+    const int E = p.search_ht + 12, cd = (pl.D + 3) / 4;
+    B4D_TRY(range_reset(h->sink, s));
+    EventSet owned;
+    cudaEvent_t evs[UPLOAD_CHUNKS];
+    int zprev = 0, odone = 0, cdone = 0, tdone = 0;
+    for (int k = 0; k < UPLOAD_CHUNKS; ++k) {
+        int zu = (k + 1 == UPLOAD_CHUNKS) ? pl.D : (int)(((long long)(k + 1) * pl.D / UPLOAD_CHUNKS + 3) & ~3ll);
+        zu = std::min(zu, pl.D);
+        CU_TRY(copy_in(h, ps.u + zprev * P, host_src + zprev * P, (size_t)(zu - zprev) * P * sizeof(uint16_t), 0,
+                       h->copy_stream));
+        CU_TRY(owned.make(&evs[k]));
+        CU_TRY(cudaEventRecord(evs[k], h->copy_stream));
+        CU_TRY(cudaStreamWaitEvent(s, evs[k], 0));
+        // planes [0, zu) are on the device: everything that needs no plane beyond zu - 1
+        b4d_launch_u16_to_f32(ps.u + zprev * P, ps.zf + zprev * P, (long long)(zu - zprev) * P, h->sink.as<unsigned>(),
+                              s);
+        const int o1 = (zu == pl.D) ? pl.D - 3 : zu - 3;            // block origins with all 4 planes present
+        b4d_launch_block_energy_range(ps.u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, 1, odone, o1, s);
+        odone = std::max(odone, o1);
+        const int c1 = (zu == pl.D) ? cd : zu / 4;                   // complete 4-plane cells
+        int t1 = tdone;                                              // tile layers whose neighbourhood is complete
+        while (t1 < ps.g1.tz && std::min(pl.rz1[4 * t1] - p.search_ht / 2 + E - 1, pl.D - 1) < zu) ++t1;
+        b4d_launch_match_range(ps.mp1, p.search_ht, cdone, c1, (long long)tdone * ps.g1.ty * ps.g1.tx,
+                               (long long)t1 * ps.g1.ty * ps.g1.tx, s);
+        cdone = c1;
+        tdone = t1;
+        zprev = zu;
     }
+    double lo = 0, hi = 0;
+    B4D_TRY(range_read(h->sink, s, &lo, &hi));
+    ps.mm.ishift = centre_shift(lo, hi);
+    return 0;
+}
+
+// Stage 1, hard thresholding: block energies and matching on the uint16 image, filter, normalise into the basic
+// estimate.  `host_src`: the uint16 volume is still in host memory and is uploaded here (can_stream_upload
+// holds).  `fuse_match`: the normalise also writes the stage-2 matching image rint(basic * scale) + shift, so that
+// the separate conversion pass (4 B read + 2 B write per voxel) is not needed.
+int stage1(Pass &ps, const uint16_t *host_src, bool fuse_match) {
+    b4d_handle *h = ps.h;
+    const Plan &pl = *ps.pl;
+    const b4d_profile &p = h->prof;
+    cudaStream_t s = h->stream;
+    StageClock &clk = *ps.clk;
+    CU_TRY(cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), s));
+    B4D_TRY(zero_acc(ps));
+    clk.mark(B4D_T_PREP, 1);
+    if (!host_src) b4d_launch_block_energy(ps.u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, pl.nvol, s);
+    clk.mark(B4D_T_K0, 1);
+    if (host_src)
+        B4D_TRY(stage1_streamed_front(ps, host_src));
+    else if (ps.R1 > 0)
+        b4d_launch_match(ps.mp1, p.search_ht, s);
+    clk.mark(B4D_T_MATCH1, 4);
+    if (ps.R1 > 0) b4d_launch_filter(ps.fp1, false, s);
+    clk.mark(B4D_T_FILTER1, 1);
+    if (fuse_match)
+        b4d_launch_normalise_match(h->numq.as<long long>(), h->gmap.as<uint32_t>(), ps.zf, ps.basic, ps.u,
+                                   ps.mm.scale, ps.mm.ishift, pl.D, pl.H, pl.W, pl.nvol, 1.0f / ps.mm.scale,
+                                   ps.tab.kf, s);
+    else
+        normalise(ps, ps.zf, ps.basic, 0, pl.D, nullptr, s);
     clk.mark(B4D_T_NORM1, 1);
     CU_TRY(cudaGetLastError());
-    }
-    if (p.stages == 1 || phase == 1) return 0;
-    if (phase >= 2) {  // the stage-1 call filled everything but the stage-2 specific fields
-        mp.u = d_u;
-        mp.s21 = h->s2.as<uint2>();
-        mp.cells = h->cells.as<uint32_t>();
-        mp.tcls = h->tcls.as<uint32_t>();
-        mp.widx = h->widx.as<uint16_t>();
-        mp.cnt = h->cnt.as<uint8_t>();
-        mp.ssd_out = nullptr;
-        mp.stats = h->stats.as<unsigned long long>();
-        fp.zf = d_zf;
-        fp.widx = mp.widx;
-        fp.cnt = mp.cnt;
-        fp.nseg = 1;
-        fp.psd = h->psd ? 1 : 0;
-        fp.qscale = mm.scale;
-        fp.numq = h->numq.as<long long>();
-        fp.gmap = h->gmap.as<uint32_t>();
-    }
+    return 0;
+}
 
-    // ---- stage 2: Wiener, matching on the basic estimate
-    mp.g = g2;
-    mp.tau = tau2;
-    mp.K = p.k_wie;
-    const long long Pv = (long long)pl.H * pl.W;
-    const long long tiles_per_layer = (long long)g2.ty * g2.tx;
-    const int cd2 = (pl.D + 3) / 4;
-    if (phase == 3) {
-        // Two-call slab form, part 1 (b4d_slab_stage2_begin): everything of the stage-2 front end that does not
-        // read a plane outside [pre_o0, pre_o1) — the planes a neighbour exchange is about to overwrite lie
-        // outside.  Launched and left running: the exchange overlaps it.
-        const int o0 = h->pre_o0, o1 = h->pre_o1, E2 = p.search_wie + 12, r2 = p.search_wie / 2;
-        h->pre_cz0 = (o0 + 3) / 4;
-        h->pre_cz1 = (o1 == pl.D) ? cd2 : o1 / 4;
-        int t0 = 0, t1 = g2.tz;
-        auto layer_inside = [&](int tz) {
-            const int bz = pl.rz2[4 * tz] - r2;
-            const int zlo = std::max(bz, 0), zhi = std::min(bz + E2 - 1, pl.D - 1);
-            return zlo / 4 >= h->pre_cz0 && zhi / 4 < h->pre_cz1 && zlo >= o0 && zhi < o1;
-        };
-        while (t0 < g2.tz && !layer_inside(t0)) ++t0;
-        t1 = t0;
-        while (t1 < g2.tz && layer_inside(t1)) ++t1;
-        h->pre_tz0 = t0;
-        h->pre_tz1 = t1;
-        if (o1 > o0)
-            b4d_launch_to_match(d_basic + (long long)o0 * Pv, d_u + (long long)o0 * Pv, (long long)(o1 - o0) * Pv, 0.0f,
-                                mm.scale, mm.ishift, s);
-        B4D_TRY(zero_acc());
-        b4d_launch_block_energy_range(d_u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, 1, o0, std::max(o0, o1 - 3), s);
-        if (R2 > 0)
-            b4d_launch_match_range(mp, p.search_wie, h->pre_cz0, std::max(h->pre_cz0, h->pre_cz1), t0 * tiles_per_layer,
-                                   t1 * tiles_per_layer, s);
-        h->pre_done = true;
-        CU_TRY(cudaGetLastError());
-        return 0;
+// Stage-2 front end on the whole basic estimate: its matching image (unless stage 1 already wrote it), block
+// energies, matching.
+int stage2_front_whole(Pass &ps, bool already_converted) {
+    b4d_handle *h = ps.h;
+    const Plan &pl = *ps.pl;
+    cudaStream_t s = h->stream;
+    if (!already_converted) b4d_launch_to_match(ps.basic, ps.u, ps.TV, 0.0f, ps.mm.scale, ps.mm.ishift, s);
+    B4D_TRY(zero_acc(ps));
+    ps.clk->mark(B4D_T_PREP, 2);
+    b4d_launch_block_energy(ps.u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, pl.nvol, s);
+    ps.clk->mark(B4D_T_K0, 1);
+    if (ps.R2 > 0) b4d_launch_match(ps.mp2, h->prof.search_wie, s);
+    ps.clk->mark(B4D_T_MATCH2, 4);
+    return 0;
+}
+
+// Two-call slab form, part 1 (b4d_slab_stage2_begin): everything of the stage-2 front end that reads no plane
+// outside the owned planes [o0, o1) — the planes a neighbour exchange is about to overwrite lie outside.
+// Launched and left running: the exchange overlaps it.  h->pre records the ranges for stage2_front_rest.
+int stage2_front_owned(Pass &ps, int o0, int o1) {
+    b4d_handle *h = ps.h;
+    const Plan &pl = *ps.pl;
+    cudaStream_t s = h->stream;
+    OwnedFront &f = h->pre;
+    const long long Pv = (long long)pl.H * pl.W, tiles_per_layer = (long long)ps.g2.ty * ps.g2.tx;
+    const int E2 = h->prof.search_wie + 12, r2 = h->prof.search_wie / 2;
+    f.o0 = o0;
+    f.o1 = o1;
+    f.cz0 = (o0 + 3) / 4;
+    f.cz1 = (o1 == pl.D) ? (pl.D + 3) / 4 : o1 / 4;
+    auto layer_inside = [&](int tz) {
+        const int bz = pl.rz2[4 * tz] - r2;
+        const int zlo = std::max(bz, 0), zhi = std::min(bz + E2 - 1, pl.D - 1);
+        return zlo / 4 >= f.cz0 && zhi / 4 < f.cz1 && zlo >= o0 && zhi < o1;
+    };
+    f.tz0 = 0;
+    while (f.tz0 < ps.g2.tz && !layer_inside(f.tz0)) ++f.tz0;
+    f.tz1 = f.tz0;
+    while (f.tz1 < ps.g2.tz && layer_inside(f.tz1)) ++f.tz1;
+    if (o1 > o0)
+        b4d_launch_to_match(ps.basic + o0 * Pv, ps.u + o0 * Pv, (long long)(o1 - o0) * Pv, 0.0f, ps.mm.scale,
+                            ps.mm.ishift, s);
+    B4D_TRY(zero_acc(ps));
+    b4d_launch_block_energy_range(ps.u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, 1, o0, std::max(o0, o1 - 3), s);
+    if (ps.R2 > 0)
+        b4d_launch_match_range(ps.mp2, h->prof.search_wie, f.cz0, std::max(f.cz0, f.cz1), f.tz0 * tiles_per_layer,
+                               f.tz1 * tiles_per_layer, s);
+    f.done = true;
+    CU_TRY(cudaGetLastError());
+    return 0;
+}
+
+// Part 2: the rest of the stage-2 front end (planes, origins, cells and tile layers outside the ranges of part 1).
+int stage2_front_rest(Pass &ps) {
+    b4d_handle *h = ps.h;
+    const Plan &pl = *ps.pl;
+    cudaStream_t s = h->stream;
+    OwnedFront &f = h->pre;
+    const long long Pv = (long long)pl.H * pl.W, tiles_per_layer = (long long)ps.g2.ty * ps.g2.tx;
+    const int o0 = f.o0, o1 = f.o1;
+    if (o0 > 0) b4d_launch_to_match(ps.basic, ps.u, o0 * Pv, 0.0f, ps.mm.scale, ps.mm.ishift, s);
+    if (o1 < pl.D)
+        b4d_launch_to_match(ps.basic + o1 * Pv, ps.u + o1 * Pv, (pl.D - o1) * Pv, 0.0f, ps.mm.scale, ps.mm.ishift, s);
+    b4d_launch_block_energy_range(ps.u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, 1, 0, std::min(o0, pl.D - 3), s);
+    b4d_launch_block_energy_range(ps.u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, 1, std::max(o0, o1 - 3), pl.D - 3, s);
+    ps.clk->mark(B4D_T_PREP, 4);
+    if (ps.R2 > 0) {
+        b4d_launch_match_range(ps.mp2, h->prof.search_wie, 0, f.cz0, 0, f.tz0 * tiles_per_layer, s);
+        b4d_launch_match_range(ps.mp2, h->prof.search_wie, std::max(f.cz0, f.cz1), (pl.D + 3) / 4,
+                               f.tz1 * tiles_per_layer, (long long)ps.g2.tz * tiles_per_layer, s);
     }
-    if (phase == 2 && h->pre_done) {
-        // part 2: the rest of the front end (planes, origins, cells and tile layers outside the ranges of part 1)
-        const int o0 = h->pre_o0, o1 = h->pre_o1;
-        if (o0 > 0) b4d_launch_to_match(d_basic, d_u, (long long)o0 * Pv, 0.0f, mm.scale, mm.ishift, s);
-        if (o1 < pl.D)
-            b4d_launch_to_match(d_basic + (long long)o1 * Pv, d_u + (long long)o1 * Pv, (long long)(pl.D - o1) * Pv, 0.0f,
-                                mm.scale, mm.ishift, s);
-        b4d_launch_block_energy_range(d_u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, 1, 0, std::min(o0, pl.D - 3), s);
-        b4d_launch_block_energy_range(d_u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, 1, std::max(o0, o1 - 3), pl.D - 3, s);
-        clk.mark(B4D_T_PREP, 4);
-        if (R2 > 0) {
-            b4d_launch_match_range(mp, p.search_wie, 0, h->pre_cz0, 0, h->pre_tz0 * tiles_per_layer, s);
-            b4d_launch_match_range(mp, p.search_wie, std::max(h->pre_cz0, h->pre_cz1), cd2, h->pre_tz1 * tiles_per_layer,
-                                   (long long)g2.tz * tiles_per_layer, s);
-        }
-        clk.mark(B4D_T_MATCH2, 8);
-        h->pre_done = false;
-    } else {
-        if (!fused_match) b4d_launch_to_match(d_basic, d_u, TV, 0.0f, mm.scale, mm.ishift, s);
-        B4D_TRY(zero_acc());
-        clk.mark(B4D_T_PREP, 2);
-        b4d_launch_block_energy(d_u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, pl.nvol, s);
-        clk.mark(B4D_T_K0, 1);
-        if (R2 > 0) b4d_launch_match(mp, p.search_wie, s);
-        clk.mark(B4D_T_MATCH2, 4);
-    }
-    fp.g = g2;
-    fp.basic = d_basic;
-    fp.K = p.k_wie;
-    fp.Ns = p.search_wie;
+    ps.clk->mark(B4D_T_MATCH2, 8);
+    f.done = false;
+    return 0;
+}
+
+// Stage 2, Wiener: the filter and the normalise into `out` (quantized with `q`).  A large single volume whose
+// result goes to host memory (`sink`) is filtered in z chunks, see HostSink.
+int stage2_back(Pass &ps, HostSink *sink, const QuantSpec *q) {
+    b4d_handle *h = ps.h;
+    const Plan &pl = *ps.pl;
+    cudaStream_t s = h->stream;
+    StageClock &clk = *ps.clk;
     const long long P = (long long)pl.H * pl.W;
     constexpr int NCH = 8;
-    const int nseg_ch = (sink && sink->host && pl.nvol == 1 && R2 > 0 && (P & 3) == 0 && TV >= h->pipeline_min_voxels)
-                            ? b4d_filter_segments(fp, true, NCH)
+    const int nseg_ch = (sink && sink->host && pl.nvol == 1 && ps.R2 > 0 && (P & 3) == 0 &&
+                         ps.TV >= h->pipeline_min_voxels)
+                            ? b4d_filter_segments(ps.fp2, true, NCH)
                             : 0;
     if (nseg_ch >= NCH && nseg_ch % NCH == 0) {
         // chunked: launch everything on the compute stream first (events between the chunks), then
         // queue normalise + copy of the planes each chunk finishes on the copy stream
-        const int spc = nseg_ch / NCH, r2 = p.search_wie / 2;
+        const int spc = nseg_ch / NCH, r2 = h->prof.search_wie / 2;
         EventSet owned;
         cudaEvent_t evs[NCH];
         for (int c = 0; c < NCH; ++c) {
-            b4d_launch_filter_segments(fp, true, nseg_ch, c * spc, spc, s);
+            b4d_launch_filter_segments(ps.fp2, true, nseg_ch, c * spc, spc, s);
             CU_TRY(owned.make(&evs[c]));
             CU_TRY(cudaEventRecord(evs[c], s));
         }
         clk.mark(B4D_T_FILTER2, NCH);
+        const size_t esz = q ? sizeof(uint16_t) : sizeof(float);
         long long zdone = 0;
         for (int c = 0; c < NCH; ++c) {
             // after chunk c: no later segment touches a plane below the window of its first reference
             long long zfin = pl.D;
             if (c + 1 < NCH) {
-                const int iz_next = (int)((long long)(c + 1) * spc * g2.nrz / nseg_ch);
+                const int iz_next = (int)((long long)(c + 1) * spc * ps.g2.nrz / nseg_ch);
                 zfin = std::max<long long>(0, (long long)pl.rz2[iz_next] - r2);
             }
             CU_TRY(cudaStreamWaitEvent(h->copy_stream, evs[c], 0));
             if (zfin > zdone) {
                 // origins below zfin are final as well: a block touches its own origin plane
-                if (q)
-                    b4d_launch_normalise_q16(h->numq.as<long long>(), h->gmap.as<uint32_t>(), d_basic,
-                                             reinterpret_cast<uint16_t *>(d_out), pl.D, pl.H, pl.W, 1, (int)zdone, (int)zfin,
-                                             1.0f / mm.scale, tab.kf, q->sub, q->add, q->step, q->trunc, h->copy_stream);
-                else
-                    b4d_launch_normalise_wm(h->numq.as<long long>(), h->gmap.as<uint32_t>(), d_basic, d_out, pl.D, pl.H,
-                                            pl.W, 1, (int)zdone, (int)zfin, 1.0f / mm.scale, tab.kf, h->copy_stream);
+                normalise(ps, ps.basic, ps.out, (int)zdone, (int)zfin, q, h->copy_stream);
                 const long long a = std::max(zdone, sink->p0), b = std::min(zfin, sink->p1);
-                const size_t esz = q ? sizeof(uint16_t) : sizeof(float);
                 if (b > a)
                     CU_TRY(copy_out(h, static_cast<char *>(sink->host) + (size_t)(a - sink->p0) * P * esz,
-                                    reinterpret_cast<char *>(d_out) + (size_t)a * P * esz, (size_t)(b - a) * P * esz, 0,
-                                    h->copy_stream));
+                                    reinterpret_cast<char *>(ps.out) + (size_t)a * P * esz, (size_t)(b - a) * P * esz,
+                                    0, h->copy_stream));
                 zdone = zfin;
             }
         }
@@ -651,17 +724,21 @@ int run_pipeline(b4d_handle *h, const Plan &pl, const float *d_zf, uint16_t *d_u
         CU_TRY(cudaGetLastError());
         return 0;
     }
-    if (R2 > 0) b4d_launch_filter(fp, true, s);
+    if (ps.R2 > 0) b4d_launch_filter(ps.fp2, true, s);
     clk.mark(B4D_T_FILTER2, 1);
-    if (q)
-        b4d_launch_normalise_q16(h->numq.as<long long>(), h->gmap.as<uint32_t>(), d_basic,
-                                 reinterpret_cast<uint16_t *>(d_out), pl.D, pl.H, pl.W, pl.nvol, 0, pl.D, 1.0f / mm.scale,
-                                 tab.kf, q->sub, q->add, q->step, q->trunc, s);
-    else
-        normalise(d_basic, d_out);
+    normalise(ps, ps.basic, ps.out, 0, pl.D, q, s);
     clk.mark(B4D_T_NORM2, 1);
     CU_TRY(cudaGetLastError());
     return 0;
+}
+
+// Both stages of one pass (stage 1 alone when profile.stages = 1).
+int denoise_pass(Pass &ps, const uint16_t *host_src, HostSink *sink, const QuantSpec *q) {
+    const bool two = ps.h->prof.stages == 2;
+    B4D_TRY(stage1(ps, host_src, two));
+    if (!two) return 0;
+    B4D_TRY(stage2_front_whole(ps, true));
+    return stage2_back(ps, sink, q);
 }
 
 // float32 input -> matching map (shift, scale); mirrors oracle derive_match_map.
@@ -718,18 +795,11 @@ int derive_match_map(b4d_handle *h, const float *d_in, long long n, float sigma,
 // uint16 input: float copy + the centring shift of the stage-2 matching image
 // (stage 1 matches on the raw integers; mirrors oracle denoise_one).
 int convert_u16(b4d_handle *h, const uint16_t *d_in, float *d_zf, long long n, MatchMap *mm) {
-    cudaStream_t s = h->stream;
-    B4D_TRY(h->sink.ensure(64));
-    const unsigned init[2] = {0xFFFFu, 0u};
-    CU_TRY(cudaMemcpyAsync(h->sink.p, init, sizeof(init), cudaMemcpyHostToDevice, s));
-    b4d_launch_u16_to_f32(d_in, d_zf, n, h->sink.as<unsigned>(), s);
-    unsigned got[2] = {0, 0};
-    CU_TRY(cudaMemcpyAsync(got, h->sink.p, sizeof(got), cudaMemcpyDeviceToHost, s));
-    CU_TRY(cudaStreamSynchronize(s));
-    const double lo = got[0], hi = got[1];
-    mm->integral = 1;
-    mm->scale = 1.0f;
-    mm->cf = 0.0f;
+    B4D_TRY(range_reset(h->sink, h->stream));
+    b4d_launch_u16_to_f32(d_in, d_zf, n, h->sink.as<unsigned>(), h->stream);
+    double lo = 0, hi = 0;
+    B4D_TRY(range_read(h->sink, h->stream, &lo, &hi));
+    *mm = MatchMap();  // integral, unit scale
     mm->ishift = centre_shift(lo, hi);
     return 0;
 }
@@ -749,6 +819,36 @@ void reset_timings(b4d_handle *h) {
     }
 }
 
+// The end of a denoise call: wait for the compute stream, book the stage timings, fetch the matcher statistics.
+int finish(b4d_handle *h, StageClock &clk) {
+    CU_TRY(cudaStreamSynchronize(h->stream));
+    clk.resolve();
+    CU_TRY(cudaMemcpy(h->match_stats, h->stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+// One uint16 volume or slab in: from host memory and large enough, it stays there for stage 1 to upload behind
+// the matcher (*host_src = in); otherwise it is copied to h->in and converted into h->zf with its matching map.
+int stage_u16_input(b4d_handle *h, const Plan &pl, const uint16_t *in, int in_on_device, StageClock &clk,
+                    MatchMap *mm, const uint16_t **host_src) {
+    const long long V = (long long)pl.D * pl.H * pl.W;
+    B4D_TRY(h->in.ensure((size_t)V * sizeof(uint16_t)));
+    B4D_TRY(h->u16.ensure((size_t)V * sizeof(uint16_t) + 16));
+    B4D_TRY(h->zf.ensure((size_t)V * sizeof(float)));
+    B4D_TRY(h->out.ensure((size_t)V * sizeof(float)));
+    *host_src = nullptr;
+    if (!in_on_device && can_stream_upload(h, pl)) {
+        *host_src = in;
+        clk.mark(-1, 0);
+    } else {
+        CU_TRY(copy_in(h, h->in.p, in, (size_t)V * sizeof(uint16_t), in_on_device, h->stream));
+        clk.mark(-1, 0);
+        B4D_TRY(convert_u16(h, h->in.as<uint16_t>(), h->zf.as<float>(), V, mm));
+    }
+    clk.mark(B4D_T_PREP, 1);
+    return 0;
+}
+
 // Batched denoise, chunked so scratch stays bounded.
 template <class T>
 int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3], float sigma, float *out,
@@ -759,13 +859,7 @@ int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3],
     const long long V = shape[0] * shape[1] * shape[2];
     const int64_t per = std::max<int64_t>(1, std::min<int64_t>(n, h->pass_voxels / V));
     cudaStream_t s = h->stream;
-    Plan pl;
-    pl.D = (int)shape[0];
-    pl.H = (int)shape[1];
-    pl.W = (int)shape[2];
-    pl.rz1 = pl.rz2 = ref_origins(shape[0]);
-    pl.ry = ref_origins(shape[1]);
-    pl.rx = ref_origins(shape[2]);
+    Plan pl = make_plan(shape, 0, shape[0], 1, h->prof);
     StageClock clk(h);
     for (int64_t i0 = 0; i0 < n; i0 += per) {
         const int64_t nb = std::min<int64_t>(per, n - i0);
@@ -773,12 +867,9 @@ int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3],
         pl.nvol = (int)nb;
         // input -> device (always into an aligned scratch copy)
         B4D_TRY(h->in.ensure((size_t)TV * sizeof(T)));
-        HostSource src;
         // one uint16 volume from host memory: uploaded in chunks behind the stage-1 matcher
-        const bool stream_in = sizeof(T) == 2 && !in_dev && nb == 1 && can_stream_upload(h, pl);
-        if (stream_in) src.host = reinterpret_cast<const uint16_t *>(in + i0 * V);
-        else
-            CU_TRY(copy_in(h, h->in.p, in + i0 * V, (size_t)TV * sizeof(T), in_dev, s));
+        const bool stream_in = sizeof(T) == 2 && !in_dev && can_stream_upload(h, pl);
+        if (!stream_in) CU_TRY(copy_in(h, h->in.p, in + i0 * V, (size_t)TV * sizeof(T), in_dev, s));
         B4D_TRY(h->u16.ensure((size_t)TV * sizeof(uint16_t) + 16));
         float *d_out = nullptr;
         if (out_dev && (reinterpret_cast<uintptr_t>(out + i0 * V) & 15) == 0) {
@@ -789,7 +880,7 @@ int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3],
         }
         MatchMap mm;
         float centre = 0.0f;
-        const float *d_zf = nullptr;
+        float *d_zf = nullptr;
         uint16_t *d_u = h->u16.as<uint16_t>();
         clk.mark(-1, 0);
         if (sizeof(T) == 2) {
@@ -807,21 +898,30 @@ int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3],
             d_zf = h->in.as<float>();
         }
         clk.mark(B4D_T_PREP, 2);
-        HostSink sink;
-        if (!out_dev && nb == 1 && h->prof.stages == 2 && centre == 0.0f) {
-            sink.host = out + i0 * V;
-            sink.p0 = 0;
-            sink.p1 = pl.D;
-        }
-        B4D_TRY(run_pipeline(h, pl, d_zf, d_u, mm, sigma, d_out, clk, 0, &sink, &src));
+        const bool to_host = !out_dev && nb == 1 && h->prof.stages == 2 && centre == 0.0f;
+        HostSink sink{to_host ? out + i0 * V : nullptr, 0, pl.D};
+        Pass ps;
+        B4D_TRY(make_pass(h, pl, sigma, mm, d_zf, d_u, d_out, clk, ps));
+        B4D_TRY(denoise_pass(ps, stream_in ? reinterpret_cast<const uint16_t *>(in + i0 * V) : nullptr, &sink,
+                             nullptr));
         if (centre != 0.0f) b4d_launch_add_scalar(d_out, TV, centre, s);
         if (!sink.done && d_out != out + i0 * V)
             CU_TRY(copy_out(h, out + i0 * V, d_out, (size_t)TV * sizeof(float), out_dev, s));
-        CU_TRY(cudaStreamSynchronize(s));
-        clk.resolve();
+        B4D_TRY(finish(h, clk));
     }
-    CU_TRY(cudaMemcpy(h->match_stats, h->stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     return 0;
+}
+
+// The open slab of the two-call form and an owned range inside it.
+int check_open_slab(const b4d_handle *h, int64_t own_begin, int64_t own_end) {
+    if (!h->slab_open) return fail(B4D_ERR_INVALID, "b4d_slab_stage1_u16 has not been called");
+    if (own_begin < h->slab_z_begin || own_end > h->slab_z_begin + h->slab.D || own_begin >= own_end)
+        return fail(B4D_ERR_INVALID, "owned range outside the slab");
+    return 0;
+}
+int make_slab_pass(b4d_handle *h, StageClock &clk, Pass &ps) {
+    return make_pass(h, h->slab, h->slab_sigma, h->slab_mm, h->zf.as<float>(), h->in.as<uint16_t>(),
+                     h->out.as<float>(), clk, ps);
 }
 
 }  // namespace
@@ -880,6 +980,8 @@ void b4d_destroy(b4d_handle *h) {
                       &h->ssd, &h->refs, &h->hist, &h->partial, &h->sink, &h->stats, &h->s2, &h->cells, &h->tcls,
                       &h->alt_in, &h->alt_zf, &h->alt_out, &h->alt_partial, &h->alt_sink})
         b->release();
+    if (h->pre.ev0) cudaEventDestroy(h->pre.ev0);
+    if (h->pre.ev1) cudaEventDestroy(h->pre.ev1);
     if (h->stream) cudaStreamDestroy(h->stream);
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
     delete h;
@@ -910,11 +1012,12 @@ int b4d_set_pass_voxels(b4d_handle *h, int64_t voxels) {
     return 0;
 }
 
-// One uint16 volume larger than a pass: z-slabs with the no-exchange halo, one after the other on this
-// GPU (b4d_denoise_slab_u16); equal to the one-pass result bit for bit, like the multi-GPU slabs.
-static int denoise_oversize_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3], float sigma, float *out,
-                                int in_on_device, int out_on_device) {
-    const int64_t D = shape[0], P = shape[1] * shape[2];
+// `n` uint16 volumes, each larger than a pass: z-slabs with the no-exchange halo, one after the other on this
+// GPU (b4d_denoise_slab_u16); equal to the one-pass result bit for bit, like the multi-GPU slabs.  The timings
+// and match statistics are summed over all slabs.
+static int denoise_oversize_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3], float sigma,
+                                float *out, int in_on_device, int out_on_device) {
+    const int64_t D = shape[0], P = shape[1] * shape[2], V = D * P;
     const int64_t halo = (h->prof.search_ht + 2) + (h->prof.stages == 2 ? h->prof.search_wie + 2 : 0);
     const int64_t planes = h->pass_voxels / P;
     if (planes < 2 * halo + 4)
@@ -925,22 +1028,21 @@ static int denoise_oversize_u16(b4d_handle *h, const uint16_t *in, const int64_t
     float t_ms[B4D_T_COUNT] = {};
     int64_t launches[B4D_T_COUNT] = {};
     unsigned long long stats[4] = {};
-    for (int64_t ob = 0; ob < D; ob += own) {
-        const int64_t oe = std::min(D, ob + own), zb = std::max<int64_t>(0, ob - halo), ze = std::min(D, oe + halo);
-        const int64_t sshape[3] = {ze - zb, shape[1], shape[2]};
-        B4D_TRY(b4d_denoise_slab_u16(h, in + zb * P, sshape, zb, D, ob, oe, sigma, out + ob * P, in_on_device,
-                                     out_on_device));
-        for (int i = 0; i < B4D_T_COUNT; ++i) {
-            t_ms[i] += h->t_ms[i];
-            launches[i] += h->launches[i];
+    for (int64_t i = 0; i < n; ++i)
+        for (int64_t ob = 0; ob < D; ob += own) {
+            const int64_t oe = std::min(D, ob + own), zb = std::max<int64_t>(0, ob - halo), ze = std::min(D, oe + halo);
+            const int64_t sshape[3] = {ze - zb, shape[1], shape[2]};
+            B4D_TRY(b4d_denoise_slab_u16(h, in + i * V + zb * P, sshape, zb, D, ob, oe, sigma, out + i * V + ob * P,
+                                         in_on_device, out_on_device));
+            for (int k = 0; k < B4D_T_COUNT; ++k) {
+                t_ms[k] += h->t_ms[k];
+                launches[k] += h->launches[k];
+            }
+            for (int k = 0; k < 4; ++k) stats[k] += h->match_stats[k];
         }
-        for (int i = 0; i < 4; ++i) stats[i] += h->match_stats[i];
-    }
-    for (int i = 0; i < B4D_T_COUNT; ++i) {
-        h->t_ms[i] = t_ms[i];
-        h->launches[i] = launches[i];
-    }
-    for (int i = 0; i < 4; ++i) h->match_stats[i] = stats[i];
+    std::memcpy(h->t_ms, t_ms, sizeof(t_ms));
+    std::memcpy(h->launches, launches, sizeof(launches));
+    std::memcpy(h->match_stats, stats, sizeof(stats));
     return 0;
 }
 
@@ -949,24 +1051,7 @@ int b4d_denoise_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t 
     if (h && in && out && shape && n >= 1 && shape[0] > 0 && shape[1] > 0 && shape[2] > 0 &&
         shape[0] * shape[1] * shape[2] > h->pass_voxels) {
         B4D_TRY(common_checks(h, in, out, shape, sigma));
-        const int64_t V = shape[0] * shape[1] * shape[2];
-        float t_ms[B4D_T_COUNT] = {};
-        int64_t launches[B4D_T_COUNT] = {};
-        unsigned long long stats[4] = {};
-        for (int64_t i = 0; i < n; ++i) {  // every volume of the batch is larger than a pass
-            B4D_TRY(denoise_oversize_u16(h, in + i * V, shape, sigma, out + i * V, in_on_device, out_on_device));
-            for (int k = 0; k < B4D_T_COUNT; ++k) {
-                t_ms[k] += h->t_ms[k];
-                launches[k] += h->launches[k];
-            }
-            for (int k = 0; k < 4; ++k) stats[k] += h->match_stats[k];
-        }
-        for (int k = 0; k < B4D_T_COUNT; ++k) {
-            h->t_ms[k] = t_ms[k];
-            h->launches[k] = launches[k];
-        }
-        for (int k = 0; k < 4; ++k) h->match_stats[k] = stats[k];
-        return 0;
+        return denoise_oversize_u16(h, in, n, shape, sigma, out, in_on_device, out_on_device);
     }
     return denoise_batch<uint16_t>(h, in, n, shape, sigma, out, in_on_device, out_on_device);
 }
@@ -988,13 +1073,7 @@ int b4d_targets_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t 
     // teacher of chunk c - 1 and the raw of chunk c go back and chunk c + 1 comes up on the copy stream.
     if ((!in_on_device || !out_on_device) && per >= 8 && V * per >= h->pipeline_min_voxels) per = (per + 3) / 4;
     cudaStream_t s = h->stream, cs = h->copy_stream;
-    Plan pl;
-    pl.D = (int)shape[0];
-    pl.H = (int)shape[1];
-    pl.W = (int)shape[2];
-    pl.rz1 = pl.rz2 = ref_origins(shape[0]);
-    pl.ry = ref_origins(shape[1]);
-    pl.rx = ref_origins(shape[2]);
+    Plan pl = make_plan(shape, 0, shape[0], 1, h->prof);
     StageClock clk(h);
     EventSet owned;
     DevBuf *b_in[2] = {&h->in, &h->alt_in}, *b_zf[2] = {&h->zf, &h->alt_zf}, *b_out[2] = {&h->out, &h->alt_out};
@@ -1019,18 +1098,15 @@ int b4d_targets_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t 
         B4D_TRY(b_zf[set]->ensure((size_t)TV * sizeof(float)));
         B4D_TRY(b_out[set]->ensure((size_t)TV * sizeof(float)));
         B4D_TRY(b_par[set]->ensure((size_t)nb * sizeof(float)));
-        B4D_TRY(b_sink[set]->ensure(64));
         // copy stream: counts up, raw = float32(counts) - offset, range of the counts.  In stream order this
         // follows the copy-out of chunk c - 2, the last reader of this buffer set.
         CU_TRY(copy_in(h, b_in[set]->p, in + i0 * V, (size_t)TV * sizeof(uint16_t), in_on_device, cs));
         CU_TRY(cudaMemcpyAsync(b_par[set]->p, offsets + i0, (size_t)nb * sizeof(float), cudaMemcpyHostToDevice, cs));
-        const unsigned init[2] = {0xFFFFu, 0u};
-        CU_TRY(cudaMemcpyAsync(b_sink[set]->p, init, sizeof(init), cudaMemcpyHostToDevice, cs));
+        B4D_TRY(range_reset(*b_sink[set], cs));
         b4d_launch_u16_sub_offset(b_in[set]->as<uint16_t>(), b_par[set]->as<float>(), b_zf[set]->as<float>(), V, TV,
                                   b_sink[set]->as<unsigned>(), cs);
-        unsigned got[2] = {0, 0};
-        CU_TRY(cudaMemcpyAsync(got, b_sink[set]->p, sizeof(got), cudaMemcpyDeviceToHost, cs));
-        CU_TRY(cudaStreamSynchronize(cs));
+        double lo = 0, hi = 0;
+        B4D_TRY(range_read(*b_sink[set], cs, &lo, &hi));
         float omin = offsets[i0], omax = offsets[i0];
         for (int64_t k = 0; k < nb; ++k) {
             omin = std::min(omin, offsets[i0 + k]);
@@ -1040,15 +1116,14 @@ int b4d_targets_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t 
         // Matching is invariant to a constant shift per volume: stage 1 matches on the counts themselves,
         // the stage-2 matching image rint(basic) + ishift only has to stay inside uint16.
         MatchMap mm;
-        mm.integral = 1;
-        mm.scale = 1.0f;
-        mm.cf = 0.0f;
-        mm.ishift = centre_shift((double)got[0] - std::ceil((double)omax), (double)got[1] - std::floor((double)omin));
+        mm.ishift = centre_shift(lo - std::ceil((double)omax), hi - std::floor((double)omin));
         // compute stream: the chunk's two stages and the clip (its inputs are complete: the copy stream was
         // synchronised above)
         clk.mark(-1, 0);
-        B4D_TRY(run_pipeline(h, pl, b_zf[set]->as<float>(), b_in[set]->as<uint16_t>(), mm, sigma,
-                             b_out[set]->as<float>(), clk));
+        Pass ps;
+        B4D_TRY(make_pass(h, pl, sigma, mm, b_zf[set]->as<float>(), b_in[set]->as<uint16_t>(),
+                          b_out[set]->as<float>(), clk, ps));
+        B4D_TRY(denoise_pass(ps, nullptr, nullptr, nullptr));
         b4d_launch_clip(b_out[set]->as<float>(), TV, max_count, s);
         cudaEvent_t done;
         CU_TRY(owned.make(&done));
@@ -1064,10 +1139,7 @@ int b4d_targets_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t 
     }
     B4D_TRY(teacher_back());
     CU_TRY(cudaStreamSynchronize(cs));
-    CU_TRY(cudaStreamSynchronize(s));
-    clk.resolve();
-    CU_TRY(cudaMemcpy(h->match_stats, h->stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    return 0;
+    return finish(h, clk);
 }
 
 static int denoise_slab_impl(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
@@ -1081,48 +1153,20 @@ static int denoise_slab_impl(b4d_handle *h, const uint16_t *in, const int64_t sh
         own_begin >= own_end)
         return fail(B4D_ERR_INVALID, "slab / owned range inconsistent");
     reset_timings(h);
-    cudaStream_t s = h->stream;
-    const long long V = shape[0] * shape[1] * shape[2], P = shape[1] * shape[2];
-    Plan pl;
-    pl.D = (int)shape[0];
-    pl.H = (int)shape[1];
-    pl.W = (int)shape[2];
-    pl.nvol = 1;
-    pl.rz1 = slab_origins(z_total, z_begin, shape[0], h->prof.search_ht / 2);
-    pl.rz2 = slab_origins(z_total, z_begin, shape[0], h->prof.search_wie / 2);
-    pl.ry = ref_origins(shape[1]);
-    pl.rx = ref_origins(shape[2]);
-    B4D_TRY(h->in.ensure((size_t)V * sizeof(uint16_t)));
-    B4D_TRY(h->u16.ensure((size_t)V * sizeof(uint16_t) + 16));
-    B4D_TRY(h->zf.ensure((size_t)V * sizeof(float)));
-    B4D_TRY(h->out.ensure((size_t)V * sizeof(float)));
+    const long long P = shape[1] * shape[2];
+    const Plan pl = make_plan(shape, z_begin, z_total, 1, h->prof);
     StageClock clk(h);
     MatchMap mm;
-    HostSource src;
-    if (!in_on_device && can_stream_upload(h, pl) && !pl.rz1.empty()) {
-        src.host = in;  // uploaded in chunks behind the stage-1 matcher (run_pipeline)
-        clk.mark(-1, 0);
-    } else {
-        CU_TRY(copy_in(h, h->in.p, in, (size_t)V * sizeof(uint16_t), in_on_device, s));
-        clk.mark(-1, 0);
-        B4D_TRY(convert_u16(h, h->in.as<uint16_t>(), h->zf.as<float>(), V, &mm));
-    }
-    clk.mark(B4D_T_PREP, 1);
-    HostSink sink;
-    if (!out_on_device) {
-        sink.host = out;
-        sink.p0 = own_begin - z_begin;
-        sink.p1 = own_end - z_begin;
-    }
-    B4D_TRY(run_pipeline(h, pl, h->zf.as<float>(), h->in.as<uint16_t>(), mm, sigma, h->out.as<float>(), clk, 0, &sink,
-                         &src, q));
+    const uint16_t *host_src = nullptr;
+    B4D_TRY(stage_u16_input(h, pl, in, in_on_device, clk, &mm, &host_src));
+    HostSink sink{out_on_device ? nullptr : out, own_begin - z_begin, own_end - z_begin};
+    Pass ps;
+    B4D_TRY(make_pass(h, pl, sigma, mm, h->zf.as<float>(), h->in.as<uint16_t>(), h->out.as<float>(), clk, ps));
+    B4D_TRY(denoise_pass(ps, host_src, &sink, q));
     if (!sink.done)
-        CU_TRY(copy_out(h, out, h->out.as<char>() + (size_t)(own_begin - z_begin) * P * esz,
-                        (size_t)(own_end - own_begin) * P * esz, out_on_device, s));
-    CU_TRY(cudaStreamSynchronize(s));
-    clk.resolve();
-    CU_TRY(cudaMemcpy(h->match_stats, h->stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    return 0;
+        CU_TRY(copy_out(h, out, h->out.as<char>() + (size_t)sink.p0 * P * esz, (size_t)(sink.p1 - sink.p0) * P * esz,
+                        out_on_device, h->stream));
+    return finish(h, clk);
 }
 int b4d_denoise_slab_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
                          int64_t z_total, int64_t own_begin, int64_t own_end, float sigma, float *out,
@@ -1134,11 +1178,7 @@ int b4d_denoise_slab_q16_u16(b4d_handle *h, const uint16_t *in, const int64_t sh
                              int64_t z_total, int64_t own_begin, int64_t own_end, float sigma, float offset_sub,
                              float offset_add, float step, int truncate, uint16_t *out, int in_on_device,
                              int out_on_device) {
-    QuantSpec q;
-    q.sub = offset_sub;
-    q.add = offset_add;
-    q.step = step;
-    q.trunc = truncate;
+    const QuantSpec q{offset_sub, offset_add, step, truncate};
     return denoise_slab_impl(h, in, shape, z_begin, z_total, own_begin, own_end, sigma, out, in_on_device,
                              out_on_device, &q);
 }
@@ -1150,57 +1190,27 @@ int b4d_denoise_q16_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3
                                     truncate, out, in_on_device, out_on_device);
 }
 
-static Plan slab_plan_of(const b4d_handle *h) {
-    Plan pl;
-    pl.D = (int)h->slab_shape[0];
-    pl.H = (int)h->slab_shape[1];
-    pl.W = (int)h->slab_shape[2];
-    pl.nvol = 1;
-    pl.rz1 = slab_origins(h->slab_z_total, h->slab_z_begin, h->slab_shape[0], h->prof.search_ht / 2);
-    pl.rz2 = slab_origins(h->slab_z_total, h->slab_z_begin, h->slab_shape[0], h->prof.search_wie / 2);
-    pl.ry = ref_origins(h->slab_shape[1]);
-    pl.rx = ref_origins(h->slab_shape[2]);
-    return pl;
-}
-
 int b4d_slab_stage1_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin, int64_t z_total,
                         float sigma, int in_on_device) {
     B4D_TRY(common_checks(h, in, in, shape, sigma));
     if (z_begin < 0 || z_begin + shape[0] > z_total) return fail(B4D_ERR_INVALID, "slab range inconsistent");
     if (h->prof.stages != 2) return fail(B4D_ERR_INVALID, "the two-call slab form needs stages = 2");
     reset_timings(h);
-    cudaStream_t s = h->stream;
-    const long long V = shape[0] * shape[1] * shape[2];
-    for (int i = 0; i < 3; ++i) h->slab_shape[i] = shape[i];
-    h->slab_z_begin = z_begin;
-    h->slab_z_total = z_total;
-    h->slab_sigma = sigma;
     h->slab_open = false;
-    const Plan pl = slab_plan_of(h);
-    B4D_TRY(h->in.ensure((size_t)V * sizeof(uint16_t)));
-    B4D_TRY(h->u16.ensure((size_t)V * sizeof(uint16_t) + 16));
-    B4D_TRY(h->zf.ensure((size_t)V * sizeof(float)));
-    B4D_TRY(h->out.ensure((size_t)V * sizeof(float)));
+    h->slab = make_plan(shape, z_begin, z_total, 1, h->prof);
+    h->slab_z_begin = z_begin;
+    h->slab_sigma = sigma;
     StageClock clk(h);
     MatchMap mm;
-    HostSource src;
-    if (!in_on_device && can_stream_upload(h, pl) && !pl.rz1.empty()) {
-        src.host = in;  // uploaded in chunks behind the stage-1 matcher (run_pipeline)
-        clk.mark(-1, 0);
-    } else {
-        CU_TRY(copy_in(h, h->in.p, in, (size_t)V * sizeof(uint16_t), in_on_device, s));
-        clk.mark(-1, 0);
-        B4D_TRY(convert_u16(h, h->in.as<uint16_t>(), h->zf.as<float>(), V, &mm));
-    }
-    clk.mark(B4D_T_PREP, 1);
-    B4D_TRY(run_pipeline(h, pl, h->zf.as<float>(), h->in.as<uint16_t>(), mm, sigma, h->out.as<float>(), clk, 1, nullptr,
-                         &src));
-    CU_TRY(cudaStreamSynchronize(s));
+    const uint16_t *host_src = nullptr;
+    B4D_TRY(stage_u16_input(h, h->slab, in, in_on_device, clk, &mm, &host_src));
+    Pass ps;
+    B4D_TRY(make_pass(h, h->slab, sigma, mm, h->zf.as<float>(), h->in.as<uint16_t>(), h->out.as<float>(), clk, ps));
+    B4D_TRY(stage1(ps, host_src, false));
+    CU_TRY(cudaStreamSynchronize(h->stream));
     clk.resolve();
-    h->pre_done = false;
-    h->slab_cf = mm.cf;
-    h->slab_scale = mm.scale;
-    h->slab_ishift = src.used ? src.ishift : mm.ishift;
+    h->pre.done = false;
+    h->slab_mm = ps.mm;
     h->slab_open = true;
     return 0;
 }
@@ -1209,10 +1219,10 @@ int b4d_slab_basic_planes(b4d_handle *h, int64_t plane0, int64_t nplanes, float 
                           int buf_on_device) {
     if (!h || !buf) return fail(B4D_ERR_INVALID, "NULL argument");
     if (!h->slab_open) return fail(B4D_ERR_INVALID, "b4d_slab_stage1_u16 has not been called");
-    if (plane0 < 0 || nplanes < 0 || plane0 + nplanes > h->slab_shape[0])
+    if (plane0 < 0 || nplanes < 0 || plane0 + nplanes > h->slab.D)
         return fail(B4D_ERR_INVALID, "plane range outside the slab");
     CU_TRY(cudaSetDevice(h->device));
-    const size_t P = (size_t)h->slab_shape[1] * h->slab_shape[2];
+    const size_t P = (size_t)h->slab.H * h->slab.W;
     float *dev = h->basic.as<float>() + (size_t)plane0 * P;
     const size_t bytes = (size_t)nplanes * P * sizeof(float);
     if (to_handle)
@@ -1224,48 +1234,34 @@ int b4d_slab_basic_planes(b4d_handle *h, int64_t plane0, int64_t nplanes, float 
 }
 
 static int slab_stage2_impl(b4d_handle *h, int64_t own_begin, int64_t own_end, void *out, int out_on_device,
-                           const QuantSpec *q) {
+                            const QuantSpec *q) {
     if (!h || !out) return fail(B4D_ERR_INVALID, "NULL argument");
     if (q && !(q->step >= 1.0f)) return fail(B4D_ERR_INVALID, "step must be >= 1");
     const size_t esz = q ? sizeof(uint16_t) : sizeof(float);
-    if (!h->slab_open) return fail(B4D_ERR_INVALID, "b4d_slab_stage1_u16 has not been called");
-    const int64_t zb = h->slab_z_begin, D = h->slab_shape[0];
-    if (own_begin < zb || own_end > zb + D || own_begin >= own_end)
-        return fail(B4D_ERR_INVALID, "owned range outside the slab");
+    B4D_TRY(check_open_slab(h, own_begin, own_end));
     CU_TRY(cudaSetDevice(h->device));
-    cudaStream_t s = h->stream;
-    const long long P = h->slab_shape[1] * h->slab_shape[2];
-    const Plan pl = slab_plan_of(h);
-    const bool had_pre = h->pre_done;
-    MatchMap mm;
-    mm.cf = h->slab_cf;
-    mm.scale = h->slab_scale;
-    mm.ishift = h->slab_ishift;
+    const long long P = (long long)h->slab.H * h->slab.W;
+    const bool had_pre = h->pre.done;
     StageClock clk(h);
     clk.mark(-1, 0);
-    HostSink sink;
-    if (!out_on_device) {
-        sink.host = out;
-        sink.p0 = own_begin - zb;
-        sink.p1 = own_end - zb;
-    }
-    B4D_TRY(run_pipeline(h, pl, h->zf.as<float>(), h->in.as<uint16_t>(), mm, h->slab_sigma, h->out.as<float>(), clk, 2,
-                         &sink, nullptr, q));
+    HostSink sink{out_on_device ? nullptr : out, own_begin - h->slab_z_begin, own_end - h->slab_z_begin};
+    Pass ps;
+    B4D_TRY(make_slab_pass(h, clk, ps));
+    B4D_TRY(had_pre ? stage2_front_rest(ps) : stage2_front_whole(ps, false));
+    B4D_TRY(stage2_back(ps, &sink, q));
     if (!sink.done)
-        CU_TRY(copy_out(h, out, h->out.as<char>() + (size_t)(own_begin - zb) * P * esz,
-                        (size_t)(own_end - own_begin) * P * esz, out_on_device, s));
-    CU_TRY(cudaStreamSynchronize(s));
-    clk.resolve();
+        CU_TRY(copy_out(h, out, h->out.as<char>() + (size_t)sink.p0 * P * esz, (size_t)(sink.p1 - sink.p0) * P * esz,
+                        out_on_device, h->stream));
+    B4D_TRY(finish(h, clk));
     if (had_pre) {
         float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, h->pre_ev0, h->pre_ev1) == cudaSuccess) {
+        if (cudaEventElapsedTime(&ms, h->pre.ev0, h->pre.ev1) == cudaSuccess) {
             h->t_ms[B4D_T_MATCH2] += ms;
             h->launches[B4D_T_MATCH2] += 5;
         } else {
             cudaGetLastError();
         }
     }
-    CU_TRY(cudaMemcpy(h->match_stats, h->stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     h->slab_open = false;
     return 0;
 }
@@ -1274,11 +1270,7 @@ int b4d_slab_stage2(b4d_handle *h, int64_t own_begin, int64_t own_end, float *ou
 }
 int b4d_slab_stage2_q16(b4d_handle *h, int64_t own_begin, int64_t own_end, float offset_sub, float offset_add,
                         float step, int truncate, uint16_t *out, int out_on_device) {
-    QuantSpec q;
-    q.sub = offset_sub;
-    q.add = offset_add;
-    q.step = step;
-    q.trunc = truncate;
+    const QuantSpec q{offset_sub, offset_add, step, truncate};
     return slab_stage2_impl(h, own_begin, own_end, out, out_on_device, &q);
 }
 
@@ -1292,27 +1284,19 @@ float *b4d_slab_basic_ptr(b4d_handle *h) {
 
 int b4d_slab_stage2_begin(b4d_handle *h, int64_t own_begin, int64_t own_end) {
     if (!h) return fail(B4D_ERR_INVALID, "NULL argument");
-    if (!h->slab_open) return fail(B4D_ERR_INVALID, "b4d_slab_stage1_u16 has not been called");
-    const int64_t zb = h->slab_z_begin, D = h->slab_shape[0];
-    if (own_begin < zb || own_end > zb + D || own_begin >= own_end)
-        return fail(B4D_ERR_INVALID, "owned range outside the slab");
+    B4D_TRY(check_open_slab(h, own_begin, own_end));
     CU_TRY(cudaSetDevice(h->device));
-    const Plan pl = slab_plan_of(h);
-    MatchMap mm;
-    mm.cf = h->slab_cf;
-    mm.scale = h->slab_scale;
-    mm.ishift = h->slab_ishift;
     StageClock clk(h);
     clk.mark(-1, 0);
-    h->pre_o0 = (int)(own_begin - zb);
-    h->pre_o1 = (int)(own_end - zb);
-    if (!h->pre_ev0) {
-        CU_TRY(cudaEventCreate(&h->pre_ev0));
-        CU_TRY(cudaEventCreate(&h->pre_ev1));
+    if (!h->pre.ev0) {
+        CU_TRY(cudaEventCreate(&h->pre.ev0));
+        CU_TRY(cudaEventCreate(&h->pre.ev1));
     }
-    CU_TRY(cudaEventRecord(h->pre_ev0, h->stream));
-    B4D_TRY(run_pipeline(h, pl, h->zf.as<float>(), h->in.as<uint16_t>(), mm, h->slab_sigma, h->out.as<float>(), clk, 3));
-    CU_TRY(cudaEventRecord(h->pre_ev1, h->stream));
+    CU_TRY(cudaEventRecord(h->pre.ev0, h->stream));
+    Pass ps;
+    B4D_TRY(make_slab_pass(h, clk, ps));
+    B4D_TRY(stage2_front_owned(ps, (int)(own_begin - h->slab_z_begin), (int)(own_end - h->slab_z_begin)));
+    CU_TRY(cudaEventRecord(h->pre.ev1, h->stream));
     return 0;  // no synchronisation: the launches run while the caller exchanges planes
 }
 
@@ -1325,25 +1309,12 @@ int b4d_match_stage1(b4d_handle *h, const uint16_t *in, const int64_t shape[3], 
     const b4d_profile &p = h->prof;
     cudaStream_t s = h->stream;
     reset_timings(h);
-    Plan pl;
-    pl.D = (int)shape[0];
-    pl.H = (int)shape[1];
-    pl.W = (int)shape[2];
-    pl.nvol = 1;
-    pl.rz1 = pl.rz2 = ref_origins(shape[0]);
-    pl.ry = ref_origins(shape[1]);
-    pl.rx = ref_origins(shape[2]);
-    std::vector<int> refs;
-    refs.insert(refs.end(), pl.rz1.begin(), pl.rz1.end());
-    refs.insert(refs.end(), pl.ry.begin(), pl.ry.end());
-    refs.insert(refs.end(), pl.rx.begin(), pl.rx.end());
+    const Plan pl = make_plan(shape, 0, shape[0], 1, p);
+    B4dGeom g, g_unused;
+    B4D_TRY(upload_geometry(h, pl, &g, &g_unused));
     const long long V = shape[0] * shape[1] * shape[2];
-    B4D_TRY(h->refs.ensure(refs.size() * sizeof(int)));
     B4D_TRY(h->u16.ensure((size_t)V * sizeof(uint16_t) + 16));
-    CU_TRY(cudaMemcpyAsync(h->refs.p, refs.data(), refs.size() * sizeof(int), cudaMemcpyHostToDevice, s));
     CU_TRY(cudaMemcpyAsync(h->u16.p, in, (size_t)V * sizeof(uint16_t), cudaMemcpyHostToDevice, s));
-    B4dGeom g;
-    fill_geom(pl, pl.rz1, h->refs.as<int>(), &g);
     const long long R = g.refs_per_vol;
     const int K = p.k_ht, Ns = p.search_ht, r = Ns / 2;
     B4D_TRY(h->widx.ensure((size_t)R * std::max(p.k_ht, p.k_wie) * sizeof(uint16_t)));
