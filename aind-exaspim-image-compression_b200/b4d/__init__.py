@@ -19,6 +19,8 @@ from .api import (  # noqa: F401
     patch_has_incoherent_segment,
     denoise_quantized,
     tile_stats,
+    noise_sigma,
+    noise_sigma_from_hist,
 )
 from .cache import load_patch_cache, write_patch_cache  # noqa: F401
 from .codec import chunk_grid, chunk_shuffle, compute_cratio, entropy_bytes, estimate_cratio  # noqa: F401
@@ -48,6 +50,8 @@ __all__ = [
     "patch_has_incoherent_segment",
     "denoise_quantized",
     "tile_stats",
+    "noise_sigma",
+    "noise_sigma_from_hist",
     "slab_plan",
     "bind_to_gpu_numa",
     "denoise_volume_sharded",

@@ -52,6 +52,12 @@ EXPORTS = (
     "b4d_coherence_gate",
     "b4d_set_noise_model",
 )
+# include/b4d_noise.h: the noise-level extension (no counterpart in the CPU oracle library)
+NOISE_EXPORTS = (
+    "b4d_noise_sigma_u16",
+    "b4d_noise_sigma_from_hist",
+)
+NOISE_HIST_BINS = 262141  # B4D_NOISE_HIST_BINS: |d| <= 4 * 65535
 
 
 class Profile(ctypes.Structure):
@@ -114,6 +120,9 @@ def load():
     lib.b4d_stream.restype = ctypes.c_void_p
     lib.b4d_slab_basic_ptr.restype = ctypes.c_void_p
     lib.b4d_default_profile.restype = None
+    i64p, vp = ctypes.POINTER(ctypes.c_int64), ctypes.c_void_p
+    lib.b4d_noise_sigma_u16.argtypes = [vp, vp, ctypes.c_int64, i64p, i64p, vp, vp, vp, vp, ctypes.c_int]
+    lib.b4d_noise_sigma_from_hist.argtypes = [vp, vp, vp, vp]
     if lib.b4d_version() != ABI_VERSION:
         raise B4DLibraryError("libb4d.so ABI %d != binding ABI %d" % (lib.b4d_version(), ABI_VERSION))
     _lib = lib

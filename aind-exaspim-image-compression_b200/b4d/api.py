@@ -603,6 +603,44 @@ class Denoiser:
         d = {k: getattr(st, k) for k, _ in _lib.Stats._fields_}
         return (d, hist) if return_hist else d
 
+    def noise_sigma(self, x, tile=None, return_hist=False):
+        """Noise standard deviation per tile from the MAD of the finest 3-D Haar detail (DESIGN §3.11).
+
+        x     (D,H,W) or (N,D,H,W) uint16, NumPy or torch (host or CUDA).
+        tile  (tz, ty, tx), even sides: a C-order grid anchored at the origin, ragged at the far faces;
+              None: one tile per volume.
+        Returns {"sigma", "mad", "cells"} (float64, float64, int64) shaped (N,)? + tile grid (the grid axes are
+        dropped when tile is None); with return_hist, also the exact 262141-bin histogram of |d| over every cell
+        of the call (int64), the payload to sum across ranks for noise_sigma_from_hist."""
+        x, shape, tile, grid = _noise_sigma_args(x, tile)
+        if _is_torch(x):
+            import torch
+
+            xc = x.contiguous()
+            on_dev = xc.is_cuda
+            if on_dev:
+                torch.cuda.current_stream(xc.device).synchronize()
+            in_ptr = xc.data_ptr()
+        else:
+            xc = np.ascontiguousarray(x)
+            on_dev = False
+            in_ptr = xc.ctypes.data
+        n = 1 if len(shape) == 3 else shape[0]
+        out_shape = (() if len(shape) == 3 else (n,)) + grid
+        sigma = np.empty(out_shape, np.float64)
+        mad = np.empty(out_shape, np.float64)
+        cells = np.empty(out_shape, np.int64)
+        hist = np.empty(_lib.NOISE_HIST_BINS, np.int64) if return_hist else None
+        _lib.check(
+            self.lib.b4d_noise_sigma_u16(
+                self._h, in_ptr, n, _lib.shape3(shape[-3:]), _lib.shape3(tile) if tile is not None else None,
+                sigma.ctypes.data, mad.ctypes.data, cells.ctypes.data, hist.ctypes.data if return_hist else None,
+                int(on_dev),
+            )
+        )
+        d = {"sigma": sigma[()], "mad": mad[()], "cells": cells[()]}
+        return (d, hist) if return_hist else d
+
     def coherence_scores(self, labels, raw, smooth_sigma=1.0, coherence_lag=2, min_autocorr=0.4,
                          max_highfreq_frac=0.35, min_segment_voxels=50, max_segments=1024):
         """The spatial-coherence gate of the sampler (metrics.py:189-260) on the device, for one patch (3-D arrays)
@@ -840,3 +878,48 @@ def noise_scaled_step(sigma_tile, kappa):
 
 def tile_stats(x, percentile=1.0, device=None, return_hist=False):
     return get_denoiser(device).tile_stats(x, percentile, return_hist)
+
+
+def _noise_sigma_args(x, tile):
+    """Argument checks of noise_sigma, before any device work: (x, shape, tile tuple or None, tile grid)."""
+    if _is_torch(x):
+        import torch
+
+        ok = x.dtype == torch.uint16
+        shape = tuple(int(s) for s in x.shape)
+    else:
+        x = np.asarray(x)
+        ok = x.dtype == np.uint16
+        shape = x.shape
+    if not ok:
+        raise ValueError("noise_sigma expects uint16, got %s" % (x.dtype,))
+    if len(shape) not in (3, 4):
+        raise ValueError("noise_sigma expects a 3-D volume or a 4-D batch, got %d-D" % len(shape))
+    if tile is None:
+        return x, shape, None, ()
+    tile = tuple(int(t) for t in tile)
+    if len(tile) != 3 or any(t < 2 or t % 2 for t in tile):
+        raise ValueError("tile must be three even sides >= 2, got %r" % (tile,))
+    return x, shape, tile, tuple(-(-s // t) for s, t in zip(shape[-3:], tile))
+
+
+def noise_sigma(x, tile=None, device=None, return_hist=False):
+    """Noise standard deviation per tile from the MAD of the finest 3-D Haar detail; see Denoiser.noise_sigma.
+    Feeds noise_scaled_step and bm4d(z, sigma) with a measured sigma."""
+    _noise_sigma_args(x, tile)
+    return get_denoiser(device).noise_sigma(x, tile, return_hist)
+
+
+def noise_sigma_from_hist(hist):
+    """{"sigma", "mad", "cells"} of an exact |d| histogram (262141 bins, e.g. the sum of the per-rank histograms of
+    noise_sigma(..., return_hist=True)): the same rule as noise_sigma, host arithmetic only."""
+    if _is_torch(hist):
+        hist = hist.detach().cpu().numpy()
+    h = np.ascontiguousarray(hist, dtype=np.int64)
+    if h.shape != (_lib.NOISE_HIST_BINS,):
+        raise ValueError("hist must have %d bins" % _lib.NOISE_HIST_BINS)
+    out = np.empty(2, np.float64)
+    cells = np.empty(1, np.int64)
+    _lib.check(_lib.load().b4d_noise_sigma_from_hist(h.ctypes.data, out.ctypes.data, out[1:].ctypes.data,
+                                                     cells.ctypes.data))
+    return {"sigma": out[0], "mad": out[1], "cells": cells[0]}

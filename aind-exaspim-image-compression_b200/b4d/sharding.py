@@ -158,9 +158,11 @@ def bind_to_gpu_numa(device):
 
 
 def merge_histograms(hist, group=None):
-    """All-gather + sum of per-rank 65536-bin histograms (the path's only
-    collective).  `hist` is an int64 torch tensor on the rank's device (NCCL) or
-    on the CPU (gloo).  Without an initialised process group it is returned as is."""
+    """All-gather + sum of per-rank histograms of any length (the path's only
+    collective): the 65536-bin intensity histograms of tile_stats or the 262141-bin
+    |d| histograms of noise_sigma.  `hist` is an int64 torch tensor on the rank's
+    device (NCCL) or on the CPU (gloo).  Without an initialised process group it is
+    returned as is."""
     import torch
     import torch.distributed as dist
 

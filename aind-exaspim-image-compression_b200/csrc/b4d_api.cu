@@ -1,4 +1,4 @@
-// b4d_api.cu — the C ABI of include/b4d.h over the sm_100a kernels: handle,
+// b4d_api.cu — the C ABI of include/b4d.h (and b4d_noise.h) over the sm_100a kernels: handle,
 // scratch buffers, the two-stage pipeline, slab geometry, statistics.
 //
 // There is NO CPU fallback here: every entry point that computes needs a CUDA
@@ -94,6 +94,7 @@ struct b4d_handle {
     DevBuf coh_x, coh_sm, coh_tmp, coh_keys, coh_sums, coh_lab, coh_w;
     DevBuf in, u16, zf, numq, gmap, basic, out, widx, cnt, ssd, refs, hist, partial, sink, stats, s2, cells, tcls;
     DevBuf alt_in, alt_zf, alt_out, alt_partial, alt_sink;  // second buffer set of b4d_targets_u16
+    DevBuf nz_hist, nz_sel, nz_res, nz_full;  // b4d_noise_sigma_u16: per-tile digit histograms, selections, results
     float t_ms[B4D_T_COUNT];
     int64_t launches[B4D_T_COUNT];
     unsigned long long match_stats[4];
@@ -978,7 +979,8 @@ void b4d_destroy(b4d_handle *h) {
     for (DevBuf *b : {&h->coh_x, &h->coh_sm, &h->coh_tmp, &h->coh_keys, &h->coh_sums, &h->coh_lab, &h->coh_w}) b->release();
     for (DevBuf *b : {&h->in, &h->u16, &h->zf, &h->numq, &h->gmap, &h->basic, &h->out, &h->widx, &h->cnt,
                       &h->ssd, &h->refs, &h->hist, &h->partial, &h->sink, &h->stats, &h->s2, &h->cells, &h->tcls,
-                      &h->alt_in, &h->alt_zf, &h->alt_out, &h->alt_partial, &h->alt_sink})
+                      &h->alt_in, &h->alt_zf, &h->alt_out, &h->alt_partial, &h->alt_sink, &h->nz_hist, &h->nz_sel,
+                      &h->nz_res, &h->nz_full})
         b->release();
     if (h->pre.ev0) cudaEventDestroy(h->pre.ev0);
     if (h->pre.ev1) cudaEventDestroy(h->pre.ev1);
@@ -1656,6 +1658,116 @@ int b4d_stats_from_hist(const int64_t *hist_in, double pct, b4d_stats *out) {
     }
     if (n < 1) return fail(B4D_ERR_INVALID, "empty histogram");
     return stats_of_hist(hist, n, pct, out);
+}
+
+// DESIGN §3.11: from the two middle order statistics a <= b of |d| over m cells, in this order in float64 so that
+// the result equals np.median(|d|) / (np.sqrt(8.0) * 0.6744897501960817) bit for bit.
+static void noise_of_order_stats(int64_t a, int64_t b, int64_t m, double *sigma, double *mad, int64_t *cells) {
+    *cells = m;
+    if (m == 0) {
+        *mad = *sigma = std::nan("");
+        return;
+    }
+    *mad = ((double)a + (double)b) / 2.0;
+    *sigma = *mad / (std::sqrt(8.0) * 0.6744897501960817);
+}
+
+int b4d_noise_sigma_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3], const int64_t tile[3],
+                        double *sigma, double *mad, int64_t *cells, int64_t *hist_out, int in_on_device) {
+    if (!h || !in || !shape || !sigma || !mad || !cells || n < 1) return fail(B4D_ERR_INVALID, "NULL argument or n < 1");
+    B4D_TRY(check_shape(shape));
+    int64_t side[3];  // tile sides in voxels; one tile per volume: the shape rounded up to even
+    for (int a = 0; a < 3; ++a) {
+        if (tile && (tile[a] < 2 || (tile[a] & 1))) return fail(B4D_ERR_INVALID, "tile sides must be even and >= 2");
+        side[a] = tile ? tile[a] : shape[a] + (shape[a] & 1);
+    }
+    const int64_t vox = shape[0] * shape[1] * shape[2];
+    if (n > (INT64_MAX / 2) / vox) return fail(B4D_ERR_TOO_LARGE, "input too large");
+    NoiseGeom g{};
+    g.vol_stride = vox;
+    g.H = (int)shape[1];
+    g.W = (int)shape[2];
+    int nc[3], tc[3], nt[3];
+    for (int a = 0; a < 3; ++a) {
+        nc[a] = (int)(shape[a] / 2);
+        nt[a] = side[a] >= shape[a] ? 1 : (int)((shape[a] + side[a] - 1) / side[a]);
+        tc[a] = (int)std::min<int64_t>(side[a] / 2, nc[a]);  // a tile wider than the volume is the one tile
+    }
+    g.ncz = nc[0], g.ncy = nc[1], g.ncx = nc[2];
+    g.tcz = tc[0], g.tcy = tc[1], g.tcx = tc[2];
+    g.ntz = nt[0], g.nty = nt[1], g.ntx = nt[2];
+    if ((int64_t)tc[0] * tc[1] * tc[2] > (int64_t)UINT32_MAX)
+        return fail(B4D_ERR_TOO_LARGE, "a tile may hold at most 2^32 - 1 cells (32-bit counts)");
+    // launch shape: a CTA takes about 4096 cells of one tile, as whole cell rows
+    const int max_rows = tc[0] * tc[1];
+    g.rows_per_cta = std::max(1, std::min(max_rows, 4096 / tc[2]));
+    g.warps = std::min(8, g.rows_per_cta);
+    g.ctas_per_tile = (max_rows + g.rows_per_cta - 1) / g.rows_per_cta;
+    const long long ntiles = n * (long long)nt[0] * nt[1] * nt[2];
+    // tiles per launch: bounds the scratch (4 KB per tile) and the grid
+    const long long group = std::min<long long>(ntiles, std::min<long long>(1 << 16, INT32_MAX / g.ctas_per_tile));
+
+    CU_TRY(cudaSetDevice(h->device));
+    cudaStream_t s = h->stream;
+    g.in = in;
+    if (!in_on_device) {
+        B4D_TRY(h->in.ensure((size_t)(n * vox) * sizeof(uint16_t)));
+        CU_TRY(copy_in(h, h->in.p, in, (size_t)(n * vox) * sizeof(uint16_t), 0, s));
+        g.in = h->in.as<uint16_t>();
+    }
+    B4D_TRY(h->nz_hist.ensure((size_t)group * 1024 * sizeof(uint32_t)));
+    B4D_TRY(h->nz_sel.ensure((size_t)group * 5 * sizeof(uint32_t)));
+    B4D_TRY(h->nz_res.ensure((size_t)ntiles * 3 * sizeof(uint32_t)));
+    uint32_t *d_hist = h->nz_hist.as<uint32_t>(), *d_sel = h->nz_sel.as<uint32_t>();
+    for (long long t0 = 0; t0 < ntiles; t0 += group) {
+        const long long cnt = std::min(group, ntiles - t0);
+        g.tile0 = t0;
+        CU_TRY(cudaMemsetAsync(d_hist, 0, (size_t)cnt * 1024 * sizeof(uint32_t), s));
+        b4d_launch_noise_pass(g, 1, cnt, d_hist, nullptr, s);
+        b4d_launch_noise_select(1, d_hist, d_sel, nullptr, cnt, s);
+        CU_TRY(cudaMemsetAsync(d_hist, 0, (size_t)cnt * 1024 * sizeof(uint32_t), s));
+        b4d_launch_noise_pass(g, 2, cnt, d_hist, d_sel, s);
+        b4d_launch_noise_select(2, d_hist, d_sel, h->nz_res.as<uint32_t>() + t0 * 3, cnt, s);
+        CU_TRY(cudaGetLastError());
+    }
+    std::vector<unsigned long long> full;
+    if (hist_out) {
+        B4D_TRY(h->nz_full.ensure(B4D_NOISE_HIST_BINS * sizeof(unsigned long long)));
+        CU_TRY(cudaMemsetAsync(h->nz_full.p, 0, B4D_NOISE_HIST_BINS * sizeof(unsigned long long), s));
+        b4d_launch_noise_hist(g, n, h->nz_full.as<unsigned long long>(), s);
+        CU_TRY(cudaGetLastError());
+        full.resize(B4D_NOISE_HIST_BINS);
+        CU_TRY(cudaMemcpyAsync(full.data(), h->nz_full.p, B4D_NOISE_HIST_BINS * sizeof(unsigned long long),
+                               cudaMemcpyDeviceToHost, s));
+    }
+    std::vector<uint32_t> res((size_t)ntiles * 3);
+    CU_TRY(cudaMemcpyAsync(res.data(), h->nz_res.p, res.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CU_TRY(cudaStreamSynchronize(s));
+    for (long long t = 0; t < ntiles; ++t)
+        noise_of_order_stats(res[3 * t], res[3 * t + 1], res[3 * t + 2], sigma + t, mad + t, cells + t);
+    if (hist_out)
+        for (int v = 0; v < B4D_NOISE_HIST_BINS; ++v) hist_out[v] = (int64_t)full[v];
+    return 0;
+}
+
+// The statistics of an exact |d| histogram (any sum of per-call or per-slab histograms); host arithmetic only.
+int b4d_noise_sigma_from_hist(const int64_t *hist, double *sigma, double *mad, int64_t *cells) {
+    if (!hist || !sigma || !mad || !cells) return fail(B4D_ERR_INVALID, "NULL argument");
+    int64_t m = 0;
+    for (int v = 0; v < B4D_NOISE_HIST_BINS; ++v) {
+        if (hist[v] < 0) return fail(B4D_ERR_INVALID, "negative count");
+        m += hist[v];
+    }
+    int64_t ab[2] = {0, 0};
+    const int64_t rank[2] = {(m - 1) / 2, m / 2};
+    for (int k = 0; k < 2 && m > 0; ++k) {
+        int64_t c = 0;
+        int v = 0;
+        while (c + hist[v] <= rank[k]) c += hist[v++];
+        ab[k] = v;
+    }
+    noise_of_order_stats(ab[0], ab[1], m, sigma, mad, cells);
+    return 0;
 }
 
 int b4d_last_timings(b4d_handle *h, float ms[B4D_T_COUNT], int64_t launches[B4D_T_COUNT]) {

@@ -4,6 +4,7 @@
 #include <stdint.h>
 
 #include "../../include/b4d.h"
+#include "../../include/b4d_noise.h"
 
 #define B4D_L 4
 #define B4D_LV 64
@@ -123,6 +124,26 @@ void b4d_launch_fg_mask(const uint16_t *in, const float *off, const float *thr, 
 // K9: C-order chunk gather + 2-byte shuffle (+ per-chunk byte histograms [nchunks][2][256])
 void b4d_launch_chunk_shuffle(const uint16_t *in, int D, int H, int W, int cz, int cy, int cx, uint8_t *out,
                               uint32_t *hist, cudaStream_t s);
+// noise level (b4d_noise.cu): Haar-detail median per tile, DESIGN §3.11.  Cells are 2x2x2 at even origins, counted
+// per axis (ncz, ncy, ncx); tiles are tcz x tcy x tcx cells, ntz x nty x ntx per volume, numbered over all volumes.
+struct NoiseGeom {
+    const uint16_t *in;
+    long long vol_stride;  // voxels per volume
+    int H, W;
+    int ncz, ncy, ncx;
+    int tcz, tcy, tcx;
+    int ntz, nty, ntx;
+    long long tile0;       // first tile of the launch (passes): scratch entries are relative to it
+    int rows_per_cta, ctas_per_tile, warps;
+};
+// pass 1 (high digit) or 2 (low digit of the chosen bins) over `ntiles` tiles from g.tile0: hist[ntiles][1024]
+void b4d_launch_noise_pass(const NoiseGeom &g, int pass, long long ntiles, uint32_t *hist, const uint32_t *sel,
+                           cudaStream_t s);
+// select 1 (sel[ntiles][5] = m, bin / rank of (m-1)/2, bin / rank of m/2) or 2 (res[ntiles][3] = a, b, m)
+void b4d_launch_noise_select(int which, const uint32_t *hist, uint32_t *sel, uint32_t *res, long long ntiles,
+                             cudaStream_t s);
+// whole-call histogram of |d| over every cell of `nvol` volumes: hist[B4D_NOISE_HIST_BINS], accumulated
+void b4d_launch_noise_hist(const NoiseGeom &g, long long nvol, unsigned long long *hist, cudaStream_t s);
 // coherence gate (b4d_coherence.cu): 23 sums per (patch, label slot), see there
 void b4d_launch_coherence(const float *raw, const unsigned long long *labels, int D, int H, int W, long long npatch,
                           int lag, int radius, const double *w, double *x, double *sm, double *tmp,
