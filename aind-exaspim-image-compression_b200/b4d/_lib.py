@@ -56,8 +56,14 @@ EXPORTS = (
 NOISE_EXPORTS = (
     "b4d_noise_sigma_u16",
     "b4d_noise_sigma_from_hist",
+    "b4d_noise_level_u16",
+    "b4d_gat_forward_u16",
+    "b4d_gat_inverse_f32",
+    "b4d_denoise_vst_u16",
+    "b4d_denoise_vst_q16_u16",
 )
 NOISE_HIST_BINS = 262141  # B4D_NOISE_HIST_BINS: |d| <= 4 * 65535
+NLF_MAX_BINS = 64  # B4D_NLF_MAX_BINS
 
 
 class Profile(ctypes.Structure):
@@ -123,10 +129,22 @@ def load():
     i64p, vp = ctypes.POINTER(ctypes.c_int64), ctypes.c_void_p
     lib.b4d_noise_sigma_u16.argtypes = [vp, vp, ctypes.c_int64, i64p, i64p, vp, vp, vp, vp, ctypes.c_int]
     lib.b4d_noise_sigma_from_hist.argtypes = [vp, vp, vp, vp]
+    i64, f32, c_int = ctypes.c_int64, ctypes.c_float, ctypes.c_int
+    lib.b4d_noise_level_u16.argtypes = [vp, vp, i64, i64p, vp, c_int, i64, vp, vp, vp, vp, vp, vp, vp, c_int]
+    lib.b4d_gat_forward_u16.argtypes = [vp, vp, vp, i64, vp, c_int, c_int]
+    lib.b4d_gat_inverse_f32.argtypes = [vp, vp, vp, i64, vp, c_int, c_int]
+    lib.b4d_denoise_vst_u16.argtypes = [vp, vp, i64, i64p, vp, f32, vp, c_int, c_int]
+    lib.b4d_denoise_vst_q16_u16.argtypes = [vp, vp, i64, i64p, vp, f32, f32, f32, f32, c_int, vp, c_int, c_int]
     if lib.b4d_version() != ABI_VERSION:
         raise B4DLibraryError("libb4d.so ABI %d != binding ABI %d" % (lib.b4d_version(), ABI_VERSION))
     _lib = lib
     return lib
+
+
+class PgModel(ctypes.Structure):
+    """Mirror of ``struct b4d_pg_model`` (include/b4d_noise.h)."""
+
+    _fields_ = [("gain", ctypes.c_double), ("offset", ctypes.c_double), ("read_sigma", ctypes.c_double)]
 
 
 class SegmentScore(ctypes.Structure):

@@ -17,6 +17,7 @@ point (``ValueError`` for shape/dtype, ``RuntimeError`` for CUDA,
 torch out on the same device.  Everything computes on the GPU through the C ABI;
 there is no CPU fallback.
 """
+import collections
 import ctypes
 import enum
 import os
@@ -641,6 +642,108 @@ class Denoiser:
         d = {"sigma": sigma[()], "mad": mad[()], "cells": cells[()]}
         return (d, hist) if return_hist else d
 
+    # ---- Poisson-Gaussian noise (DESIGN §3.12) -------------------------------
+    def _io(self, x, out_dtype):
+        """(contiguous input, its pointer, on device, output of out_dtype ("float32" / "uint16") in the same place,
+        its pointer) for the elementwise and VST calls; a CUDA tensor must live on the handle's device."""
+        if _is_torch(x):
+            import torch
+
+            xc = x.contiguous()
+            on_dev = xc.is_cuda
+            if on_dev and xc.device.index != self.device:
+                raise ValueError("tensor lives on cuda:%s, handle on cuda:%d" % (xc.device.index, self.device))
+            out = torch.empty(xc.shape, dtype=getattr(torch, out_dtype), device=xc.device)
+            if on_dev:
+                torch.cuda.current_stream(xc.device).synchronize()
+            return xc, xc.data_ptr(), on_dev, out, out.data_ptr()
+        xc = np.ascontiguousarray(x)
+        out = np.empty(xc.shape, dtype=out_dtype)
+        return xc, xc.ctypes.data, False, out, out.ctypes.data
+
+    def noise_level_function(self, x, edges=None, min_cells=256):
+        """Noise-level function var(z) = a E[z] + b of Poisson-Gaussian counts (DESIGN §3.12): the Haar-detail MAD of
+        noise_sigma per intensity bin of the 2x2x2 cells, and a weighted least-squares line through the bins.
+
+        x          (D,H,W) or (N,D,H,W) uint16, NumPy or torch (host or CUDA); one set of bins for every volume.
+        edges      nb + 1 strictly increasing finite bin edges in counts (1 <= nb <= 64); a cell whose 8 voxels sum to
+                   s is in bin k iff 8 edges[k] <= s < 8 edges[k + 1].  None: default_nlf_edges().
+        min_cells  bins with fewer cells stay out of the fit.
+        Returns {"edges", "cells", "level_sum", "level", "mad", "sigma", "a", "b", "usable"}: per-bin int64 / float64
+        arrays (level = mean intensity of the bin's cells, NaN when empty), the fitted a, b (NaN when fewer than 2
+        bins are usable) and the number of usable bins."""
+        x, shape, edges, min_cells = _nlf_args(x, edges, min_cells)
+        if _is_torch(x):
+            xc = x.contiguous()
+            on_dev = xc.is_cuda
+            if on_dev:
+                import torch
+
+                torch.cuda.current_stream(xc.device).synchronize()
+            in_ptr = xc.data_ptr()
+        else:
+            xc = np.ascontiguousarray(x)
+            on_dev, in_ptr = False, xc.ctypes.data
+        nb = edges.size - 1
+        cells = np.empty(nb, np.int64)
+        level_sum = np.empty(nb, np.int64)
+        mad = np.empty(nb, np.float64)
+        sigma = np.empty(nb, np.float64)
+        level = np.empty(nb, np.float64)
+        fit = np.empty(2, np.float64)
+        usable = np.empty(1, np.int64)
+        n = 1 if len(shape) == 3 else shape[0]
+        _lib.check(
+            self.lib.b4d_noise_level_u16(
+                self._h, in_ptr, n, _lib.shape3(shape[-3:]), edges.ctypes.data, nb, min_cells, cells.ctypes.data,
+                level_sum.ctypes.data, mad.ctypes.data, sigma.ctypes.data, level.ctypes.data, fit.ctypes.data,
+                usable.ctypes.data, int(on_dev),
+            )
+        )
+        return {"edges": edges, "cells": cells, "level_sum": level_sum, "level": level, "mad": mad, "sigma": sigma,
+                "a": fit[0], "b": fit[1], "usable": int(usable[0])}
+
+    def gat_forward(self, x, model):
+        """Generalized Anscombe transform of uint16 counts under `model` (PoissonGaussian) -> float32, elementwise:
+        2 sqrt(max((z - offset)/gain + 3/8 + (read_sigma/gain)^2, 0)), float64 inside.  NumPy or torch (host or
+        CUDA) -> the same kind, same shape."""
+        _elementwise_args(x, "uint16", "gat_forward")
+        m = _model_c(model)
+        xc, in_ptr, on_dev, out, out_ptr = self._io(x, "float32")
+        _lib.check(self.lib.b4d_gat_forward_u16(self._h, ctypes.byref(m), in_ptr, int(np.prod(xc.shape)), out_ptr,
+                                                int(on_dev), int(on_dev)))
+        return out
+
+    def gat_inverse(self, y, model):
+        """Closed-form approximation of the exact unbiased inverse of gat_forward (Makitalo & Foi 2013), float32 ->
+        float32 counts gain * lambda + offset; lambda = 0 for y <= sqrt(1.5)."""
+        _elementwise_args(y, "float32", "gat_inverse")
+        m = _model_c(model)
+        yc, in_ptr, on_dev, out, out_ptr = self._io(y, "float32")
+        _lib.check(self.lib.b4d_gat_inverse_f32(self._h, ctypes.byref(m), in_ptr, int(np.prod(yc.shape)), out_ptr,
+                                                int(on_dev), int(on_dev)))
+        return out
+
+    def denoise_vst(self, x, model, sigma=1.0, quantize=None):
+        """Denoise Poisson-Gaussian uint16 counts: gat_inverse(denoise(gat_forward(x, model), sigma), model), with the
+        intermediate float32 volume never leaving the device.  sigma is the noise level after the transform: 1 for an
+        exact model.  (D,H,W) or (N,D,H,W), NumPy or torch -> float32; quantize = (offset_sub, offset_add, step[,
+        truncate]): the uint16 volume quantize() gives on that float32 result instead."""
+        _vst_args(x, sigma, quantize)
+        m = _model_c(model)
+        shape = tuple(int(v) for v in x.shape)
+        n = 1 if len(shape) == 3 else shape[0]
+        xc, in_ptr, on_dev, out, out_ptr = self._io(x, "float32" if quantize is None else "uint16")
+        if quantize is None:
+            _lib.check(self.lib.b4d_denoise_vst_u16(self._h, in_ptr, n, _lib.shape3(shape[-3:]), ctypes.byref(m),
+                                                    float(sigma), out_ptr, int(on_dev), int(on_dev)))
+            return out
+        q = tuple(quantize) + (False,) * (4 - len(quantize))
+        _lib.check(self.lib.b4d_denoise_vst_q16_u16(self._h, in_ptr, n, _lib.shape3(shape[-3:]), ctypes.byref(m),
+                                                    float(sigma), float(q[0]), float(q[1]), float(q[2]),
+                                                    int(bool(q[3])), out_ptr, int(on_dev), int(on_dev)))
+        return out
+
     def coherence_scores(self, labels, raw, smooth_sigma=1.0, coherence_lag=2, min_autocorr=0.4,
                          max_highfreq_frac=0.35, min_segment_voxels=50, max_segments=1024):
         """The spatial-coherence gate of the sampler (metrics.py:189-260) on the device, for one patch (3-D arrays)
@@ -923,3 +1026,110 @@ def noise_sigma_from_hist(hist):
     _lib.check(_lib.load().b4d_noise_sigma_from_hist(h.ctypes.data, out.ctypes.data, out[1:].ctypes.data,
                                                      cells.ctypes.data))
     return {"sigma": out[0], "mad": out[1], "cells": cells[0]}
+
+
+# --------------------------------------------------------------------------
+# Poisson-Gaussian noise (DESIGN §3.12)
+# --------------------------------------------------------------------------
+class PoissonGaussian(collections.namedtuple("PoissonGaussian", "gain offset read_sigma")):
+    """Camera model z = gain * Poisson(lambda) + N(offset, read_sigma^2) of the generalized Anscombe transform:
+    gain > 0 (counts per photo-electron), offset (the dark level), read_sigma >= 0 (counts), all finite."""
+
+    __slots__ = ()
+
+    @classmethod
+    def from_nlf(cls, a, b, offset):
+        """The model of a noise-level function var(z) = a E[z] + b (noise_level_function) and an offset measured
+        elsewhere, e.g. tile_stats(x)["offset"]: gain = a, read_sigma = sqrt(max(b + a offset, 0))."""
+        a, b, mu = float(a), float(b), float(offset)
+        return cls(a, mu, float(np.sqrt(max(b + a * mu, 0.0))))
+
+
+def default_nlf_edges():
+    """0, then 32 * 2^(k/3) for k = 0 .. 33: three bins per octave from 32 to 65536 counts, 34 bins."""
+    return np.array([0.0] + [32.0 * 2.0 ** (k / 3.0) for k in range(34)], np.float64)
+
+
+def _model_c(model):
+    """PoissonGaussian (or any (gain, offset, read_sigma)) -> _lib.PgModel; ValueError outside the domain."""
+    try:
+        gain, offset, read_sigma = (float(v) for v in model)
+    except (TypeError, ValueError):
+        raise ValueError("model must be a PoissonGaussian (gain, offset, read_sigma), got %r" % (model,))
+    if not (np.isfinite(gain) and gain > 0):
+        raise ValueError("gain must be positive and finite, got %r" % gain)
+    if not np.isfinite(offset):
+        raise ValueError("offset must be finite, got %r" % offset)
+    if not (np.isfinite(read_sigma) and read_sigma >= 0):
+        raise ValueError("read_sigma must be non-negative and finite, got %r" % read_sigma)
+    return _lib.PgModel(gain, offset, read_sigma)
+
+
+def _dtype_name(x):
+    return str(x.dtype).replace("torch.", "") if _is_torch(x) else np.asarray(x).dtype.name
+
+
+def _elementwise_args(x, dtype, what):
+    if not _is_torch(x) and not isinstance(x, np.ndarray):
+        x = np.asarray(x)
+    if _dtype_name(x) != dtype:
+        raise ValueError("%s expects %s, got %s" % (what, dtype, _dtype_name(x)))
+
+
+def _nlf_args(x, edges, min_cells):
+    """Argument checks of noise_level_function, before any device work: (x, shape, edges float64, min_cells)."""
+    if not _is_torch(x):
+        x = np.asarray(x)
+    if _dtype_name(x) != "uint16":
+        raise ValueError("noise_level_function expects uint16, got %s" % _dtype_name(x))
+    shape = tuple(int(s) for s in x.shape)
+    if len(shape) not in (3, 4):
+        raise ValueError("noise_level_function expects a 3-D volume or a 4-D batch, got %d-D" % len(shape))
+    e = default_nlf_edges() if edges is None else np.ascontiguousarray(edges, dtype=np.float64)
+    if e.ndim != 1 or not 2 <= e.size <= _lib.NLF_MAX_BINS + 1:
+        raise ValueError("edges must be 2 .. %d values (1 .. %d bins)" % (_lib.NLF_MAX_BINS + 1, _lib.NLF_MAX_BINS))
+    if not np.all(np.isfinite(e)) or not np.all(np.diff(e) > 0):
+        raise ValueError("edges must be finite and strictly increasing")
+    if int(min_cells) < 1:
+        raise ValueError("min_cells must be >= 1")
+    return x, shape, e, int(min_cells)
+
+
+def _vst_args(x, sigma, quantize):
+    if not _is_torch(x):
+        x = np.asarray(x)
+    if _dtype_name(x) != "uint16":
+        raise ValueError("denoise_vst expects uint16 counts, got %s" % _dtype_name(x))
+    if x.ndim not in (3, 4):
+        raise ValueError("expected a 3-D volume or a 4-D batch, got %d-D" % x.ndim)
+    if not (np.isfinite(sigma) and sigma > 0):
+        raise ValueError("sigma must be positive and finite, got %r" % (sigma,))
+    if quantize is not None and not (3 <= len(quantize) <= 4 and float(quantize[2]) >= 1.0):
+        raise ValueError("quantize must be (offset_sub, offset_add, step >= 1[, truncate])")
+
+
+def noise_level_function(x, edges=None, min_cells=256, device=None):
+    """Noise-level function of Poisson-Gaussian counts; see Denoiser.noise_level_function."""
+    _nlf_args(x, edges, min_cells)
+    return get_denoiser(device).noise_level_function(x, edges, min_cells)
+
+
+def gat_forward(x, model, device=None):
+    """Generalized Anscombe transform; see Denoiser.gat_forward."""
+    _elementwise_args(x, "uint16", "gat_forward")
+    _model_c(model)
+    return get_denoiser(device).gat_forward(x, model)
+
+
+def gat_inverse(y, model, device=None):
+    """Inverse of gat_forward; see Denoiser.gat_inverse."""
+    _elementwise_args(y, "float32", "gat_inverse")
+    _model_c(model)
+    return get_denoiser(device).gat_inverse(y, model)
+
+
+def denoise_vst(x, model, sigma=1.0, quantize=None, device=None):
+    """Denoise Poisson-Gaussian uint16 counts through the GAT; see Denoiser.denoise_vst."""
+    _vst_args(x, sigma, quantize)
+    _model_c(model)
+    return get_denoiser(device).denoise_vst(x, model, sigma, quantize)

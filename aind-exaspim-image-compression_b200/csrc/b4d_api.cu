@@ -95,6 +95,7 @@ struct b4d_handle {
     DevBuf in, u16, zf, numq, gmap, basic, out, widx, cnt, ssd, refs, hist, partial, sink, stats, s2, cells, tcls;
     DevBuf alt_in, alt_zf, alt_out, alt_partial, alt_sink;  // second buffer set of b4d_targets_u16
     DevBuf nz_hist, nz_sel, nz_res, nz_full;  // b4d_noise_sigma_u16: per-tile digit histograms, selections, results
+    DevBuf nlf_sum;  // b4d_noise_level_u16: per-bin sums of the cell intensities
     float t_ms[B4D_T_COUNT];
     int64_t launches[B4D_T_COUNT];
     unsigned long long match_stats[4];
@@ -850,6 +851,19 @@ int stage_u16_input(b4d_handle *h, const Plan &pl, const uint16_t *in, int in_on
     return 0;
 }
 
+// The float32 batch staged in h->in (TV voxels): its matching map, the centring shift of a large DC level (the
+// staged copy then holds z - c0 and *centre = c0 is added back after the pass) and the uint16 matching image
+// in h->u16.
+int prepare_f32(b4d_handle *h, long long TV, float sigma, MatchMap *mm, float *centre) {
+    B4D_TRY(derive_match_map(h, h->in.as<float>(), TV, sigma, mm, centre));
+    if (*centre != 0.0f) {
+        b4d_launch_add_scalar(h->in.as<float>(), TV, -*centre, h->stream);
+        B4D_TRY(derive_match_map(h, h->in.as<float>(), TV, sigma, mm));
+    }
+    b4d_launch_to_match(h->in.as<float>(), h->u16.as<uint16_t>(), TV, mm->cf, mm->scale, mm->ishift, h->stream);
+    return 0;
+}
+
 // Batched denoise, chunked so scratch stays bounded.
 template <class T>
 int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3], float sigma, float *out,
@@ -890,12 +904,7 @@ int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3],
             d_zf = h->zf.as<float>();
             d_u = h->in.as<uint16_t>();  // the staged copy doubles as the matching image
         } else {
-            B4D_TRY(derive_match_map(h, h->in.as<float>(), TV, sigma, &mm, &centre));
-            if (centre != 0.0f) {  // large DC level: denoise z - c0 (in the scratch copy), add c0 back at the end
-                b4d_launch_add_scalar(h->in.as<float>(), TV, -centre, s);
-                B4D_TRY(derive_match_map(h, h->in.as<float>(), TV, sigma, &mm));
-            }
-            b4d_launch_to_match(h->in.as<float>(), h->u16.as<uint16_t>(), TV, mm.cf, mm.scale, mm.ishift, s);
+            B4D_TRY(prepare_f32(h, TV, sigma, &mm, &centre));
             d_zf = h->in.as<float>();
         }
         clk.mark(B4D_T_PREP, 2);
@@ -908,6 +917,84 @@ int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3],
         if (centre != 0.0f) b4d_launch_add_scalar(d_out, TV, centre, s);
         if (!sink.done && d_out != out + i0 * V)
             CU_TRY(copy_out(h, out + i0 * V, d_out, (size_t)TV * sizeof(float), out_dev, s));
+        B4D_TRY(finish(h, clk));
+    }
+    return 0;
+}
+
+// DESIGN §3.12: the camera model as the GAT kernels take it; B4D_ERR_INVALID outside its domain.
+int gat_params(const b4d_pg_model *m, GatParams *p) {
+    if (!m) return fail(B4D_ERR_INVALID, "NULL model");
+    if (!(m->gain > 0) || !std::isfinite(m->gain)) return fail(B4D_ERR_INVALID, "gain must be positive and finite");
+    if (!std::isfinite(m->offset)) return fail(B4D_ERR_INVALID, "offset must be finite");
+    if (!(m->read_sigma >= 0) || !std::isfinite(m->read_sigma))
+        return fail(B4D_ERR_INVALID, "read_sigma must be non-negative and finite");
+    const double q = m->read_sigma / m->gain;
+    p->gain = m->gain;
+    p->offset = m->offset;
+    p->qq = q * q;
+    p->s15 = std::sqrt(1.5);
+    p->c1 = 0.25 * p->s15;
+    p->c2 = 0.625 * p->s15;
+    return 0;
+}
+
+// Batched denoise of uint16 counts through the GAT: forward into the float32 scratch, the float32 pipeline of
+// denoise_batch on it, then the inverse into `out` (float32, or uint16 through K7 with `q`).  Chunked like
+// denoise_batch, with the same scratch.
+int denoise_vst(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3], const b4d_pg_model *model,
+                float sigma, void *out, const QuantSpec *q, int in_dev, int out_dev) {
+    GatParams gp;
+    B4D_TRY(gat_params(model, &gp));
+    if (q && !(q->step >= 1.0f)) return fail(B4D_ERR_INVALID, "step must be >= 1");
+    B4D_TRY(common_checks(h, in, out, shape, sigma));
+    if (n < 1) return fail(B4D_ERR_INVALID, "n must be >= 1");
+    reset_timings(h);
+    const long long V = shape[0] * shape[1] * shape[2];
+    const int64_t per = std::max<int64_t>(1, std::min<int64_t>(n, h->pass_voxels / V));
+    const size_t osz = q ? sizeof(uint16_t) : sizeof(float);
+    cudaStream_t s = h->stream;
+    Plan pl = make_plan(shape, 0, shape[0], 1, h->prof);
+    StageClock clk(h);
+    const int norm_slot = h->prof.stages == 2 ? B4D_T_NORM2 : B4D_T_NORM1;
+    for (int64_t i0 = 0; i0 < n; i0 += per) {
+        const int64_t nb = std::min<int64_t>(per, n - i0);
+        const long long TV = V * nb;
+        pl.nvol = (int)nb;
+        B4D_TRY(h->in.ensure((size_t)TV * sizeof(float)));
+        B4D_TRY(h->u16.ensure((size_t)TV * sizeof(uint16_t) + 16));
+        B4D_TRY(h->out.ensure((size_t)TV * sizeof(float)));
+        char *user_out = static_cast<char *>(out) + (size_t)i0 * V * osz;
+        // the float32 result: in place in a device output of float32 when it is 16-byte aligned
+        float *d_res = h->out.as<float>();
+        if (!q && out_dev && (reinterpret_cast<uintptr_t>(user_out) & 15) == 0) d_res = reinterpret_cast<float *>(user_out);
+        // host input is staged in h->u16, which to_match overwrites with the matching image after the forward
+        const uint16_t *src = in + i0 * V;
+        if (!in_dev) {
+            CU_TRY(copy_in(h, h->u16.p, src, (size_t)TV * sizeof(uint16_t), 0, s));
+            src = h->u16.as<uint16_t>();
+        }
+        clk.mark(-1, 0);
+        b4d_launch_gat_forward(src, h->in.as<float>(), TV, gp, s);
+        MatchMap mm;
+        float centre = 0.0f;
+        B4D_TRY(prepare_f32(h, TV, sigma, &mm, &centre));
+        clk.mark(B4D_T_PREP, centre != 0.0f ? 5 : 3);
+        HostSink sink{nullptr, 0, pl.D};
+        Pass ps;
+        B4D_TRY(make_pass(h, pl, sigma, mm, h->in.as<float>(), h->u16.as<uint16_t>(), d_res, clk, ps));
+        B4D_TRY(denoise_pass(ps, nullptr, &sink, nullptr));
+        if (centre != 0.0f) b4d_launch_add_scalar(d_res, TV, centre, s);
+        clk.mark(-1, 0);
+        // inverse: in place, or K7 into uint16 (the user's device buffer, else h->u16: the pass is done with it)
+        uint16_t *d_q = nullptr;
+        if (q) d_q = out_dev ? reinterpret_cast<uint16_t *>(user_out) : h->u16.as<uint16_t>();
+        b4d_launch_gat_inverse(d_res, d_res, d_q, TV, gp, q ? q->sub : 0.f, q ? q->add : 0.f, q ? q->step : 1.f,
+                               q ? q->trunc : 0, s);
+        CU_TRY(cudaGetLastError());
+        clk.mark(norm_slot, 1);
+        const void *d_final = q ? static_cast<const void *>(d_q) : static_cast<const void *>(d_res);
+        if (d_final != user_out) CU_TRY(copy_out(h, user_out, d_final, (size_t)TV * osz, out_dev, s));
         B4D_TRY(finish(h, clk));
     }
     return 0;
@@ -1768,6 +1855,165 @@ int b4d_noise_sigma_from_hist(const int64_t *hist, double *sigma, double *mad, i
     }
     noise_of_order_stats(ab[0], ab[1], m, sigma, mad, cells);
     return 0;
+}
+
+// DESIGN §3.12: noise-level function.  The passes of b4d_noise_sigma_u16 with the intensity bin of a cell as its
+// key; k_noise_select1/2 run on the [nb][1024] histograms as on per-tile ones.  The statistics and the fit are
+// host arithmetic in float64 in the order of the contract.
+int b4d_noise_level_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3], const double *edges,
+                        int nbins, int64_t min_cells, int64_t *cells, int64_t *level_sum, double *mad, double *sigma,
+                        double *level, double fit[2], int64_t *usable, int in_on_device) {
+    if (!h || !in || !shape || !edges || !cells || !level_sum || !mad || !sigma || !level || !fit || !usable || n < 1)
+        return fail(B4D_ERR_INVALID, "NULL argument or n < 1");
+    B4D_TRY(check_shape(shape));
+    if (nbins < 1 || nbins > B4D_NLF_MAX_BINS) return fail(B4D_ERR_INVALID, "nbins must be in 1 .. 64");
+    if (min_cells < 1) return fail(B4D_ERR_INVALID, "min_cells must be >= 1");
+    for (int k = 0; k <= nbins; ++k) {
+        if (!std::isfinite(edges[k])) return fail(B4D_ERR_INVALID, "bin edges must be finite");
+        if (k && !(edges[k] > edges[k - 1])) return fail(B4D_ERR_INVALID, "bin edges must be strictly increasing");
+    }
+    const int64_t vox = shape[0] * shape[1] * shape[2];
+    if (n > (INT64_MAX / 2) / vox) return fail(B4D_ERR_TOO_LARGE, "input too large");
+    NlfGeom g{};
+    g.vol_stride = vox;
+    g.nvol = n;
+    g.H = (int)shape[1];
+    g.W = (int)shape[2];
+    g.ncz = (int)(shape[0] / 2), g.ncy = (int)(shape[1] / 2), g.ncx = (int)(shape[2] / 2);
+    if ((int64_t)g.ncz * g.ncy * g.ncx * n > (int64_t)UINT32_MAX)
+        return fail(B4D_ERR_TOO_LARGE, "a call may hold at most 2^32 - 1 cells (32-bit counts)");
+    g.nb = nbins;
+    // ceil(8 e_k) (8 e is exact), clamped to the range of s = 0 .. 524280: the integer test keeps its meaning
+    for (int k = 0; k < NLF_THR; ++k)
+        g.thr[k] = k > nbins ? INT32_MAX : (int)std::min(524281.0, std::max(0.0, std::ceil(8.0 * edges[k])));
+
+    CU_TRY(cudaSetDevice(h->device));
+    cudaStream_t s = h->stream;
+    g.in = in;
+    if (!in_on_device) {
+        B4D_TRY(h->in.ensure((size_t)(n * vox) * sizeof(uint16_t)));
+        CU_TRY(copy_in(h, h->in.p, in, (size_t)(n * vox) * sizeof(uint16_t), 0, s));
+        g.in = h->in.as<uint16_t>();
+    }
+    B4D_TRY(h->nz_hist.ensure((size_t)nbins * 1024 * sizeof(uint32_t)));
+    B4D_TRY(h->nz_sel.ensure((size_t)nbins * 5 * sizeof(uint32_t)));
+    B4D_TRY(h->nz_res.ensure((size_t)nbins * 3 * sizeof(uint32_t)));
+    B4D_TRY(h->nlf_sum.ensure((size_t)nbins * sizeof(unsigned long long)));
+    uint32_t *d_hist = h->nz_hist.as<uint32_t>(), *d_sel = h->nz_sel.as<uint32_t>();
+    CU_TRY(cudaMemsetAsync(d_hist, 0, (size_t)nbins * 1024 * sizeof(uint32_t), s));
+    CU_TRY(cudaMemsetAsync(h->nlf_sum.p, 0, (size_t)nbins * sizeof(unsigned long long), s));
+    for (int pass = 1; pass <= 2; ++pass) {
+        const int group = b4d_nlf_bins_per_launch(pass);
+        const int launches = (nbins + group - 1) / group;
+        for (int i = 0; i < launches; ++i) {  // equal shares of the bins
+            g.kb0 = (int)((int64_t)nbins * i / launches);
+            g.kb1 = (int)((int64_t)nbins * (i + 1) / launches);
+            b4d_launch_nlf_pass(g, pass, d_hist, h->nlf_sum.as<unsigned long long>(), d_sel, s);
+        }
+        if (pass == 1) {
+            b4d_launch_noise_select(1, d_hist, d_sel, nullptr, nbins, s);
+            CU_TRY(cudaMemsetAsync(d_hist, 0, (size_t)nbins * 1024 * sizeof(uint32_t), s));
+        } else {
+            b4d_launch_noise_select(2, d_hist, d_sel, h->nz_res.as<uint32_t>(), nbins, s);
+        }
+        CU_TRY(cudaGetLastError());
+    }
+    std::vector<uint32_t> res((size_t)nbins * 3);
+    std::vector<unsigned long long> lsum(nbins);
+    CU_TRY(cudaMemcpyAsync(res.data(), h->nz_res.p, res.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CU_TRY(cudaMemcpyAsync(lsum.data(), h->nlf_sum.p, lsum.size() * sizeof(unsigned long long),
+                           cudaMemcpyDeviceToHost, s));
+    CU_TRY(cudaStreamSynchronize(s));
+    double W = 0, Sx = 0, Sy = 0, Sxx = 0, Sxy = 0;
+    int64_t used = 0;
+    for (int k = 0; k < nbins; ++k) {
+        noise_of_order_stats(res[3 * k], res[3 * k + 1], res[3 * k + 2], sigma + k, mad + k, cells + k);
+        level_sum[k] = (int64_t)lsum[k];
+        level[k] = cells[k] ? (double)level_sum[k] / (8.0 * (double)cells[k]) : std::nan("");
+        if (cells[k] < min_cells) continue;
+        const double w = (double)cells[k], x = level[k], y = sigma[k] * sigma[k];
+        W += w;
+        Sx += w * x;
+        Sy += w * y;
+        Sxx += w * x * x;
+        Sxy += w * x * y;
+        ++used;
+    }
+    *usable = used;
+    fit[0] = fit[1] = std::nan("");
+    if (used >= 2) {
+        fit[0] = (W * Sxy - Sx * Sy) / (W * Sxx - Sx * Sx);
+        fit[1] = (Sy - fit[0] * Sx) / W;
+    }
+    return 0;
+}
+
+int b4d_gat_forward_u16(b4d_handle *h, const b4d_pg_model *model, const uint16_t *in, int64_t n, float *out,
+                        int in_on_device, int out_on_device) {
+    GatParams gp;
+    B4D_TRY(gat_params(model, &gp));
+    if (!h || !in || !out || n < 0) return fail(B4D_ERR_INVALID, "NULL argument");
+    CU_TRY(cudaSetDevice(h->device));
+    if (n == 0) return 0;
+    cudaStream_t s = h->stream;
+    const uint16_t *d_in = in;
+    float *d_out = out;
+    if (!in_on_device) {
+        B4D_TRY(h->u16.ensure((size_t)n * sizeof(uint16_t) + 16));
+        CU_TRY(copy_in(h, h->u16.p, in, (size_t)n * sizeof(uint16_t), 0, s));
+        d_in = h->u16.as<uint16_t>();
+    }
+    if (!out_on_device) {
+        B4D_TRY(h->out.ensure((size_t)n * sizeof(float)));
+        d_out = h->out.as<float>();
+    }
+    b4d_launch_gat_forward(d_in, d_out, n, gp, s);
+    CU_TRY(cudaGetLastError());
+    if (d_out != out) CU_TRY(copy_out(h, out, d_out, (size_t)n * sizeof(float), 0, s));
+    CU_TRY(cudaStreamSynchronize(s));
+    return 0;
+}
+
+int b4d_gat_inverse_f32(b4d_handle *h, const b4d_pg_model *model, const float *in, int64_t n, float *out,
+                        int in_on_device, int out_on_device) {
+    GatParams gp;
+    B4D_TRY(gat_params(model, &gp));
+    if (!h || !in || !out || n < 0) return fail(B4D_ERR_INVALID, "NULL argument");
+    CU_TRY(cudaSetDevice(h->device));
+    if (n == 0) return 0;
+    cudaStream_t s = h->stream;
+    const float *d_in = in;
+    float *d_out = out;
+    if (!in_on_device) {
+        B4D_TRY(h->in.ensure((size_t)n * sizeof(float)));
+        CU_TRY(copy_in(h, h->in.p, in, (size_t)n * sizeof(float), 0, s));
+        d_in = h->in.as<float>();
+    }
+    if (!out_on_device) {
+        B4D_TRY(h->out.ensure((size_t)n * sizeof(float)));
+        d_out = h->out.as<float>();
+    }
+    b4d_launch_gat_inverse(d_in, d_out, nullptr, n, gp, 0.f, 0.f, 1.f, 0, s);
+    CU_TRY(cudaGetLastError());
+    if (d_out != out) CU_TRY(copy_out(h, out, d_out, (size_t)n * sizeof(float), 0, s));
+    CU_TRY(cudaStreamSynchronize(s));
+    return 0;
+}
+
+int b4d_denoise_vst_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3],
+                        const b4d_pg_model *model, float sigma_vst, float *out, int in_on_device, int out_on_device) {
+    return denoise_vst(h, in, n, shape, model, sigma_vst, out, nullptr, in_on_device, out_on_device);
+}
+
+int b4d_denoise_vst_q16_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3],
+                            const b4d_pg_model *model, float sigma_vst, float offset_sub, float offset_add,
+                            float step, int truncate, uint16_t *out, int in_on_device, int out_on_device) {
+    QuantSpec q;
+    q.sub = offset_sub;
+    q.add = offset_add;
+    q.step = step;
+    q.trunc = truncate ? 1 : 0;
+    return denoise_vst(h, in, n, shape, model, sigma_vst, out, &q, in_on_device, out_on_device);
 }
 
 int b4d_last_timings(b4d_handle *h, float ms[B4D_T_COUNT], int64_t launches[B4D_T_COUNT]) {

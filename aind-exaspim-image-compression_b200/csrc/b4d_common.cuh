@@ -144,6 +144,54 @@ void b4d_launch_noise_select(int which, const uint32_t *hist, uint32_t *sel, uin
                              cudaStream_t s);
 // whole-call histogram of |d| over every cell of `nvol` volumes: hist[B4D_NOISE_HIST_BINS], accumulated
 void b4d_launch_noise_hist(const NoiseGeom &g, long long nvol, unsigned long long *hist, cudaStream_t s);
+// noise-level function (b4d_noise.cu, DESIGN §3.12): the same passes keyed by the intensity bin of each cell.
+// thr[k] = ceil(8 e_k) clamped to [0, 524281] for k <= nb, INT32_MAX beyond: a cell of sum s is in bin k iff
+// thr[k] <= s < thr[k + 1].  A launch covers bins [kb0, kb1).
+constexpr int NLF_THR = 128;
+struct NlfGeom {
+    const uint16_t *in;
+    long long vol_stride, nvol;
+    int H, W;
+    int ncz, ncy, ncx;
+    int nb, kb0, kb1;
+    int thr[NLF_THR];
+};
+// bins per launch of pass 1 / pass 2 (shared-memory histograms of 2 KB / 4 KB per bin)
+int b4d_nlf_bins_per_launch(int pass);
+// pass 1: hist[k][0, 512) and lsum[k] (sum s); pass 2: hist[k][0, 1024) from sel[k][5] of select 1
+void b4d_launch_nlf_pass(const NlfGeom &g, int pass, uint32_t *hist, unsigned long long *lsum, const uint32_t *sel,
+                         cudaStream_t s);
+// generalized Anscombe transform (b4d_vst.cu, DESIGN §3.12): qq = (read_sigma / gain)^2, s15 = sqrt(1.5),
+// c1 = 0.25 s15, c2 = 0.625 s15, all float64 from the host
+struct GatParams {
+    double gain, offset, qq, s15, c1, c2;
+};
+void b4d_launch_gat_forward(const uint16_t *in, float *out, long long n, const GatParams &p, cudaStream_t s);
+// float32 result into `out`, or (q16 non-null) K7 of it into q16
+void b4d_launch_gat_inverse(const float *in, float *out, uint16_t *q16, long long n, const GatParams &p,
+                            float offset_sub, float offset_add, float step, int trunc, cudaStream_t s);
+
+// K7: q = rint(clip((x - offset_sub + offset_add) / step, 0, 65535/step)).
+// float32, clip BEFORE round, round-half-to-even: transforms.py:403-411.
+__device__ __forceinline__ uint32_t quant1(float x, float osub, float oadd, float step, float hi, bool unit) {
+    float v = __fadd_rn(__fsub_rn(x, osub), oadd);
+    if (!unit) v = __fdiv_rn(v, step);
+    v = fminf(fmaxf(v, 0.0f), hi);
+    return (uint32_t)__float2int_rn(v);
+}
+// truncating variant: np.maximum(x, 0).astype(int) (evaluate.py:202) followed by the uint16 cast of
+// compute_cratio (utils/img_util.py:420-423): toward zero, no upper clip, int64 -> uint16 wraps modulo 2^16
+__device__ __forceinline__ uint32_t quant1_trunc(float x, float osub, float oadd, float step, float hi, bool unit) {
+    (void)hi;
+    float v = __fadd_rn(__fsub_rn(x, osub), oadd);
+    if (!unit) v = __fdiv_rn(v, step);
+    v = fmaxf(v, 0.0f);  // NaN -> 0
+    return (uint32_t)(__float2ll_rz(v) & 0xFFFFll);
+}
+template <bool TRUNC>
+__device__ __forceinline__ uint32_t quantq(float x, float osub, float oadd, float step, float hi, bool unit) {
+    return TRUNC ? quant1_trunc(x, osub, oadd, step, hi, unit) : quant1(x, osub, oadd, step, hi, unit);
+}
 // coherence gate (b4d_coherence.cu): 23 sums per (patch, label slot), see there
 void b4d_launch_coherence(const float *raw, const unsigned long long *labels, int D, int H, int W, long long npatch,
                           int lag, int radius, const double *w, double *x, double *sm, double *tmp,

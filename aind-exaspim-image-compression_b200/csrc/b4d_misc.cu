@@ -175,8 +175,6 @@ struct NormOut {
     float q_sub, q_add, q_step, q_hi;
     int q_unit, q_trunc;
 };
-__device__ __forceinline__ uint32_t quant1(float x, float osub, float oadd, float step, float hi, bool unit);
-__device__ __forceinline__ uint32_t quant1_trunc(float x, float osub, float oadd, float step, float hi, bool unit);
 // One WARP owns an 8 x 29 (y, x) tile and marches along z over WM_NZ planes (+3 planes of run-in); no shared memory,
 // no barrier.  Lane i holds column X0 - 3 + i of the uint32 map for the 11 rows Y0 - 3 .. Y0 + 7 (lanes 0-2 are the
 // x halo); the x pass takes the three left neighbours by warp shuffles of the uint32 values, the y pass runs on the
@@ -371,27 +369,7 @@ __global__ void __launch_bounds__(WMT_WARPS * 32, 4) k_normalise_wm_tma(const __
 }
 
 // -------------------------------------------------------------- quantize ----
-// K7: q = rint(clip((x - offset_sub + offset_add) / step, 0, 65535/step)).
-// float32, clip BEFORE round, round-half-to-even: transforms.py:403-411.
-__device__ __forceinline__ uint32_t quant1(float x, float osub, float oadd, float step, float hi, bool unit) {
-    float v = __fadd_rn(__fsub_rn(x, osub), oadd);
-    if (!unit) v = __fdiv_rn(v, step);
-    v = fminf(fmaxf(v, 0.0f), hi);
-    return (uint32_t)__float2int_rn(v);
-}
-// truncating variant: np.maximum(x, 0).astype(int) (evaluate.py:202) followed by the uint16 cast of
-// compute_cratio (utils/img_util.py:420-423): toward zero, no upper clip, int64 -> uint16 wraps modulo 2^16
-__device__ __forceinline__ uint32_t quant1_trunc(float x, float osub, float oadd, float step, float hi, bool unit) {
-    (void)hi;
-    float v = __fadd_rn(__fsub_rn(x, osub), oadd);
-    if (!unit) v = __fdiv_rn(v, step);
-    v = fmaxf(v, 0.0f);  // NaN -> 0
-    return (uint32_t)(__float2ll_rz(v) & 0xFFFFll);
-}
-template <bool TRUNC>
-__device__ __forceinline__ uint32_t quantq(float x, float osub, float oadd, float step, float hi, bool unit) {
-    return TRUNC ? quant1_trunc(x, osub, oadd, step, hi, unit) : quant1(x, osub, oadd, step, hi, unit);
-}
+// K7 (quant1, quant1_trunc: b4d_common.cuh, shared with the fused GAT inverse of b4d_vst.cu)
 template <bool TRUNC>
 __global__ void __launch_bounds__(256) k_quantize(const float *__restrict__ in, uint16_t *__restrict__ out,
                                                   long long n, float osub, float oadd, float step) {

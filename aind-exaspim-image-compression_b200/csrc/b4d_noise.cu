@@ -8,6 +8,8 @@
 //
 // Traversal: a CTA takes a run of cell rows (fixed z, y) of one tile, a warp one row at a time, lane = cell along
 // x, so consecutive lanes read consecutive 4-byte words (W even, 4-byte aligned base) or 2-byte pairs otherwise.
+#include <algorithm>
+
 #include "b4d_common.cuh"
 
 namespace {
@@ -235,6 +237,125 @@ __global__ void __launch_bounds__(256) k_noise_hist(NoiseGeom g, long long nvol,
         if (sh[i]) atomicAdd(&hist[i], (unsigned long long)sh[i]);
 }
 
+// ---------------------------------------------------------------- noise-level function (DESIGN §3.12) ----
+// The passes above keyed by the intensity bin of each cell instead of its tile.  A CTA keeps the histograms of
+// its bins in dynamic shared memory ([nr][512] in pass 1, [nr][1024] in pass 2) and flushes the non-zero entries
+// once; its warps stride over every cell row of every volume.
+constexpr int NLF_THREADS = 1024;
+constexpr int NLF_SMEM_CAP = 200 * 1024;  // bytes of dynamic shared memory per CTA: 50 bins in pass 2
+
+// |d| of the cell at (cz, cy, cx) and the sum s of its 8 voxels (s == 0: all zero, padding)
+template <bool WIDE>
+__device__ __forceinline__ uint32_t cell_detail_sum(const uint16_t *__restrict__ vol, int H, int W, int cz, int cy,
+                                                    int cx, uint32_t &s) {
+    const long long plane = (long long)H * W;
+    const uint16_t *p = vol + (2ll * cz * H + 2ll * cy) * W + 2ll * cx;
+    int a0, b0, a1, b1, a2, b2, a3, b3;
+    if (WIDE) {
+        const uint32_t w0 = __ldcs(reinterpret_cast<const unsigned int *>(p));
+        const uint32_t w1 = __ldcs(reinterpret_cast<const unsigned int *>(p + W));
+        const uint32_t w2 = __ldcs(reinterpret_cast<const unsigned int *>(p + plane));
+        const uint32_t w3 = __ldcs(reinterpret_cast<const unsigned int *>(p + plane + W));
+        a0 = (int)(w0 & 0xFFFFu), b0 = (int)(w0 >> 16);
+        a1 = (int)(w1 & 0xFFFFu), b1 = (int)(w1 >> 16);
+        a2 = (int)(w2 & 0xFFFFu), b2 = (int)(w2 >> 16);
+        a3 = (int)(w3 & 0xFFFFu), b3 = (int)(w3 >> 16);
+    } else {
+        a0 = __ldcs(p), b0 = __ldcs(p + 1);
+        a1 = __ldcs(p + W), b1 = __ldcs(p + W + 1);
+        a2 = __ldcs(p + plane), b2 = __ldcs(p + plane + 1);
+        a3 = __ldcs(p + plane + W), b3 = __ldcs(p + plane + W + 1);
+    }
+    s = (uint32_t)((a0 + b0) + (a1 + b1) + (a2 + b2) + (a3 + b3));
+    const int d = (a0 - b0) - (a1 - b1) - (a2 - b2) + (a3 - b3);
+    return (uint32_t)(d < 0 ? -d : d);
+}
+
+// Intensity bin of a cell sum: the last k with thr[k] <= s (thr non-decreasing, padded with INT32_MAX), -1 below
+// thr[0].  Bin k exists for k < nb only.
+__device__ __forceinline__ int nlf_bin(const int *thr, uint32_t s) {
+    int lo = 0;
+#pragma unroll
+    for (int st = NLF_THR / 2; st; st >>= 1)
+        if (thr[lo + st - 1] <= (int)s) lo += st;
+    return lo - 1;
+}
+
+// sh[key] += v summed over the warp's lanes with `ok`, one 64-bit shared atomic per distinct key (nearly every
+// cell of a warp lies in the same background bin).  Uniform over the warp.
+__device__ __forceinline__ void warp_sum_add(unsigned long long *sh, uint32_t key, uint32_t v, bool ok) {
+    uint32_t pending = __ballot_sync(B4D_FULL, ok);
+    while (pending) {
+        const int leader = __ffs(pending) - 1;
+        const uint32_t k = __shfl_sync(B4D_FULL, key, leader);
+        const bool mine = ok && key == k;
+        const uint32_t sum = __reduce_add_sync(B4D_FULL, mine ? v : 0u);  // <= 32 * 524280 < 2^32
+        if ((int)(threadIdx.x & 31) == leader) atomicAdd(&sh[k], (unsigned long long)sum);
+        pending &= ~__ballot_sync(B4D_FULL, mine);
+    }
+}
+
+template <int PASS, bool WIDE>
+__global__ void __launch_bounds__(NLF_THREADS) k_nlf_pass(NlfGeom g, uint32_t *__restrict__ hist,
+                                                          unsigned long long *__restrict__ lsum,
+                                                          const uint32_t *__restrict__ sel) {
+    constexpr int PER = PASS == 1 ? 512 : 1024;
+    extern __shared__ uint32_t dsh[];  // [nr][PER] counts; pass 1 then [nr] 64-bit level sums
+    __shared__ int thr[NLF_THR];
+    __shared__ uint32_t hi_a[B4D_NLF_MAX_BINS], hi_b[B4D_NLF_MAX_BINS];  // pass 2: high digits of the two ranks
+    const int nr = g.kb1 - g.kb0;
+    unsigned long long *ssum = reinterpret_cast<unsigned long long *>(dsh + nr * PER);
+    for (int i = threadIdx.x; i < NLF_THR; i += blockDim.x) thr[i] = g.thr[i];
+    for (int i = threadIdx.x; i < nr * PER; i += blockDim.x) dsh[i] = 0u;
+    for (int i = threadIdx.x; i < nr; i += blockDim.x) {
+        if (PASS == 1) {
+            ssum[i] = 0ull;
+        } else {
+            const uint32_t *s = sel + (long long)(g.kb0 + i) * 5;
+            hi_a[i] = s[0] ? s[1] : 0xFFFFFFFFu;  // a bin without cells matches no high digit
+            hi_b[i] = s[0] ? s[3] : 0xFFFFFFFFu;
+        }
+    }
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const long long rows_per_vol = (long long)g.ncz * g.ncy, rows = rows_per_vol * g.nvol;
+    const long long nw = (long long)gridDim.x * (blockDim.x >> 5);
+    for (long long r = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); r < rows; r += nw) {
+        const long long v = r / rows_per_vol;
+        const int rr = (int)(r - v * rows_per_vol);
+        const int cz = rr / g.ncy, cy = rr % g.ncy;
+        const uint16_t *vol = g.in + v * g.vol_stride;
+        for (int x = 0; x < g.ncx; x += 64) {  // two cells per lane in flight
+            const bool in0 = x + lane < g.ncx, in1 = x + 32 + lane < g.ncx;
+            uint32_t d0 = 0, d1 = 0, s0 = 0, s1 = 0;
+            if (in0) d0 = cell_detail_sum<WIDE>(vol, g.H, g.W, cz, cy, x + lane, s0);
+            if (in1) d1 = cell_detail_sum<WIDE>(vol, g.H, g.W, cz, cy, x + 32 + lane, s1);
+            const int k0 = nlf_bin(thr, s0) - g.kb0, k1 = nlf_bin(thr, s1) - g.kb0;
+            bool ok0 = s0 != 0u && k0 >= 0 && k0 < nr, ok1 = s1 != 0u && k1 >= 0 && k1 < nr;
+            if (PASS == 1) {
+                warp_hist_add(dsh, (uint32_t)k0 * 512u + (d0 >> 9), ok0);
+                warp_hist_add(dsh, (uint32_t)k1 * 512u + (d1 >> 9), ok1);
+                warp_sum_add(ssum, (uint32_t)k0, s0, ok0);
+                warp_sum_add(ssum, (uint32_t)k1, s1, ok1);
+            } else {
+                const uint32_t h0 = d0 >> 9, h1 = d1 >> 9;
+                const uint32_t a0 = ok0 ? hi_a[k0] : 0u, b0 = ok0 ? hi_b[k0] : 0u;
+                const uint32_t a1 = ok1 ? hi_a[k1] : 0u, b1 = ok1 ? hi_b[k1] : 0u;
+                ok0 = ok0 && (h0 == a0 || h0 == b0);
+                ok1 = ok1 && (h1 == a1 || h1 == b1);
+                warp_hist_add(dsh, (uint32_t)k0 * 1024u + (h0 == a0 ? 0u : 512u) + (d0 & 511u), ok0);
+                warp_hist_add(dsh, (uint32_t)k1 * 1024u + (h1 == a1 ? 0u : 512u) + (d1 & 511u), ok1);
+            }
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < nr * PER; i += blockDim.x)
+        if (dsh[i]) atomicAdd(&hist[(long long)(g.kb0 + i / PER) * 1024 + i % PER], dsh[i]);
+    if (PASS == 1)
+        for (int i = threadIdx.x; i < nr; i += blockDim.x)
+            if (ssum[i]) atomicAdd(&lsum[g.kb0 + i], ssum[i]);
+}
+
 int sm_count() {
     static int sms = 0;
     if (!sms) {
@@ -248,7 +369,37 @@ int sm_count() {
 
 bool wide_ok(const NoiseGeom &g) { return (g.W & 1) == 0 && (reinterpret_cast<uintptr_t>(g.in) & 3) == 0; }
 
+// A persistent grid: as many CTAs as fit on the device at this launch's shared-memory size, fewer for small calls.
+template <int PASS, bool WIDE>
+void launch_nlf(const NlfGeom &g, uint32_t *hist, unsigned long long *lsum, const uint32_t *sel, cudaStream_t s) {
+    const int nr = g.kb1 - g.kb0;
+    const size_t smem = (size_t)nr * (PASS == 1 ? 512 * 4 + 8 : 1024 * 4);
+    cudaFuncSetAttribute(k_nlf_pass<PASS, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    int per_sm = 0;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_nlf_pass<PASS, WIDE>, NLF_THREADS, smem);
+    const long long rows = (long long)g.ncz * g.ncy * g.nvol;
+    long long blocks = (rows + NLF_THREADS / 32 - 1) / (NLF_THREADS / 32);
+    blocks = std::min<long long>(blocks, (long long)std::max(1, per_sm) * sm_count());
+    k_nlf_pass<PASS, WIDE><<<(unsigned)std::max(1ll, blocks), NLF_THREADS, smem, s>>>(g, hist, lsum, sel);
+}
+
 }  // namespace
+
+int b4d_nlf_bins_per_launch(int pass) {
+    return pass == 1 ? B4D_NLF_MAX_BINS : NLF_SMEM_CAP / (1024 * 4);
+}
+
+void b4d_launch_nlf_pass(const NlfGeom &g, int pass, uint32_t *hist, unsigned long long *lsum, const uint32_t *sel,
+                         cudaStream_t s) {
+    const bool w = (g.W & 1) == 0 && (reinterpret_cast<uintptr_t>(g.in) & 3) == 0;
+    if (pass == 1) {
+        if (w) launch_nlf<1, true>(g, hist, lsum, sel, s);
+        else launch_nlf<1, false>(g, hist, lsum, sel, s);
+    } else {
+        if (w) launch_nlf<2, true>(g, hist, lsum, sel, s);
+        else launch_nlf<2, false>(g, hist, lsum, sel, s);
+    }
+}
 
 void b4d_launch_noise_pass(const NoiseGeom &g, int pass, long long ntiles, uint32_t *hist, const uint32_t *sel,
                            cudaStream_t s) {
