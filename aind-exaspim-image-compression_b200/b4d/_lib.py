@@ -15,53 +15,61 @@ ABI_VERSION = 1
 T_NAMES = ("prep", "match1", "filter1", "norm1", "match2", "filter2", "norm2", "k0")
 T_COUNT = 8
 
-EXPORTS = (
-    "b4d_version",
-    "b4d_last_error",
-    "b4d_default_profile",
-    "b4d_create",
-    "b4d_destroy",
-    "b4d_set_profile",
-    "b4d_denoise_u16",
-    "b4d_denoise_f32",
-    "b4d_targets_u16",
-    "b4d_set_pass_voxels",
-    "b4d_set_pipeline_min_voxels",
-    "b4d_chunk_shuffle_u16",
-    "b4d_foreground_mask_u16",
-    "b4d_denoise_slab_u16",
-    "b4d_slab_stage1_u16",
-    "b4d_slab_basic_planes",
-    "b4d_slab_stage2",
-    "b4d_match_stage1",
-    "b4d_num_refs",
-    "b4d_quantize_u16",
-    "b4d_tile_stats",
-    "b4d_last_timings",
-    "b4d_stream",
-    "b4d_last_match_stats",
-    "b4d_measure_pipe_peaks",
-    "b4d_debug_accumulators",
-    "b4d_quantize_trunc_u16",
-    "b4d_denoise_q16_u16",
-    "b4d_denoise_slab_q16_u16",
-    "b4d_slab_stage2_q16",
-    "b4d_slab_basic_ptr",
-    "b4d_slab_stage2_begin",
-    "b4d_stats_from_hist",
-    "b4d_coherence_gate",
-    "b4d_set_noise_model",
-)
+# Prototypes of the C ABI, name -> (restype, argtypes), in header order.  load() applies them, so every call converts
+# its arguments through ctypes: int64_t / int / float / double take plain Python numbers, and every pointer or array
+# parameter is a c_void_p that takes an address (int), None, a ctypes array or byref(struct) -- an ndarray is refused.
+_I64, _INT, _F32, _F64, _P = ctypes.c_int64, ctypes.c_int, ctypes.c_float, ctypes.c_double, ctypes.c_void_p
+_CORE = {
+    "b4d_version": (_INT, []),
+    "b4d_last_error": (ctypes.c_char_p, []),
+    "b4d_default_profile": (None, [_P]),
+    "b4d_create": (_INT, [_INT, _P, _P]),
+    "b4d_destroy": (None, [_P]),
+    "b4d_set_profile": (_INT, [_P, _P]),
+    "b4d_denoise_u16": (_INT, [_P, _P, _I64, _P, _F32, _P, _INT, _INT]),
+    "b4d_denoise_f32": (_INT, [_P, _P, _I64, _P, _F32, _P, _INT, _INT]),
+    "b4d_set_pass_voxels": (_INT, [_P, _I64]),
+    "b4d_set_pipeline_min_voxels": (_INT, [_P, _I64]),
+    "b4d_targets_u16": (_INT, [_P, _P, _I64, _P, _P, _F32, _F32, _P, _P, _INT, _INT]),
+    "b4d_denoise_slab_u16": (_INT, [_P, _P, _P, _I64, _I64, _I64, _I64, _F32, _P, _INT, _INT]),
+    "b4d_slab_stage1_u16": (_INT, [_P, _P, _P, _I64, _I64, _F32, _INT]),
+    "b4d_slab_basic_planes": (_INT, [_P, _I64, _I64, _P, _INT, _INT]),
+    "b4d_slab_stage2": (_INT, [_P, _I64, _I64, _P, _INT]),
+    "b4d_slab_basic_ptr": (_P, [_P]),
+    "b4d_slab_stage2_begin": (_INT, [_P, _I64, _I64]),
+    "b4d_slab_stage2_q16": (_INT, [_P, _I64, _I64, _F32, _F32, _F32, _INT, _P, _INT]),
+    "b4d_match_stage1": (_INT, [_P, _P, _P, _F32, _P, _P, _P]),
+    "b4d_num_refs": (_I64, [_P]),
+    "b4d_quantize_u16": (_INT, [_P, _P, _I64, _F32, _F32, _F32, _P, _INT, _INT]),
+    "b4d_quantize_trunc_u16": (_INT, [_P, _P, _I64, _F32, _F32, _F32, _P, _INT, _INT]),
+    "b4d_denoise_slab_q16_u16": (_INT, [_P, _P, _P, _I64, _I64, _I64, _I64, _F32, _F32, _F32, _F32, _INT, _P, _INT,
+                                         _INT]),
+    "b4d_denoise_q16_u16": (_INT, [_P, _P, _P, _F32, _F32, _F32, _F32, _INT, _P, _INT, _INT]),
+    "b4d_foreground_mask_u16": (_INT, [_P, _P, _I64, _P, _P, _F32, _INT, _P, _INT, _INT]),
+    "b4d_chunk_shuffle_u16": (_INT, [_P, _P, _P, _P, _P, _P, _INT, _INT]),
+    "b4d_tile_stats": (_INT, [_P, _P, _I64, _F64, _P, _P, _INT]),
+    "b4d_stats_from_hist": (_INT, [_P, _F64, _P]),
+    "b4d_last_timings": (_INT, [_P, _P, _P]),
+    "b4d_stream": (_P, [_P]),
+    "b4d_last_match_stats": (_INT, [_P, _P]),
+    "b4d_measure_pipe_peaks": (_INT, [_P, _P]),
+    "b4d_set_noise_model": (_INT, [_P, _P, _P]),
+    "b4d_coherence_gate": (_INT, [_P, _P, _P, _I64, _P, _F64, _F64, _I64, _F64, _INT, _P, _P, _I64, _P, _INT]),
+    "b4d_debug_accumulators": (_INT, [_P, _P, _P, _I64]),
+}
 # include/b4d_noise.h: the noise-level extension (no counterpart in the CPU oracle library)
-NOISE_EXPORTS = (
-    "b4d_noise_sigma_u16",
-    "b4d_noise_sigma_from_hist",
-    "b4d_noise_level_u16",
-    "b4d_gat_forward_u16",
-    "b4d_gat_inverse_f32",
-    "b4d_denoise_vst_u16",
-    "b4d_denoise_vst_q16_u16",
-)
+_NOISE = {
+    "b4d_noise_sigma_u16": (_INT, [_P, _P, _I64, _P, _P, _P, _P, _P, _P, _INT]),
+    "b4d_noise_sigma_from_hist": (_INT, [_P, _P, _P, _P]),
+    "b4d_noise_level_u16": (_INT, [_P, _P, _I64, _P, _P, _INT, _I64, _P, _P, _P, _P, _P, _P, _P, _INT]),
+    "b4d_gat_forward_u16": (_INT, [_P, _P, _P, _I64, _P, _INT, _INT]),
+    "b4d_gat_inverse_f32": (_INT, [_P, _P, _P, _I64, _P, _INT, _INT]),
+    "b4d_denoise_vst_u16": (_INT, [_P, _P, _I64, _P, _P, _F32, _P, _INT, _INT]),
+    "b4d_denoise_vst_q16_u16": (_INT, [_P, _P, _I64, _P, _P, _F32, _F32, _F32, _F32, _INT, _P, _INT, _INT]),
+}
+SIGNATURES = {**_CORE, **_NOISE}
+EXPORTS = tuple(_CORE)
+NOISE_EXPORTS = tuple(_NOISE)
 NOISE_HIST_BINS = 262141  # B4D_NOISE_HIST_BINS: |d| <= 4 * 65535
 NLF_MAX_BINS = 64  # B4D_NLF_MAX_BINS
 
@@ -120,21 +128,9 @@ def load():
             "or `make -C aind-exaspim-image-compression_b200/csrc`. There is no CPU fallback." % LIB_PATH
         )
     lib = ctypes.CDLL(LIB_PATH)
-    lib.b4d_last_error.restype = ctypes.c_char_p
-    lib.b4d_num_refs.restype = ctypes.c_int64
-    lib.b4d_destroy.restype = None
-    lib.b4d_stream.restype = ctypes.c_void_p
-    lib.b4d_slab_basic_ptr.restype = ctypes.c_void_p
-    lib.b4d_default_profile.restype = None
-    i64p, vp = ctypes.POINTER(ctypes.c_int64), ctypes.c_void_p
-    lib.b4d_noise_sigma_u16.argtypes = [vp, vp, ctypes.c_int64, i64p, i64p, vp, vp, vp, vp, ctypes.c_int]
-    lib.b4d_noise_sigma_from_hist.argtypes = [vp, vp, vp, vp]
-    i64, f32, c_int = ctypes.c_int64, ctypes.c_float, ctypes.c_int
-    lib.b4d_noise_level_u16.argtypes = [vp, vp, i64, i64p, vp, c_int, i64, vp, vp, vp, vp, vp, vp, vp, c_int]
-    lib.b4d_gat_forward_u16.argtypes = [vp, vp, vp, i64, vp, c_int, c_int]
-    lib.b4d_gat_inverse_f32.argtypes = [vp, vp, vp, i64, vp, c_int, c_int]
-    lib.b4d_denoise_vst_u16.argtypes = [vp, vp, i64, i64p, vp, f32, vp, c_int, c_int]
-    lib.b4d_denoise_vst_q16_u16.argtypes = [vp, vp, i64, i64p, vp, f32, f32, f32, f32, c_int, vp, c_int, c_int]
+    for name, (restype, argtypes) in SIGNATURES.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     if lib.b4d_version() != ABI_VERSION:
         raise B4DLibraryError("libb4d.so ABI %d != binding ABI %d" % (lib.b4d_version(), ABI_VERSION))
     _lib = lib

@@ -20,6 +20,7 @@ there is no CPU fallback.
 import collections
 import ctypes
 import enum
+import math
 import os
 
 import numpy as np
@@ -98,6 +99,57 @@ def _is_torch(x):
     return type(x).__module__.split(".")[0] == "torch"
 
 
+def _dtype_name(x):
+    return str(x.dtype).replace("torch.", "")
+
+
+def _array_arg(x, dtypes, ndims, what, cast=False):
+    """Check an array argument before any handle or device work: a torch tensor, or anything np.asarray takes, of one
+    of the dtype names `dtypes` and, unless `ndims` is None, of one of the dimensionalities `ndims`; ValueError
+    otherwise.  With `cast`, NumPy input is first converted to dtypes[0] (a tensor must have it already).  Returns the
+    tensor or the ndarray."""
+    if not _is_torch(x):
+        x = np.asarray(x, dtype=dtypes[0] if cast else None)
+    dtype = _dtype_name(x)
+    if dtype not in dtypes:
+        raise ValueError("%s expects %s, got %s" % (what, " or ".join(dtypes), dtype))
+    if ndims is not None and x.ndim not in ndims:
+        raise ValueError("%s expects %s-D input, got %d-D" % (what, " or ".join(str(n) for n in ndims), x.ndim))
+    return x
+
+
+def _ptr(a):
+    """Address of an array's data for a pointer parameter of the C ABI; None stays None (NULL)."""
+    if a is None:
+        return None
+    return a.data_ptr() if _is_torch(a) else a.ctypes.data
+
+
+def _out_like(x, shape, dtype):
+    """New output of `shape` and dtype name `dtype` where the input x lives: torch on x's device, else NumPy."""
+    if _is_torch(x):
+        import torch
+
+        return torch.empty(shape, dtype=getattr(torch, dtype), device=x.device)
+    return np.empty(shape, dtype=dtype)
+
+
+def _host_out(out, shape, dtype):
+    """A caller's NumPy output (e.g. a pinned buffer), which must be C-contiguous of `shape` and `dtype`; a new array
+    when `out` is None."""
+    if out is None:
+        return np.empty(shape, dtype=dtype)
+    if out.shape != tuple(shape) or out.dtype != dtype or not out.flags.c_contiguous:
+        raise ValueError("out must be a C-contiguous %s array of shape %r" % (np.dtype(dtype).name, tuple(shape)))
+    return out
+
+
+def _quantize_args(quantize):
+    """quantize = (offset_sub, offset_add, step[, truncate]) -> the four trailing arguments of the *_q16 calls."""
+    q = tuple(quantize) + (False,) * (4 - len(quantize))
+    return q[0], q[1], q[2], int(bool(q[3]))
+
+
 class Denoiser:
     """One ``b4d_handle``: scratch buffers + a stream on one CUDA device.
     Not thread-safe; one per (process, device)."""
@@ -123,13 +175,45 @@ class Denoiser:
         except Exception:
             pass
 
+    def _check_device(self, device):
+        """ValueError unless the torch device `device` is this handle's CUDA device: the library would otherwise be
+        handed a pointer into another GPU's memory."""
+        if device.type != "cuda" or device.index != self.device:
+            raise ValueError("%s is not the handle's device cuda:%d" % (device, self.device))
+
+    def _input(self, x):
+        """(keep-alive, pointer, on-device flag, shape) of an array that passed _array_arg.  A CUDA tensor must live on
+        the handle's device; a tensor is made contiguous, and the current torch stream of its device is synchronised so
+        that the library reads finished data.  NumPy input is made C-contiguous."""
+        if not _is_torch(x):
+            xc = np.ascontiguousarray(x)
+            return xc, xc.ctypes.data, False, xc.shape
+        if x.is_cuda:
+            self._check_device(x.device)
+        xc = x.contiguous()
+        if xc.is_cuda:
+            import torch
+
+            torch.cuda.current_stream(xc.device).synchronize()
+        return xc, xc.data_ptr(), xc.is_cuda, tuple(xc.shape)
+
+    def _device_out(self, shape, dtype, device):
+        """New torch output of dtype name `dtype` on `device`, which must be the handle's CUDA device ("cuda" without
+        an index is the current device, as torch reads it)."""
+        import torch
+
+        device = torch.device(device)
+        if device.type == "cuda" and device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        self._check_device(device)
+        return torch.empty(shape, dtype=getattr(torch, dtype), device=device)
+
     def debug_accumulators(self, n):
         """(numq, wmap) int64 arrays: the fixed-point aggregation state the last filter stage of the last
         single-volume call left on the device (b4d_debug_accumulators; diagnostics for the parity tests)."""
         numq = np.empty(n, dtype=np.int64)
         wmap = np.empty(n, dtype=np.int64)
-        _lib.check(self.lib.b4d_debug_accumulators(self._h, numq.ctypes.data_as(ctypes.c_void_p),
-                                                   wmap.ctypes.data_as(ctypes.c_void_p), ctypes.c_int64(n)))
+        _lib.check(self.lib.b4d_debug_accumulators(self._h, numq.ctypes.data, wmap.ctypes.data, n))
         return numq, wmap
 
     def set_noise_model(self, nu_ht=None, nu_wie=None):
@@ -142,8 +226,7 @@ class Denoiser:
         b = np.ascontiguousarray(nu_wie, dtype=np.float32).reshape(-1)
         if a.size != 64 or b.size != 64:
             raise ValueError("nu_ht and nu_wie must hold 64 values each")
-        _lib.check(self.lib.b4d_set_noise_model(self._h, a.ctypes.data_as(ctypes.c_void_p),
-                                                b.ctypes.data_as(ctypes.c_void_p)))
+        _lib.check(self.lib.b4d_set_noise_model(self._h, a.ctypes.data, b.ctypes.data))
 
     def set_profile(self, profile=None, stages=2):
         """Switch algorithm constants (no-op when nothing changes)."""
@@ -158,205 +241,71 @@ class Denoiser:
     # ---- raw pointer level -------------------------------------------------
     def denoise_ptr(self, in_ptr, dtype, n, shape, sigma, out_ptr, in_dev, out_dev):
         fn = self.lib.b4d_denoise_u16 if dtype == np.uint16 else self.lib.b4d_denoise_f32
-        _lib.check(
-            fn(
-                self._h,
-                ctypes.c_void_p(in_ptr),
-                ctypes.c_int64(n),
-                _lib.shape3(shape),
-                ctypes.c_float(sigma),
-                ctypes.c_void_p(out_ptr),
-                int(in_dev),
-                int(out_dev),
-            )
-        )
+        _lib.check(fn(self._h, in_ptr, n, _lib.shape3(shape), sigma, out_ptr, int(in_dev), int(out_dev)))
 
     # ---- array level ---------------------------------------------------------
     def denoise(self, z, sigma):
         """(D,H,W) or (N,D,H,W); uint16 or float32; NumPy or torch -> float32."""
-        if _is_torch(z):
-            import torch
-
-            if z.dtype not in (torch.uint16, torch.float32):
-                raise ValueError("torch input must be uint16 or float32, got %s" % z.dtype)
-            zc = z.contiguous()
-            if zc.ndim not in (3, 4):
-                raise ValueError("expected a 3-D volume or a 4-D batch, got %d-D" % zc.ndim)
-            n = zc.shape[0] if zc.ndim == 4 else 1
-            on_dev = zc.is_cuda
-            if on_dev and zc.device.index != self.device:
-                raise ValueError("tensor lives on cuda:%s, handle on cuda:%d" % (zc.device.index, self.device))
-            out = torch.empty(zc.shape, dtype=torch.float32, device=zc.device)
-            if on_dev:
-                torch.cuda.current_stream(zc.device).synchronize()
-            self.denoise_ptr(
-                zc.data_ptr(),
-                np.uint16 if zc.dtype == torch.uint16 else np.float32,
-                n,
-                tuple(zc.shape[-3:]),
-                sigma,
-                out.data_ptr(),
-                on_dev,
-                on_dev,
-            )
-            return out
-        z = np.asarray(z)
-        if z.ndim not in (3, 4):
-            raise ValueError("expected a 3-D volume or a 4-D batch, got %d-D" % z.ndim)
-        zc = np.ascontiguousarray(z)
-        n = zc.shape[0] if zc.ndim == 4 else 1
-        out = np.empty(zc.shape, dtype=np.float32)
-        self.denoise_ptr(zc.ctypes.data, zc.dtype.type, n, zc.shape[-3:], sigma, out.ctypes.data, 0, 0)
+        zc, ptr, on_dev, shape = self._input(_array_arg(z, ("uint16", "float32"), (3, 4), "denoise"))
+        out = _out_like(zc, shape, "float32")
+        n = shape[0] if len(shape) == 4 else 1
+        self.denoise_ptr(ptr, np.dtype(_dtype_name(zc)), n, shape[-3:], sigma, _ptr(out), on_dev, on_dev)
         return out
 
     def targets(self, raw_u16, offsets, sigma, max_count=65535.0, raw_out=None, teacher_out=None):
         """(N,D,H,W) uint16 patches + per-patch offsets -> (raw, teacher) float32 in one call
         (b4d_targets_u16: subtraction, BM4D and clip all on the device).  `raw_out` / `teacher_out`
         may be preallocated C-contiguous float32 arrays (e.g. the cache's memmaps)."""
-        zc = np.ascontiguousarray(raw_u16)
-        if zc.ndim != 4 or zc.dtype != np.uint16:
-            raise ValueError("raw_u16 must be (N, D, H, W) uint16")
+        zc = np.ascontiguousarray(_array_arg(raw_u16, ("uint16",), (4,), "targets"))
         off = np.ascontiguousarray(np.broadcast_to(np.asarray(offsets, dtype=np.float32), (zc.shape[0],)))
-        outs = []
-        for o in (raw_out, teacher_out):
-            if o is None:
-                o = np.empty(zc.shape, dtype=np.float32)
-            elif o.shape != zc.shape or o.dtype != np.float32 or not o.flags.c_contiguous:
-                raise ValueError("output must be a C-contiguous float32 array of shape %r" % (zc.shape,))
-            outs.append(o)
-        _lib.check(
-            self.lib.b4d_targets_u16(
-                self._h,
-                ctypes.c_void_p(zc.ctypes.data),
-                ctypes.c_int64(zc.shape[0]),
-                _lib.shape3(zc.shape[1:]),
-                ctypes.c_void_p(off.ctypes.data),
-                ctypes.c_float(sigma),
-                ctypes.c_float(max_count),
-                ctypes.c_void_p(outs[0].ctypes.data),
-                ctypes.c_void_p(outs[1].ctypes.data),
-                0,
-                0,
-            )
-        )
-        return outs[0], outs[1]
+        raw_out = _host_out(raw_out, zc.shape, np.float32)
+        teacher_out = _host_out(teacher_out, zc.shape, np.float32)
+        _lib.check(self.lib.b4d_targets_u16(self._h, zc.ctypes.data, zc.shape[0], _lib.shape3(zc.shape[1:]),
+                                            off.ctypes.data, sigma, max_count, raw_out.ctypes.data,
+                                            teacher_out.ctypes.data, 0, 0))
+        return raw_out, teacher_out
 
     def denoise_slab(self, slab, z_begin, z_total, own_begin, own_end, sigma, out=None, quantize=None):
         """One z-slab (uint16, with halos) of a larger volume -> float32 owned planes.
         `out` (NumPy path only) receives the result in place, e.g. a pinned buffer.
         quantize = (offset_sub, offset_add, step[, truncate]): the fused denoise -> offset -> quantize path, the
         result is the uint16 volume K7 would give on the float32 output (2 bytes per voxel leave the device)."""
-        odt_np, odt_t = (np.float32, "float32") if quantize is None else (np.uint16, "uint16")
-        if _is_torch(slab):
-            import torch
-
-            sc = slab.contiguous()
-            if sc.dtype != torch.uint16 or sc.ndim != 3:
-                raise ValueError("slab must be a 3-D uint16 tensor")
-            out = torch.empty((own_end - own_begin,) + tuple(sc.shape[1:]), dtype=getattr(torch, odt_t), device=sc.device)
-            on_dev = sc.is_cuda
-            if on_dev:
-                torch.cuda.current_stream(sc.device).synchronize()
-            in_ptr, out_ptr, shape = sc.data_ptr(), out.data_ptr(), tuple(sc.shape)
+        sc, in_ptr, on_dev, shape = self._input(_array_arg(slab, ("uint16",), (3,), "denoise_slab"))
+        odt = "float32" if quantize is None else "uint16"
+        oshape = (own_end - own_begin,) + shape[1:]
+        out = _out_like(sc, oshape, odt) if _is_torch(sc) else _host_out(out, oshape, odt)
+        if quantize is None:
+            _lib.check(self.lib.b4d_denoise_slab_u16(self._h, in_ptr, _lib.shape3(shape), z_begin, z_total, own_begin,
+                                                     own_end, sigma, _ptr(out), on_dev, on_dev))
         else:
-            sc = np.ascontiguousarray(slab)
-            if sc.dtype != np.uint16 or sc.ndim != 3:
-                raise ValueError("slab must be a 3-D uint16 array")
-            oshape = (own_end - own_begin,) + sc.shape[1:]
-            if out is None:
-                out = np.empty(oshape, dtype=odt_np)
-            elif out.shape != oshape or out.dtype != odt_np or not out.flags.c_contiguous:
-                raise ValueError("out must be a C-contiguous %s array of shape %r" % (odt_t, oshape))
-            on_dev = False
-            in_ptr, out_ptr, shape = sc.ctypes.data, out.ctypes.data, sc.shape
-        if quantize is not None:
-            q = tuple(quantize) + (False,) * (4 - len(quantize))
-            _lib.check(
-                self.lib.b4d_denoise_slab_q16_u16(
-                    self._h, ctypes.c_void_p(in_ptr), _lib.shape3(shape), ctypes.c_int64(z_begin),
-                    ctypes.c_int64(z_total), ctypes.c_int64(own_begin), ctypes.c_int64(own_end), ctypes.c_float(sigma),
-                    ctypes.c_float(q[0]), ctypes.c_float(q[1]), ctypes.c_float(q[2]), int(bool(q[3])),
-                    ctypes.c_void_p(out_ptr), int(on_dev), int(on_dev),
-                )
-            )
-            return out
-        _lib.check(
-            self.lib.b4d_denoise_slab_u16(
-                self._h,
-                ctypes.c_void_p(in_ptr),
-                _lib.shape3(shape),
-                ctypes.c_int64(z_begin),
-                ctypes.c_int64(z_total),
-                ctypes.c_int64(own_begin),
-                ctypes.c_int64(own_end),
-                ctypes.c_float(sigma),
-                ctypes.c_void_p(out_ptr),
-                int(on_dev),
-                int(on_dev),
-            )
-        )
+            _lib.check(self.lib.b4d_denoise_slab_q16_u16(self._h, in_ptr, _lib.shape3(shape), z_begin, z_total,
+                                                         own_begin, own_end, sigma, *_quantize_args(quantize),
+                                                         _ptr(out), on_dev, on_dev))
         return out
 
     # ---- the slab in two calls, for one neighbour exchange between the stages ----
     def slab_stage1(self, slab, z_begin, z_total, sigma):
         """Stage 1 on a uint16 slab (NumPy or torch); the basic estimate stays on the device."""
-        if _is_torch(slab):
-            import torch
-
-            sc = slab.contiguous()
-            if sc.dtype != torch.uint16 or sc.ndim != 3:
-                raise ValueError("slab must be a 3-D uint16 tensor")
-            on_dev = sc.is_cuda
-            if on_dev:
-                torch.cuda.current_stream(sc.device).synchronize()
-            ptr, shape = sc.data_ptr(), tuple(sc.shape)
-        else:
-            sc = np.ascontiguousarray(slab)
-            if sc.dtype != np.uint16 or sc.ndim != 3:
-                raise ValueError("slab must be a 3-D uint16 array")
-            on_dev, ptr, shape = False, sc.ctypes.data, sc.shape
+        sc, ptr, on_dev, shape = self._input(_array_arg(slab, ("uint16",), (3,), "slab_stage1"))
         self._slab_shape = tuple(int(v) for v in shape)
-        _lib.check(
-            self.lib.b4d_slab_stage1_u16(self._h, ctypes.c_void_p(ptr), _lib.shape3(shape), ctypes.c_int64(z_begin),
-                                         ctypes.c_int64(z_total), ctypes.c_float(sigma), int(on_dev))
-        )
+        _lib.check(self.lib.b4d_slab_stage1_u16(self._h, ptr, _lib.shape3(shape), z_begin, z_total, sigma, on_dev))
 
     def slab_basic(self, plane0, nplanes, device=None):
         """Planes [plane0, plane0 + nplanes) (slab-local) of the basic estimate: a torch CUDA
         tensor when `device` is given, else a NumPy array."""
         shape = (int(nplanes),) + self._slab_shape[1:]
-        if device is not None:
-            import torch
-
-            buf = torch.empty(shape, dtype=torch.float32, device=device)
-            ptr, on_dev = buf.data_ptr(), True
-        else:
-            buf = np.empty(shape, dtype=np.float32)
-            ptr, on_dev = buf.ctypes.data, False
+        buf = np.empty(shape, dtype=np.float32) if device is None else self._device_out(shape, "float32", device)
         if nplanes:
-            _lib.check(self.lib.b4d_slab_basic_planes(self._h, ctypes.c_int64(plane0), ctypes.c_int64(nplanes),
-                                                      ctypes.c_void_p(ptr), 0, int(on_dev)))
+            _lib.check(self.lib.b4d_slab_basic_planes(self._h, plane0, nplanes, _ptr(buf), 0, device is not None))
         return buf
 
     def slab_set_basic(self, plane0, planes):
         """Overwrite planes of the basic estimate (the neighbour's exact halo planes)."""
-        if _is_torch(planes):
-            import torch
-
-            pc = planes.contiguous()
-            if pc.dtype != torch.float32:
-                raise ValueError("planes must be float32")
-            if pc.is_cuda:
-                torch.cuda.current_stream(pc.device).synchronize()
-            ptr, on_dev, n = pc.data_ptr(), pc.is_cuda, pc.shape[0]
-        else:
-            pc = np.ascontiguousarray(planes, dtype=np.float32)
-            ptr, on_dev, n = pc.ctypes.data, False, pc.shape[0]
-        if tuple(pc.shape[1:]) != self._slab_shape[1:]:
+        pc, ptr, on_dev, shape = self._input(_array_arg(planes, ("float32",), None, "slab_set_basic", cast=True))
+        if tuple(shape[1:]) != self._slab_shape[1:]:
             raise ValueError("planes must have the slab's (H, W)")
-        if n:
-            _lib.check(self.lib.b4d_slab_basic_planes(self._h, ctypes.c_int64(plane0), ctypes.c_int64(n),
-                                                      ctypes.c_void_p(ptr), 1, int(on_dev)))
+        if shape[0]:
+            _lib.check(self.lib.b4d_slab_basic_planes(self._h, plane0, shape[0], ptr, 1, on_dev))
 
     def slab_basic_tensor(self, device):
         """Zero-copy torch view (D, H, W) float32 of the open slab's basic estimate on `device`: a neighbour
@@ -376,33 +325,21 @@ class Denoiser:
 
     def slab_stage2_begin(self, own_begin, own_end):
         """Launch, without waiting, the part of the stage-2 front end that reads owned planes only."""
-        _lib.check(self.lib.b4d_slab_stage2_begin(self._h, ctypes.c_int64(own_begin), ctypes.c_int64(own_end)))
+        _lib.check(self.lib.b4d_slab_stage2_begin(self._h, own_begin, own_end))
 
     def slab_stage2(self, own_begin, own_end, out=None, device=None, quantize=None):
         """Stage 2 on the completed basic estimate -> float32 owned planes (NumPy, or torch on
         `device`; `out` may be a preallocated NumPy array, e.g. pinned).  quantize = (offset_sub, offset_add,
         step[, truncate]): uint16 output of the fused quantizer instead (see denoise_slab)."""
         oshape = (int(own_end - own_begin),) + self._slab_shape[1:]
-        odt_np, odt_t = (np.float32, "float32") if quantize is None else (np.uint16, "uint16")
-        if device is not None:
-            import torch
-
-            out = torch.empty(oshape, dtype=getattr(torch, odt_t), device=device)
-            ptr, on_dev = out.data_ptr(), True
+        odt = "float32" if quantize is None else "uint16"
+        out = _host_out(out, oshape, odt) if device is None else self._device_out(oshape, odt, device)
+        on_dev = device is not None
+        if quantize is None:
+            _lib.check(self.lib.b4d_slab_stage2(self._h, own_begin, own_end, _ptr(out), on_dev))
         else:
-            if out is None:
-                out = np.empty(oshape, dtype=odt_np)
-            elif out.shape != oshape or out.dtype != odt_np or not out.flags.c_contiguous:
-                raise ValueError("out must be a C-contiguous %s array of shape %r" % (odt_t, oshape))
-            ptr, on_dev = out.ctypes.data, False
-        if quantize is not None:
-            q = tuple(quantize) + (False,) * (4 - len(quantize))
-            _lib.check(self.lib.b4d_slab_stage2_q16(self._h, ctypes.c_int64(own_begin), ctypes.c_int64(own_end),
-                                                    ctypes.c_float(q[0]), ctypes.c_float(q[1]), ctypes.c_float(q[2]),
-                                                    int(bool(q[3])), ctypes.c_void_p(ptr), int(on_dev)))
-            return out
-        _lib.check(self.lib.b4d_slab_stage2(self._h, ctypes.c_int64(own_begin), ctypes.c_int64(own_end),
-                                            ctypes.c_void_p(ptr), int(on_dev)))
+            _lib.check(self.lib.b4d_slab_stage2_q16(self._h, own_begin, own_end, *_quantize_args(quantize), _ptr(out),
+                                                    on_dev))
         return out
 
     def denoise_quantized(self, vol, sigma, offset_sub=0.0, offset_add=0.0, step=1.0, truncate=False, out=None):
@@ -413,194 +350,73 @@ class Denoiser:
 
     def match_stage1(self, vol, sigma):
         """Instrumented stage-1 matcher: (idx[R,K] int32, ssd[R,K] uint64, count[R] int32)."""
-        vol = np.ascontiguousarray(vol)
-        if vol.dtype != np.uint16 or vol.ndim != 3:
-            raise ValueError("match_stage1 expects a 3-D uint16 array")
+        vol = np.ascontiguousarray(_array_arg(vol, ("uint16",), (3,), "match_stage1"))
         shape = _lib.shape3(vol.shape)
         R = self.lib.b4d_num_refs(shape)
         K = int(self.profile.max_stack_size_ht)
         idx = np.empty((R, K), dtype=np.int32)
         ssd = np.empty((R, K), dtype=np.uint64)
         cnt = np.empty((R,), dtype=np.int32)
-        _lib.check(
-            self.lib.b4d_match_stage1(
-                self._h,
-                ctypes.c_void_p(vol.ctypes.data),
-                shape,
-                ctypes.c_float(sigma),
-                ctypes.c_void_p(idx.ctypes.data),
-                ctypes.c_void_p(ssd.ctypes.data),
-                ctypes.c_void_p(cnt.ctypes.data),
-            )
-        )
+        _lib.check(self.lib.b4d_match_stage1(self._h, vol.ctypes.data, shape, sigma, idx.ctypes.data, ssd.ctypes.data,
+                                             cnt.ctypes.data))
         return idx, ssd, cnt
 
     def quantize(self, x, offset_sub=0.0, offset_add=0.0, step=1.0, truncate=False):
         """K7: rint(clip((x - offset_sub + offset_add)/step, 0, 65535/step)) -> uint16.
         truncate=True: the evaluator's variant, np.maximum(v, 0).astype(int) cast to uint16 (evaluate.py:202,
         utils/img_util.py:420-423): toward zero, no upper clip, wrapping modulo 2^16."""
-        if _is_torch(x):
-            import torch
-
-            xc = x.contiguous()
-            if xc.dtype != torch.float32:
-                raise ValueError("quantize expects float32")
-            out = torch.empty(xc.shape, dtype=torch.uint16, device=xc.device)
-            on_dev = xc.is_cuda
-            if on_dev:
-                torch.cuda.current_stream(xc.device).synchronize()
-            in_ptr, out_ptr, n = xc.data_ptr(), out.data_ptr(), xc.numel()
-        else:
-            xc = np.ascontiguousarray(x, dtype=np.float32)
-            out = np.empty(xc.shape, dtype=np.uint16)
-            on_dev = False
-            in_ptr, out_ptr, n = xc.ctypes.data, out.ctypes.data, xc.size
+        xc, in_ptr, on_dev, shape = self._input(_array_arg(x, ("float32",), None, "quantize", cast=True))
+        out = _out_like(xc, shape, "uint16")
         fn = self.lib.b4d_quantize_trunc_u16 if truncate else self.lib.b4d_quantize_u16
-        _lib.check(
-            fn(
-                self._h,
-                ctypes.c_void_p(in_ptr),
-                ctypes.c_int64(n),
-                ctypes.c_float(offset_sub),
-                ctypes.c_float(offset_add),
-                ctypes.c_float(step),
-                ctypes.c_void_p(out_ptr),
-                int(on_dev),
-                int(on_dev),
-            )
-        )
+        _lib.check(fn(self._h, in_ptr, math.prod(shape), offset_sub, offset_add, step, _ptr(out), on_dev, on_dev))
         return out
 
     def set_pass_voxels(self, voxels):
         """Voxels per pass (scratch ~45 B each; 0 = default 1.25 Gi).  A uint16 volume larger than a
         pass is denoised as consecutive z-slabs with halos; the result does not change."""
-        _lib.check(self.lib.b4d_set_pass_voxels(self._h, ctypes.c_int64(int(voxels))))
+        _lib.check(self.lib.b4d_set_pass_voxels(self._h, int(voxels)))
 
     def set_pipeline_min_voxels(self, voxels):
         """Volume size from which host transfers are pipelined against the kernels (default 2^26)."""
-        _lib.check(self.lib.b4d_set_pipeline_min_voxels(self._h, ctypes.c_int64(int(voxels))))
+        _lib.check(self.lib.b4d_set_pipeline_min_voxels(self._h, int(voxels)))
 
     def foreground_mask(self, raw_u16, offsets=0.0, k=6.0, dilate=1):
         """make_foreground_mask (metrics.py:32-61) of uint16 patches after the offset subtraction
         (data_handling.py:353-354): (D,H,W) or (N,D,H,W) uint16 -> bool mask of the same shape."""
-        zc = np.ascontiguousarray(raw_u16)
-        if zc.dtype != np.uint16 or zc.ndim not in (3, 4):
-            raise ValueError("raw_u16 must be a uint16 volume or a (N, D, H, W) batch")
+        zc = np.ascontiguousarray(_array_arg(raw_u16, ("uint16",), (3, 4), "foreground_mask"))
         n = zc.shape[0] if zc.ndim == 4 else 1
         off = np.ascontiguousarray(np.broadcast_to(np.asarray(offsets, dtype=np.float32), (n,)))
         out = np.empty(zc.shape, dtype=np.uint8)
-        _lib.check(
-            self.lib.b4d_foreground_mask_u16(
-                self._h,
-                ctypes.c_void_p(zc.ctypes.data),
-                ctypes.c_int64(n),
-                _lib.shape3(zc.shape[-3:]),
-                ctypes.c_void_p(off.ctypes.data),
-                ctypes.c_float(k),
-                ctypes.c_int(int(dilate)),
-                ctypes.c_void_p(out.ctypes.data),
-                0,
-                0,
-            )
-        )
+        _lib.check(self.lib.b4d_foreground_mask_u16(self._h, zc.ctypes.data, n, _lib.shape3(zc.shape[-3:]),
+                                                    off.ctypes.data, k, int(dilate), out.ctypes.data, 0, 0))
         return out.view(np.bool_)
 
     def chunk_shuffle(self, x, chunk=(64, 64, 64), want_bytes=True, want_hist=True):
         """K9: C-order chunk gather + Blosc 2-byte shuffle of a uint16 volume, plus per-piece byte
-        histograms [pieces, 2, 256] (uint32).  Returns (bytes or None, hist or None)."""
+        histograms [pieces, 2, 256] (uint32; int32 for torch input).  Returns (bytes or None, hist or None)."""
         if len(chunk) != 3:
             raise ValueError("chunk must have three entries")
         if not (want_bytes or want_hist):
             raise ValueError("nothing requested")
-        torch_in = _is_torch(x)
-        if torch_in:
-            import torch
-
-            xc = x.contiguous()
-            if xc.dtype != torch.uint16 or xc.ndim != 3:
-                raise ValueError("chunk_shuffle expects a 3-D uint16 volume")
-            on_dev = xc.is_cuda
-            if on_dev:
-                torch.cuda.current_stream(xc.device).synchronize()
-            shape, in_ptr = tuple(xc.shape), xc.data_ptr()
-        else:
-            xc = np.ascontiguousarray(x)
-            if xc.dtype != np.uint16 or xc.ndim != 3:
-                raise ValueError("chunk_shuffle expects a 3-D uint16 volume")
-            on_dev = False
-            shape, in_ptr = xc.shape, xc.ctypes.data
+        xc, in_ptr, on_dev, shape = self._input(_array_arg(x, ("uint16",), (3,), "chunk_shuffle"))
         npieces = 1
         for s_, c_ in zip(shape, chunk):
             if int(c_) < 1:
                 raise ValueError("chunk sides must be >= 1")
             npieces *= -(-int(s_) // int(c_))
-        nvox = int(shape[0]) * int(shape[1]) * int(shape[2])
-        out = hist = None
-        out_ptr = hist_ptr = None
-        if on_dev:
-            if want_bytes:
-                out = torch.empty(2 * nvox, dtype=torch.uint8, device=xc.device)
-                out_ptr = out.data_ptr()
-            if want_hist:
-                hist = torch.empty((npieces, 2, 256), dtype=torch.int32, device=xc.device)
-                hist_ptr = hist.data_ptr()
-        else:
-            if want_bytes:
-                out = np.empty(2 * nvox, dtype=np.uint8)
-                out_ptr = out.ctypes.data
-            if want_hist:
-                hist = np.empty((npieces, 2, 256), dtype=np.uint32)
-                hist_ptr = hist.ctypes.data
-        _lib.check(
-            self.lib.b4d_chunk_shuffle_u16(
-                self._h,
-                ctypes.c_void_p(in_ptr),
-                _lib.shape3(shape),
-                _lib.shape3(chunk),
-                ctypes.c_void_p(out_ptr),
-                ctypes.c_void_p(hist_ptr),
-                int(on_dev),
-                int(on_dev),
-            )
-        )
-        if torch_in and not on_dev:
-            import torch
-
-            out = torch.from_numpy(out) if out is not None else None
-            hist = torch.from_numpy(hist.view(np.int32)) if hist is not None else None
+        out = _out_like(xc, (2 * math.prod(shape),), "uint8") if want_bytes else None
+        hist = _out_like(xc, (npieces, 2, 256), "int32" if _is_torch(xc) else "uint32") if want_hist else None
+        _lib.check(self.lib.b4d_chunk_shuffle_u16(self._h, in_ptr, _lib.shape3(shape), _lib.shape3(chunk), _ptr(out),
+                                                  _ptr(hist), on_dev, on_dev))
         return out, hist
 
     def tile_stats(self, x, percentile=1.0, return_hist=False):
         """K8: offset percentile over non-zero voxels + median / MAD sigma of a uint16 tile."""
-        if _is_torch(x):
-            import torch
-
-            xc = x.contiguous()
-            if xc.dtype != torch.uint16:
-                raise ValueError("tile_stats expects uint16")
-            on_dev = xc.is_cuda
-            if on_dev:
-                torch.cuda.current_stream(xc.device).synchronize()
-            in_ptr, n = xc.data_ptr(), xc.numel()
-        else:
-            xc = np.ascontiguousarray(x)
-            if xc.dtype != np.uint16:
-                raise ValueError("tile_stats expects uint16")
-            on_dev = False
-            in_ptr, n = xc.ctypes.data, xc.size
+        xc, in_ptr, on_dev, shape = self._input(_array_arg(x, ("uint16",), None, "tile_stats"))
         st = _lib.Stats()
         hist = np.empty(65536, dtype=np.int64) if return_hist else None
-        _lib.check(
-            self.lib.b4d_tile_stats(
-                self._h,
-                ctypes.c_void_p(in_ptr),
-                ctypes.c_int64(n),
-                ctypes.c_double(percentile),
-                ctypes.byref(st),
-                ctypes.c_void_p(hist.ctypes.data) if return_hist else None,
-                int(on_dev),
-            )
-        )
+        _lib.check(self.lib.b4d_tile_stats(self._h, in_ptr, math.prod(shape), percentile, ctypes.byref(st), _ptr(hist),
+                                           on_dev))
         d = {k: getattr(st, k) for k, _ in _lib.Stats._fields_}
         return (d, hist) if return_hist else d
 
@@ -613,19 +429,8 @@ class Denoiser:
         Returns {"sigma", "mad", "cells"} (float64, float64, int64) shaped (N,)? + tile grid (the grid axes are
         dropped when tile is None); with return_hist, also the exact 262141-bin histogram of |d| over every cell
         of the call (int64), the payload to sum across ranks for noise_sigma_from_hist."""
-        x, shape, tile, grid = _noise_sigma_args(x, tile)
-        if _is_torch(x):
-            import torch
-
-            xc = x.contiguous()
-            on_dev = xc.is_cuda
-            if on_dev:
-                torch.cuda.current_stream(xc.device).synchronize()
-            in_ptr = xc.data_ptr()
-        else:
-            xc = np.ascontiguousarray(x)
-            on_dev = False
-            in_ptr = xc.ctypes.data
+        x, tile, grid = _noise_sigma_args(x, tile)
+        xc, in_ptr, on_dev, shape = self._input(x)
         n = 1 if len(shape) == 3 else shape[0]
         out_shape = (() if len(shape) == 3 else (n,)) + grid
         sigma = np.empty(out_shape, np.float64)
@@ -635,32 +440,13 @@ class Denoiser:
         _lib.check(
             self.lib.b4d_noise_sigma_u16(
                 self._h, in_ptr, n, _lib.shape3(shape[-3:]), _lib.shape3(tile) if tile is not None else None,
-                sigma.ctypes.data, mad.ctypes.data, cells.ctypes.data, hist.ctypes.data if return_hist else None,
-                int(on_dev),
+                sigma.ctypes.data, mad.ctypes.data, cells.ctypes.data, _ptr(hist), on_dev,
             )
         )
         d = {"sigma": sigma[()], "mad": mad[()], "cells": cells[()]}
         return (d, hist) if return_hist else d
 
     # ---- Poisson-Gaussian noise (DESIGN §3.12) -------------------------------
-    def _io(self, x, out_dtype):
-        """(contiguous input, its pointer, on device, output of out_dtype ("float32" / "uint16") in the same place,
-        its pointer) for the elementwise and VST calls; a CUDA tensor must live on the handle's device."""
-        if _is_torch(x):
-            import torch
-
-            xc = x.contiguous()
-            on_dev = xc.is_cuda
-            if on_dev and xc.device.index != self.device:
-                raise ValueError("tensor lives on cuda:%s, handle on cuda:%d" % (xc.device.index, self.device))
-            out = torch.empty(xc.shape, dtype=getattr(torch, out_dtype), device=xc.device)
-            if on_dev:
-                torch.cuda.current_stream(xc.device).synchronize()
-            return xc, xc.data_ptr(), on_dev, out, out.data_ptr()
-        xc = np.ascontiguousarray(x)
-        out = np.empty(xc.shape, dtype=out_dtype)
-        return xc, xc.ctypes.data, False, out, out.ctypes.data
-
     def noise_level_function(self, x, edges=None, min_cells=256):
         """Noise-level function var(z) = a E[z] + b of Poisson-Gaussian counts (DESIGN §3.12): the Haar-detail MAD of
         noise_sigma per intensity bin of the 2x2x2 cells, and a weighted least-squares line through the bins.
@@ -672,18 +458,8 @@ class Denoiser:
         Returns {"edges", "cells", "level_sum", "level", "mad", "sigma", "a", "b", "usable"}: per-bin int64 / float64
         arrays (level = mean intensity of the bin's cells, NaN when empty), the fitted a, b (NaN when fewer than 2
         bins are usable) and the number of usable bins."""
-        x, shape, edges, min_cells = _nlf_args(x, edges, min_cells)
-        if _is_torch(x):
-            xc = x.contiguous()
-            on_dev = xc.is_cuda
-            if on_dev:
-                import torch
-
-                torch.cuda.current_stream(xc.device).synchronize()
-            in_ptr = xc.data_ptr()
-        else:
-            xc = np.ascontiguousarray(x)
-            on_dev, in_ptr = False, xc.ctypes.data
+        x, edges, min_cells = _nlf_args(x, edges, min_cells)
+        xc, in_ptr, on_dev, shape = self._input(x)
         nb = edges.size - 1
         cells = np.empty(nb, np.int64)
         level_sum = np.empty(nb, np.int64)
@@ -697,7 +473,7 @@ class Denoiser:
             self.lib.b4d_noise_level_u16(
                 self._h, in_ptr, n, _lib.shape3(shape[-3:]), edges.ctypes.data, nb, min_cells, cells.ctypes.data,
                 level_sum.ctypes.data, mad.ctypes.data, sigma.ctypes.data, level.ctypes.data, fit.ctypes.data,
-                usable.ctypes.data, int(on_dev),
+                usable.ctypes.data, on_dev,
             )
         )
         return {"edges": edges, "cells": cells, "level_sum": level_sum, "level": level, "mad": mad, "sigma": sigma,
@@ -707,21 +483,23 @@ class Denoiser:
         """Generalized Anscombe transform of uint16 counts under `model` (PoissonGaussian) -> float32, elementwise:
         2 sqrt(max((z - offset)/gain + 3/8 + (read_sigma/gain)^2, 0)), float64 inside.  NumPy or torch (host or
         CUDA) -> the same kind, same shape."""
-        _elementwise_args(x, "uint16", "gat_forward")
+        x = _array_arg(x, ("uint16",), None, "gat_forward")
         m = _model_c(model)
-        xc, in_ptr, on_dev, out, out_ptr = self._io(x, "float32")
-        _lib.check(self.lib.b4d_gat_forward_u16(self._h, ctypes.byref(m), in_ptr, int(np.prod(xc.shape)), out_ptr,
-                                                int(on_dev), int(on_dev)))
+        xc, in_ptr, on_dev, shape = self._input(x)
+        out = _out_like(xc, shape, "float32")
+        _lib.check(self.lib.b4d_gat_forward_u16(self._h, ctypes.byref(m), in_ptr, math.prod(shape), _ptr(out), on_dev,
+                                                on_dev))
         return out
 
     def gat_inverse(self, y, model):
         """Closed-form approximation of the exact unbiased inverse of gat_forward (Makitalo & Foi 2013), float32 ->
         float32 counts gain * lambda + offset; lambda = 0 for y <= sqrt(1.5)."""
-        _elementwise_args(y, "float32", "gat_inverse")
+        y = _array_arg(y, ("float32",), None, "gat_inverse")
         m = _model_c(model)
-        yc, in_ptr, on_dev, out, out_ptr = self._io(y, "float32")
-        _lib.check(self.lib.b4d_gat_inverse_f32(self._h, ctypes.byref(m), in_ptr, int(np.prod(yc.shape)), out_ptr,
-                                                int(on_dev), int(on_dev)))
+        yc, in_ptr, on_dev, shape = self._input(y)
+        out = _out_like(yc, shape, "float32")
+        _lib.check(self.lib.b4d_gat_inverse_f32(self._h, ctypes.byref(m), in_ptr, math.prod(shape), _ptr(out), on_dev,
+                                                on_dev))
         return out
 
     def denoise_vst(self, x, model, sigma=1.0, quantize=None):
@@ -729,19 +507,17 @@ class Denoiser:
         intermediate float32 volume never leaving the device.  sigma is the noise level after the transform: 1 for an
         exact model.  (D,H,W) or (N,D,H,W), NumPy or torch -> float32; quantize = (offset_sub, offset_add, step[,
         truncate]): the uint16 volume quantize() gives on that float32 result instead."""
-        _vst_args(x, sigma, quantize)
+        x = _vst_args(x, sigma, quantize)
         m = _model_c(model)
-        shape = tuple(int(v) for v in x.shape)
+        xc, in_ptr, on_dev, shape = self._input(x)
         n = 1 if len(shape) == 3 else shape[0]
-        xc, in_ptr, on_dev, out, out_ptr = self._io(x, "float32" if quantize is None else "uint16")
+        out = _out_like(xc, shape, "float32" if quantize is None else "uint16")
         if quantize is None:
-            _lib.check(self.lib.b4d_denoise_vst_u16(self._h, in_ptr, n, _lib.shape3(shape[-3:]), ctypes.byref(m),
-                                                    float(sigma), out_ptr, int(on_dev), int(on_dev)))
-            return out
-        q = tuple(quantize) + (False,) * (4 - len(quantize))
-        _lib.check(self.lib.b4d_denoise_vst_q16_u16(self._h, in_ptr, n, _lib.shape3(shape[-3:]), ctypes.byref(m),
-                                                    float(sigma), float(q[0]), float(q[1]), float(q[2]),
-                                                    int(bool(q[3])), out_ptr, int(on_dev), int(on_dev)))
+            _lib.check(self.lib.b4d_denoise_vst_u16(self._h, in_ptr, n, _lib.shape3(shape[-3:]), ctypes.byref(m), sigma,
+                                                    _ptr(out), on_dev, on_dev))
+        else:
+            _lib.check(self.lib.b4d_denoise_vst_q16_u16(self._h, in_ptr, n, _lib.shape3(shape[-3:]), ctypes.byref(m),
+                                                        sigma, *_quantize_args(quantize), _ptr(out), on_dev, on_dev))
         return out
 
     def coherence_scores(self, labels, raw, smooth_sigma=1.0, coherence_lag=2, min_autocorr=0.4,
@@ -759,11 +535,9 @@ class Denoiser:
         cnt = np.zeros(n, dtype=np.int64)
         _lib.check(
             self.lib.b4d_coherence_gate(
-                self._h, x.ctypes.data_as(ctypes.c_void_p), lab.ctypes.data_as(ctypes.c_void_p), ctypes.c_int64(n),
-                _lib.shape3(shape), ctypes.c_double(min_autocorr), ctypes.c_double(max_highfreq_frac),
-                ctypes.c_int64(min_segment_voxels), ctypes.c_double(smooth_sigma), ctypes.c_int(coherence_lag),
-                reject.ctypes.data_as(ctypes.c_void_p), seg, ctypes.c_int64(max_segments),
-                cnt.ctypes.data_as(ctypes.c_void_p), 0,
+                self._h, x.ctypes.data, lab.ctypes.data, n, _lib.shape3(shape), min_autocorr, max_highfreq_frac,
+                min_segment_voxels, smooth_sigma, coherence_lag, reject.ctypes.data, seg, max_segments,
+                cnt.ctypes.data, 0,
             )
         )
         tables = []
@@ -943,9 +717,7 @@ def precompute_targets(raw_u16, offsets, sigma, max_count=65535.0, device=None):
     Returns (raw float32, teacher float32) as the cache stores them
     (scripts/precompute.py:204-228).
     """
-    raw_u16 = np.asarray(raw_u16)
-    if raw_u16.ndim != 4 or raw_u16.dtype != np.uint16:
-        raise ValueError("raw_u16 must be (N, D, H, W) uint16")
+    raw_u16 = _array_arg(raw_u16, ("uint16",), (4,), "precompute_targets")
     h = get_denoiser(device)
     h.set_profile("np", 2)
     return h.targets(raw_u16, offsets, _sigma_scalar(sigma), max_count)
@@ -984,26 +756,14 @@ def tile_stats(x, percentile=1.0, device=None, return_hist=False):
 
 
 def _noise_sigma_args(x, tile):
-    """Argument checks of noise_sigma, before any device work: (x, shape, tile tuple or None, tile grid)."""
-    if _is_torch(x):
-        import torch
-
-        ok = x.dtype == torch.uint16
-        shape = tuple(int(s) for s in x.shape)
-    else:
-        x = np.asarray(x)
-        ok = x.dtype == np.uint16
-        shape = x.shape
-    if not ok:
-        raise ValueError("noise_sigma expects uint16, got %s" % (x.dtype,))
-    if len(shape) not in (3, 4):
-        raise ValueError("noise_sigma expects a 3-D volume or a 4-D batch, got %d-D" % len(shape))
+    """Argument checks of noise_sigma, before any device work: (x, tile tuple or None, tile grid)."""
+    x = _array_arg(x, ("uint16",), (3, 4), "noise_sigma")
     if tile is None:
-        return x, shape, None, ()
+        return x, None, ()
     tile = tuple(int(t) for t in tile)
     if len(tile) != 3 or any(t < 2 or t % 2 for t in tile):
         raise ValueError("tile must be three even sides >= 2, got %r" % (tile,))
-    return x, shape, tile, tuple(-(-s // t) for s, t in zip(shape[-3:], tile))
+    return x, tile, tuple(-(-int(s) // t) for s, t in zip(x.shape[-3:], tile))
 
 
 def noise_sigma(x, tile=None, device=None, return_hist=False):
@@ -1065,26 +825,9 @@ def _model_c(model):
     return _lib.PgModel(gain, offset, read_sigma)
 
 
-def _dtype_name(x):
-    return str(x.dtype).replace("torch.", "") if _is_torch(x) else np.asarray(x).dtype.name
-
-
-def _elementwise_args(x, dtype, what):
-    if not _is_torch(x) and not isinstance(x, np.ndarray):
-        x = np.asarray(x)
-    if _dtype_name(x) != dtype:
-        raise ValueError("%s expects %s, got %s" % (what, dtype, _dtype_name(x)))
-
-
 def _nlf_args(x, edges, min_cells):
-    """Argument checks of noise_level_function, before any device work: (x, shape, edges float64, min_cells)."""
-    if not _is_torch(x):
-        x = np.asarray(x)
-    if _dtype_name(x) != "uint16":
-        raise ValueError("noise_level_function expects uint16, got %s" % _dtype_name(x))
-    shape = tuple(int(s) for s in x.shape)
-    if len(shape) not in (3, 4):
-        raise ValueError("noise_level_function expects a 3-D volume or a 4-D batch, got %d-D" % len(shape))
+    """Argument checks of noise_level_function, before any device work: (x, edges float64, min_cells)."""
+    x = _array_arg(x, ("uint16",), (3, 4), "noise_level_function")
     e = default_nlf_edges() if edges is None else np.ascontiguousarray(edges, dtype=np.float64)
     if e.ndim != 1 or not 2 <= e.size <= _lib.NLF_MAX_BINS + 1:
         raise ValueError("edges must be 2 .. %d values (1 .. %d bins)" % (_lib.NLF_MAX_BINS + 1, _lib.NLF_MAX_BINS))
@@ -1092,20 +835,17 @@ def _nlf_args(x, edges, min_cells):
         raise ValueError("edges must be finite and strictly increasing")
     if int(min_cells) < 1:
         raise ValueError("min_cells must be >= 1")
-    return x, shape, e, int(min_cells)
+    return x, e, int(min_cells)
 
 
 def _vst_args(x, sigma, quantize):
-    if not _is_torch(x):
-        x = np.asarray(x)
-    if _dtype_name(x) != "uint16":
-        raise ValueError("denoise_vst expects uint16 counts, got %s" % _dtype_name(x))
-    if x.ndim not in (3, 4):
-        raise ValueError("expected a 3-D volume or a 4-D batch, got %d-D" % x.ndim)
+    """Argument checks of denoise_vst, before any device work: returns x."""
+    x = _array_arg(x, ("uint16",), (3, 4), "denoise_vst")
     if not (np.isfinite(sigma) and sigma > 0):
         raise ValueError("sigma must be positive and finite, got %r" % (sigma,))
     if quantize is not None and not (3 <= len(quantize) <= 4 and float(quantize[2]) >= 1.0):
         raise ValueError("quantize must be (offset_sub, offset_add, step >= 1[, truncate])")
+    return x
 
 
 def noise_level_function(x, edges=None, min_cells=256, device=None):
@@ -1116,14 +856,14 @@ def noise_level_function(x, edges=None, min_cells=256, device=None):
 
 def gat_forward(x, model, device=None):
     """Generalized Anscombe transform; see Denoiser.gat_forward."""
-    _elementwise_args(x, "uint16", "gat_forward")
+    _array_arg(x, ("uint16",), None, "gat_forward")
     _model_c(model)
     return get_denoiser(device).gat_forward(x, model)
 
 
 def gat_inverse(y, model, device=None):
     """Inverse of gat_forward; see Denoiser.gat_inverse."""
-    _elementwise_args(y, "float32", "gat_inverse")
+    _array_arg(y, ("float32",), None, "gat_inverse")
     _model_c(model)
     return get_denoiser(device).gat_inverse(y, model)
 

@@ -185,8 +185,7 @@ def stats_from_hist_lib(hist, percentile=1.0):
     if h.shape != (65536,):
         raise ValueError("hist must have 65536 bins")
     st = _lib.Stats()
-    _lib.check(_lib.load().b4d_stats_from_hist(h.ctypes.data_as(ctypes.c_void_p), ctypes.c_double(percentile),
-                                               ctypes.byref(st)))
+    _lib.check(_lib.load().b4d_stats_from_hist(h.ctypes.data, percentile, ctypes.byref(st)))
     return {k: getattr(st, k) for k, _ in _lib.Stats._fields_}
 
 
