@@ -76,11 +76,28 @@ struct Plan {
     std::vector<int> rz1, rz2, ry, rx;
 };
 
+// Stage timings of a call: an event at every stage boundary, resolved after the final synchronise.  The interval
+// that ends at mark(slot) is booked to `slot` (to none for -1): its device time and the kernels enqueued in it.
+struct StageClock {
+    b4d_handle *h;
+    std::vector<cudaEvent_t> evs;
+    std::vector<std::pair<int, long long>> tags;  // (slot, kernels enqueued) of the interval ending at evs[i]
+    long long enqueued = 0;                       // b4d_kernels_enqueued at the last mark
+    explicit StageClock(b4d_handle *hh) : h(hh) {}
+    StageClock(const StageClock &) = delete;
+    StageClock &operator=(const StageClock &) = delete;
+    ~StageClock() { discard(); }  // an error return before resolve()
+    void mark(int slot);
+    void resolve();  // after a synchronise: book every interval, then discard the marks
+    void discard();
+};
+
 // Two-call slab form: what b4d_slab_stage2_begin already launched of the stage-2 front end (planes [o0, o1) of
 // the matching image, cell planes [cz0, cz1), tile layers [tz0, tz1) classified and matched).
 struct OwnedFront {
+    explicit OwnedFront(b4d_handle *h) : clk(h) {}
     bool done = false;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // device time of part 1, added to the stage-2 matching slot
+    StageClock clk;  // part 1, booked to the stage-2 matching slot by b4d_slab_stage2
     int o0 = 0, o1 = 0, cz0 = 0, cz1 = 0, tz0 = 0, tz1 = 0;
 };
 
@@ -96,9 +113,9 @@ struct b4d_handle {
     DevBuf alt_in, alt_zf, alt_out, alt_partial, alt_sink;  // second buffer set of b4d_targets_u16
     DevBuf nz_hist, nz_sel, nz_res, nz_full;  // b4d_noise_sigma_u16: per-tile digit histograms, selections, results
     DevBuf nlf_sum;  // b4d_noise_level_u16: per-bin sums of the cell intensities
-    float t_ms[B4D_T_COUNT];
-    int64_t launches[B4D_T_COUNT];
-    unsigned long long match_stats[4];
+    float t_ms[B4D_T_COUNT] = {};
+    int64_t launches[B4D_T_COUNT] = {};
+    unsigned long long match_stats[4] = {};
     long long pass_voxels = CHUNK_VOXELS;  // voxels per pass (b4d_set_pass_voxels)
     long long pipeline_min_voxels = 1ll << 26;  // host transfers are pipelined from this volume size up
     HostMover mover;  // pageable host arrays <-> device (pinned ring + copy threads)
@@ -111,7 +128,7 @@ struct b4d_handle {
     int64_t slab_z_begin = 0;
     float slab_sigma = 0.f;
     MatchMap slab_mm;
-    OwnedFront pre;
+    OwnedFront pre{this};
 };
 
 namespace {
@@ -328,40 +345,31 @@ struct EventSet {
     }
 };
 
-// One stage boundary timing: we record an event after each kernel family and
-// resolve all of them after the final synchronise.
-struct StageClock {
-    b4d_handle *h;
-    std::vector<cudaEvent_t> evs;
-    std::vector<std::pair<int, int>> tags;  // (slot, launches) for interval i -> i+1
-    explicit StageClock(b4d_handle *hh) : h(hh) {}
-    StageClock(const StageClock &) = delete;
-    StageClock &operator=(const StageClock &) = delete;
-    ~StageClock() {  // an error return before resolve()
-        for (auto e : evs) cudaEventDestroy(e);
-    }
-    void mark(int slot, int launches) {
-        cudaEvent_t e;
-        cudaEventCreate(&e);
-        cudaEventRecord(e, h->stream);
-        evs.push_back(e);
-        tags.push_back({slot, launches});
-    }
-    void resolve() {
-        for (size_t i = 1; i < evs.size(); ++i) {
-            float ms = 0.f;
-            cudaEventElapsedTime(&ms, evs[i - 1], evs[i]);
-            const int slot = tags[i].first;
-            if (slot >= 0 && slot < B4D_T_COUNT) {
-                h->t_ms[slot] += ms;
-                h->launches[slot] += tags[i].second;
-            }
+void StageClock::mark(int slot) {
+    cudaEvent_t e;
+    cudaEventCreate(&e);
+    cudaEventRecord(e, h->stream);
+    evs.push_back(e);
+    tags.push_back({slot, b4d_kernels_enqueued - enqueued});  // the first interval is never booked
+    enqueued = b4d_kernels_enqueued;
+}
+void StageClock::resolve() {
+    for (size_t i = 1; i < evs.size(); ++i) {
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, evs[i - 1], evs[i]);
+        const int slot = tags[i].first;
+        if (slot >= 0 && slot < B4D_T_COUNT) {
+            h->t_ms[slot] += ms;
+            h->launches[slot] += tags[i].second;
         }
-        for (auto e : evs) cudaEventDestroy(e);
-        evs.clear();
-        tags.clear();
     }
-};
+    discard();
+}
+void StageClock::discard() {
+    for (auto e : evs) cudaEventDestroy(e);
+    evs.clear();
+    tags.clear();
+}
 
 // Where the result goes when it is wanted in HOST memory: planes [p0, p1) of the (single) volume, to `host`
 // (p1 - p0 planes).  stage2_back then runs the filter in z chunks and every chunk of finished planes is
@@ -450,7 +458,6 @@ int make_pass(b4d_handle *h, const Plan &pl, float sigma, const MatchMap &mm, fl
     const size_t ntile = (size_t)pl.nvol * std::max(ps.g1.tz, ps.g2.tz) * ps.g1.ty * ps.g1.tx;
     B4D_TRY(h->cells.ensure(ncell * sizeof(uint32_t)));
     B4D_TRY(h->tcls.ensure(ntile * sizeof(uint32_t)));
-    B4D_TRY(h->stats.ensure(4 * sizeof(unsigned long long)));
     // Both stages aggregate in order-independent fixed point (int64): the result does not
     // depend on scheduling, a slab equals the whole volume bit for bit, and the basic estimate
     // that feeds the stage-2 matching (a discontinuous decision) is reproducible.
@@ -575,25 +582,24 @@ int stage1(Pass &ps, const uint16_t *host_src, bool fuse_match) {
     const b4d_profile &p = h->prof;
     cudaStream_t s = h->stream;
     StageClock &clk = *ps.clk;
-    CU_TRY(cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), s));
     B4D_TRY(zero_acc(ps));
-    clk.mark(B4D_T_PREP, 1);
+    clk.mark(B4D_T_PREP);
     if (!host_src) b4d_launch_block_energy(ps.u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, pl.nvol, s);
-    clk.mark(B4D_T_K0, 1);
+    clk.mark(B4D_T_K0);
     if (host_src)
         B4D_TRY(stage1_streamed_front(ps, host_src));
     else if (ps.R1 > 0)
         b4d_launch_match(ps.mp1, p.search_ht, s);
-    clk.mark(B4D_T_MATCH1, 4);
+    clk.mark(B4D_T_MATCH1);
     if (ps.R1 > 0) b4d_launch_filter(ps.fp1, false, s);
-    clk.mark(B4D_T_FILTER1, 1);
+    clk.mark(B4D_T_FILTER1);
     if (fuse_match)
         b4d_launch_normalise_match(h->numq.as<long long>(), h->gmap.as<uint32_t>(), ps.zf, ps.basic, ps.u,
                                    ps.mm.scale, ps.mm.ishift, pl.D, pl.H, pl.W, pl.nvol, 1.0f / ps.mm.scale,
                                    ps.tab.kf, s);
     else
         normalise(ps, ps.zf, ps.basic, 0, pl.D, nullptr, s);
-    clk.mark(B4D_T_NORM1, 1);
+    clk.mark(B4D_T_NORM1);
     CU_TRY(cudaGetLastError());
     return 0;
 }
@@ -606,11 +612,11 @@ int stage2_front_whole(Pass &ps, bool already_converted) {
     cudaStream_t s = h->stream;
     if (!already_converted) b4d_launch_to_match(ps.basic, ps.u, ps.TV, 0.0f, ps.mm.scale, ps.mm.ishift, s);
     B4D_TRY(zero_acc(ps));
-    ps.clk->mark(B4D_T_PREP, 2);
+    ps.clk->mark(B4D_T_PREP);
     b4d_launch_block_energy(ps.u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, pl.nvol, s);
-    ps.clk->mark(B4D_T_K0, 1);
+    ps.clk->mark(B4D_T_K0);
     if (ps.R2 > 0) b4d_launch_match(ps.mp2, h->prof.search_wie, s);
-    ps.clk->mark(B4D_T_MATCH2, 4);
+    ps.clk->mark(B4D_T_MATCH2);
     return 0;
 }
 
@@ -663,13 +669,13 @@ int stage2_front_rest(Pass &ps) {
         b4d_launch_to_match(ps.basic + o1 * Pv, ps.u + o1 * Pv, (pl.D - o1) * Pv, 0.0f, ps.mm.scale, ps.mm.ishift, s);
     b4d_launch_block_energy_range(ps.u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, 1, 0, std::min(o0, pl.D - 3), s);
     b4d_launch_block_energy_range(ps.u, h->s2.as<uint2>(), pl.D, pl.H, pl.W, 1, std::max(o0, o1 - 3), pl.D - 3, s);
-    ps.clk->mark(B4D_T_PREP, 4);
+    ps.clk->mark(B4D_T_PREP);
     if (ps.R2 > 0) {
         b4d_launch_match_range(ps.mp2, h->prof.search_wie, 0, f.cz0, 0, f.tz0 * tiles_per_layer, s);
         b4d_launch_match_range(ps.mp2, h->prof.search_wie, std::max(f.cz0, f.cz1), (pl.D + 3) / 4,
                                f.tz1 * tiles_per_layer, (long long)ps.g2.tz * tiles_per_layer, s);
     }
-    ps.clk->mark(B4D_T_MATCH2, 8);
+    ps.clk->mark(B4D_T_MATCH2);
     f.done = false;
     return 0;
 }
@@ -698,7 +704,7 @@ int stage2_back(Pass &ps, HostSink *sink, const QuantSpec *q) {
             CU_TRY(owned.make(&evs[c]));
             CU_TRY(cudaEventRecord(evs[c], s));
         }
-        clk.mark(B4D_T_FILTER2, NCH);
+        clk.mark(B4D_T_FILTER2);
         const size_t esz = q ? sizeof(uint16_t) : sizeof(float);
         long long zdone = 0;
         for (int c = 0; c < NCH; ++c) {
@@ -721,15 +727,15 @@ int stage2_back(Pass &ps, HostSink *sink, const QuantSpec *q) {
             }
         }
         CU_TRY(cudaStreamSynchronize(h->copy_stream));
-        clk.mark(B4D_T_NORM2, NCH);
+        clk.mark(B4D_T_NORM2);
         sink->done = true;
         CU_TRY(cudaGetLastError());
         return 0;
     }
     if (ps.R2 > 0) b4d_launch_filter(ps.fp2, true, s);
-    clk.mark(B4D_T_FILTER2, 1);
+    clk.mark(B4D_T_FILTER2);
     normalise(ps, ps.basic, ps.out, 0, pl.D, q, s);
-    clk.mark(B4D_T_NORM2, 1);
+    clk.mark(B4D_T_NORM2);
     CU_TRY(cudaGetLastError());
     return 0;
 }
@@ -814,18 +820,23 @@ int common_checks(b4d_handle *h, const void *in, const void *out, const int64_t 
     return 0;
 }
 
-void reset_timings(b4d_handle *h) {
-    for (int i = 0; i < B4D_T_COUNT; ++i) {
-        h->t_ms[i] = 0.f;
-        h->launches[i] = 0;
-    }
+// Every b4d_last_* value describes the whole last public call: a denoising entry point resets the timings and the
+// matcher statistics (host copies and device counters) here, once, and all it runs afterwards only adds to them.
+int reset_last(b4d_handle *h) {
+    std::fill(h->t_ms, h->t_ms + B4D_T_COUNT, 0.f);
+    std::fill(h->launches, h->launches + B4D_T_COUNT, 0);
+    std::fill(h->match_stats, h->match_stats + 4, 0ull);
+    B4D_TRY(h->stats.ensure(sizeof(h->match_stats)));
+    CU_TRY(cudaMemsetAsync(h->stats.p, 0, sizeof(h->match_stats), h->stream));
+    return 0;
 }
 
-// The end of a denoise call: wait for the compute stream, book the stage timings, fetch the matcher statistics.
+// The end of a denoise pass: wait for the compute stream, book the stage timings, fetch the matcher statistics
+// accumulated since reset_last.
 int finish(b4d_handle *h, StageClock &clk) {
     CU_TRY(cudaStreamSynchronize(h->stream));
     clk.resolve();
-    CU_TRY(cudaMemcpy(h->match_stats, h->stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    CU_TRY(cudaMemcpy(h->match_stats, h->stats.p, sizeof(h->match_stats), cudaMemcpyDeviceToHost));
     return 0;
 }
 
@@ -841,13 +852,13 @@ int stage_u16_input(b4d_handle *h, const Plan &pl, const uint16_t *in, int in_on
     *host_src = nullptr;
     if (!in_on_device && can_stream_upload(h, pl)) {
         *host_src = in;
-        clk.mark(-1, 0);
+        clk.mark(-1);
     } else {
         CU_TRY(copy_in(h, h->in.p, in, (size_t)V * sizeof(uint16_t), in_on_device, h->stream));
-        clk.mark(-1, 0);
+        clk.mark(-1);
         B4D_TRY(convert_u16(h, h->in.as<uint16_t>(), h->zf.as<float>(), V, mm));
     }
-    clk.mark(B4D_T_PREP, 1);
+    clk.mark(B4D_T_PREP);
     return 0;
 }
 
@@ -870,7 +881,7 @@ int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3],
                   int in_dev, int out_dev) {
     B4D_TRY(common_checks(h, in, out, shape, sigma));
     if (n < 1) return fail(B4D_ERR_INVALID, "n must be >= 1");
-    reset_timings(h);
+    B4D_TRY(reset_last(h));
     const long long V = shape[0] * shape[1] * shape[2];
     const int64_t per = std::max<int64_t>(1, std::min<int64_t>(n, h->pass_voxels / V));
     cudaStream_t s = h->stream;
@@ -897,7 +908,7 @@ int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3],
         float centre = 0.0f;
         float *d_zf = nullptr;
         uint16_t *d_u = h->u16.as<uint16_t>();
-        clk.mark(-1, 0);
+        clk.mark(-1);
         if (sizeof(T) == 2) {
             B4D_TRY(h->zf.ensure((size_t)TV * sizeof(float)));
             if (!stream_in) B4D_TRY(convert_u16(h, h->in.as<uint16_t>(), h->zf.as<float>(), TV, &mm));
@@ -907,7 +918,7 @@ int denoise_batch(b4d_handle *h, const T *in, int64_t n, const int64_t shape[3],
             B4D_TRY(prepare_f32(h, TV, sigma, &mm, &centre));
             d_zf = h->in.as<float>();
         }
-        clk.mark(B4D_T_PREP, 2);
+        clk.mark(B4D_T_PREP);
         const bool to_host = !out_dev && nb == 1 && h->prof.stages == 2 && centre == 0.0f;
         HostSink sink{to_host ? out + i0 * V : nullptr, 0, pl.D};
         Pass ps;
@@ -949,7 +960,7 @@ int denoise_vst(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shap
     if (q && !(q->step >= 1.0f)) return fail(B4D_ERR_INVALID, "step must be >= 1");
     B4D_TRY(common_checks(h, in, out, shape, sigma));
     if (n < 1) return fail(B4D_ERR_INVALID, "n must be >= 1");
-    reset_timings(h);
+    B4D_TRY(reset_last(h));
     const long long V = shape[0] * shape[1] * shape[2];
     const int64_t per = std::max<int64_t>(1, std::min<int64_t>(n, h->pass_voxels / V));
     const size_t osz = q ? sizeof(uint16_t) : sizeof(float);
@@ -974,25 +985,25 @@ int denoise_vst(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shap
             CU_TRY(copy_in(h, h->u16.p, src, (size_t)TV * sizeof(uint16_t), 0, s));
             src = h->u16.as<uint16_t>();
         }
-        clk.mark(-1, 0);
+        clk.mark(-1);
         b4d_launch_gat_forward(src, h->in.as<float>(), TV, gp, s);
         MatchMap mm;
         float centre = 0.0f;
         B4D_TRY(prepare_f32(h, TV, sigma, &mm, &centre));
-        clk.mark(B4D_T_PREP, centre != 0.0f ? 5 : 3);
+        clk.mark(B4D_T_PREP);
         HostSink sink{nullptr, 0, pl.D};
         Pass ps;
         B4D_TRY(make_pass(h, pl, sigma, mm, h->in.as<float>(), h->u16.as<uint16_t>(), d_res, clk, ps));
         B4D_TRY(denoise_pass(ps, nullptr, &sink, nullptr));
         if (centre != 0.0f) b4d_launch_add_scalar(d_res, TV, centre, s);
-        clk.mark(-1, 0);
+        clk.mark(-1);
         // inverse: in place, or K7 into uint16 (the user's device buffer, else h->u16: the pass is done with it)
         uint16_t *d_q = nullptr;
         if (q) d_q = out_dev ? reinterpret_cast<uint16_t *>(user_out) : h->u16.as<uint16_t>();
         b4d_launch_gat_inverse(d_res, d_res, d_q, TV, gp, q ? q->sub : 0.f, q ? q->add : 0.f, q ? q->step : 1.f,
                                q ? q->trunc : 0, s);
         CU_TRY(cudaGetLastError());
-        clk.mark(norm_slot, 1);
+        clk.mark(norm_slot);
         const void *d_final = q ? static_cast<const void *>(d_q) : static_cast<const void *>(d_res);
         if (d_final != user_out) CU_TRY(copy_out(h, user_out, d_final, (size_t)TV * osz, out_dev, s));
         B4D_TRY(finish(h, clk));
@@ -1054,8 +1065,6 @@ int b4d_create(int device, const b4d_profile *profile, b4d_handle **out) {
         delete h;
         return fail(B4D_ERR_CUDA, std::string("cudaStreamCreate: ") + cudaGetErrorString(es));
     }
-    reset_timings(h);
-    std::memset(h->match_stats, 0, sizeof(h->match_stats));
     *out = h;
     return 0;
 }
@@ -1069,8 +1078,6 @@ void b4d_destroy(b4d_handle *h) {
                       &h->alt_in, &h->alt_zf, &h->alt_out, &h->alt_partial, &h->alt_sink, &h->nz_hist, &h->nz_sel,
                       &h->nz_res, &h->nz_full})
         b->release();
-    if (h->pre.ev0) cudaEventDestroy(h->pre.ev0);
-    if (h->pre.ev1) cudaEventDestroy(h->pre.ev1);
     if (h->stream) cudaStreamDestroy(h->stream);
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
     delete h;
@@ -1101,9 +1108,35 @@ int b4d_set_pass_voxels(b4d_handle *h, int64_t voxels) {
     return 0;
 }
 
+// One slab, after common_checks and reset_last: its stages add to the timings and match statistics of the call.
+static int denoise_slab_impl(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
+                             int64_t z_total, int64_t own_begin, int64_t own_end, float sigma, void *out,
+                             int in_on_device, int out_on_device, const QuantSpec *q) {
+    if (q && h->prof.stages != 2) return fail(B4D_ERR_INVALID, "quantized output needs stages = 2");
+    if (q && !(q->step >= 1.0f)) return fail(B4D_ERR_INVALID, "step must be >= 1");
+    const size_t esz = q ? sizeof(uint16_t) : sizeof(float);
+    if (z_begin < 0 || z_begin + shape[0] > z_total || own_begin < z_begin || own_end > z_begin + shape[0] ||
+        own_begin >= own_end)
+        return fail(B4D_ERR_INVALID, "slab / owned range inconsistent");
+    const long long P = shape[1] * shape[2];
+    const Plan pl = make_plan(shape, z_begin, z_total, 1, h->prof);
+    StageClock clk(h);
+    MatchMap mm;
+    const uint16_t *host_src = nullptr;
+    B4D_TRY(stage_u16_input(h, pl, in, in_on_device, clk, &mm, &host_src));
+    HostSink sink{out_on_device ? nullptr : out, own_begin - z_begin, own_end - z_begin};
+    Pass ps;
+    B4D_TRY(make_pass(h, pl, sigma, mm, h->zf.as<float>(), h->in.as<uint16_t>(), h->out.as<float>(), clk, ps));
+    B4D_TRY(denoise_pass(ps, host_src, &sink, q));
+    if (!sink.done)
+        CU_TRY(copy_out(h, out, h->out.as<char>() + (size_t)sink.p0 * P * esz, (size_t)(sink.p1 - sink.p0) * P * esz,
+                        out_on_device, h->stream));
+    return finish(h, clk);
+}
+
 // `n` uint16 volumes, each larger than a pass: z-slabs with the no-exchange halo, one after the other on this
-// GPU (b4d_denoise_slab_u16); equal to the one-pass result bit for bit, like the multi-GPU slabs.  The timings
-// and match statistics are summed over all slabs.
+// GPU (as b4d_denoise_slab_u16); equal to the one-pass result bit for bit, like the multi-GPU slabs.  The timings
+// and match statistics cover all slabs.
 static int denoise_oversize_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3], float sigma,
                                 float *out, int in_on_device, int out_on_device) {
     const int64_t D = shape[0], P = shape[1] * shape[2], V = D * P;
@@ -1114,24 +1147,14 @@ static int denoise_oversize_u16(b4d_handle *h, const uint16_t *in, int64_t n, co
                                        "or shard the volume in y / x");
     const int64_t nslab = (D + (planes - 2 * halo) - 1) / (planes - 2 * halo);
     const int64_t own = (D + nslab - 1) / nslab;
-    float t_ms[B4D_T_COUNT] = {};
-    int64_t launches[B4D_T_COUNT] = {};
-    unsigned long long stats[4] = {};
+    B4D_TRY(reset_last(h));
     for (int64_t i = 0; i < n; ++i)
         for (int64_t ob = 0; ob < D; ob += own) {
             const int64_t oe = std::min(D, ob + own), zb = std::max<int64_t>(0, ob - halo), ze = std::min(D, oe + halo);
             const int64_t sshape[3] = {ze - zb, shape[1], shape[2]};
-            B4D_TRY(b4d_denoise_slab_u16(h, in + i * V + zb * P, sshape, zb, D, ob, oe, sigma, out + i * V + ob * P,
-                                         in_on_device, out_on_device));
-            for (int k = 0; k < B4D_T_COUNT; ++k) {
-                t_ms[k] += h->t_ms[k];
-                launches[k] += h->launches[k];
-            }
-            for (int k = 0; k < 4; ++k) stats[k] += h->match_stats[k];
+            B4D_TRY(denoise_slab_impl(h, in + i * V + zb * P, sshape, zb, D, ob, oe, sigma, out + i * V + ob * P,
+                                      in_on_device, out_on_device, nullptr));
         }
-    std::memcpy(h->t_ms, t_ms, sizeof(t_ms));
-    std::memcpy(h->launches, launches, sizeof(launches));
-    std::memcpy(h->match_stats, stats, sizeof(stats));
     return 0;
 }
 
@@ -1155,7 +1178,7 @@ int b4d_targets_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t 
     B4D_TRY(common_checks(h, in, teacher_out, shape, sigma));
     if (n < 1 || !offsets) return fail(B4D_ERR_INVALID, "n must be >= 1 and offsets non-NULL");
     if (h->prof.stages != 2) return fail(B4D_ERR_INVALID, "target generation needs stages = 2");
-    reset_timings(h);
+    B4D_TRY(reset_last(h));
     const long long V = shape[0] * shape[1] * shape[2];
     int64_t per = std::max<int64_t>(1, std::min<int64_t>(n, h->pass_voxels / V));
     // With host buffers a pass is cut into four chunks on two buffer sets: while chunk c computes, the
@@ -1208,7 +1231,7 @@ int b4d_targets_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t 
         mm.ishift = centre_shift(lo - std::ceil((double)omax), hi - std::floor((double)omin));
         // compute stream: the chunk's two stages and the clip (its inputs are complete: the copy stream was
         // synchronised above)
-        clk.mark(-1, 0);
+        clk.mark(-1);
         Pass ps;
         B4D_TRY(make_pass(h, pl, sigma, mm, b_zf[set]->as<float>(), b_in[set]->as<uint16_t>(),
                           b_out[set]->as<float>(), clk, ps));
@@ -1231,35 +1254,11 @@ int b4d_targets_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t 
     return finish(h, clk);
 }
 
-static int denoise_slab_impl(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
-                             int64_t z_total, int64_t own_begin, int64_t own_end, float sigma, void *out,
-                             int in_on_device, int out_on_device, const QuantSpec *q) {
-    B4D_TRY(common_checks(h, in, out, shape, sigma));
-    if (q && h->prof.stages != 2) return fail(B4D_ERR_INVALID, "quantized output needs stages = 2");
-    if (q && !(q->step >= 1.0f)) return fail(B4D_ERR_INVALID, "step must be >= 1");
-    const size_t esz = q ? sizeof(uint16_t) : sizeof(float);
-    if (z_begin < 0 || z_begin + shape[0] > z_total || own_begin < z_begin || own_end > z_begin + shape[0] ||
-        own_begin >= own_end)
-        return fail(B4D_ERR_INVALID, "slab / owned range inconsistent");
-    reset_timings(h);
-    const long long P = shape[1] * shape[2];
-    const Plan pl = make_plan(shape, z_begin, z_total, 1, h->prof);
-    StageClock clk(h);
-    MatchMap mm;
-    const uint16_t *host_src = nullptr;
-    B4D_TRY(stage_u16_input(h, pl, in, in_on_device, clk, &mm, &host_src));
-    HostSink sink{out_on_device ? nullptr : out, own_begin - z_begin, own_end - z_begin};
-    Pass ps;
-    B4D_TRY(make_pass(h, pl, sigma, mm, h->zf.as<float>(), h->in.as<uint16_t>(), h->out.as<float>(), clk, ps));
-    B4D_TRY(denoise_pass(ps, host_src, &sink, q));
-    if (!sink.done)
-        CU_TRY(copy_out(h, out, h->out.as<char>() + (size_t)sink.p0 * P * esz, (size_t)(sink.p1 - sink.p0) * P * esz,
-                        out_on_device, h->stream));
-    return finish(h, clk);
-}
 int b4d_denoise_slab_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
                          int64_t z_total, int64_t own_begin, int64_t own_end, float sigma, float *out,
                          int in_on_device, int out_on_device) {
+    B4D_TRY(common_checks(h, in, out, shape, sigma));
+    B4D_TRY(reset_last(h));
     return denoise_slab_impl(h, in, shape, z_begin, z_total, own_begin, own_end, sigma, out, in_on_device,
                              out_on_device, nullptr);
 }
@@ -1267,6 +1266,8 @@ int b4d_denoise_slab_q16_u16(b4d_handle *h, const uint16_t *in, const int64_t sh
                              int64_t z_total, int64_t own_begin, int64_t own_end, float sigma, float offset_sub,
                              float offset_add, float step, int truncate, uint16_t *out, int in_on_device,
                              int out_on_device) {
+    B4D_TRY(common_checks(h, in, out, shape, sigma));
+    B4D_TRY(reset_last(h));
     const QuantSpec q{offset_sub, offset_add, step, truncate};
     return denoise_slab_impl(h, in, shape, z_begin, z_total, own_begin, own_end, sigma, out, in_on_device,
                              out_on_device, &q);
@@ -1284,8 +1285,9 @@ int b4d_slab_stage1_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3
     B4D_TRY(common_checks(h, in, in, shape, sigma));
     if (z_begin < 0 || z_begin + shape[0] > z_total) return fail(B4D_ERR_INVALID, "slab range inconsistent");
     if (h->prof.stages != 2) return fail(B4D_ERR_INVALID, "the two-call slab form needs stages = 2");
-    reset_timings(h);
+    B4D_TRY(reset_last(h));
     h->slab_open = false;
+    h->pre.clk.discard();
     h->slab = make_plan(shape, z_begin, z_total, 1, h->prof);
     h->slab_z_begin = z_begin;
     h->slab_sigma = sigma;
@@ -1332,7 +1334,7 @@ static int slab_stage2_impl(b4d_handle *h, int64_t own_begin, int64_t own_end, v
     const long long P = (long long)h->slab.H * h->slab.W;
     const bool had_pre = h->pre.done;
     StageClock clk(h);
-    clk.mark(-1, 0);
+    clk.mark(-1);
     HostSink sink{out_on_device ? nullptr : out, own_begin - h->slab_z_begin, own_end - h->slab_z_begin};
     Pass ps;
     B4D_TRY(make_slab_pass(h, clk, ps));
@@ -1342,15 +1344,7 @@ static int slab_stage2_impl(b4d_handle *h, int64_t own_begin, int64_t own_end, v
         CU_TRY(copy_out(h, out, h->out.as<char>() + (size_t)sink.p0 * P * esz, (size_t)(sink.p1 - sink.p0) * P * esz,
                         out_on_device, h->stream));
     B4D_TRY(finish(h, clk));
-    if (had_pre) {
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, h->pre.ev0, h->pre.ev1) == cudaSuccess) {
-            h->t_ms[B4D_T_MATCH2] += ms;
-            h->launches[B4D_T_MATCH2] += 5;
-        } else {
-            cudaGetLastError();
-        }
-    }
+    h->pre.clk.resolve();  // part 1, if b4d_slab_stage2_begin ran
     h->slab_open = false;
     return 0;
 }
@@ -1375,17 +1369,13 @@ int b4d_slab_stage2_begin(b4d_handle *h, int64_t own_begin, int64_t own_end) {
     if (!h) return fail(B4D_ERR_INVALID, "NULL argument");
     B4D_TRY(check_open_slab(h, own_begin, own_end));
     CU_TRY(cudaSetDevice(h->device));
-    StageClock clk(h);
-    clk.mark(-1, 0);
-    if (!h->pre.ev0) {
-        CU_TRY(cudaEventCreate(&h->pre.ev0));
-        CU_TRY(cudaEventCreate(&h->pre.ev1));
-    }
-    CU_TRY(cudaEventRecord(h->pre.ev0, h->stream));
+    StageClock &clk = h->pre.clk;
+    clk.discard();  // a repeated call: only the last part 1 counts
+    clk.mark(-1);
     Pass ps;
     B4D_TRY(make_slab_pass(h, clk, ps));
     B4D_TRY(stage2_front_owned(ps, (int)(own_begin - h->slab_z_begin), (int)(own_end - h->slab_z_begin)));
-    CU_TRY(cudaEventRecord(h->pre.ev1, h->stream));
+    clk.mark(B4D_T_MATCH2);
     return 0;  // no synchronisation: the launches run while the caller exchanges planes
 }
 
@@ -1397,7 +1387,7 @@ int b4d_match_stage1(b4d_handle *h, const uint16_t *in, const int64_t shape[3], 
     if (Dc * Hc * Wc > INT32_MAX) return fail(B4D_ERR_TOO_LARGE, "candidate index space exceeds int32");
     const b4d_profile &p = h->prof;
     cudaStream_t s = h->stream;
-    reset_timings(h);
+    B4D_TRY(reset_last(h));
     const Plan pl = make_plan(shape, 0, shape[0], 1, p);
     B4dGeom g, g_unused;
     B4D_TRY(upload_geometry(h, pl, &g, &g_unused));
@@ -1409,8 +1399,6 @@ int b4d_match_stage1(b4d_handle *h, const uint16_t *in, const int64_t shape[3], 
     B4D_TRY(h->widx.ensure((size_t)R * std::max(p.k_ht, p.k_wie) * sizeof(uint16_t)));
     B4D_TRY(h->cnt.ensure((size_t)R));
     B4D_TRY(h->ssd.ensure((size_t)R * K * sizeof(uint32_t)));
-    B4D_TRY(h->stats.ensure(4 * sizeof(unsigned long long)));
-    CU_TRY(cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), s));
     B4D_TRY(h->s2.ensure((size_t)V * sizeof(uint2)));
     B4D_TRY(h->cells.ensure((size_t)pl.D * g.ty * g.tx * sizeof(uint32_t)));
     B4D_TRY(h->tcls.ensure((size_t)g.tz * g.ty * g.tx * sizeof(uint32_t)));
@@ -1428,9 +1416,9 @@ int b4d_match_stage1(b4d_handle *h, const uint16_t *in, const int64_t shape[3], 
     mp.ssd_out = h->ssd.as<uint32_t>();
     mp.stats = h->stats.as<unsigned long long>();
     StageClock clk(h);
-    clk.mark(-1, 0);
+    clk.mark(-1);
     b4d_launch_match(mp, Ns, s);
-    clk.mark(B4D_T_MATCH1, 4);
+    clk.mark(B4D_T_MATCH1);
     CU_TRY(cudaGetLastError());
     std::vector<uint16_t> hw((size_t)R * K);
     std::vector<uint32_t> hs((size_t)R * K);

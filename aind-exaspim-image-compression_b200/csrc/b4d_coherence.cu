@@ -184,10 +184,10 @@ void b4d_launch_coherence(const float *raw, const unsigned long long *labels, in
     cudaMemsetAsync(keys, 0, (size_t)npatch * cap * sizeof(unsigned long long), s);
     cudaMemsetAsync(sums, 0, (size_t)npatch * cap * COH_NSUM * sizeof(double), s);
     cudaMemsetAsync(overflow, 0, sizeof(int), s);
-    k_coh_centre<<<grid_of(total), 256, 0, s>>>(raw, x, V, npatch);
-    k_coh_gauss<<<grid_of(total), 256, 0, s>>>(x, sm, D, H, W, npatch, 0, radius, w);
-    k_coh_gauss<<<grid_of(total), 256, 0, s>>>(sm, tmp, D, H, W, npatch, 1, radius, w);
-    k_coh_gauss<<<grid_of(total), 256, 0, s>>>(tmp, sm, D, H, W, npatch, 2, radius, w);
-    k_coh_labels<<<grid_of(total), 256, 0, s>>>(labels, V, npatch, keys, cap, overflow);
-    k_coh_sums<<<grid_of(total), 256, 0, s>>>(x, sm, labels, D, H, W, npatch, lag, keys, cap, sums);
+    b4d_launch(k_coh_centre, grid_of(total), 256, 0, s, raw, x, V, npatch);
+    b4d_launch(k_coh_gauss, grid_of(total), 256, 0, s, x, sm, D, H, W, npatch, 0, radius, w);
+    b4d_launch(k_coh_gauss, grid_of(total), 256, 0, s, sm, tmp, D, H, W, npatch, 1, radius, w);
+    b4d_launch(k_coh_gauss, grid_of(total), 256, 0, s, tmp, sm, D, H, W, npatch, 2, radius, w);
+    b4d_launch(k_coh_labels, grid_of(total), 256, 0, s, labels, V, npatch, keys, cap, overflow);
+    b4d_launch(k_coh_sums, grid_of(total), 256, 0, s, x, sm, labels, D, H, W, npatch, lag, keys, cap, sums);
 }

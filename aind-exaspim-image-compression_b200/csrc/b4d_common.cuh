@@ -3,8 +3,22 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <utility>
+
 #include "../../include/b4d.h"
 #include "../../include/b4d_noise.h"
+
+// Kernels this host thread has enqueued.  A stage mark of the host pipeline books the kernels enqueued since the
+// previous mark as that stage's launch count.  Per thread because the launchers do not see the handle; a call
+// runs on one thread (the transfer threads only copy).
+inline thread_local long long b4d_kernels_enqueued = 0;
+
+// The one place that enqueues a kernel (every launcher goes through it, so every kernel is counted).
+template <class... P, class... A>
+inline void b4d_launch(void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, A &&...args) {
+    kernel<<<grid, block, smem, s>>>(std::forward<A>(args)...);
+    ++b4d_kernels_enqueued;
+}
 
 #define B4D_L 4
 #define B4D_LV 64

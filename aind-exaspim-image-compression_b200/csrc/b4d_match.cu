@@ -1280,9 +1280,9 @@ void launch_k(const MatchParams &pin, long long tile0, long long tile1, cudaStre
     const unsigned tiles = (unsigned)(tile1 - tile0);
     // byte tiles first (cheap), then everything else; each kernel exits at once on a foreign tile
     cudaFuncSetAttribute(k_match<NS, K32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G::SMEM_B);
-    k_match<NS, K32, true><<<tiles, WARPS * 32, G::SMEM_B, s>>>(p, tmap, emap);
+    b4d_launch(k_match<NS, K32, true>, tiles, WARPS * 32, G::SMEM_B, s, p, tmap, emap);
     cudaFuncSetAttribute(k_match<NS, K32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G::SMEM);
-    k_match<NS, K32, false><<<tiles, WARPS * 32, G::SMEM, s>>>(p, tmap, emap);
+    b4d_launch(k_match<NS, K32, false>, tiles, WARPS * 32, G::SMEM, s, p, tmap, emap);
 }
 // cell planes [cz0, cz1) (min/max table) and tiles [tile0, tile1) (classification + both matcher
 // kernels); the whole volume in one go is cz = [0, cd), tiles = [0, all)
@@ -1291,9 +1291,11 @@ void launch_ns(const MatchParams &p, int cz0, int cz1, long long tile0, long lon
     // cz0, cz1 count 4-plane layers (the callers' unit): voxel planes [4 cz0, min(4 cz1, D))
     const int z0 = 4 * cz0, z1 = std::min(4 * cz1, p.g.D);
     if (z1 > z0)
-        k_plane_ranges<NS><<<(unsigned)((long long)p.g.nvol * (z1 - z0) * p.g.ty), 256, 0, s>>>(p.u, p.g, p.cells, z0, z1);
+        b4d_launch(k_plane_ranges<NS>, (unsigned)((long long)p.g.nvol * (z1 - z0) * p.g.ty), 256, 0, s, p.u, p.g,
+                   p.cells, z0, z1);
     if (tile1 > tile0) {
-        k_tile_class<NS><<<(unsigned)((tile1 - tile0 + 7) / 8), 256, 0, s>>>(p.cells, p.g, p.tcls, tile0, tile1);
+        b4d_launch(k_tile_class<NS>, (unsigned)((tile1 - tile0 + 7) / 8), 256, 0, s, p.cells, p.g, p.tcls, tile0,
+                   tile1);
         if (p.K > 16) launch_k<NS, true>(p, tile0, tile1, s);
         else launch_k<NS, false>(p, tile0, tile1, s);
     }
@@ -1316,13 +1318,13 @@ void b4d_launch_block_energy_range(const uint16_t *u, uint2 *s21, int D, int H, 
                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS) {
             const long long blocks = (long long)((W - 3 + K0T_TX - 1) / K0T_TX) * ((H - 3 + K0_TY - 1) / K0_TY) * nzc * nvol;
-            k_block_energy_tma<<<(unsigned)blocks, K0T_WARPS * 32, 0, s>>>(map, s21, D, H, W, nvol, zo0, zo1);
+            b4d_launch(k_block_energy_tma, (unsigned)blocks, K0T_WARPS * 32, 0, s, map, s21, D, H, W, nvol, zo0, zo1);
             return;
         }
     }
     const long long warps = (long long)((W - 3 + K0_TX - 1) / K0_TX) * ((H - 3 + K0_TY - 1) / K0_TY) * nzc * nvol;
     const long long blocks = (warps + K0_WARPS - 1) / K0_WARPS;
-    k_block_energy<<<(unsigned)blocks, K0_WARPS * 32, 0, s>>>(u, s21, D, H, W, nvol, zo0, zo1);
+    b4d_launch(k_block_energy, (unsigned)blocks, K0_WARPS * 32, 0, s, u, s21, D, H, W, nvol, zo0, zo1);
 }
 void b4d_launch_block_energy(const uint16_t *u, uint2 *s21, int D, int H, int W, int nvol, cudaStream_t s) {
     b4d_launch_block_energy_range(u, s21, D, H, W, nvol, 0, D - 3, s);

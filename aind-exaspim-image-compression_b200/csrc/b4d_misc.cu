@@ -717,25 +717,26 @@ __global__ void __launch_bounds__(1024) k_pipe(int iters, unsigned *sink) {
 }  // namespace
 
 void b4d_launch_u16_to_f32(const uint16_t *in, float *out, long long n, unsigned *minmax, cudaStream_t s) {
-    k_u16_to_f32<<<grid_for(n >> 3, 256, 8), 256, 0, s>>>(in, out, n, minmax);
+    b4d_launch(k_u16_to_f32, grid_for(n >> 3, 256, 8), 256, 0, s, in, out, n, minmax);
 }
 void b4d_launch_u16_sub_offset(const uint16_t *in, const float *off, float *out, long long vol_stride, long long n,
                                unsigned *minmax, cudaStream_t s) {
-    k_u16_sub_offset<<<grid_for((vol_stride & 7) ? n : (n >> 3), 256, 8), 256, 0, s>>>(in, off, out, vol_stride, n, minmax);
+    b4d_launch(k_u16_sub_offset, grid_for((vol_stride & 7) ? n : (n >> 3), 256, 8), 256, 0, s, in, off, out,
+               vol_stride, n, minmax);
 }
 __global__ void __launch_bounds__(256) k_add_scalar(float *__restrict__ x, long long n, float c) {
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) x[i] = __fadd_rn(x[i], c);
 }
 void b4d_launch_add_scalar(float *x, long long n, float c, cudaStream_t s) {
-    k_add_scalar<<<grid_for(n, 256, 8), 256, 0, s>>>(x, n, c);
+    b4d_launch(k_add_scalar, grid_for(n, 256, 8), 256, 0, s, x, n, c);
 }
 void b4d_launch_clip(float *x, long long n, float hi, cudaStream_t s) {
-    k_clip<<<grid_for(n >> 2, 256, 8), 256, 0, s>>>(x, n, hi);
+    b4d_launch(k_clip, grid_for(n >> 2, 256, 8), 256, 0, s, x, n, hi);
 }
 void b4d_launch_to_match(const float *in, uint16_t *out, long long n, float cf, float scale, int ishift,
                          cudaStream_t s) {
-    k_to_match<<<grid_for(n >> 3, 256, 8), 256, 0, s>>>(in, out, n, cf, scale, ishift);
+    b4d_launch(k_to_match, grid_for(n >> 3, 256, 8), 256, 0, s, in, out, n, cf, scale, ishift);
 }
 static void launch_norm(const long long *numq, const uint32_t *gmap, const float *fallback, const NormOut &o, int D,
                         int H, int W, int nvol, int z0, int z1, float inv_qscale, const float kf[4], cudaStream_t s) {
@@ -751,13 +752,13 @@ static void launch_norm(const long long *numq, const uint32_t *gmap, const float
             attr = true;
         }
         const long long blocks = (long long)nvol * ntz * nty * ((W + WMT_TX - 1) / WMT_TX);
-        k_normalise_wm_tma<<<(unsigned)blocks, WMT_WARPS * 32, WMT_NST * WMT_STAGE, s>>>(
-            mg, mn, fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf[0], kf[1], kf[2], kf[3]);
+        b4d_launch(k_normalise_wm_tma, (unsigned)blocks, WMT_WARPS * 32, WMT_NST * WMT_STAGE, s, mg, mn, fallback, o,
+                   D, H, W, nvol, z0, z1, inv_qscale, kf[0], kf[1], kf[2], kf[3]);
         return;
     }
     const long long tiles = (long long)nvol * ntz * nty * ((W + WM_TX - 1) / WM_TX);
-    k_normalise_wm<<<(unsigned)((tiles + WM_WARPS - 1) / WM_WARPS), WM_WARPS * 32, 0, s>>>(
-        numq, gmap, fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf[0], kf[1], kf[2], kf[3]);
+    b4d_launch(k_normalise_wm, (unsigned)((tiles + WM_WARPS - 1) / WM_WARPS), WM_WARPS * 32, 0, s, numq, gmap,
+               fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf[0], kf[1], kf[2], kf[3]);
 }
 void b4d_launch_normalise_wm(const long long *numq, const uint32_t *gmap, const float *fallback, float *out, int D,
                              int H, int W, int nvol, int z0, int z1, float inv_qscale, const float kf[4],
@@ -792,35 +793,35 @@ void b4d_launch_normalise_match(const long long *numq, const uint32_t *gmap, con
 }
 void b4d_launch_quantize(const float *in, uint16_t *out, long long n, float offset_sub, float offset_add,
                          float step, cudaStream_t s) {
-    k_quantize<false><<<grid_for(n >> 4, 256, 8), 256, 0, s>>>(in, out, n, offset_sub, offset_add, step);
+    b4d_launch(k_quantize<false>, grid_for(n >> 4, 256, 8), 256, 0, s, in, out, n, offset_sub, offset_add, step);
 }
 void b4d_launch_quantize_trunc(const float *in, uint16_t *out, long long n, float offset_sub, float offset_add,
                                float step, cudaStream_t s) {
-    k_quantize<true><<<grid_for(n >> 4, 256, 8), 256, 0, s>>>(in, out, n, offset_sub, offset_add, step);
+    b4d_launch(k_quantize<true>, grid_for(n >> 4, 256, 8), 256, 0, s, in, out, n, offset_sub, offset_add, step);
 }
 void b4d_launch_chunk_shuffle(const uint16_t *in, int D, int H, int W, int cz, int cy, int cx, uint8_t *out,
                               uint32_t *hist, cudaStream_t s) {
     const long long nchunks = (long long)((D + cz - 1) / cz) * ((H + cy - 1) / cy) * ((W + cx - 1) / cx);
-    k_chunk_shuffle<<<grid_for(nchunks * 256, 256, 8), 256, 0, s>>>(in, D, H, W, cz, cy, cx, out, hist);
+    b4d_launch(k_chunk_shuffle, grid_for(nchunks * 256, 256, 8), 256, 0, s, in, D, H, W, cz, cy, cx, out, hist);
 }
 void b4d_launch_fg_mask(const uint16_t *in, const float *off, const float *thr, int D, int H, int W, long long n,
                         int dilate, uint8_t *out, cudaStream_t s) {
-    k_fg_mask<<<grid_for(n, 256, 8), 256, 0, s>>>(in, off, thr, D, H, W, n, dilate, out);
+    b4d_launch(k_fg_mask, grid_for(n, 256, 8), 256, 0, s, in, off, thr, D, H, W, n, dilate, out);
 }
 void b4d_launch_hist(const uint16_t *in, long long n, unsigned long long *hist, cudaStream_t s) {
-    k_hist<<<grid_for(n >> 3, 512, 2), 512, 0, s>>>(in, n, hist);
+    b4d_launch(k_hist, grid_for(n >> 3, 512, 2), 512, 0, s, in, n, hist);
 }
 int b4d_analyze_blocks() { return AN_BLOCKS; }
 void b4d_launch_analyze(const float *in, long long n, double c, double *partial, cudaStream_t s) {
-    k_analyze<<<AN_BLOCKS, 256, 0, s>>>(in, n, c, partial);
+    b4d_launch(k_analyze, AN_BLOCKS, 256, 0, s, in, n, c, partial);
 }
 double b4d_launch_pipe_bench(int which, int iters, unsigned *sink, cudaStream_t s) {
     const int blocks = sm_count() * 2;
     switch (which) {
-        case 0: k_pipe<0><<<blocks, 1024, 0, s>>>(iters, sink); break;
-        case 1: k_pipe<1><<<blocks, 1024, 0, s>>>(iters, sink); break;
-        case 2: k_pipe<2><<<blocks, 1024, 0, s>>>(iters, sink); break;
-        default: k_pipe<3><<<blocks, 1024, 0, s>>>(iters, sink); break;
+        case 0: b4d_launch(k_pipe<0>, blocks, 1024, 0, s, iters, sink); break;
+        case 1: b4d_launch(k_pipe<1>, blocks, 1024, 0, s, iters, sink); break;
+        case 2: b4d_launch(k_pipe<2>, blocks, 1024, 0, s, iters, sink); break;
+        default: b4d_launch(k_pipe<3>, blocks, 1024, 0, s, iters, sink); break;
     }
     const double per_iter = (which == 2) ? 2.0 : 1.0;
     return (double)blocks * 1024.0 * (double)iters * 16.0 * 8.0 * per_iter;

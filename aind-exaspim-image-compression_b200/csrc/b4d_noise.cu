@@ -380,7 +380,7 @@ void launch_nlf(const NlfGeom &g, uint32_t *hist, unsigned long long *lsum, cons
     const long long rows = (long long)g.ncz * g.ncy * g.nvol;
     long long blocks = (rows + NLF_THREADS / 32 - 1) / (NLF_THREADS / 32);
     blocks = std::min<long long>(blocks, (long long)std::max(1, per_sm) * sm_count());
-    k_nlf_pass<PASS, WIDE><<<(unsigned)std::max(1ll, blocks), NLF_THREADS, smem, s>>>(g, hist, lsum, sel);
+    b4d_launch(k_nlf_pass<PASS, WIDE>, (unsigned)std::max(1ll, blocks), NLF_THREADS, smem, s, g, hist, lsum, sel);
 }
 
 }  // namespace
@@ -407,25 +407,25 @@ void b4d_launch_noise_pass(const NoiseGeom &g, int pass, long long ntiles, uint3
     const int threads = 32 * g.warps;
     const bool w = wide_ok(g);
     if (pass == 1) {
-        if (w) k_noise_pass<1, true><<<blocks, threads, 0, s>>>(g, hist, sel);
-        else k_noise_pass<1, false><<<blocks, threads, 0, s>>>(g, hist, sel);
+        if (w) b4d_launch(k_noise_pass<1, true>, blocks, threads, 0, s, g, hist, sel);
+        else b4d_launch(k_noise_pass<1, false>, blocks, threads, 0, s, g, hist, sel);
     } else {
-        if (w) k_noise_pass<2, true><<<blocks, threads, 0, s>>>(g, hist, sel);
-        else k_noise_pass<2, false><<<blocks, threads, 0, s>>>(g, hist, sel);
+        if (w) b4d_launch(k_noise_pass<2, true>, blocks, threads, 0, s, g, hist, sel);
+        else b4d_launch(k_noise_pass<2, false>, blocks, threads, 0, s, g, hist, sel);
     }
 }
 
 void b4d_launch_noise_select(int which, const uint32_t *hist, uint32_t *sel, uint32_t *res, long long ntiles,
                              cudaStream_t s) {
     const unsigned blocks = (unsigned)((ntiles + 7) / 8);
-    if (which == 1) k_noise_select1<<<blocks, 256, 0, s>>>(hist, sel, ntiles);
-    else k_noise_select2<<<blocks, 256, 0, s>>>(hist, sel, res, ntiles);
+    if (which == 1) b4d_launch(k_noise_select1, blocks, 256, 0, s, hist, sel, ntiles);
+    else b4d_launch(k_noise_select2, blocks, 256, 0, s, hist, sel, res, ntiles);
 }
 
 void b4d_launch_noise_hist(const NoiseGeom &g, long long nvol, unsigned long long *hist, cudaStream_t s) {
     const long long rows = (long long)g.ncz * g.ncy * nvol;
     long long blocks = (rows + 7) / 8;
     if (blocks > 4ll * sm_count()) blocks = 4ll * sm_count();
-    if (wide_ok(g)) k_noise_hist<true><<<(unsigned)blocks, 256, 0, s>>>(g, nvol, hist);
-    else k_noise_hist<false><<<(unsigned)blocks, 256, 0, s>>>(g, nvol, hist);
+    if (wide_ok(g)) b4d_launch(k_noise_hist<true>, (unsigned)blocks, 256, 0, s, g, nvol, hist);
+    else b4d_launch(k_noise_hist<false>, (unsigned)blocks, 256, 0, s, g, nvol, hist);
 }

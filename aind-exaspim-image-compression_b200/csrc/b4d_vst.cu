@@ -69,13 +69,14 @@ __global__ void __launch_bounds__(256) k_gat_inverse(const float *in, float *out
 }  // namespace
 
 void b4d_launch_gat_forward(const uint16_t *in, float *out, long long n, const GatParams &p, cudaStream_t s) {
-    k_gat_forward<<<grid_for(n), 256, 0, s>>>(in, out, n, p);
+    b4d_launch(k_gat_forward, grid_for(n), 256, 0, s, in, out, n, p);
 }
 
 void b4d_launch_gat_inverse(const float *in, float *out, uint16_t *q16, long long n, const GatParams &p,
                             float offset_sub, float offset_add, float step, int trunc, cudaStream_t s) {
     const unsigned g = grid_for(n);
-    if (!q16) k_gat_inverse<false, false><<<g, 256, 0, s>>>(in, out, q16, n, p, offset_sub, offset_add, step);
-    else if (trunc) k_gat_inverse<true, true><<<g, 256, 0, s>>>(in, out, q16, n, p, offset_sub, offset_add, step);
-    else k_gat_inverse<true, false><<<g, 256, 0, s>>>(in, out, q16, n, p, offset_sub, offset_add, step);
+    if (!q16) b4d_launch(k_gat_inverse<false, false>, g, 256, 0, s, in, out, q16, n, p, offset_sub, offset_add, step);
+    else if (trunc)
+        b4d_launch(k_gat_inverse<true, true>, g, 256, 0, s, in, out, q16, n, p, offset_sub, offset_add, step);
+    else b4d_launch(k_gat_inverse<true, false>, g, 256, 0, s, in, out, q16, n, p, offset_sub, offset_add, step);
 }

@@ -239,8 +239,12 @@ int b4d_tile_stats(b4d_handle *h, const uint16_t *in, int64_t n, double pct, b4d
  * ranks all-gather): host arithmetic only, no device work. */
 int b4d_stats_from_hist(const int64_t *hist, double pct, b4d_stats *out);
 
-/* Device time of the last denoise call, per kernel family, in milliseconds
- * (CUDA events on the handle's stream).  names: see B4D_T_* below. */
+/* The last public denoise call as a whole (every chunk, pass and slab of it; the two-call slab form from
+ * b4d_slab_stage1_u16 to b4d_slab_stage2), per kernel family (B4D_T_* below): ms = device time in milliseconds
+ * (CUDA events on the handle's stream), launches = the kernels enqueued in the intervals that family books.
+ * Memsets and copies are not launches.  A few kernels are booked to no family: the add-back of the DC shift of
+ * centred float input, the clip and offset subtraction of b4d_targets_u16, the block energies of
+ * b4d_match_stage1. */
 #define B4D_T_PREP 0
 #define B4D_T_MATCH1 1
 #define B4D_T_FILTER1 2
@@ -257,7 +261,8 @@ int b4d_last_timings(b4d_handle *h, float ms[B4D_T_COUNT], int64_t launches[B4D_
  * a call.  NULL for the CPU oracle build. */
 void *b4d_stream(b4d_handle *h);
 
-/* Diagnostics of the last matching launch(es): out[0] = reference blocks that
+/* Diagnostics of the matching launches of the last public call, summed over all of them (as b4d_last_timings):
+ * out[0] = reference blocks that
  * took the survivor-list overflow fallback, out[1] = tiles on the uint64 path,
  * out[2] = reference blocks on the exact-but-slow selection, out[3] = tiles matched
  * on the byte (dp4a) path. */
