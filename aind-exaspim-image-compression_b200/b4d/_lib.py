@@ -70,6 +70,14 @@ _NOISE = {
 SIGNATURES = {**_CORE, **_NOISE}
 EXPORTS = tuple(_CORE)
 NOISE_EXPORTS = tuple(_NOISE)
+# include/b4d_vst_slab.h: the z-slab forms of the VST path, a table of their own
+VST_SLAB_SIGNATURES = {
+    "b4d_denoise_slab_vst_u16": (_INT, [_P, _P, _P, _I64, _I64, _I64, _I64, _P, _F32, _P, _INT, _P, _INT, _INT]),
+    "b4d_denoise_slab_vst_q16_u16": (_INT, [_P, _P, _P, _I64, _I64, _I64, _I64, _P, _F32, _P, _INT, _F32, _F32, _F32,
+                                             _INT, _P, _INT, _INT]),
+    "b4d_slab_stage1_vst_u16": (_INT, [_P, _P, _P, _I64, _I64, _P, _F32, _P, _INT, _INT]),
+}
+VST_SLAB_EXPORTS = tuple(VST_SLAB_SIGNATURES)
 NOISE_HIST_BINS = 262141  # B4D_NOISE_HIST_BINS: |d| <= 4 * 65535
 NLF_MAX_BINS = 64  # B4D_NLF_MAX_BINS
 
@@ -128,7 +136,7 @@ def load():
             "or `make -C aind-exaspim-image-compression_b200/csrc`. There is no CPU fallback." % LIB_PATH
         )
     lib = ctypes.CDLL(LIB_PATH)
-    for name, (restype, argtypes) in SIGNATURES.items():
+    for name, (restype, argtypes) in {**SIGNATURES, **VST_SLAB_SIGNATURES}.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
     if lib.b4d_version() != ABI_VERSION:

@@ -373,7 +373,8 @@ class Denoiser:
 
     def set_pass_voxels(self, voxels):
         """Voxels per pass (scratch ~45 B each; 0 = default 1.25 Gi).  A uint16 volume larger than a
-        pass is denoised as consecutive z-slabs with halos; the result does not change."""
+        pass is denoised as consecutive z-slabs with halos, by denoise and by denoise_vst (which first
+        takes the value set of the whole volume); the result does not change."""
         _lib.check(self.lib.b4d_set_pass_voxels(self._h, int(voxels)))
 
     def set_pipeline_min_voxels(self, voxels):
@@ -506,7 +507,8 @@ class Denoiser:
         """Denoise Poisson-Gaussian uint16 counts: gat_inverse(denoise(gat_forward(x, model), sigma), model), with the
         intermediate float32 volume never leaving the device.  sigma is the noise level after the transform: 1 for an
         exact model.  (D,H,W) or (N,D,H,W), NumPy or torch -> float32; quantize = (offset_sub, offset_add, step[,
-        truncate]): the uint16 volume quantize() gives on that float32 result instead."""
+        truncate]): the uint16 volume quantize() gives on that float32 result instead.  A volume larger than a pass
+        (set_pass_voxels) is denoised as z-slabs with the value set of the whole volume: the same result."""
         x = _vst_args(x, sigma, quantize)
         m = _model_c(model)
         xc, in_ptr, on_dev, shape = self._input(x)
@@ -519,6 +521,37 @@ class Denoiser:
             _lib.check(self.lib.b4d_denoise_vst_q16_u16(self._h, in_ptr, n, _lib.shape3(shape[-3:]), ctypes.byref(m),
                                                         sigma, *_quantize_args(quantize), _ptr(out), on_dev, on_dev))
         return out
+
+    def denoise_slab_vst(self, slab, z_begin, z_total, own_begin, own_end, model, value_hist, first, sigma=1.0,
+                         out=None, quantize=None):
+        """denoise_slab through the GAT: one z-slab (uint16, with halos) of a larger volume -> its owned planes of
+        denoise_vst on the whole volume, bit for bit (DESIGN §3.12, map rule).  value_hist: the 65536 counts of every
+        uint16 value of the WHOLE volume (tile_stats(..., return_hist=True), or such histograms summed across ranks);
+        first: the whole volume's voxel (0, 0, 0).  out / quantize as denoise_slab."""
+        sc, in_ptr, on_dev, shape = self._input(_vst_args(slab, sigma, quantize, (3,), "denoise_slab_vst"))
+        m, hist, first = _model_c(model), _value_hist(value_hist), int(first)
+        odt = "float32" if quantize is None else "uint16"
+        oshape = (own_end - own_begin,) + shape[1:]
+        out = _out_like(sc, oshape, odt) if _is_torch(sc) else _host_out(out, oshape, odt)
+        if quantize is None:
+            _lib.check(self.lib.b4d_denoise_slab_vst_u16(self._h, in_ptr, _lib.shape3(shape), z_begin, z_total,
+                                                         own_begin, own_end, ctypes.byref(m), sigma, hist.ctypes.data,
+                                                         first, _ptr(out), on_dev, on_dev))
+        else:
+            _lib.check(self.lib.b4d_denoise_slab_vst_q16_u16(self._h, in_ptr, _lib.shape3(shape), z_begin, z_total,
+                                                             own_begin, own_end, ctypes.byref(m), sigma,
+                                                             hist.ctypes.data, first, *_quantize_args(quantize),
+                                                             _ptr(out), on_dev, on_dev))
+        return out
+
+    def slab_stage1_vst(self, slab, z_begin, z_total, model, value_hist, first, sigma=1.0):
+        """slab_stage1 through the GAT (value_hist, first as denoise_slab_vst); slab_basic / slab_set_basic /
+        slab_basic_tensor / slab_stage2_begin / slab_stage2 complete it, and stage 2 ends in the inverse."""
+        sc, ptr, on_dev, shape = self._input(_vst_args(slab, sigma, None, (3,), "slab_stage1_vst"))
+        m, hist, first = _model_c(model), _value_hist(value_hist), int(first)
+        self._slab_shape = tuple(int(v) for v in shape)
+        _lib.check(self.lib.b4d_slab_stage1_vst_u16(self._h, ptr, _lib.shape3(shape), z_begin, z_total,
+                                                    ctypes.byref(m), sigma, hist.ctypes.data, first, on_dev))
 
     def coherence_scores(self, labels, raw, smooth_sigma=1.0, coherence_lag=2, min_autocorr=0.4,
                          max_highfreq_frac=0.35, min_segment_voxels=50, max_segments=1024):
@@ -838,14 +871,25 @@ def _nlf_args(x, edges, min_cells):
     return x, e, int(min_cells)
 
 
-def _vst_args(x, sigma, quantize):
-    """Argument checks of denoise_vst, before any device work: returns x."""
-    x = _array_arg(x, ("uint16",), (3, 4), "denoise_vst")
+def _vst_args(x, sigma, quantize, ndims=(3, 4), what="denoise_vst"):
+    """Argument checks of denoise_vst (and its slab forms), before any device work: returns x."""
+    x = _array_arg(x, ("uint16",), ndims, what)
     if not (np.isfinite(sigma) and sigma > 0):
         raise ValueError("sigma must be positive and finite, got %r" % (sigma,))
     if quantize is not None and not (3 <= len(quantize) <= 4 and float(quantize[2]) >= 1.0):
         raise ValueError("quantize must be (offset_sub, offset_add, step >= 1[, truncate])")
     return x
+
+
+def _value_hist(value_hist):
+    """The value set of a VST slab (NumPy or torch, host or CUDA) -> C-contiguous int64 NumPy array of 65536 counts;
+    ValueError for another length."""
+    if _is_torch(value_hist):
+        value_hist = value_hist.detach().cpu().numpy()
+    h = np.ascontiguousarray(value_hist, dtype=np.int64)
+    if h.shape != (65536,):
+        raise ValueError("value_hist must hold 65536 counts (one per uint16 value), got shape %r" % (h.shape,))
+    return h
 
 
 def noise_level_function(x, edges=None, min_cells=256, device=None):

@@ -6,7 +6,9 @@ whole-volume result and no volume data crosses GPUs.  The only exchange is the
 all-gather of per-slab uint16 histograms (256 KiB per rank) from which every
 rank derives the same global offset percentile / median / MAD sigma — a
 percentile is not decomposable from per-rank percentiles, a histogram is
-(transforms.py:433-438, metrics.py:54-58).
+(transforms.py:433-438, metrics.py:54-58).  The VST path (DESIGN §3.12) uses the
+same merged histogram as the value set of the whole volume, from which every rank
+derives the same matching map.
 """
 import os
 
@@ -65,15 +67,48 @@ def exchange_planes(send_down, send_up, recv_below, recv_above, rank, world, gro
             req.wait()
 
 
+def _process_group_ready():
+    import torch.distributed as dist
+
+    return dist.is_available() and dist.is_initialized()
+
+
+def vst_value_hist(denoiser, owned, world, value_hist=None, device=None, group=None):
+    """The value set of the whole volume for the VST slab forms (int64 NumPy, 65536 counts): `value_hist` as given,
+    else the histogram of this rank's `owned` planes summed over the ranks with merge_histograms.  ValueError when
+    world > 1 and no process group is initialised: the local histogram alone would silently give another map."""
+    if value_hist is not None:
+        return value_hist
+    if world > 1 and not _process_group_ready():
+        raise ValueError("world > 1 needs an initialised process group, or the whole volume's value_hist")
+    import torch
+
+    _, hist = denoiser.tile_stats(owned, return_hist=True)
+    merged = merge_histograms(torch.from_numpy(hist).to(device) if device is not None else torch.from_numpy(hist),
+                              group)
+    return merged.cpu().numpy()
+
+
 def denoise_slab_exchange(denoiser, slab, z_begin, z_total, own_begin, own_end, sigma, rank, world, device=None,
-                          out=None, group=None, quantize=None):
+                          out=None, group=None, quantize=None, model=None, value_hist=None, first=None):
     """One rank's part of the exchange variant: stage 1 on the slab (halo `exchange_halo`), swap
     the exact basic-estimate planes next to each interior face with the neighbours, stage 2.
     `device` = the rank's torch CUDA device (planes then travel device to device).
-    quantize = (offset_sub, offset_add, step[, truncate]): uint16 output of the fused quantizer."""
+    quantize = (offset_sub, offset_add, step[, truncate]): uint16 output of the fused quantizer.
+    model (PoissonGaussian, the same on every rank): through the GAT, `sigma` is then sigma_vst; value_hist as
+    vst_value_hist; first = the whole volume's voxel (0, 0, 0), taken from the slab when it starts at plane 0."""
     import torch
 
-    denoiser.slab_stage1(slab, z_begin, z_total, sigma)
+    if model is None:
+        denoiser.slab_stage1(slab, z_begin, z_total, sigma)
+    else:
+        if first is None:
+            if z_begin != 0:
+                raise ValueError("the VST slab form needs `first`, the whole volume's voxel (0, 0, 0)")
+            first = int(slab[0, 0, 0])
+        value_hist = vst_value_hist(denoiser, slab[own_begin - z_begin : own_end - z_begin], world, value_hist,
+                                    device, group)
+        denoiser.slab_stage1_vst(slab, z_begin, z_total, model, value_hist, first, sigma)
     lo_h, hi_h = own_begin - z_begin, (z_begin + slab.shape[0]) - own_end
     if (rank > 0 and own_end - own_begin < lo_h) or (rank < world - 1 and own_end - own_begin < hi_h):
         raise ValueError("every rank must own at least as many planes as the halo")
@@ -109,24 +144,37 @@ def denoise_slab_exchange(denoiser, slab, z_begin, z_total, own_begin, own_end, 
     return denoiser.slab_stage2(own_begin, own_end, out=out, device=device if out is None else None, quantize=quantize)
 
 
-def denoise_volume_sharded(get_slab, z_total, sigma, denoiser, world=1, rank=0, exchange=False, device=None):
+def denoise_volume_sharded(get_slab, z_total, sigma, denoiser, world=1, rank=0, exchange=False, device=None,
+                           model=None, value_hist=None):
     """Denoise this rank's share of a (z_total, H, W) uint16 volume.
 
     get_slab(z_begin, z_end) -> uint16 array/tensor of those planes (host or
     device).  Returns (own_begin, own_end, float32 planes).  With `exchange`
     (needs an initialised process group when world > 1) the slabs carry half the
     halo and neighbours swap basic-estimate planes between the stages.
+    model (PoissonGaussian, the same on every rank): denoise through the GAT
+    (DESIGN §3.12) with `sigma` as sigma_vst; the value set is `value_hist` (the
+    whole volume's 65536 counts) or, when None, the owned planes' histograms
+    merged across the ranks (world > 1 then needs an initialised process group).
     """
     p = denoiser.profile
     ns1, ns2 = 2 * int(np.ravel(p.search_window_ht)[0]) + 1, 2 * int(np.ravel(p.search_window_wiener)[0]) + 1
+    if model is not None and value_hist is None and world > 1 and not _process_group_ready():
+        raise ValueError("world > 1 needs an initialised process group, or the whole volume's value_hist")
+    first = None if model is None else int(get_slab(0, 1)[0, 0, 0])
     if exchange and denoiser._stages == 2 and world > 1:
         own_begin, own_end, z_begin, z_end = slab_plan(z_total, world, rank, exchange_halo(ns1, ns2))
         out = denoise_slab_exchange(denoiser, get_slab(z_begin, z_end), z_begin, z_total, own_begin, own_end, sigma,
-                                    rank, world, device=device)
+                                    rank, world, device=device, model=model, value_hist=value_hist, first=first)
         return own_begin, own_end, out
     own_begin, own_end, z_begin, z_end = slab_plan(z_total, world, rank, halo_planes(ns1, ns2, denoiser._stages))
     slab = get_slab(z_begin, z_end)
-    out = denoiser.denoise_slab(slab, z_begin, z_total, own_begin, own_end, sigma)
+    if model is None:
+        out = denoiser.denoise_slab(slab, z_begin, z_total, own_begin, own_end, sigma)
+    else:
+        value_hist = vst_value_hist(denoiser, slab[own_begin - z_begin : own_end - z_begin], world, value_hist,
+                                    device)
+        out = denoiser.denoise_slab_vst(slab, z_begin, z_total, own_begin, own_end, model, value_hist, first, sigma)
     return own_begin, own_end, out
 
 

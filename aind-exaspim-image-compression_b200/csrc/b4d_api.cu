@@ -10,6 +10,7 @@
 #include <string>
 #include <vector>
 
+#include "../../include/b4d_vst_slab.h"
 #include "b4d_common.cuh"
 #include "b4d_host.cuh"
 
@@ -113,6 +114,7 @@ struct b4d_handle {
     DevBuf alt_in, alt_zf, alt_out, alt_partial, alt_sink;  // second buffer set of b4d_targets_u16
     DevBuf nz_hist, nz_sel, nz_res, nz_full;  // b4d_noise_sigma_u16: per-tile digit histograms, selections, results
     DevBuf nlf_sum;  // b4d_noise_level_u16: per-bin sums of the cell intensities
+    DevBuf vst;      // VST passes: value table [65536 f32] | value list [65537 f32] | absent flag | value codes
     float t_ms[B4D_T_COUNT] = {};
     int64_t launches[B4D_T_COUNT] = {};
     unsigned long long match_stats[4] = {};
@@ -128,6 +130,8 @@ struct b4d_handle {
     int64_t slab_z_begin = 0;
     float slab_sigma = 0.f;
     MatchMap slab_mm;
+    bool slab_vst = false;  // a VST slab (b4d_slab_stage1_vst_u16): data in `in`, matching image in `u16`
+    GatEpilogue slab_gat{};  // ... and the inverse its stage 2 ends in
     OwnedFront pre{this};
 };
 
@@ -422,6 +426,7 @@ struct Pass {
     const Plan *pl;
     StageClock *clk;
     MatchMap mm;  // a streamed stage-1 upload sets ishift from the data range
+    const GatEpilogue *gat = nullptr;  // a VST pass: the normalise into `out` ends in the GAT inverse
     float *zf;
     uint16_t *u;
     float *basic, *out;
@@ -515,17 +520,18 @@ int zero_acc(const Pass &ps) {
 }
 
 // Planes [z0, z1) of every volume of the accumulators divided out: num / den from `fallback` into `dst`, or
-// quantized into `dst` as uint16 with `q`.
+// quantized into `dst` as uint16 with `q`.  The normalise into the pass's result of a VST pass ends in the inverse.
 void normalise(const Pass &ps, const float *fallback, float *dst, int z0, int z1, const QuantSpec *q, cudaStream_t s) {
     const Plan &pl = *ps.pl;
     const long long *numq = ps.h->numq.as<long long>();
     const uint32_t *gmap = ps.h->gmap.as<uint32_t>();
+    const GatEpilogue *epi = dst == ps.out ? ps.gat : nullptr;
     if (q)
         b4d_launch_normalise_q16(numq, gmap, fallback, reinterpret_cast<uint16_t *>(dst), pl.D, pl.H, pl.W, pl.nvol,
-                                 z0, z1, 1.0f / ps.mm.scale, ps.tab.kf, q->sub, q->add, q->step, q->trunc, s);
+                                 z0, z1, 1.0f / ps.mm.scale, ps.tab.kf, q->sub, q->add, q->step, q->trunc, epi, s);
     else
         b4d_launch_normalise_wm(numq, gmap, fallback, dst, pl.D, pl.H, pl.W, pl.nvol, z0, z1, 1.0f / ps.mm.scale,
-                                ps.tab.kf, s);
+                                ps.tab.kf, epi, s);
 }
 
 // Stage-1 front end of one uint16 volume in host memory: it is uploaded in z chunks on the copy stream and the
@@ -575,8 +581,9 @@ int stage1_streamed_front(Pass &ps, const uint16_t *host_src) {
 // Stage 1, hard thresholding: block energies and matching on the uint16 image, filter, normalise into the basic
 // estimate.  `host_src`: the uint16 volume is still in host memory and is uploaded here (can_stream_upload
 // holds).  `fuse_match`: the normalise also writes the stage-2 matching image rint(basic * scale) + shift, so that
-// the separate conversion pass (4 B read + 2 B write per voxel) is not needed.
-int stage1(Pass &ps, const uint16_t *host_src, bool fuse_match) {
+// the separate conversion pass (4 B read + 2 B write per voxel) is not needed.  `q`: profile.stages = 1, the basic
+// estimate is the result and is quantized.
+int stage1(Pass &ps, const uint16_t *host_src, bool fuse_match, const QuantSpec *q = nullptr) {
     b4d_handle *h = ps.h;
     const Plan &pl = *ps.pl;
     const b4d_profile &p = h->prof;
@@ -598,7 +605,7 @@ int stage1(Pass &ps, const uint16_t *host_src, bool fuse_match) {
                                    ps.mm.scale, ps.mm.ishift, pl.D, pl.H, pl.W, pl.nvol, 1.0f / ps.mm.scale,
                                    ps.tab.kf, s);
     else
-        normalise(ps, ps.zf, ps.basic, 0, pl.D, nullptr, s);
+        normalise(ps, ps.zf, ps.basic, 0, pl.D, q, s);
     clk.mark(B4D_T_NORM1);
     CU_TRY(cudaGetLastError());
     return 0;
@@ -743,7 +750,7 @@ int stage2_back(Pass &ps, HostSink *sink, const QuantSpec *q) {
 // Both stages of one pass (stage 1 alone when profile.stages = 1).
 int denoise_pass(Pass &ps, const uint16_t *host_src, HostSink *sink, const QuantSpec *q) {
     const bool two = ps.h->prof.stages == 2;
-    B4D_TRY(stage1(ps, host_src, two));
+    B4D_TRY(stage1(ps, host_src, two, two ? nullptr : q));
     if (!two) return 0;
     B4D_TRY(stage2_front_whole(ps, true));
     return stage2_back(ps, sink, q);
@@ -950,62 +957,157 @@ int gat_params(const b4d_pg_model *m, GatParams *p) {
     return 0;
 }
 
-// Batched denoise of uint16 counts through the GAT: forward into the float32 scratch, the float32 pipeline of
-// denoise_batch on it, then the inverse into `out` (float32, or uint16 through K7 with `q`).  Chunked like
-// denoise_batch, with the same scratch.
-int denoise_vst(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3], const b4d_pg_model *model,
-                float sigma, void *out, const QuantSpec *q, int in_dev, int out_dev) {
+// A VST pass's value set as the caller gives it (DESIGN §3.12, map rule): the camera model, the counts of every uint16
+// value of the whole volume (host, 65536 x int64; only > 0 matters) and the volume's first voxel.  hist == nullptr:
+// the pass's own input is the whole volume (or batch chunk) and provides both.
+struct VstInput {
     GatParams gp;
-    B4D_TRY(gat_params(model, &gp));
+    const int64_t *hist = nullptr;
+    int first = 0;
+};
+int vst_input(const b4d_pg_model *model, const int64_t *hist, int first, VstInput *v) {
+    B4D_TRY(gat_params(model, &v->gp));
+    if (!hist) return fail(B4D_ERR_INVALID, "NULL value_hist");
+    if (first < 0 || first > 65535) return fail(B4D_ERR_INVALID, "first_value must be in [0, 65535]");
+    for (int u = 0; u < 65536; ++u)
+        if (hist[u] < 0) return fail(B4D_ERR_INVALID, "negative count in value_hist");
+    if (hist[first] == 0) return fail(B4D_ERR_INVALID, "first_value has a count of 0 in value_hist");
+    v->hist = hist;
+    v->first = first;
+    return 0;
+}
+
+// Layout of h->vst: the value table, the value list, the absent flag, the value codes.
+constexpr size_t VST_LIST = 65536, VST_FLAG = VST_LIST + 65537, VST_CODES_BYTES = (VST_FLAG + 1) * sizeof(float);
+constexpr size_t VST_BYTES = VST_CODES_BYTES + 65537 * sizeof(uint16_t);
+
+// DESIGN §3.12, map rule: the matching map *mm and the centring c0 of a VST pass are what derive_match_map and the
+// centring of prepare_f32 yield on the short list [f(first), f(u) for every u present], GAT-forwarded on the device.
+// Every statistic derive_match_map reduces is a min or a max, and c = rint(z0) - z0 comes from the first value, so
+// this equals the derivation on the data itself.  Then the fused forward of the n voxels at `src`: data f(u) - c0 into
+// h->in, matching image into h->u16 (src may be h->u16), the absent flag set by a value outside the set.
+int vst_front(b4d_handle *h, const uint16_t *src, long long n, const int64_t *hist, int first, const GatParams &gp,
+              float sigma, MatchMap *mm, float *centre) {
+    cudaStream_t s = h->stream;
+    std::vector<uint16_t> vals{(uint16_t)first};
+    for (int u = 0; u < 65536; ++u)
+        if (hist[u] > 0) vals.push_back((uint16_t)u);
+    const int m = (int)vals.size();
+    B4D_TRY(h->vst.ensure(VST_BYTES));
+    float *table = h->vst.as<float>(), *list = table + VST_LIST;
+    unsigned *absent = h->vst.as<unsigned>() + VST_FLAG;
+    uint16_t *codes = reinterpret_cast<uint16_t *>(h->vst.as<char>() + VST_CODES_BYTES);
+    CU_TRY(cudaMemcpyAsync(codes, vals.data(), (size_t)m * sizeof(uint16_t), cudaMemcpyHostToDevice, s));
+    CU_TRY(cudaMemsetAsync(table, 0xFF, VST_LIST * sizeof(float), s));  // NaN: not in the value set
+    CU_TRY(cudaMemsetAsync(absent, 0, sizeof(unsigned), s));
+    b4d_launch_gat_values(codes, m, gp, list, table, s);
+    B4D_TRY(derive_match_map(h, list, m, sigma, mm, centre));  // synchronises: `vals` may go
+    if (*centre != 0.0f) {  // the list and the table hold z - c0, as prepare_f32's staged copy would
+        b4d_launch_add_scalar(list, m, -*centre, s);
+        b4d_launch_add_scalar(table, (long long)VST_LIST, -*centre, s);
+        B4D_TRY(derive_match_map(h, list, m, sigma, mm));
+    }
+    b4d_launch_gat_forward_map(src, table, h->in.as<float>(), h->u16.as<uint16_t>(), n, mm->cf, mm->scale, mm->ishift,
+                               absent, s);
+    CU_TRY(cudaGetLastError());
+    return 0;
+}
+// After the pass has finished: B4D_ERR_INVALID when the input held a value outside the value set it was given.
+int vst_check_absent(b4d_handle *h) {
+    unsigned absent = 0;
+    CU_TRY(cudaMemcpy(&absent, h->vst.as<unsigned>() + VST_FLAG, sizeof(absent), cudaMemcpyDeviceToHost));
+    if (absent) return fail(B4D_ERR_INVALID, "the input holds a value whose count in value_hist is 0");
+    return 0;
+}
+
+// Counts of every uint16 value of n voxels on the device, added to the histogram in h->hist (zeroed by the caller).
+void count_values(b4d_handle *h, const uint16_t *d_src, long long n) {
+    b4d_launch_hist(d_src, n, h->hist.as<unsigned long long>(), h->stream);
+}
+int zero_value_hist(b4d_handle *h) {
+    B4D_TRY(h->hist.ensure(65536 * sizeof(unsigned long long)));
+    CU_TRY(cudaMemsetAsync(h->hist.p, 0, 65536 * sizeof(unsigned long long), h->stream));
+    return 0;
+}
+// h->hist to the host, and the first voxel of the volume from `d_first` unless that is null (synchronises the stream)
+int read_value_hist(b4d_handle *h, const uint16_t *d_first, std::vector<int64_t> *hist, int *first) {
+    hist->resize(65536);
+    uint16_t f = 0;
+    CU_TRY(cudaMemcpyAsync(hist->data(), h->hist.p, 65536 * sizeof(int64_t), cudaMemcpyDeviceToHost, h->stream));
+    if (d_first) CU_TRY(cudaMemcpyAsync(&f, d_first, sizeof(f), cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(cudaStreamSynchronize(h->stream));
+    *first = f;
+    return 0;
+}
+
+// The input of one VST pass (n voxels of uint16 counts, host or device): staged in h->u16 when on the host, value set
+// (the input's own when v.hist is null), map, fused forward; *epi receives the inverse the pass ends in.
+int stage_vst_input(b4d_handle *h, const uint16_t *in, long long n, int in_on_device, const VstInput &v, float sigma,
+                    StageClock &clk, MatchMap *mm, GatEpilogue *epi) {
+    B4D_TRY(h->in.ensure((size_t)n * sizeof(float)));
+    B4D_TRY(h->u16.ensure((size_t)n * sizeof(uint16_t) + 16));
+    B4D_TRY(h->out.ensure((size_t)n * sizeof(float)));
+    const uint16_t *src = in;
+    if (!in_on_device) {
+        CU_TRY(copy_in(h, h->u16.p, in, (size_t)n * sizeof(uint16_t), 0, h->stream));
+        src = h->u16.as<uint16_t>();
+    }
+    clk.mark(-1);
+    std::vector<int64_t> own;
+    const int64_t *hist = v.hist;
+    int first = v.first;
+    if (!hist) {
+        B4D_TRY(zero_value_hist(h));
+        count_values(h, src, n);
+        B4D_TRY(read_value_hist(h, src, &own, &first));
+        hist = own.data();
+    }
+    epi->p = v.gp;
+    B4D_TRY(vst_front(h, src, n, hist, first, v.gp, sigma, mm, &epi->centre));
+    clk.mark(B4D_T_PREP);
+    return 0;
+}
+
+// The argument checks of b4d_denoise_vst_u16 / _q16_u16, before any device work; *gp receives the model.
+int vst_checks(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3], const b4d_pg_model *model,
+               float sigma, const void *out, const QuantSpec *q, GatParams *gp) {
+    B4D_TRY(gat_params(model, gp));
     if (q && !(q->step >= 1.0f)) return fail(B4D_ERR_INVALID, "step must be >= 1");
     B4D_TRY(common_checks(h, in, out, shape, sigma));
     if (n < 1) return fail(B4D_ERR_INVALID, "n must be >= 1");
-    B4D_TRY(reset_last(h));
+    return 0;
+}
+// Batched denoise of uint16 counts through the GAT (DESIGN §3.12), chunked like denoise_batch: per chunk its value
+// set, the map from the value list, the fused forward into the float32 data and the matching image, the float32
+// pipeline, and the inverse (and K7 with `q`) in the last normalise.  After vst_checks; each volume fits a pass.
+int denoise_vst(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3], const GatParams &gp,
+                float sigma, void *out, const QuantSpec *q, int in_dev, int out_dev) {
+    VstInput v;
+    v.gp = gp;
     const long long V = shape[0] * shape[1] * shape[2];
+    B4D_TRY(reset_last(h));
     const int64_t per = std::max<int64_t>(1, std::min<int64_t>(n, h->pass_voxels / V));
     const size_t osz = q ? sizeof(uint16_t) : sizeof(float);
-    cudaStream_t s = h->stream;
     Plan pl = make_plan(shape, 0, shape[0], 1, h->prof);
     StageClock clk(h);
-    const int norm_slot = h->prof.stages == 2 ? B4D_T_NORM2 : B4D_T_NORM1;
     for (int64_t i0 = 0; i0 < n; i0 += per) {
         const int64_t nb = std::min<int64_t>(per, n - i0);
         const long long TV = V * nb;
         pl.nvol = (int)nb;
-        B4D_TRY(h->in.ensure((size_t)TV * sizeof(float)));
-        B4D_TRY(h->u16.ensure((size_t)TV * sizeof(uint16_t) + 16));
-        B4D_TRY(h->out.ensure((size_t)TV * sizeof(float)));
-        char *user_out = static_cast<char *>(out) + (size_t)i0 * V * osz;
-        // the float32 result: in place in a device output of float32 when it is 16-byte aligned
-        float *d_res = h->out.as<float>();
-        if (!q && out_dev && (reinterpret_cast<uintptr_t>(user_out) & 15) == 0) d_res = reinterpret_cast<float *>(user_out);
-        // host input is staged in h->u16, which to_match overwrites with the matching image after the forward
-        const uint16_t *src = in + i0 * V;
-        if (!in_dev) {
-            CU_TRY(copy_in(h, h->u16.p, src, (size_t)TV * sizeof(uint16_t), 0, s));
-            src = h->u16.as<uint16_t>();
-        }
-        clk.mark(-1);
-        b4d_launch_gat_forward(src, h->in.as<float>(), TV, gp, s);
         MatchMap mm;
-        float centre = 0.0f;
-        B4D_TRY(prepare_f32(h, TV, sigma, &mm, &centre));
-        clk.mark(B4D_T_PREP);
-        HostSink sink{nullptr, 0, pl.D};
+        GatEpilogue epi;
+        B4D_TRY(stage_vst_input(h, in + i0 * V, TV, in_dev, v, sigma, clk, &mm, &epi));
+        char *user_out = static_cast<char *>(out) + (size_t)i0 * V * osz;
+        // the result in place in a device output (float32 only when 16-byte aligned), else in h->out
+        void *d_res = h->out.p;
+        if (out_dev && (q || (reinterpret_cast<uintptr_t>(user_out) & 15) == 0)) d_res = user_out;
+        HostSink sink{out_dev || nb > 1 ? nullptr : user_out, 0, pl.D};
         Pass ps;
-        B4D_TRY(make_pass(h, pl, sigma, mm, h->in.as<float>(), h->u16.as<uint16_t>(), d_res, clk, ps));
-        B4D_TRY(denoise_pass(ps, nullptr, &sink, nullptr));
-        if (centre != 0.0f) b4d_launch_add_scalar(d_res, TV, centre, s);
-        clk.mark(-1);
-        // inverse: in place, or K7 into uint16 (the user's device buffer, else h->u16: the pass is done with it)
-        uint16_t *d_q = nullptr;
-        if (q) d_q = out_dev ? reinterpret_cast<uint16_t *>(user_out) : h->u16.as<uint16_t>();
-        b4d_launch_gat_inverse(d_res, d_res, d_q, TV, gp, q ? q->sub : 0.f, q ? q->add : 0.f, q ? q->step : 1.f,
-                               q ? q->trunc : 0, s);
-        CU_TRY(cudaGetLastError());
-        clk.mark(norm_slot);
-        const void *d_final = q ? static_cast<const void *>(d_q) : static_cast<const void *>(d_res);
-        if (d_final != user_out) CU_TRY(copy_out(h, user_out, d_final, (size_t)TV * osz, out_dev, s));
+        B4D_TRY(make_pass(h, pl, sigma, mm, h->in.as<float>(), h->u16.as<uint16_t>(), static_cast<float *>(d_res), clk,
+                          ps));
+        ps.gat = &epi;
+        B4D_TRY(denoise_pass(ps, nullptr, &sink, q));
+        if (!sink.done && d_res != user_out) CU_TRY(copy_out(h, user_out, d_res, (size_t)TV * osz, out_dev, h->stream));
         B4D_TRY(finish(h, clk));
     }
     return 0;
@@ -1019,6 +1121,12 @@ int check_open_slab(const b4d_handle *h, int64_t own_begin, int64_t own_end) {
     return 0;
 }
 int make_slab_pass(b4d_handle *h, StageClock &clk, Pass &ps) {
+    if (h->slab_vst) {
+        B4D_TRY(make_pass(h, h->slab, h->slab_sigma, h->slab_mm, h->in.as<float>(), h->u16.as<uint16_t>(),
+                          h->out.as<float>(), clk, ps));
+        ps.gat = &h->slab_gat;
+        return 0;
+    }
     return make_pass(h, h->slab, h->slab_sigma, h->slab_mm, h->zf.as<float>(), h->in.as<uint16_t>(),
                      h->out.as<float>(), clk, ps);
 }
@@ -1076,7 +1184,7 @@ void b4d_destroy(b4d_handle *h) {
     for (DevBuf *b : {&h->in, &h->u16, &h->zf, &h->numq, &h->gmap, &h->basic, &h->out, &h->widx, &h->cnt,
                       &h->ssd, &h->refs, &h->hist, &h->partial, &h->sink, &h->stats, &h->s2, &h->cells, &h->tcls,
                       &h->alt_in, &h->alt_zf, &h->alt_out, &h->alt_partial, &h->alt_sink, &h->nz_hist, &h->nz_sel,
-                      &h->nz_res, &h->nz_full})
+                      &h->nz_res, &h->nz_full, &h->vst})
         b->release();
     if (h->stream) cudaStreamDestroy(h->stream);
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
@@ -1109,9 +1217,10 @@ int b4d_set_pass_voxels(b4d_handle *h, int64_t voxels) {
 }
 
 // One slab, after common_checks and reset_last: its stages add to the timings and match statistics of the call.
+// `vst`: a VST slab with the whole volume's value set.
 static int denoise_slab_impl(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
                              int64_t z_total, int64_t own_begin, int64_t own_end, float sigma, void *out,
-                             int in_on_device, int out_on_device, const QuantSpec *q) {
+                             int in_on_device, int out_on_device, const QuantSpec *q, const VstInput *vst = nullptr) {
     if (q && h->prof.stages != 2) return fail(B4D_ERR_INVALID, "quantized output needs stages = 2");
     if (q && !(q->step >= 1.0f)) return fail(B4D_ERR_INVALID, "step must be >= 1");
     const size_t esz = q ? sizeof(uint16_t) : sizeof(float);
@@ -1122,23 +1231,32 @@ static int denoise_slab_impl(b4d_handle *h, const uint16_t *in, const int64_t sh
     const Plan pl = make_plan(shape, z_begin, z_total, 1, h->prof);
     StageClock clk(h);
     MatchMap mm;
+    GatEpilogue epi;
     const uint16_t *host_src = nullptr;
-    B4D_TRY(stage_u16_input(h, pl, in, in_on_device, clk, &mm, &host_src));
+    if (vst)
+        B4D_TRY(stage_vst_input(h, in, shape[0] * P, in_on_device, *vst, sigma, clk, &mm, &epi));
+    else
+        B4D_TRY(stage_u16_input(h, pl, in, in_on_device, clk, &mm, &host_src));
     HostSink sink{out_on_device ? nullptr : out, own_begin - z_begin, own_end - z_begin};
     Pass ps;
-    B4D_TRY(make_pass(h, pl, sigma, mm, h->zf.as<float>(), h->in.as<uint16_t>(), h->out.as<float>(), clk, ps));
+    B4D_TRY(make_pass(h, pl, sigma, mm, vst ? h->in.as<float>() : h->zf.as<float>(),
+                      vst ? h->u16.as<uint16_t>() : h->in.as<uint16_t>(), h->out.as<float>(), clk, ps));
+    if (vst) ps.gat = &epi;
     B4D_TRY(denoise_pass(ps, host_src, &sink, q));
     if (!sink.done)
         CU_TRY(copy_out(h, out, h->out.as<char>() + (size_t)sink.p0 * P * esz, (size_t)(sink.p1 - sink.p0) * P * esz,
                         out_on_device, h->stream));
-    return finish(h, clk);
+    B4D_TRY(finish(h, clk));
+    return vst ? vst_check_absent(h) : 0;
 }
 
 // `n` uint16 volumes, each larger than a pass: z-slabs with the no-exchange halo, one after the other on this
 // GPU (as b4d_denoise_slab_u16); equal to the one-pass result bit for bit, like the multi-GPU slabs.  The timings
-// and match statistics cover all slabs.
-static int denoise_oversize_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3], float sigma,
-                                float *out, int in_on_device, int out_on_device) {
+// and match statistics cover all slabs.  `gp`: through the GAT (b4d_denoise_vst_u16); a pass first takes the value
+// set of the whole volume (host input uploaded in pass-sized pieces and discarded after counting), and every slab
+// uses it.  `out`: float32, or uint16 with `q`.
+static int denoise_oversize(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3], float sigma,
+                            void *out, int in_on_device, int out_on_device, const QuantSpec *q, const GatParams *gp) {
     const int64_t D = shape[0], P = shape[1] * shape[2], V = D * P;
     const int64_t halo = (h->prof.search_ht + 2) + (h->prof.stages == 2 ? h->prof.search_wie + 2 : 0);
     const int64_t planes = h->pass_voxels / P;
@@ -1147,14 +1265,42 @@ static int denoise_oversize_u16(b4d_handle *h, const uint16_t *in, int64_t n, co
                                        "or shard the volume in y / x");
     const int64_t nslab = (D + (planes - 2 * halo) - 1) / (planes - 2 * halo);
     const int64_t own = (D + nslab - 1) / nslab;
+    const size_t esz = q ? sizeof(uint16_t) : sizeof(float);
     B4D_TRY(reset_last(h));
-    for (int64_t i = 0; i < n; ++i)
+    for (int64_t i = 0; i < n; ++i) {
+        const uint16_t *vin = in + i * V;
+        VstInput v;
+        std::vector<int64_t> hist;
+        if (gp) {
+            StageClock clk(h);
+            clk.mark(-1);
+            B4D_TRY(zero_value_hist(h));
+            if (in_on_device) {
+                count_values(h, vin, V);
+            } else {
+                const long long piece = std::min<long long>(V, h->pass_voxels);
+                B4D_TRY(h->u16.ensure((size_t)piece * sizeof(uint16_t) + 16));
+                for (long long p0 = 0; p0 < V; p0 += piece) {  // the stream orders each upload after the last count
+                    const long long np = std::min(piece, V - p0);
+                    CU_TRY(copy_in(h, h->u16.p, vin + p0, (size_t)np * sizeof(uint16_t), 0, h->stream));
+                    count_values(h, h->u16.as<uint16_t>(), np);
+                }
+            }
+            clk.mark(B4D_T_PREP);
+            B4D_TRY(read_value_hist(h, in_on_device ? vin : nullptr, &hist, &v.first));
+            if (!in_on_device) v.first = vin[0];
+            clk.resolve();
+            v.gp = *gp;
+            v.hist = hist.data();
+        }
         for (int64_t ob = 0; ob < D; ob += own) {
             const int64_t oe = std::min(D, ob + own), zb = std::max<int64_t>(0, ob - halo), ze = std::min(D, oe + halo);
             const int64_t sshape[3] = {ze - zb, shape[1], shape[2]};
-            B4D_TRY(denoise_slab_impl(h, in + i * V + zb * P, sshape, zb, D, ob, oe, sigma, out + i * V + ob * P,
-                                      in_on_device, out_on_device, nullptr));
+            B4D_TRY(denoise_slab_impl(h, vin + zb * P, sshape, zb, D, ob, oe, sigma,
+                                      static_cast<char *>(out) + (size_t)(i * V + ob * P) * esz, in_on_device,
+                                      out_on_device, q, gp ? &v : nullptr));
         }
+    }
     return 0;
 }
 
@@ -1163,7 +1309,7 @@ int b4d_denoise_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t 
     if (h && in && out && shape && n >= 1 && shape[0] > 0 && shape[1] > 0 && shape[2] > 0 &&
         shape[0] * shape[1] * shape[2] > h->pass_voxels) {
         B4D_TRY(common_checks(h, in, out, shape, sigma));
-        return denoise_oversize_u16(h, in, n, shape, sigma, out, in_on_device, out_on_device);
+        return denoise_oversize(h, in, n, shape, sigma, out, in_on_device, out_on_device, nullptr, nullptr);
     }
     return denoise_batch<uint16_t>(h, in, n, shape, sigma, out, in_on_device, out_on_device);
 }
@@ -1280,8 +1426,9 @@ int b4d_denoise_q16_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3
                                     truncate, out, in_on_device, out_on_device);
 }
 
-int b4d_slab_stage1_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin, int64_t z_total,
-                        float sigma, int in_on_device) {
+// Part 1 of the two-call slab form: stage 1 of the slab, left open on the handle (`vst`: a VST slab).
+static int slab_stage1_impl(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
+                            int64_t z_total, float sigma, int in_on_device, const VstInput *vst) {
     B4D_TRY(common_checks(h, in, in, shape, sigma));
     if (z_begin < 0 || z_begin + shape[0] > z_total) return fail(B4D_ERR_INVALID, "slab range inconsistent");
     if (h->prof.stages != 2) return fail(B4D_ERR_INVALID, "the two-call slab form needs stages = 2");
@@ -1291,19 +1438,29 @@ int b4d_slab_stage1_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3
     h->slab = make_plan(shape, z_begin, z_total, 1, h->prof);
     h->slab_z_begin = z_begin;
     h->slab_sigma = sigma;
+    h->slab_vst = vst != nullptr;
+    h->slab_mm = MatchMap();
     StageClock clk(h);
-    MatchMap mm;
     const uint16_t *host_src = nullptr;
-    B4D_TRY(stage_u16_input(h, h->slab, in, in_on_device, clk, &mm, &host_src));
+    if (vst)
+        B4D_TRY(stage_vst_input(h, in, shape[0] * shape[1] * shape[2], in_on_device, *vst, sigma, clk, &h->slab_mm,
+                                &h->slab_gat));
+    else
+        B4D_TRY(stage_u16_input(h, h->slab, in, in_on_device, clk, &h->slab_mm, &host_src));
     Pass ps;
-    B4D_TRY(make_pass(h, h->slab, sigma, mm, h->zf.as<float>(), h->in.as<uint16_t>(), h->out.as<float>(), clk, ps));
+    B4D_TRY(make_slab_pass(h, clk, ps));
     B4D_TRY(stage1(ps, host_src, false));
     CU_TRY(cudaStreamSynchronize(h->stream));
     clk.resolve();
+    if (vst) B4D_TRY(vst_check_absent(h));
     h->pre.done = false;
     h->slab_mm = ps.mm;
     h->slab_open = true;
     return 0;
+}
+int b4d_slab_stage1_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin, int64_t z_total,
+                        float sigma, int in_on_device) {
+    return slab_stage1_impl(h, in, shape, z_begin, z_total, sigma, in_on_device, nullptr);
 }
 
 int b4d_slab_basic_planes(b4d_handle *h, int64_t plane0, int64_t nplanes, float *buf, int to_handle,
@@ -1988,9 +2145,20 @@ int b4d_gat_inverse_f32(b4d_handle *h, const b4d_pg_model *model, const float *i
     return 0;
 }
 
+// One volume larger than a pass goes through denoise_oversize: the value set of the whole volume, then z-slabs.
+static int denoise_vst_any(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3],
+                           const b4d_pg_model *model, float sigma, void *out, const QuantSpec *q, int in_on_device,
+                           int out_on_device) {
+    GatParams gp;
+    B4D_TRY(vst_checks(h, in, n, shape, model, sigma, out, q, &gp));
+    if (shape[0] * shape[1] * shape[2] > h->pass_voxels)
+        return denoise_oversize(h, in, n, shape, sigma, out, in_on_device, out_on_device, q, &gp);
+    return denoise_vst(h, in, n, shape, gp, sigma, out, q, in_on_device, out_on_device);
+}
+
 int b4d_denoise_vst_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3],
                         const b4d_pg_model *model, float sigma_vst, float *out, int in_on_device, int out_on_device) {
-    return denoise_vst(h, in, n, shape, model, sigma_vst, out, nullptr, in_on_device, out_on_device);
+    return denoise_vst_any(h, in, n, shape, model, sigma_vst, out, nullptr, in_on_device, out_on_device);
 }
 
 int b4d_denoise_vst_q16_u16(b4d_handle *h, const uint16_t *in, int64_t n, const int64_t shape[3],
@@ -2001,7 +2169,40 @@ int b4d_denoise_vst_q16_u16(b4d_handle *h, const uint16_t *in, int64_t n, const 
     q.add = offset_add;
     q.step = step;
     q.trunc = truncate ? 1 : 0;
-    return denoise_vst(h, in, n, shape, model, sigma_vst, out, &q, in_on_device, out_on_device);
+    return denoise_vst_any(h, in, n, shape, model, sigma_vst, out, &q, in_on_device, out_on_device);
+}
+
+// include/b4d_vst_slab.h: the slab forms of the VST path, with the whole volume's value set (DESIGN §3.12)
+int b4d_denoise_slab_vst_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
+                             int64_t z_total, int64_t own_begin, int64_t own_end, const b4d_pg_model *model,
+                             float sigma_vst, const int64_t *value_hist, int first_value, float *out, int in_on_device,
+                             int out_on_device) {
+    VstInput v;
+    B4D_TRY(vst_input(model, value_hist, first_value, &v));
+    B4D_TRY(common_checks(h, in, out, shape, sigma_vst));
+    B4D_TRY(reset_last(h));
+    return denoise_slab_impl(h, in, shape, z_begin, z_total, own_begin, own_end, sigma_vst, out, in_on_device,
+                             out_on_device, nullptr, &v);
+}
+int b4d_denoise_slab_vst_q16_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
+                                 int64_t z_total, int64_t own_begin, int64_t own_end, const b4d_pg_model *model,
+                                 float sigma_vst, const int64_t *value_hist, int first_value, float offset_sub,
+                                 float offset_add, float step, int truncate, uint16_t *out, int in_on_device,
+                                 int out_on_device) {
+    VstInput v;
+    B4D_TRY(vst_input(model, value_hist, first_value, &v));
+    B4D_TRY(common_checks(h, in, out, shape, sigma_vst));
+    B4D_TRY(reset_last(h));
+    const QuantSpec q{offset_sub, offset_add, step, truncate ? 1 : 0};
+    return denoise_slab_impl(h, in, shape, z_begin, z_total, own_begin, own_end, sigma_vst, out, in_on_device,
+                             out_on_device, &q, &v);
+}
+int b4d_slab_stage1_vst_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
+                            int64_t z_total, const b4d_pg_model *model, float sigma_vst, const int64_t *value_hist,
+                            int first_value, int in_on_device) {
+    VstInput v;
+    B4D_TRY(vst_input(model, value_hist, first_value, &v));
+    return slab_stage1_impl(h, in, shape, z_begin, z_total, sigma_vst, in_on_device, &v);
 }
 
 int b4d_last_timings(b4d_handle *h, float ms[B4D_T_COUNT], int64_t launches[B4D_T_COUNT]) {

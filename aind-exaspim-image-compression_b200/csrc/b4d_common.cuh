@@ -121,16 +121,19 @@ void b4d_launch_normalise_match(const long long *numq, const uint32_t *gmap, con
                                 uint16_t *match, float mscale, int ishift, int D, int H, int W, int nvol,
                                 float inv_qscale, const float kf[4], cudaStream_t s);
 // weight-map contract: den = G (*) (kf x kf x kf) over planes [z0, z1) of every volume, out = num / den / qscale
+// (with `epi`: the GAT inverse of that, see GatEpilogue)
+struct GatEpilogue;
 void b4d_launch_normalise_wm(const long long *numq, const uint32_t *gmap, const float *fallback, float *out, int D,
                              int H, int W, int nvol, int z0, int z1, float inv_qscale, const float kf[4],
-                             cudaStream_t s);
+                             const GatEpilogue *epi, cudaStream_t s);
 void b4d_launch_quantize(const float *in, uint16_t *out, long long n, float offset_sub, float offset_add,
                          float step, cudaStream_t s);
 void b4d_launch_quantize_trunc(const float *in, uint16_t *out, long long n, float offset_sub, float offset_add,
                                float step, cudaStream_t s);
 void b4d_launch_normalise_q16(const long long *numq, const uint32_t *gmap, const float *fallback, uint16_t *q16, int D,
                               int H, int W, int nvol, int z0, int z1, float inv_qscale, const float kf[4],
-                              float offset_sub, float offset_add, float step, int trunc, cudaStream_t s);
+                              float offset_sub, float offset_add, float step, int trunc, const GatEpilogue *epi,
+                              cudaStream_t s);
 void b4d_launch_hist(const uint16_t *in, long long n, unsigned long long *hist, cudaStream_t s);
 // make_foreground_mask after the statistic: threshold + L1-ball dilation, per patch thr / off
 void b4d_launch_fg_mask(const uint16_t *in, const float *off, const float *thr, int D, int H, int W, long long n,
@@ -184,6 +187,18 @@ void b4d_launch_gat_forward(const uint16_t *in, float *out, long long n, const G
 // float32 result into `out`, or (q16 non-null) K7 of it into q16
 void b4d_launch_gat_inverse(const float *in, float *out, uint16_t *q16, long long n, const GatParams &p,
                             float offset_sub, float offset_add, float step, int trunc, cudaStream_t s);
+// The value set of a VST pass (DESIGN §3.12, map rule): list[i] = forward(vals[i]) for the m values, and the same
+// value in table[vals[i]] (table: 65536 floats, NaN where no value was written).
+void b4d_launch_gat_values(const uint16_t *vals, int m, const GatParams &p, float *list, float *table, cudaStream_t s);
+// Forward with a known map: zf[i] = table[in[i]], match[i] = to_match(zf[i], cf, scale, ishift); *absent |= 1 when
+// a value's entry is NaN (not in the value set).  `match` may be `in` (in place).
+void b4d_launch_gat_forward_map(const uint16_t *in, const float *table, float *zf, uint16_t *match, long long n,
+                                float cf, float scale, int ishift, unsigned *absent, cudaStream_t s);
+// Epilogue of the last normalise of a VST pass: y = gat_inverse1(y + centre) (the add only when centre != 0).
+struct GatEpilogue {
+    GatParams p;
+    float centre;
+};
 
 // K7: q = rint(clip((x - offset_sub + offset_add) / step, 0, 65535/step)).
 // float32, clip BEFORE round, round-half-to-even: transforms.py:403-411.
@@ -205,6 +220,25 @@ __device__ __forceinline__ uint32_t quant1_trunc(float x, float osub, float oadd
 template <bool TRUNC>
 __device__ __forceinline__ uint32_t quantq(float x, float osub, float oadd, float step, float hi, bool unit) {
     return TRUNC ? quant1_trunc(x, osub, oadd, step, hi, unit) : quant1(x, osub, oadd, step, hi, unit);
+}
+// GAT inverse of one value (DESIGN §3.12): float64, every operation in the order of the contract (-fmad=false)
+__device__ __forceinline__ float gat_inverse1(float D, const GatParams &p) {
+    const double d = (double)D;
+    double lam = 0.0;
+    if (!(d <= p.s15)) {  // P(sqrt(1.5)) = 0: the floor below is continuous; NaN takes this branch and gives 0
+        const double r = 1.0 / d;
+        const double P = 0.25 * d * d + p.c1 * r - 1.375 * r * r + p.c2 * r * r * r - 0.125;
+        const double l = P - p.qq;
+        lam = l > 0.0 ? l : 0.0;
+    }
+    return (float)(p.gain * lam + p.offset);
+}
+// Matching image: u = clamp(int(rint((v + cf) * scale)) + ishift, 0, 65535): the integer shift is applied after
+// rounding so that rounding never depends on it.
+__device__ __forceinline__ uint32_t to_match(float v, float cf, float scale, int ishift) {
+    long long q = (long long)__float2ll_rn((v + cf) * scale) + ishift;
+    q = min(max(q, 0ll), 65535ll);
+    return (uint32_t)q;
 }
 // coherence gate (b4d_coherence.cu): 23 sums per (patch, label slot), see there
 void b4d_launch_coherence(const float *raw, const unsigned long long *labels, int D, int H, int W, long long npatch,

@@ -70,13 +70,7 @@ __global__ void __launch_bounds__(256) k_u16_to_f32(const uint16_t *__restrict__
 }
 
 // ---------------------------------------------- f32 -> matching image (u16) --
-// u = clamp(int(rint((v + cf) * scale)) + ishift, 0, 65535): the integer shift is
-// applied after rounding so that rounding never depends on it.
-__device__ __forceinline__ uint32_t to_match(float v, float cf, float scale, int ishift) {
-    long long q = (long long)__float2ll_rn((v + cf) * scale) + ishift;
-    q = min(max(q, 0ll), 65535ll);
-    return (uint32_t)q;
-}
+// (to_match: b4d_common.cuh, shared with the fused GAT forward of b4d_vst.cu)
 __global__ void __launch_bounds__(256) k_to_match(const float *__restrict__ in, uint16_t *__restrict__ out,
                                                   long long n, float shift, float scale, int ishift) {
     const long long nv = n >> 3;
@@ -174,11 +168,21 @@ struct NormOut {
     int ishift;
     float q_sub, q_add, q_step, q_hi;
     int q_unit, q_trunc;
+    GatEpilogue gat;     // VST instantiations: y = gat_inverse1(y + centre) before the outputs
 };
+// The result of one voxel as the outputs take it: y itself, or in a VST pass its GAT inverse (bit-identical to a
+// separate k_add_scalar + k_gat_inverse on the stored y: the same float32 add and float64 operations).
+template <bool VST>
+__device__ __forceinline__ float norm_epilogue(float y, const NormOut &o) {
+    if (!VST) return y;
+    if (o.gat.centre != 0.0f) y = __fadd_rn(y, o.gat.centre);
+    return gat_inverse1(y, o.gat.p);
+}
 // One WARP owns an 8 x 29 (y, x) tile and marches along z over WM_NZ planes (+3 planes of run-in); no shared memory,
 // no barrier.  Lane i holds column X0 - 3 + i of the uint32 map for the 11 rows Y0 - 3 .. Y0 + 7 (lanes 0-2 are the
 // x halo); the x pass takes the three left neighbours by warp shuffles of the uint32 values, the y pass runs on the
 // 11 x-convolved rows in registers, the z pass on a rolling window of three earlier xy-convolved values per row.
+template <bool VST>
 __global__ void __launch_bounds__(WM_WARPS * 32) k_normalise_wm(const long long *__restrict__ numq,
                                                                 const uint32_t *__restrict__ gmap,
                                                                 const float *__restrict__ fb, NormOut o, int D, int H,
@@ -246,7 +250,7 @@ __global__ void __launch_bounds__(WM_WARPS * 32) k_normalise_wm(const long long 
                 den = fma(k[2], h2[r], den);
                 den = fma(k[3], h3[r], den);
                 const long long a = a0 + (long long)r * W;
-                const float y = den > 0.0 ? (float)(((double)nq[r] / den) * inv) : fb[a];
+                const float y = norm_epilogue<VST>(den > 0.0 ? (float)(((double)nq[r] / den) * inv) : fb[a], o);
                 if (o.out) o.out[a] = y;
                 if (o.match) o.match[a] = (uint16_t)to_match(y, 0.0f, o.mscale, o.ishift);
                 if (o.q16)
@@ -271,6 +275,7 @@ constexpr uint32_t WMT_G_BYTES = WMT_GW * WM_EY * 4, WMT_N_BYTES = WMT_TX * WM_T
 constexpr int WMT_G_STAGE = ((int)WMT_G_BYTES + 127) / 128 * 128;
 constexpr int WMT_STAGE = WMT_G_STAGE + (int)WMT_N_BYTES;
 static_assert(WMT_TX % 4 == 0 && WMT_GW % 4 == 0 && WMT_GW >= WMT_TX + 4 && WMT_N_BYTES % 128 == 0, "TMA boxes of the normalise kernel");
+template <bool VST>
 __global__ void __launch_bounds__(WMT_WARPS * 32, 4) k_normalise_wm_tma(const __grid_constant__ CUtensorMap gmap_t,
                                                                        const __grid_constant__ CUtensorMap numq_t,
                                                                        const float *__restrict__ fb, NormOut o, int D, int H,
@@ -354,7 +359,7 @@ __global__ void __launch_bounds__(WMT_WARPS * 32, 4) k_normalise_wm_tma(const __
                 den = fma(k[2], h2[r], den);
                 den = fma(k[3], h3[r], den);
                 const long long a = a0 + (long long)r * W;
-                const float y = den > 0.0 ? (float)(((double)nq[r] / den) * inv) : fb[a];
+                const float y = norm_epilogue<VST>(den > 0.0 ? (float)(((double)nq[r] / den) * inv) : fb[a], o);
                 if (o.out) o.out[a] = y;
                 if (o.match) o.match[a] = (uint16_t)to_match(y, 0.0f, o.mscale, o.ishift);
                 if (o.q16)
@@ -369,7 +374,7 @@ __global__ void __launch_bounds__(WMT_WARPS * 32, 4) k_normalise_wm_tma(const __
 }
 
 // -------------------------------------------------------------- quantize ----
-// K7 (quant1, quant1_trunc: b4d_common.cuh, shared with the fused GAT inverse of b4d_vst.cu)
+// K7 (quant1, quant1_trunc: b4d_common.cuh, shared with b4d_gat_inverse_f32's kernel in b4d_vst.cu)
 template <bool TRUNC>
 __global__ void __launch_bounds__(256) k_quantize(const float *__restrict__ in, uint16_t *__restrict__ out,
                                                   long long n, float osub, float oadd, float step) {
@@ -738,39 +743,45 @@ void b4d_launch_to_match(const float *in, uint16_t *out, long long n, float cf, 
                          cudaStream_t s) {
     b4d_launch(k_to_match, grid_for(n >> 3, 256, 8), 256, 0, s, in, out, n, cf, scale, ishift);
 }
-static void launch_norm(const long long *numq, const uint32_t *gmap, const float *fallback, const NormOut &o, int D,
-                        int H, int W, int nvol, int z0, int z1, float inv_qscale, const float kf[4], cudaStream_t s) {
+static void launch_norm(const long long *numq, const uint32_t *gmap, const float *fallback, NormOut o, int D,
+                        int H, int W, int nvol, int z0, int z1, float inv_qscale, const float kf[4],
+                        const GatEpilogue *epi, cudaStream_t s) {
     if (z1 <= z0) return;
+    const int vst = epi ? 1 : 0;
+    if (epi) o.gat = *epi;
     const long long ntz = (z1 - z0 + WM_NZ - 1) / WM_NZ, nty = (H + WM_TY - 1) / WM_TY;
     CUtensorMap mg, mn;
     if ((W & 3) == 0 && !getenv("B4D_NO_TMA") &&
         make_map_4d(&mg, CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, gmap, W, H, D, nvol, WMT_GW, WM_EY, 1) &&
         make_map_4d(&mn, CU_TENSOR_MAP_DATA_TYPE_INT64, 8, numq, W, H, D, nvol, WMT_TX, WM_TY, 1)) {
-        static bool attr = false;
-        if (!attr) {
-            cudaFuncSetAttribute(k_normalise_wm_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, WMT_NST * WMT_STAGE);
-            attr = true;
+        auto kernel = vst ? k_normalise_wm_tma<true> : k_normalise_wm_tma<false>;
+        static bool attr[2] = {false, false};
+        if (!attr[vst]) {
+            cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WMT_NST * WMT_STAGE);
+            attr[vst] = true;
         }
         const long long blocks = (long long)nvol * ntz * nty * ((W + WMT_TX - 1) / WMT_TX);
-        b4d_launch(k_normalise_wm_tma, (unsigned)blocks, WMT_WARPS * 32, WMT_NST * WMT_STAGE, s, mg, mn, fallback, o,
-                   D, H, W, nvol, z0, z1, inv_qscale, kf[0], kf[1], kf[2], kf[3]);
+        b4d_launch(kernel, (unsigned)blocks, WMT_WARPS * 32, WMT_NST * WMT_STAGE, s, mg, mn, fallback, o, D, H, W,
+                   nvol, z0, z1, inv_qscale, kf[0], kf[1], kf[2], kf[3]);
         return;
     }
     const long long tiles = (long long)nvol * ntz * nty * ((W + WM_TX - 1) / WM_TX);
-    b4d_launch(k_normalise_wm, (unsigned)((tiles + WM_WARPS - 1) / WM_WARPS), WM_WARPS * 32, 0, s, numq, gmap,
-               fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf[0], kf[1], kf[2], kf[3]);
+    b4d_launch(vst ? k_normalise_wm<true> : k_normalise_wm<false>, (unsigned)((tiles + WM_WARPS - 1) / WM_WARPS),
+               WM_WARPS * 32, 0, s, numq, gmap, fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf[0], kf[1], kf[2],
+               kf[3]);
 }
 void b4d_launch_normalise_wm(const long long *numq, const uint32_t *gmap, const float *fallback, float *out, int D,
                              int H, int W, int nvol, int z0, int z1, float inv_qscale, const float kf[4],
-                             cudaStream_t s) {
+                             const GatEpilogue *epi, cudaStream_t s) {
     NormOut o{};
     o.out = out;
-    launch_norm(numq, gmap, fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf, s);
+    launch_norm(numq, gmap, fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf, epi, s);
 }
 // K6 + K7 fused: the quantized uint16 volume is written directly (float32 result never stored)
 void b4d_launch_normalise_q16(const long long *numq, const uint32_t *gmap, const float *fallback, uint16_t *q16, int D,
                               int H, int W, int nvol, int z0, int z1, float inv_qscale, const float kf[4],
-                              float offset_sub, float offset_add, float step, int trunc, cudaStream_t s) {
+                              float offset_sub, float offset_add, float step, int trunc, const GatEpilogue *epi,
+                              cudaStream_t s) {
     NormOut o{};
     o.q16 = q16;
     o.q_sub = offset_sub;
@@ -779,7 +790,7 @@ void b4d_launch_normalise_q16(const long long *numq, const uint32_t *gmap, const
     o.q_hi = 65535.0f / step;  // float32 division, as k_quantize's __fdiv_rn(65535.0f, step)
     o.q_unit = step == 1.0f;
     o.q_trunc = trunc;
-    launch_norm(numq, gmap, fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf, s);
+    launch_norm(numq, gmap, fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf, epi, s);
 }
 void b4d_launch_normalise_match(const long long *numq, const uint32_t *gmap, const float *fallback, float *out,
                                 uint16_t *match, float mscale, int ishift, int D, int H, int W, int nvol,
@@ -789,7 +800,7 @@ void b4d_launch_normalise_match(const long long *numq, const uint32_t *gmap, con
     o.match = match;
     o.mscale = mscale;
     o.ishift = ishift;
-    launch_norm(numq, gmap, fallback, o, D, H, W, nvol, 0, D, inv_qscale, kf, s);
+    launch_norm(numq, gmap, fallback, o, D, H, W, nvol, 0, D, inv_qscale, kf, nullptr, s);
 }
 void b4d_launch_quantize(const float *in, uint16_t *out, long long n, float offset_sub, float offset_add,
                          float step, cudaStream_t s) {

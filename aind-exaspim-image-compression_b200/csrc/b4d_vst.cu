@@ -32,23 +32,39 @@ __device__ __forceinline__ float gat_forward1(uint32_t z, const GatParams &p) {
     return (float)(2.0 * sqrt(t > 0.0 ? t : 0.0));
 }
 
-__device__ __forceinline__ float gat_inverse1(float D, const GatParams &p) {
-    const double d = (double)D;
-    double lam = 0.0;
-    if (!(d <= p.s15)) {  // P(sqrt(1.5)) = 0: the floor below is continuous; NaN takes this branch and gives 0
-        const double r = 1.0 / d;
-        const double P = 0.25 * d * d + p.c1 * r - 1.375 * r * r + p.c2 * r * r * r - 0.125;
-        const double l = P - p.qq;
-        lam = l > 0.0 ? l : 0.0;
-    }
-    return (float)(p.gain * lam + p.offset);
-}
-
 __global__ void __launch_bounds__(256) k_gat_forward(const uint16_t *__restrict__ in, float *__restrict__ out,
                                                      long long n, GatParams p) {
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
         __stcs(out + i, gat_forward1(__ldcs(in + i), p));
+}
+
+// The value set of a VST pass: list[i] = f(vals[i]), table[vals[i]] = f(vals[i]).
+__global__ void __launch_bounds__(256) k_gat_values(const uint16_t *__restrict__ vals, int m, GatParams p,
+                                                    float *__restrict__ list, float *__restrict__ table) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x) {
+        const uint32_t u = vals[i];
+        const float f = gat_forward1(u, p);
+        list[i] = f;
+        table[u] = f;
+    }
+}
+
+// Forward with a known map: the float32 data and the matching image of a volume in one pass, from the 256 KB value
+// table (L2- and L1-resident).  A NaN entry marks a value outside the value set.  in / match may alias: every
+// thread reads its element before it writes it.
+__global__ void __launch_bounds__(256) k_gat_forward_map(const uint16_t *in, const float *__restrict__ table,
+                                                         float *__restrict__ zf, uint16_t *match, long long n,
+                                                         float cf, float scale, int ishift, unsigned *absent) {
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    bool bad = false;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const float v = __ldg(table + in[i]);
+        bad |= isnan(v);
+        __stcs(zf + i, v);
+        match[i] = (uint16_t)to_match(v, cf, scale, ishift);
+    }
+    if (__any_sync(B4D_FULL, bad) && (threadIdx.x & 31) == 0) atomicOr(absent, 1u);
 }
 
 // Q: write K7 of the result (TRUNC: the truncating variant) into q16 instead of the float32 result into out.
@@ -79,4 +95,13 @@ void b4d_launch_gat_inverse(const float *in, float *out, uint16_t *q16, long lon
     else if (trunc)
         b4d_launch(k_gat_inverse<true, true>, g, 256, 0, s, in, out, q16, n, p, offset_sub, offset_add, step);
     else b4d_launch(k_gat_inverse<true, false>, g, 256, 0, s, in, out, q16, n, p, offset_sub, offset_add, step);
+}
+
+void b4d_launch_gat_values(const uint16_t *vals, int m, const GatParams &p, float *list, float *table, cudaStream_t s) {
+    b4d_launch(k_gat_values, grid_for(m), 256, 0, s, vals, m, p, list, table);
+}
+
+void b4d_launch_gat_forward_map(const uint16_t *in, const float *table, float *zf, uint16_t *match, long long n,
+                                float cf, float scale, int ishift, unsigned *absent, cudaStream_t s) {
+    b4d_launch(k_gat_forward_map, grid_for(n), 256, 0, s, in, table, zf, match, n, cf, scale, ishift, absent);
 }
