@@ -785,7 +785,10 @@ int derive_match_map(b4d_handle *h, const float *d_in, long long n, float sigma,
     }
     if (nonfinite > 0 || !(std::isfinite(zlo) && std::isfinite(zhi)))
         return fail(B4D_ERR_INVALID, "input contains non-finite values (NaN or infinity)");
-    if (dev <= 1.0 / 64.0 && hi - lo <= 65535.0) {
+    // Counts minus an offset: every value within min(1, sigma)/64 of an integer.  A tolerance that did not shrink
+    // with sigma would take any data whose whole range lies within 1/64 of one integer (dim [0, 1]-normalised data,
+    // sigma ~ 1e-3) for counts: a near-constant matching image, groups picked by window index, aggregation at scale 1.
+    if (dev <= std::min(1.0, (double)sigma) / 64.0 && hi - lo <= 65535.0) {
         mm->integral = 1;
         mm->scale = 1.0f;
         mm->cf = (float)c;

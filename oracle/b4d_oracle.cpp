@@ -729,7 +729,9 @@ void den_from_weight_map(const std::vector<int64_t> &G, const Geom &g, const Mir
 //  * uint16 input: stage 1 matches on the data itself.
 //  * float32 input that is uint16 counts minus one scalar (data_handling.py:
 //    353-354): cf restores the integers (|cf| <= 0.5), scale 1 — matching is then
-//    exactly the matching on the original counts (offset invariance).
+//    exactly the matching on the original counts (offset invariance).  "Counts" means
+//    every value within min(1, sigma)/64 of an integer after the shift: data whose
+//    whole range is that close to one integer only because sigma is small are not.
 //  * any other float32 input: cf 0 and a power-of-two scale that puts sigma at
 //    32..64 steps (bounded by the 16-bit range).
 // Stage 2 quantises the basic estimate with cf = 0: u = int(rint(y*scale)) + ishift.
@@ -756,7 +758,7 @@ MatchMap derive_match_map(const float *z, int64_t n, float sigma, float *centre 
         zhi = std::max(zhi, (double)z[i]);
     }
     MatchMap mm{};
-    if (dev <= 1.0 / 64.0 && hi - lo <= 65535.0) {
+    if (dev <= std::min(1.0, (double)sigma) / 64.0 && hi - lo <= 65535.0) {
         mm.integral = 1;
         mm.scale = 1.0f;
         mm.cf = (float)c;
@@ -1216,6 +1218,20 @@ int b4d_oracle_stage2_matches(b4d_handle *hh, uint16_t *widx, uint8_t *cnt, int6
         return fail(B4D_ERR_INVALID, "no stage-2 match lists of that size");
     std::memcpy(widx, h->last_widx2.data(), h->last_widx2.size() * sizeof(uint16_t));
     std::memcpy(cnt, h->last_cnt2.data(), h->last_cnt2.size());
+    return 0;
+}
+// oracle-only: the matching map denoise_one matches n float32 values with (after the centring of a large DC
+// level, which *centre receives), for the tests that assert which map a volume takes
+int b4d_oracle_match_map(const float *z, int64_t n, float sigma, int *integral, float *scale, float *centre) {
+    if (!z || n < 1 || !integral || !scale || !centre) return fail(B4D_ERR_INVALID, "NULL argument or n < 1");
+    MatchMap mm = derive_match_map(z, n, sigma, centre);
+    if (*centre != 0.0f) {
+        std::vector<float> shifted(n);
+        for (int64_t i = 0; i < n; ++i) shifted[i] = z[i] + (-*centre);
+        mm = derive_match_map(shifted.data(), n, sigma);
+    }
+    *integral = mm.integral;
+    *scale = mm.scale;
     return 0;
 }
 int b4d_debug_accumulators(b4d_handle *hh, int64_t *numq, int64_t *wmap, int64_t n) {

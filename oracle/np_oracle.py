@@ -226,6 +226,16 @@ def default_profile(**overrides):
     return p
 
 
+def match_map(z, sigma):
+    """(integral, scale, centre) of the matching map the oracle matches float32 data z with at this sigma
+    (DESIGN §3.1): integral-count map or not, its power-of-two scale, and the DC level c0 subtracted first (0: none)."""
+    z = np.ascontiguousarray(z, dtype=np.float32)
+    integral, scale, centre = ctypes.c_int(), ctypes.c_float(), ctypes.c_float()
+    _check(load().b4d_oracle_match_map(z.ctypes.data_as(ctypes.c_void_p), ctypes.c_int64(z.size), ctypes.c_float(sigma),
+                                       ctypes.byref(integral), ctypes.byref(scale), ctypes.byref(centre)))
+    return bool(integral.value), float(scale.value), float(centre.value)
+
+
 class Oracle:
     """arith='f64' (plain restatement) or 'mirror' (float32, CUDA operation order)."""
 

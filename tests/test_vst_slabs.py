@@ -22,7 +22,7 @@ def match_scale(values, first, model, sigma):
     v = z + c
     dev = np.max(np.abs(v - np.rint(v)))
     lo, hi, zlo, zhi = np.rint(v).min(), np.rint(v).max(), z.min(), z.max()
-    if dev <= 1.0 / 64.0 and hi - lo <= 65535.0:
+    if dev <= min(1.0, float(np.float32(sigma))) / 64.0 and hi - lo <= 65535.0:
         scale = 1.0
     else:
         e_range = math.floor(math.log2(65535.0 / max(zhi - zlo, 1e-30)))
