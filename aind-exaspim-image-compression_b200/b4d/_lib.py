@@ -78,6 +78,15 @@ VST_SLAB_SIGNATURES = {
     "b4d_slab_stage1_vst_u16": (_INT, [_P, _P, _P, _I64, _I64, _P, _F32, _P, _INT, _INT]),
 }
 VST_SLAB_EXPORTS = tuple(VST_SLAB_SIGNATURES)
+# include/b4d_step_table.h: per-tile quantizer steps, a table of their own
+STEP_TABLE_SIGNATURES = {
+    "b4d_quantize_tiled_u16": (_INT, [_P, _P, _P, _I64, _P, _P, _P, _F32, _F32, _INT, _P, _INT, _INT]),
+    "b4d_dequantize_tiled_f32": (_INT, [_P, _P, _P, _I64, _P, _P, _P, _F32, _F32, _P, _INT, _INT]),
+    "b4d_denoise_slab_qt16_u16": (_INT, [_P, _P, _P, _I64, _I64, _I64, _I64, _F32, _F32, _F32, _P, _P, _P, _INT, _P,
+                                          _INT, _INT]),
+    "b4d_slab_stage2_qt16": (_INT, [_P, _I64, _I64, _F32, _F32, _P, _P, _P, _INT, _P, _INT]),
+}
+STEP_TABLE_EXPORTS = tuple(STEP_TABLE_SIGNATURES)
 NOISE_HIST_BINS = 262141  # B4D_NOISE_HIST_BINS: |d| <= 4 * 65535
 NLF_MAX_BINS = 64  # B4D_NLF_MAX_BINS
 
@@ -136,7 +145,7 @@ def load():
             "or `make -C aind-exaspim-image-compression_b200/csrc`. There is no CPU fallback." % LIB_PATH
         )
     lib = ctypes.CDLL(LIB_PATH)
-    for name, (restype, argtypes) in {**SIGNATURES, **VST_SLAB_SIGNATURES}.items():
+    for name, (restype, argtypes) in {**SIGNATURES, **VST_SLAB_SIGNATURES, **STEP_TABLE_SIGNATURES}.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
     if lib.b4d_version() != ABI_VERSION:

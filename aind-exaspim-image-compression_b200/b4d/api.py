@@ -150,6 +150,54 @@ def _quantize_args(quantize):
     return q[0], q[1], q[2], int(bool(q[3]))
 
 
+class StepTable(collections.namedtuple("StepTable", "steps tile")):
+    """Per-tile quantizer steps (DESIGN §3 item 13): steps[ntz][nty][ntx] (float32) on the C-order grid of tiles of
+    sides tile = (tz, ty, tx), anchored at the volume's plane 0 and ragged at the far faces -- the grid of noise_sigma's
+    tiles and of the codec's chunks.  The voxel at global (z, y, x) is quantized with steps[z // tz][y // ty][x // tx],
+    bit for bit as the scalar quantizer with that step.  A torch tensor is copied to the host."""
+
+    __slots__ = ()
+
+    def __new__(cls, steps, tile):
+        if _is_torch(steps):
+            steps = steps.detach().cpu().numpy()
+        return super().__new__(cls, np.ascontiguousarray(steps, dtype=np.float32), tuple(int(t) for t in tile))
+
+
+def _step_table_args(table, shape, z_begin=0, z_total=None):
+    """Checks of a StepTable against the (D, H, W) planes of a call that start at global plane z_begin, before any
+    handle work (ValueError).  z_total given (slab forms): the grid covers exactly z_total planes; else it must reach
+    plane z_begin + D - 1.  Returns (steps, tile, grid) as the C ABI takes them."""
+    steps, tile = table.steps, table.tile
+    if steps.ndim != 3:
+        raise ValueError("a step table must be 3-D (ntz, nty, ntx), got %d-D" % steps.ndim)
+    if len(tile) != 3 or any(t < 1 for t in tile):
+        raise ValueError("tile must be three sides >= 1, got %r" % (tile,))
+    if not (np.all(np.isfinite(steps)) and np.all(steps >= 1)):
+        raise ValueError("every step must be finite and >= 1")
+    D, H, W = (int(v) for v in shape)
+    ntz, nty, ntx = steps.shape
+    if (nty, ntx) != (-(-H // tile[1]), -(-W // tile[2])):
+        raise ValueError("step table grid (nty, ntx) = %r does not cover (H, W) = %r in tiles of %r"
+                         % ((nty, ntx), (H, W), tile[1:]))
+    if int(z_begin) < 0:
+        raise ValueError("z_begin must be >= 0, got %r" % (z_begin,))
+    if z_total is not None and ntz != -(-int(z_total) // tile[0]):
+        raise ValueError("step table has %d tile layers; %d planes in tiles of %d need %d"
+                         % (ntz, z_total, tile[0], -(-int(z_total) // tile[0])))
+    if ntz * tile[0] < int(z_begin) + D:
+        raise ValueError("planes [%d, %d) reach beyond the step table's %d tile layers of %d"
+                         % (z_begin, int(z_begin) + D, ntz, tile[0]))
+    return steps, _lib.shape3(tile), _lib.shape3(steps.shape)
+
+
+def _table_of(quantize):
+    """The StepTable of a quantize tuple, or None for a scalar step (or no quantize)."""
+    if quantize is not None and len(quantize) >= 3 and isinstance(quantize[2], StepTable):
+        return quantize[2]
+    return None
+
+
 class Denoiser:
     """One ``b4d_handle``: scratch buffers + a stream on one CUDA device.
     Not thread-safe; one per (process, device)."""
@@ -269,12 +317,22 @@ class Denoiser:
         """One z-slab (uint16, with halos) of a larger volume -> float32 owned planes.
         `out` (NumPy path only) receives the result in place, e.g. a pinned buffer.
         quantize = (offset_sub, offset_add, step[, truncate]): the fused denoise -> offset -> quantize path, the
-        result is the uint16 volume K7 would give on the float32 output (2 bytes per voxel leave the device)."""
-        sc, in_ptr, on_dev, shape = self._input(_array_arg(slab, ("uint16",), (3,), "denoise_slab"))
+        result is the uint16 volume K7 would give on the float32 output (2 bytes per voxel leave the device).  step
+        may be a StepTable of the whole z_total-plane volume."""
+        slab = _array_arg(slab, ("uint16",), (3,), "denoise_slab")
+        table = _table_of(quantize)
+        targs = _step_table_args(table, slab.shape, z_begin, z_total) if table is not None else None
+        sc, in_ptr, on_dev, shape = self._input(slab)
         odt = "float32" if quantize is None else "uint16"
         oshape = (own_end - own_begin,) + shape[1:]
         out = _out_like(sc, oshape, odt) if _is_torch(sc) else _host_out(out, oshape, odt)
-        if quantize is None:
+        if targs is not None:
+            sub, add, _, trunc = _quantize_args(quantize)
+            steps, tile, grid = targs
+            _lib.check(self.lib.b4d_denoise_slab_qt16_u16(self._h, in_ptr, _lib.shape3(shape), z_begin, z_total,
+                                                          own_begin, own_end, sigma, sub, add, tile, grid,
+                                                          steps.ctypes.data, trunc, _ptr(out), on_dev, on_dev))
+        elif quantize is None:
             _lib.check(self.lib.b4d_denoise_slab_u16(self._h, in_ptr, _lib.shape3(shape), z_begin, z_total, own_begin,
                                                      own_end, sigma, _ptr(out), on_dev, on_dev))
         else:
@@ -288,6 +346,7 @@ class Denoiser:
         """Stage 1 on a uint16 slab (NumPy or torch); the basic estimate stays on the device."""
         sc, ptr, on_dev, shape = self._input(_array_arg(slab, ("uint16",), (3,), "slab_stage1"))
         self._slab_shape = tuple(int(v) for v in shape)
+        self._slab_z = (int(z_begin), int(z_total), False)
         _lib.check(self.lib.b4d_slab_stage1_u16(self._h, ptr, _lib.shape3(shape), z_begin, z_total, sigma, on_dev))
 
     def slab_basic(self, plane0, nplanes, device=None):
@@ -330,12 +389,25 @@ class Denoiser:
     def slab_stage2(self, own_begin, own_end, out=None, device=None, quantize=None):
         """Stage 2 on the completed basic estimate -> float32 owned planes (NumPy, or torch on
         `device`; `out` may be a preallocated NumPy array, e.g. pinned).  quantize = (offset_sub, offset_add,
-        step[, truncate]): uint16 output of the fused quantizer instead (see denoise_slab)."""
+        step[, truncate]): uint16 output of the fused quantizer instead (see denoise_slab); step may be a StepTable
+        of the whole volume (not after slab_stage1_vst)."""
+        table = _table_of(quantize)
+        if table is not None:
+            if getattr(self, "_slab_z", None) is None:
+                raise ValueError("slab_stage1 has not been called")
+            z_begin, z_total, vst = self._slab_z
+            if vst:
+                raise NotImplementedError("a step table on the VST path is not implemented")
+            steps, tile, grid = _step_table_args(table, self._slab_shape, z_begin, z_total)
         oshape = (int(own_end - own_begin),) + self._slab_shape[1:]
         odt = "float32" if quantize is None else "uint16"
         out = _host_out(out, oshape, odt) if device is None else self._device_out(oshape, odt, device)
         on_dev = device is not None
-        if quantize is None:
+        if table is not None:
+            sub, add, _, trunc = _quantize_args(quantize)
+            _lib.check(self.lib.b4d_slab_stage2_qt16(self._h, own_begin, own_end, sub, add, tile, grid,
+                                                     steps.ctypes.data, trunc, _ptr(out), on_dev))
+        elif quantize is None:
             _lib.check(self.lib.b4d_slab_stage2(self._h, own_begin, own_end, _ptr(out), on_dev))
         else:
             _lib.check(self.lib.b4d_slab_stage2_q16(self._h, own_begin, own_end, *_quantize_args(quantize), _ptr(out),
@@ -344,7 +416,8 @@ class Denoiser:
 
     def denoise_quantized(self, vol, sigma, offset_sub=0.0, offset_add=0.0, step=1.0, truncate=False, out=None):
         """denoise -> offset -> quantize of one uint16 volume in one call (b4d_denoise_q16_u16): the uint16 volume
-        `quantize(denoise(vol, sigma), offset_sub, offset_add, step, truncate)` would give, bit for bit."""
+        `quantize(denoise(vol, sigma), offset_sub, offset_add, step, truncate)` would give, bit for bit.  step may be
+        a StepTable (b4d_denoise_slab_qt16_u16 on the slab 0, D, 0, D)."""
         D = int(vol.shape[0])
         return self.denoise_slab(vol, 0, D, 0, D, sigma, out=out, quantize=(offset_sub, offset_add, step, truncate))
 
@@ -361,14 +434,41 @@ class Denoiser:
                                              cnt.ctypes.data))
         return idx, ssd, cnt
 
-    def quantize(self, x, offset_sub=0.0, offset_add=0.0, step=1.0, truncate=False):
+    def quantize(self, x, offset_sub=0.0, offset_add=0.0, step=1.0, truncate=False, z_begin=0):
         """K7: rint(clip((x - offset_sub + offset_add)/step, 0, 65535/step)) -> uint16.
         truncate=True: the evaluator's variant, np.maximum(v, 0).astype(int) cast to uint16 (evaluate.py:202,
-        utils/img_util.py:420-423): toward zero, no upper clip, wrapping modulo 2^16."""
+        utils/img_util.py:420-423): toward zero, no upper clip, wrapping modulo 2^16.
+        step may be a StepTable: x is then 3-D, planes [z_begin, z_begin + D) of the volume the table covers, and
+        every voxel takes the step of its tile (b4d_quantize_tiled_u16)."""
+        if isinstance(step, StepTable):
+            x = _array_arg(x, ("float32",), (3,), "quantize", cast=True)
+            steps, tile, grid = _step_table_args(step, x.shape, z_begin)
+            xc, in_ptr, on_dev, shape = self._input(x)
+            out = _out_like(xc, shape, "uint16")
+            _lib.check(self.lib.b4d_quantize_tiled_u16(self._h, in_ptr, _lib.shape3(shape), int(z_begin), tile, grid,
+                                                       steps.ctypes.data, offset_sub, offset_add, int(bool(truncate)),
+                                                       _ptr(out), on_dev, on_dev))
+            return out
         xc, in_ptr, on_dev, shape = self._input(_array_arg(x, ("float32",), None, "quantize", cast=True))
         out = _out_like(xc, shape, "uint16")
         fn = self.lib.b4d_quantize_trunc_u16 if truncate else self.lib.b4d_quantize_u16
         _lib.check(fn(self._h, in_ptr, math.prod(shape), offset_sub, offset_add, step, _ptr(out), on_dev, on_dev))
+        return out
+
+    def dequantize(self, q, step, offset_sub=0.0, offset_add=0.0, z_begin=0):
+        """Inverse of quantize: x = ((float)q * s) + offset_sub - offset_add per voxel, each operation one float32
+        IEEE operation (b4d_dequantize_tiled_f32).  q: 3-D uint16, planes [z_begin, z_begin + D) of the volume; step:
+        a scalar (one tile) or a StepTable.  Within the clip range of the rounding quantizer |x - original| <= s / 2
+        up to float32 rounding; the truncating quantizer's values come back biased low."""
+        q = _array_arg(q, ("uint16",), (3,), "dequantize")
+        if not isinstance(step, StepTable):
+            step = StepTable(np.full((1, 1, 1), step, np.float32), (int(z_begin) + int(q.shape[0]),) + tuple(q.shape[1:]))
+        steps, tile, grid = _step_table_args(step, q.shape, z_begin)
+        qc, in_ptr, on_dev, shape = self._input(q)
+        out = _out_like(qc, shape, "float32")
+        _lib.check(self.lib.b4d_dequantize_tiled_f32(self._h, in_ptr, _lib.shape3(shape), int(z_begin), tile, grid,
+                                                     steps.ctypes.data, offset_sub, offset_add, _ptr(out), on_dev,
+                                                     on_dev))
         return out
 
     def set_pass_voxels(self, voxels):
@@ -550,6 +650,7 @@ class Denoiser:
         sc, ptr, on_dev, shape = self._input(_vst_args(slab, sigma, None, (3,), "slab_stage1_vst"))
         m, hist, first = _model_c(model), _value_hist(value_hist), int(first)
         self._slab_shape = tuple(int(v) for v in shape)
+        self._slab_z = (int(z_begin), int(z_total), True)
         _lib.check(self.lib.b4d_slab_stage1_vst_u16(self._h, ptr, _lib.shape3(shape), z_begin, z_total,
                                                     ctypes.byref(m), sigma, hist.ctypes.data, first, on_dev))
 
@@ -763,12 +864,27 @@ def make_foreground_mask(raw_u16, offset=0.0, k=6.0, dilate=1, device=None):
     return get_denoiser(device).foreground_mask(raw_u16, offset, k, dilate)
 
 
-def quantize(x, offset_sub=0.0, offset_add=0.0, step=1.0, device=None, truncate=False):
+def quantize(x, offset_sub=0.0, offset_add=0.0, step=1.0, device=None, truncate=False, z_begin=0):
+    """K7; see Denoiser.quantize (step: a scalar or a StepTable)."""
+    if isinstance(step, StepTable):
+        _step_table_args(step, np.shape(x) if not _is_torch(x) else tuple(x.shape), z_begin)
+        return get_denoiser(device).quantize(x, offset_sub, offset_add, step, truncate, z_begin=z_begin)
     return get_denoiser(device).quantize(x, offset_sub, offset_add, step, truncate)
 
 
+def dequantize(q, step, offset_sub=0.0, offset_add=0.0, z_begin=0, device=None):
+    """Inverse of quantize; see Denoiser.dequantize."""
+    if isinstance(step, StepTable):
+        _step_table_args(step, np.shape(q) if not _is_torch(q) else tuple(q.shape), z_begin)
+    return get_denoiser(device).dequantize(q, step, offset_sub, offset_add, z_begin)
+
+
 def denoise_quantized(vol, sigma, offset_sub=0.0, offset_add=0.0, step=1.0, truncate=False, device=None):
-    """Denoise -> background-offset subtract -> (noise-scaled) quantize of one uint16 volume, fused on the device."""
+    """Denoise -> background-offset subtract -> (noise-scaled) quantize of one uint16 volume, fused on the device;
+    step: a scalar or a StepTable (per-tile steps, e.g. noise_scaled_steps)."""
+    if isinstance(step, StepTable):
+        shape = np.shape(vol) if not _is_torch(vol) else tuple(vol.shape)
+        _step_table_args(step, shape, 0, shape[0])
     return get_denoiser(device).denoise_quantized(vol, sigma, offset_sub, offset_add, step, truncate)
 
 
@@ -782,6 +898,14 @@ def patch_has_incoherent_segment(labels, raw, min_autocorr=0.4, max_highfreq_fra
 def noise_scaled_step(sigma_tile, kappa):
     """step = max(1, kappa * sigma_tile) (SURVEY §8a, K7 definition)."""
     return float(max(1.0, float(kappa) * float(sigma_tile)))
+
+
+def noise_scaled_steps(sigma, kappa, tile):
+    """StepTable of float32(noise_scaled_step(sigma, kappa)) per tile: sigma is noise_sigma(x, tile=tile)["sigma"] of
+    one volume, (ntz, nty, ntx); a NaN sigma (a tile without usable cells, DESIGN §3.11) gives step 1."""
+    s = np.asarray(sigma.detach().cpu().numpy() if _is_torch(sigma) else sigma, dtype=np.float64)
+    steps = np.where(np.isnan(s), 1.0, np.maximum(1.0, float(kappa) * s)).astype(np.float32)
+    return StepTable(steps, tile)
 
 
 def tile_stats(x, percentile=1.0, device=None, return_hist=False):
@@ -873,6 +997,8 @@ def _nlf_args(x, edges, min_cells):
 
 def _vst_args(x, sigma, quantize, ndims=(3, 4), what="denoise_vst"):
     """Argument checks of denoise_vst (and its slab forms), before any device work: returns x."""
+    if _table_of(quantize) is not None:
+        raise NotImplementedError("a step table on the VST path is not implemented")
     x = _array_arg(x, ("uint16",), ndims, what)
     if not (np.isfinite(sigma) and sigma > 0):
         raise ValueError("sigma must be positive and finite, got %r" % (sigma,))

@@ -94,11 +94,19 @@ def denoise_slab_exchange(denoiser, slab, z_begin, z_total, own_begin, own_end, 
     """One rank's part of the exchange variant: stage 1 on the slab (halo `exchange_halo`), swap
     the exact basic-estimate planes next to each interior face with the neighbours, stage 2.
     `device` = the rank's torch CUDA device (planes then travel device to device).
-    quantize = (offset_sub, offset_add, step[, truncate]): uint16 output of the fused quantizer.
+    quantize = (offset_sub, offset_add, step[, truncate]): uint16 output of the fused quantizer; step may be a
+    StepTable of the whole z_total-plane volume (checked here, before stage 1 and the exchange).
     model (PoissonGaussian, the same on every rank): through the GAT, `sigma` is then sigma_vst; value_hist as
     vst_value_hist; first = the whole volume's voxel (0, 0, 0), taken from the slab when it starts at plane 0."""
     import torch
 
+    from .api import _step_table_args, _table_of
+
+    table = _table_of(quantize)
+    if table is not None:
+        if model is not None:
+            raise NotImplementedError("a step table on the VST path is not implemented")
+        _step_table_args(table, tuple(slab.shape), z_begin, z_total)
     if model is None:
         denoiser.slab_stage1(slab, z_begin, z_total, sigma)
     else:

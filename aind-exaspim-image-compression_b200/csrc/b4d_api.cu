@@ -10,6 +10,7 @@
 #include <string>
 #include <vector>
 
+#include "../../include/b4d_step_table.h"
 #include "../../include/b4d_vst_slab.h"
 #include "b4d_common.cuh"
 #include "b4d_host.cuh"
@@ -115,6 +116,7 @@ struct b4d_handle {
     DevBuf nz_hist, nz_sel, nz_res, nz_full;  // b4d_noise_sigma_u16: per-tile digit histograms, selections, results
     DevBuf nlf_sum;  // b4d_noise_level_u16: per-bin sums of the cell intensities
     DevBuf vst;      // VST passes: value table [65536 f32] | value list [65537 f32] | absent flag | value codes
+    DevBuf steps;    // step table of the call: {s, 65535 / s} per tile (include/b4d_step_table.h)
     float t_ms[B4D_T_COUNT] = {};
     int64_t launches[B4D_T_COUNT] = {};
     unsigned long long match_stats[4] = {};
@@ -127,7 +129,7 @@ struct b4d_handle {
     // state between b4d_slab_stage1_u16 and b4d_slab_stage2: the slab (planes from slab_z_begin on) and its map
     bool slab_open = false;
     Plan slab;
-    int64_t slab_z_begin = 0;
+    int64_t slab_z_begin = 0, slab_z_total = 0;
     float slab_sigma = 0.f;
     MatchMap slab_mm;
     bool slab_vst = false;  // a VST slab (b4d_slab_stage1_vst_u16): data in `in`, matching image in `u16`
@@ -389,7 +391,50 @@ struct HostSink {
 struct QuantSpec {
     float sub = 0.f, add = 0.f, step = 1.f;
     int trunc = 0;
+    StepTab tab{};  // tab.t set: the step of each voxel's tile replaces `step` (single-volume, non-VST passes)
 };
+
+// A step table from the caller (include/b4d_step_table.h), checked on the host against the shape[0] x H x W planes of
+// a call that start at global plane z_begin: z_total > 0 demands ntz = ceil(z_total / tz) (slab forms), else the grid
+// must reach the last plane.  Indices of the kernels are int: the table and the planes stay below 2^31.
+int check_step_table(const int64_t shape[3], int64_t z_begin, int64_t z_total, const int64_t tile[3],
+                     const int64_t grid[3], const float *steps) {
+    if (!tile || !grid || !steps) return fail(B4D_ERR_INVALID, "NULL step table");
+    for (int i = 0; i < 3; ++i)
+        if (tile[i] < 1 || tile[i] > INT32_MAX || grid[i] < 1 || grid[i] > INT32_MAX)
+            return fail(B4D_ERR_INVALID, "step table: tile sides and grid must be >= 1");
+    if (z_begin < 0 || z_begin + shape[0] > INT32_MAX) return fail(B4D_ERR_INVALID, "step table: z_begin out of range");
+    auto cdiv = [](int64_t a, int64_t b) { return (a + b - 1) / b; };
+    if (grid[1] != cdiv(shape[1], tile[1]) || grid[2] != cdiv(shape[2], tile[2]))
+        return fail(B4D_ERR_INVALID, "step table: grid (nty, ntx) must be (ceil(H / ty), ceil(W / tx))");
+    if (z_total > 0 ? grid[0] != cdiv(z_total, tile[0]) : grid[0] < cdiv(z_begin + shape[0], tile[0]))
+        return fail(B4D_ERR_INVALID, z_total > 0 ? "step table: ntz must be ceil(z_total / tz)"
+                                                 : "step table: the grid does not reach plane z_begin + D - 1");
+    if (grid[0] * grid[1] * grid[2] > INT32_MAX / 2) return fail(B4D_ERR_TOO_LARGE, "step table too large");
+    const int64_t n = grid[0] * grid[1] * grid[2];
+    for (int64_t i = 0; i < n; ++i)
+        if (!(std::isfinite(steps[i]) && steps[i] >= 1.0f))
+            return fail(B4D_ERR_INVALID, "step table: every step must be finite and >= 1");
+    return 0;
+}
+// The checked table into h->steps as {s, 65535 / s} (the float32 division of K7), and its device form.
+int upload_step_table(b4d_handle *h, int64_t z_begin, const int64_t tile[3], const int64_t grid[3], const float *steps,
+                      StepTab *tab) {
+    const int64_t n = grid[0] * grid[1] * grid[2];
+    std::vector<float2> t((size_t)n);
+    for (int64_t i = 0; i < n; ++i) t[i] = make_float2(steps[i], 65535.0f / steps[i]);
+    B4D_TRY(h->steps.ensure((size_t)n * sizeof(float2)));
+    CU_TRY(cudaMemcpyAsync(h->steps.p, t.data(), (size_t)n * sizeof(float2), cudaMemcpyHostToDevice, h->stream));
+    CU_TRY(cudaStreamSynchronize(h->stream));  // `t` is a stack vector
+    tab->t = h->steps.as<float2>();
+    tab->tz = (int)tile[0];
+    tab->ty = (int)tile[1];
+    tab->tx = (int)tile[2];
+    tab->nty = (int)grid[1];
+    tab->ntx = (int)grid[2];
+    tab->z0 = (int)z_begin;
+    return 0;
+}
 
 constexpr int UPLOAD_CHUNKS = 8;
 // Chunked launches under-fill the GPU on small volumes (a 128^3 patch ran 1.5x slower in 8 chunks and its
@@ -526,7 +571,10 @@ void normalise(const Pass &ps, const float *fallback, float *dst, int z0, int z1
     const long long *numq = ps.h->numq.as<long long>();
     const uint32_t *gmap = ps.h->gmap.as<uint32_t>();
     const GatEpilogue *epi = dst == ps.out ? ps.gat : nullptr;
-    if (q)
+    if (q && q->tab.t)
+        b4d_launch_normalise_qt16(numq, gmap, fallback, reinterpret_cast<uint16_t *>(dst), pl.D, pl.H, pl.W, z0, z1,
+                                  1.0f / ps.mm.scale, ps.tab.kf, q->sub, q->add, q->tab, q->trunc, s);
+    else if (q)
         b4d_launch_normalise_q16(numq, gmap, fallback, reinterpret_cast<uint16_t *>(dst), pl.D, pl.H, pl.W, pl.nvol,
                                  z0, z1, 1.0f / ps.mm.scale, ps.tab.kf, q->sub, q->add, q->step, q->trunc, epi, s);
     else
@@ -1187,7 +1235,7 @@ void b4d_destroy(b4d_handle *h) {
     for (DevBuf *b : {&h->in, &h->u16, &h->zf, &h->numq, &h->gmap, &h->basic, &h->out, &h->widx, &h->cnt,
                       &h->ssd, &h->refs, &h->hist, &h->partial, &h->sink, &h->stats, &h->s2, &h->cells, &h->tcls,
                       &h->alt_in, &h->alt_zf, &h->alt_out, &h->alt_partial, &h->alt_sink, &h->nz_hist, &h->nz_sel,
-                      &h->nz_res, &h->nz_full, &h->vst})
+                      &h->nz_res, &h->nz_full, &h->vst, &h->steps})
         b->release();
     if (h->stream) cudaStreamDestroy(h->stream);
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
@@ -1440,6 +1488,7 @@ static int slab_stage1_impl(b4d_handle *h, const uint16_t *in, const int64_t sha
     h->pre.clk.discard();
     h->slab = make_plan(shape, z_begin, z_total, 1, h->prof);
     h->slab_z_begin = z_begin;
+    h->slab_z_total = z_total;
     h->slab_sigma = sigma;
     h->slab_vst = vst != nullptr;
     h->slab_mm = MatchMap();
@@ -1514,6 +1563,19 @@ int b4d_slab_stage2(b4d_handle *h, int64_t own_begin, int64_t own_end, float *ou
 int b4d_slab_stage2_q16(b4d_handle *h, int64_t own_begin, int64_t own_end, float offset_sub, float offset_add,
                         float step, int truncate, uint16_t *out, int out_on_device) {
     const QuantSpec q{offset_sub, offset_add, step, truncate};
+    return slab_stage2_impl(h, own_begin, own_end, out, out_on_device, &q);
+}
+int b4d_slab_stage2_qt16(b4d_handle *h, int64_t own_begin, int64_t own_end, float offset_sub, float offset_add,
+                         const int64_t tile[3], const int64_t grid[3], const float *steps, int truncate,
+                         uint16_t *out, int out_on_device) {
+    if (!h || !out) return fail(B4D_ERR_INVALID, "NULL argument");
+    if (!h->slab_open) return fail(B4D_ERR_INVALID, "b4d_slab_stage1_u16 has not been called");
+    if (h->slab_vst) return fail(B4D_ERR_UNSUPPORTED, "a step table on the VST path is not implemented");
+    const int64_t shape[3] = {h->slab.D, h->slab.H, h->slab.W};
+    B4D_TRY(check_step_table(shape, h->slab_z_begin, h->slab_z_total, tile, grid, steps));
+    CU_TRY(cudaSetDevice(h->device));
+    QuantSpec q{offset_sub, offset_add, 1.0f, truncate ? 1 : 0};
+    B4D_TRY(upload_step_table(h, h->slab_z_begin, tile, grid, steps, &q.tab));
     return slab_stage2_impl(h, own_begin, own_end, out, out_on_device, &q);
 }
 
@@ -1606,6 +1668,69 @@ int b4d_match_stage1(b4d_handle *h, const uint16_t *in, const int64_t shape[3], 
         }
     }
     return 0;
+}
+
+// Standalone K7 with a step table (float32 -> uint16) or its inverse (uint16 -> float32).
+static int tiled_impl(b4d_handle *h, const void *in, const int64_t shape[3], int64_t z_begin, const int64_t tile[3],
+                      const int64_t grid[3], const float *steps, float offset_sub, float offset_add, int trunc,
+                      void *out, int in_on_device, int out_on_device, bool dequant) {
+    if (!h || !in || !out || !shape) return fail(B4D_ERR_INVALID, "NULL argument");
+    for (int i = 0; i < 3; ++i)
+        if (shape[i] < 1 || shape[i] > INT32_MAX) return fail(B4D_ERR_INVALID, "every dimension must be >= 1");
+    B4D_TRY(check_step_table(shape, z_begin, 0, tile, grid, steps));
+    CU_TRY(cudaSetDevice(h->device));
+    const long long n = shape[0] * shape[1] * shape[2];
+    const size_t isz = dequant ? sizeof(uint16_t) : sizeof(float), osz = dequant ? sizeof(float) : sizeof(uint16_t);
+    cudaStream_t s = h->stream;
+    StepTab tab;
+    B4D_TRY(upload_step_table(h, z_begin, tile, grid, steps, &tab));
+    const void *d_in = in;
+    void *d_out = out;
+    if (!in_on_device) {
+        B4D_TRY(h->in.ensure((size_t)n * isz));
+        CU_TRY(copy_in(h, h->in.p, in, (size_t)n * isz, 0, s));
+        d_in = h->in.p;
+    }
+    if (!out_on_device) {
+        B4D_TRY(h->u16.ensure((size_t)n * osz + 16));
+        d_out = h->u16.p;
+    }
+    const int D = (int)shape[0], H = (int)shape[1], W = (int)shape[2];
+    if (dequant)
+        b4d_launch_dequantize_tiled(static_cast<const uint16_t *>(d_in), static_cast<float *>(d_out), D, H, W,
+                                    offset_sub, offset_add, tab, s);
+    else
+        b4d_launch_quantize_tiled(static_cast<const float *>(d_in), static_cast<uint16_t *>(d_out), D, H, W, offset_sub,
+                                  offset_add, tab, trunc, s);
+    CU_TRY(cudaGetLastError());
+    if (d_out != out) CU_TRY(copy_out(h, out, d_out, (size_t)n * osz, 0, s));
+    CU_TRY(cudaStreamSynchronize(s));
+    return 0;
+}
+int b4d_quantize_tiled_u16(b4d_handle *h, const float *in, const int64_t shape[3], int64_t z_begin,
+                           const int64_t tile[3], const int64_t grid[3], const float *steps, float offset_sub,
+                           float offset_add, int truncate, uint16_t *out, int in_on_device, int out_on_device) {
+    return tiled_impl(h, in, shape, z_begin, tile, grid, steps, offset_sub, offset_add, truncate ? 1 : 0, out,
+                      in_on_device, out_on_device, false);
+}
+int b4d_dequantize_tiled_f32(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
+                             const int64_t tile[3], const int64_t grid[3], const float *steps, float offset_sub,
+                             float offset_add, float *out, int in_on_device, int out_on_device) {
+    return tiled_impl(h, in, shape, z_begin, tile, grid, steps, offset_sub, offset_add, 0, out, in_on_device,
+                      out_on_device, true);
+}
+int b4d_denoise_slab_qt16_u16(b4d_handle *h, const uint16_t *in, const int64_t shape[3], int64_t z_begin,
+                              int64_t z_total, int64_t own_begin, int64_t own_end, float sigma, float offset_sub,
+                              float offset_add, const int64_t tile[3], const int64_t grid[3], const float *steps,
+                              int truncate, uint16_t *out, int in_on_device, int out_on_device) {
+    B4D_TRY(common_checks(h, in, out, shape, sigma));
+    if (z_total < 1) return fail(B4D_ERR_INVALID, "slab / owned range inconsistent");
+    B4D_TRY(check_step_table(shape, z_begin, z_total, tile, grid, steps));
+    B4D_TRY(reset_last(h));
+    QuantSpec q{offset_sub, offset_add, 1.0f, truncate ? 1 : 0};
+    B4D_TRY(upload_step_table(h, z_begin, tile, grid, steps, &q.tab));
+    return denoise_slab_impl(h, in, shape, z_begin, z_total, own_begin, own_end, sigma, out, in_on_device,
+                             out_on_device, &q);
 }
 
 static int quantize_impl(b4d_handle *h, const float *in, int64_t n, float offset_sub, float offset_add, float step,

@@ -7,6 +7,7 @@
 
 #include "../../include/b4d.h"
 #include "../../include/b4d_noise.h"
+#include "../../include/b4d_step_table.h"
 
 // Kernels this host thread has enqueued.  A stage mark of the host pipeline books the kernels enqueued since the
 // previous mark as that stage's launch count.  Per thread because the launchers do not see the handle; a call
@@ -134,6 +135,23 @@ void b4d_launch_normalise_q16(const long long *numq, const uint32_t *gmap, const
                               int H, int W, int nvol, int z0, int z1, float inv_qscale, const float kf[4],
                               float offset_sub, float offset_add, float step, int trunc, const GatEpilogue *epi,
                               cudaStream_t s);
+// Per-tile quantizer steps (include/b4d_step_table.h, DESIGN §3 item 13) on the device: t[(iz * nty + iy) * ntx + ix]
+// = {s, 65535 / s} (float32 division, as K7's __fdiv_rn) of tile (iz, iy, ix); plane z of a launch is global plane
+// z0 + z.
+struct StepTab {
+    const float2 *t;
+    int tz, ty, tx, nty, ntx;
+    int z0;
+};
+// K6 + K7 fused with a step table (single volume)
+void b4d_launch_normalise_qt16(const long long *numq, const uint32_t *gmap, const float *fallback, uint16_t *q16, int D,
+                               int H, int W, int z0, int z1, float inv_qscale, const float kf[4], float offset_sub,
+                               float offset_add, const StepTab &tab, int trunc, cudaStream_t s);
+// standalone K7 with a step table, and its inverse, over the D x H x W planes of a launch
+void b4d_launch_quantize_tiled(const float *in, uint16_t *out, int D, int H, int W, float offset_sub, float offset_add,
+                               const StepTab &tab, int trunc, cudaStream_t s);
+void b4d_launch_dequantize_tiled(const uint16_t *in, float *out, int D, int H, int W, float offset_sub,
+                                 float offset_add, const StepTab &tab, cudaStream_t s);
 void b4d_launch_hist(const uint16_t *in, long long n, unsigned long long *hist, cudaStream_t s);
 // make_foreground_mask after the statistic: threshold + L1-ball dilation, per patch thr / off
 void b4d_launch_fg_mask(const uint16_t *in, const float *off, const float *thr, int D, int H, int W, long long n,

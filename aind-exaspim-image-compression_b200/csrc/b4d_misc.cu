@@ -168,8 +168,18 @@ struct NormOut {
     int ishift;
     float q_sub, q_add, q_step, q_hi;
     int q_unit, q_trunc;
-    GatEpilogue gat;     // VST instantiations: y = gat_inverse1(y + centre) before the outputs
+    // A VST pass never quantizes with a table, so the two share storage (NormOut, and with it the parameter layout
+    // of the instantiations without a table, is what it was before tables existed).
+    union {
+        GatEpilogue gat;  // VST instantiations: y = gat_inverse1(y + centre) before the outputs
+        StepTab tab;      // TABLE instantiations: q16 with the step of each voxel's tile instead of q_step
+    };
 };
+// K7 of one voxel of the fused output with a step-table entry e = {s, 65535 / s}
+__device__ __forceinline__ uint32_t quant_entry(float y, const NormOut &o, float2 e) {
+    return o.q_trunc ? quant1_trunc(y, o.q_sub, o.q_add, e.x, e.y, e.x == 1.0f)
+                     : quant1(y, o.q_sub, o.q_add, e.x, e.y, e.x == 1.0f);
+}
 // The result of one voxel as the outputs take it: y itself, or in a VST pass its GAT inverse (bit-identical to a
 // separate k_add_scalar + k_gat_inverse on the stored y: the same float32 add and float64 operations).
 template <bool VST>
@@ -182,7 +192,8 @@ __device__ __forceinline__ float norm_epilogue(float y, const NormOut &o) {
 // no barrier.  Lane i holds column X0 - 3 + i of the uint32 map for the 11 rows Y0 - 3 .. Y0 + 7 (lanes 0-2 are the
 // x halo); the x pass takes the three left neighbours by warp shuffles of the uint32 values, the y pass runs on the
 // 11 x-convolved rows in registers, the z pass on a rolling window of three earlier xy-convolved values per row.
-template <bool VST>
+// TABLE: the quantized output takes its step from o.tab (one L1-resident table load per voxel).
+template <bool VST, bool TABLE>
 __global__ void __launch_bounds__(WM_WARPS * 32) k_normalise_wm(const long long *__restrict__ numq,
                                                                 const uint32_t *__restrict__ gmap,
                                                                 const float *__restrict__ fb, NormOut o, int D, int H,
@@ -209,6 +220,17 @@ __global__ void __launch_bounds__(WM_WARPS * 32) k_normalise_wm(const long long 
     double h1[WM_TY], h2[WM_TY], h3[WM_TY];  // xy-convolved map of the three previous planes
 #pragma unroll
     for (int r = 0; r < WM_TY; ++r) h1[r] = h2[r] = h3[r] = 0.0;
+    // TABLE: this lane's tile column and the tile rows of the 8 rows are fixed for the whole z-march; the rows are
+    // kept as the table index of row Y0 plus 4-bit tile-row deltas (three registers, not eight: the TMA form runs at
+    // its 128-register bound)
+    int tcol = 0;
+    uint32_t tdel = 0;
+    if (TABLE) {
+        const int ty0 = Y0 / o.tab.ty;
+        tcol = ty0 * o.tab.ntx + (col_in ? gx / o.tab.tx : 0);
+#pragma unroll
+        for (int r = 1; r < WM_TY; ++r) tdel |= (uint32_t)(min(Y0 + r, H - 1) / o.tab.ty - ty0) << (4 * r);
+    }
     // Memory latency is the limit of this kernel (ncu: long-scoreboard stalls, DRAM at 17 %), so every load is
     // issued well ahead of its use: the map values of plane z + 1 and the numerators of plane z before plane z is
     // convolved.
@@ -228,6 +250,7 @@ __global__ void __launch_bounds__(WM_WARPS * 32) k_normalise_wm(const long long 
         if (z + 1 < Zb) load_map(z + 1);
         const bool out_z = z >= Za && out_lane;
         const long long a0 = vol * V + (long long)z * P + (long long)Y0 * W + gx;
+        const int tlay = TABLE ? (o.tab.z0 + max(z, 0)) / o.tab.tz * (o.tab.nty * o.tab.ntx) + tcol : 0;
         long long nq[WM_TY];
 #pragma unroll
         for (int r = 0; r < WM_TY; ++r) nq[r] = (out_z && Y0 + r < H) ? __ldcs(numq + a0 + (long long)r * W) : 0ll;
@@ -253,7 +276,9 @@ __global__ void __launch_bounds__(WM_WARPS * 32) k_normalise_wm(const long long 
                 const float y = norm_epilogue<VST>(den > 0.0 ? (float)(((double)nq[r] / den) * inv) : fb[a], o);
                 if (o.out) o.out[a] = y;
                 if (o.match) o.match[a] = (uint16_t)to_match(y, 0.0f, o.mscale, o.ishift);
-                if (o.q16)
+                if (TABLE)
+                    o.q16[a] = (uint16_t)quant_entry(y, o, __ldg(o.tab.t + tlay + (int)((tdel >> (4 * r)) & 15u) * o.tab.ntx));
+                else if (o.q16)
                     o.q16[a] = (uint16_t)(o.q_trunc ? quant1_trunc(y, o.q_sub, o.q_add, o.q_step, o.q_hi, o.q_unit != 0)
                                                     : quant1(y, o.q_sub, o.q_add, o.q_step, o.q_hi, o.q_unit != 0));
             }
@@ -275,7 +300,7 @@ constexpr uint32_t WMT_G_BYTES = WMT_GW * WM_EY * 4, WMT_N_BYTES = WMT_TX * WM_T
 constexpr int WMT_G_STAGE = ((int)WMT_G_BYTES + 127) / 128 * 128;
 constexpr int WMT_STAGE = WMT_G_STAGE + (int)WMT_N_BYTES;
 static_assert(WMT_TX % 4 == 0 && WMT_GW % 4 == 0 && WMT_GW >= WMT_TX + 4 && WMT_N_BYTES % 128 == 0, "TMA boxes of the normalise kernel");
-template <bool VST>
+template <bool VST, bool TABLE>
 __global__ void __launch_bounds__(WMT_WARPS * 32, 4) k_normalise_wm_tma(const __grid_constant__ CUtensorMap gmap_t,
                                                                        const __grid_constant__ CUtensorMap numq_t,
                                                                        const float *__restrict__ fb, NormOut o, int D, int H,
@@ -320,6 +345,14 @@ __global__ void __launch_bounds__(WMT_WARPS * 32, 4) k_normalise_wm_tma(const __
     double h1[WM_TY], h2[WM_TY], h3[WM_TY];  // xy-convolved map of the three previous planes
 #pragma unroll
     for (int r = 0; r < WM_TY; ++r) h1[r] = h2[r] = h3[r] = 0.0;
+    int tcol = 0;  // TABLE: as in k_normalise_wm
+    uint32_t tdel = 0;
+    if (TABLE) {
+        const int ty0 = Y0 / o.tab.ty;
+        tcol = ty0 * o.tab.ntx + (out_lane ? gx / o.tab.tx : 0);
+#pragma unroll
+        for (int r = 1; r < WM_TY; ++r) tdel |= (uint32_t)(min(Y0 + r, H - 1) / o.tab.ty - ty0) << (4 * r);
+    }
     for (int i = 0; i < nplanes; ++i) {
         const int st = i % WMT_NST, z = Za - 3 + i;
         mbar_wait(full0 + 8u * st, (uint32_t)((i / WMT_NST) & 1));
@@ -348,6 +381,7 @@ __global__ void __launch_bounds__(WMT_WARPS * 32, 4) k_normalise_wm_tma(const __
             xr[r] = acc;
         }
         const long long a0 = (long long)vol * V + (long long)z * P + (long long)Y0 * W + gx;
+        const int tlay = TABLE ? (o.tab.z0 + max(z, 0)) / o.tab.tz * (o.tab.nty * o.tab.ntx) + tcol : 0;
 #pragma unroll
         for (int r = 0; r < WM_TY; ++r) {
             double w0 = 0.0;  // y pass
@@ -362,7 +396,9 @@ __global__ void __launch_bounds__(WMT_WARPS * 32, 4) k_normalise_wm_tma(const __
                 const float y = norm_epilogue<VST>(den > 0.0 ? (float)(((double)nq[r] / den) * inv) : fb[a], o);
                 if (o.out) o.out[a] = y;
                 if (o.match) o.match[a] = (uint16_t)to_match(y, 0.0f, o.mscale, o.ishift);
-                if (o.q16)
+                if (TABLE)
+                    o.q16[a] = (uint16_t)quant_entry(y, o, __ldg(o.tab.t + tlay + (int)((tdel >> (4 * r)) & 15u) * o.tab.ntx));
+                else if (o.q16)
                     o.q16[a] = (uint16_t)(o.q_trunc ? quant1_trunc(y, o.q_sub, o.q_add, o.q_step, o.q_hi, o.q_unit != 0)
                                                     : quant1(y, o.q_sub, o.q_add, o.q_step, o.q_hi, o.q_unit != 0));
             }
@@ -400,6 +436,131 @@ __global__ void __launch_bounds__(256) k_quantize(const float *__restrict__ in, 
     }
     for (long long i = (nv << 4) + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
         out[i] = (uint16_t)quantq<TRUNC>(in[i], osub, oadd, step, hi, unit);
+}
+
+// ---------------------------------------------- quantize with a step table --
+// One warp per (z, y) row, grid-stride over the rows: the table row of a row is two divisions, and a lane's tile
+// column is walked with carries as it steps along x (V voxels per step, 32 V apart), so no voxel costs a division.
+// V = 4 (W % 4 == 0 and aligned pointers): 16-byte float loads, 8-byte uint16 stores; QT_U steps in flight per lane.
+constexpr int QT_WARPS = 8, QT_U = 4;
+struct TileWalk {  // tile column c of x = c * tx + r
+    int c, r;
+    __device__ __forceinline__ void step(int dc, int dr, int tx) {
+        c += dc;
+        r += dr;
+        if (r >= tx) {
+            r -= tx;
+            ++c;
+        }
+    }
+    __device__ __forceinline__ int col(int k, int tx) const {  // tile column of x + k
+        int cc = c, rr = r + k;
+        while (rr >= tx) {
+            rr -= tx;
+            ++cc;
+        }
+        return cc;
+    }
+};
+// Calls f(x, trow, walk) for the start x of every step of this lane (V-voxel steps along each row of the launch).
+template <int V, class F>
+__device__ __forceinline__ void tiled_rows(int D, int H, int W, const StepTab &tab, F &&f) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int S = 32 * V, dc = S / tab.tx, dr = S % tab.tx;
+    const TileWalk w0{(V * lane) / tab.tx, (V * lane) % tab.tx};
+    const long long rows = (long long)D * H;
+    for (long long row = (long long)blockIdx.x * QT_WARPS + warp; row < rows; row += (long long)gridDim.x * QT_WARPS) {
+        const int z = (int)(row / H), y = (int)(row - (long long)z * H);
+        const float2 *trow = tab.t + ((long long)((tab.z0 + z) / tab.tz) * tab.nty + y / tab.ty) * tab.ntx;
+        TileWalk w = w0;
+        for (int xb = V * lane; xb < W; xb += QT_U * S) {
+            f(row * W, xb, trow, w, dc, dr);
+        }
+    }
+}
+template <bool TRUNC, int V>
+__global__ void __launch_bounds__(QT_WARPS * 32) k_quantize_tiled(const float *__restrict__ in, uint16_t *__restrict__ out,
+                                                                  int D, int H, int W, float osub, float oadd,
+                                                                  StepTab tab) {
+    tiled_rows<V>(D, H, W, tab, [&](long long base, int xb, const float2 *trow, TileWalk &w, int dc, int dr) {
+        float v[QT_U][V];
+#pragma unroll
+        for (int u = 0; u < QT_U; ++u) {
+            const int x = xb + u * 32 * V;
+            if (x < W) {
+                if (V == 4) {
+                    const float4 t = __ldcs(reinterpret_cast<const float4 *>(in + base + x));
+                    v[u][0] = t.x, v[u][V > 1 ? 1 : 0] = t.y, v[u][V > 2 ? 2 : 0] = t.z, v[u][V - 1] = t.w;
+                } else {
+                    v[u][0] = __ldcs(in + base + x);
+                }
+            }
+        }
+#pragma unroll
+        for (int u = 0; u < QT_U; ++u) {
+            const int x = xb + u * 32 * V;
+            if (x < W) {
+                uint32_t q[V];
+                const float2 e0 = __ldg(trow + w.c);
+                const bool one_tile = w.r + V - 1 < tab.tx;  // the common case: all V voxels in one tile
+#pragma unroll
+                for (int k = 0; k < V; ++k) {
+                    const float2 e = (k == 0 || one_tile) ? e0 : __ldg(trow + w.col(k, tab.tx));
+                    q[k] = quantq<TRUNC>(v[u][k], osub, oadd, e.x, e.y, e.x == 1.0f);
+                }
+                if (V == 4)
+                    __stcs(reinterpret_cast<uint2 *>(out + base + x),
+                           make_uint2(q[0] | (q[V > 1 ? 1 : 0] << 16), q[V > 2 ? 2 : 0] | (q[V - 1] << 16)));
+                else
+                    out[base + x] = (uint16_t)q[0];
+            }
+            w.step(dc, dr, tab.tx);
+        }
+    });
+}
+// inverse: x = ((float)q * s) + offset_sub - offset_add, one IEEE float32 operation each
+__global__ void __launch_bounds__(QT_WARPS * 32) k_dequantize_tiled(const uint16_t *__restrict__ in,
+                                                                    float *__restrict__ out, int D, int H, int W,
+                                                                    float osub, float oadd, StepTab tab, int vec) {
+    auto deq = [&](uint32_t q, float s) { return __fsub_rn(__fadd_rn(__fmul_rn((float)q, s), osub), oadd); };
+    if (vec) {
+        tiled_rows<4>(D, H, W, tab, [&](long long base, int xb, const float2 *trow, TileWalk &w, int dc, int dr) {
+            uint2 v[QT_U];
+#pragma unroll
+            for (int u = 0; u < QT_U; ++u) {
+                const int x = xb + u * 128;
+                if (x < W) v[u] = __ldcs(reinterpret_cast<const uint2 *>(in + base + x));
+            }
+#pragma unroll
+            for (int u = 0; u < QT_U; ++u) {
+                const int x = xb + u * 128;
+                if (x < W) {
+                    float4 r;
+                    r.x = deq(v[u].x & 0xFFFFu, __ldg(&trow[w.col(0, tab.tx)].x));
+                    r.y = deq(v[u].x >> 16, __ldg(&trow[w.col(1, tab.tx)].x));
+                    r.z = deq(v[u].y & 0xFFFFu, __ldg(&trow[w.col(2, tab.tx)].x));
+                    r.w = deq(v[u].y >> 16, __ldg(&trow[w.col(3, tab.tx)].x));
+                    __stcs(reinterpret_cast<float4 *>(out + base + x), r);
+                }
+                w.step(dc, dr, tab.tx);
+            }
+        });
+    } else {
+        tiled_rows<1>(D, H, W, tab, [&](long long base, int xb, const float2 *trow, TileWalk &w, int dc, int dr) {
+            uint32_t v[QT_U];
+#pragma unroll
+            for (int u = 0; u < QT_U; ++u) {
+                const int x = xb + u * 32;
+                if (x < W) v[u] = __ldcs(in + base + x);
+            }
+#pragma unroll
+            for (int u = 0; u < QT_U; ++u) {
+                const int x = xb + u * 32;
+                if (x < W) __stcs(out + base + x, deq(v[u], __ldg(&trow[w.col(0, tab.tx)].x)));
+                w.step(dc, dr, tab.tx);
+            }
+        });
+    }
 }
 
 // --------------------------------------------------- chunk byte shuffle ----
@@ -747,18 +908,20 @@ static void launch_norm(const long long *numq, const uint32_t *gmap, const float
                         int H, int W, int nvol, int z0, int z1, float inv_qscale, const float kf[4],
                         const GatEpilogue *epi, cudaStream_t s) {
     if (z1 <= z0) return;
-    const int vst = epi ? 1 : 0;
+    const int vst = epi ? 1 : 0, table = !epi && o.tab.t ? 1 : 0;
+    const int variant = vst ? 1 : table ? 2 : 0;
     if (epi) o.gat = *epi;
     const long long ntz = (z1 - z0 + WM_NZ - 1) / WM_NZ, nty = (H + WM_TY - 1) / WM_TY;
     CUtensorMap mg, mn;
     if ((W & 3) == 0 && !getenv("B4D_NO_TMA") &&
         make_map_4d(&mg, CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, gmap, W, H, D, nvol, WMT_GW, WM_EY, 1) &&
         make_map_4d(&mn, CU_TENSOR_MAP_DATA_TYPE_INT64, 8, numq, W, H, D, nvol, WMT_TX, WM_TY, 1)) {
-        auto kernel = vst ? k_normalise_wm_tma<true> : k_normalise_wm_tma<false>;
-        static bool attr[2] = {false, false};
-        if (!attr[vst]) {
+        auto kernel = vst ? k_normalise_wm_tma<true, false>
+                          : table ? k_normalise_wm_tma<false, true> : k_normalise_wm_tma<false, false>;
+        static bool attr[3] = {false, false, false};
+        if (!attr[variant]) {
             cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WMT_NST * WMT_STAGE);
-            attr[vst] = true;
+            attr[variant] = true;
         }
         const long long blocks = (long long)nvol * ntz * nty * ((W + WMT_TX - 1) / WMT_TX);
         b4d_launch(kernel, (unsigned)blocks, WMT_WARPS * 32, WMT_NST * WMT_STAGE, s, mg, mn, fallback, o, D, H, W,
@@ -766,7 +929,8 @@ static void launch_norm(const long long *numq, const uint32_t *gmap, const float
         return;
     }
     const long long tiles = (long long)nvol * ntz * nty * ((W + WM_TX - 1) / WM_TX);
-    b4d_launch(vst ? k_normalise_wm<true> : k_normalise_wm<false>, (unsigned)((tiles + WM_WARPS - 1) / WM_WARPS),
+    b4d_launch(vst ? k_normalise_wm<true, false> : table ? k_normalise_wm<false, true> : k_normalise_wm<false, false>,
+               (unsigned)((tiles + WM_WARPS - 1) / WM_WARPS),
                WM_WARPS * 32, 0, s, numq, gmap, fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf[0], kf[1], kf[2],
                kf[3]);
 }
@@ -792,6 +956,17 @@ void b4d_launch_normalise_q16(const long long *numq, const uint32_t *gmap, const
     o.q_trunc = trunc;
     launch_norm(numq, gmap, fallback, o, D, H, W, nvol, z0, z1, inv_qscale, kf, epi, s);
 }
+void b4d_launch_normalise_qt16(const long long *numq, const uint32_t *gmap, const float *fallback, uint16_t *q16, int D,
+                               int H, int W, int z0, int z1, float inv_qscale, const float kf[4], float offset_sub,
+                               float offset_add, const StepTab &tab, int trunc, cudaStream_t s) {
+    NormOut o{};
+    o.q16 = q16;
+    o.q_sub = offset_sub;
+    o.q_add = offset_add;
+    o.q_trunc = trunc;
+    o.tab = tab;
+    launch_norm(numq, gmap, fallback, o, D, H, W, 1, z0, z1, inv_qscale, kf, nullptr, s);
+}
 void b4d_launch_normalise_match(const long long *numq, const uint32_t *gmap, const float *fallback, float *out,
                                 uint16_t *match, float mscale, int ishift, int D, int H, int W, int nvol,
                                 float inv_qscale, const float kf[4], cudaStream_t s) {
@@ -809,6 +984,30 @@ void b4d_launch_quantize(const float *in, uint16_t *out, long long n, float offs
 void b4d_launch_quantize_trunc(const float *in, uint16_t *out, long long n, float offset_sub, float offset_add,
                                float step, cudaStream_t s) {
     b4d_launch(k_quantize<true>, grid_for(n >> 4, 256, 8), 256, 0, s, in, out, n, offset_sub, offset_add, step);
+}
+static unsigned tiled_grid(int D, int H) {
+    return grid_for(((long long)D * H + QT_WARPS - 1) / QT_WARPS, 1, 16);
+}
+static bool vec4_ok(const void *a, unsigned a_align, const void *b, unsigned b_align, int W) {
+    return (W & 3) == 0 && (reinterpret_cast<uintptr_t>(a) & (a_align - 1)) == 0 &&
+           (reinterpret_cast<uintptr_t>(b) & (b_align - 1)) == 0;
+}
+void b4d_launch_quantize_tiled(const float *in, uint16_t *out, int D, int H, int W, float offset_sub, float offset_add,
+                               const StepTab &tab, int trunc, cudaStream_t s) {
+    const unsigned g = tiled_grid(D, H);
+    const bool v4 = vec4_ok(in, 16, out, 8, W);
+    if (trunc) {
+        if (v4) b4d_launch(k_quantize_tiled<true, 4>, g, QT_WARPS * 32, 0, s, in, out, D, H, W, offset_sub, offset_add, tab);
+        else b4d_launch(k_quantize_tiled<true, 1>, g, QT_WARPS * 32, 0, s, in, out, D, H, W, offset_sub, offset_add, tab);
+    } else {
+        if (v4) b4d_launch(k_quantize_tiled<false, 4>, g, QT_WARPS * 32, 0, s, in, out, D, H, W, offset_sub, offset_add, tab);
+        else b4d_launch(k_quantize_tiled<false, 1>, g, QT_WARPS * 32, 0, s, in, out, D, H, W, offset_sub, offset_add, tab);
+    }
+}
+void b4d_launch_dequantize_tiled(const uint16_t *in, float *out, int D, int H, int W, float offset_sub,
+                                 float offset_add, const StepTab &tab, cudaStream_t s) {
+    b4d_launch(k_dequantize_tiled, tiled_grid(D, H), QT_WARPS * 32, 0, s, in, out, D, H, W, offset_sub, offset_add, tab,
+               vec4_ok(in, 8, out, 16, W) ? 1 : 0);
 }
 void b4d_launch_chunk_shuffle(const uint16_t *in, int D, int H, int W, int cz, int cy, int cx, uint8_t *out,
                               uint32_t *hist, cudaStream_t s) {

@@ -1,6 +1,7 @@
 """BASELINE configs[4] end to end on the GPU box: one uint16 volume (default 1024 x 2048 x 2048, z,y,x)
 sharded in z-slabs over the ranks -> tile statistics (histogram all-gather) -> BM4D denoise (13-plane
-halos + one neighbour exchange) -> offset-subtract + quantize at step 1 and at step = kappa * sigma ->
+halos + one neighbour exchange) -> offset-subtract + quantize at step 1, at step = kappa * sigma and at
+a step per 64^3 chunk (kappa * the chunk's noise_sigma, the table assembled by an all-gather of the ranks' rows) ->
 64^3 chunk gather + byte shuffle + byte counts on the device -> entropy bound of the compressed size,
 and real zstd (host, system libzstd) on a sample of the shuffled pieces.  numcodecs/Blosc is absent
 here, so the zstd figure approximates the reference's cratio (b4d/codec.py).  Developer tool.
@@ -56,6 +57,10 @@ def main():
     dn = b4d.Denoiser(local)
     slab = make_slab((D, H, W), zb, ze, dev)
     own = slab[own_b - zb : own_e - zb]
+    # the per-chunk variant: every rank measures sigma on whole 64-plane tile layers of its own planes
+    if D % (64 * world):
+        raise SystemExit("the step-per-chunk variant needs D divisible by 64 x ranks (owned planes = whole tile layers)")
+    assert own_b % 64 == 0 and (own_e - own_b) % 64 == 0, (own_b, own_e)
 
     def barrier():
         torch.cuda.synchronize()
@@ -71,19 +76,27 @@ def main():
         else:
             y = dn.denoise_slab(slab, zb, D, own_b, own_e, SIGMA)
         step_k = b4d.noise_scaled_step(st["sigma"], args.kappa)
+        rows = torch.from_numpy(dn.noise_sigma(own, tile=(64, 64, 64))["sigma"]).to(dev)
+        if world > 1:
+            parts = [torch.empty_like(rows) for _ in range(world)]
+            dist.all_gather(parts, rows)
+            rows = torch.cat(parts, 0)
+        table = b4d.noise_scaled_steps(rows, args.kappa, (64, 64, 64))
         q1 = dn.quantize(y, offset_sub=float(st["offset"]), offset_add=0.0, step=1.0)
         qk = dn.quantize(y, offset_sub=float(st["offset"]), offset_add=0.0, step=step_k)
+        qt = dn.quantize(y, offset_sub=float(st["offset"]), offset_add=0.0, step=table, z_begin=own_b)
         del y
         s1 = dn.chunk_shuffle(q1, (64, 64, 64))
         sk = dn.chunk_shuffle(qk, (64, 64, 64))
-        return st, step_k, s1, sk
+        stt = dn.chunk_shuffle(qt, (64, 64, 64))
+        return st, step_k, table, s1, sk, stt
 
     step(); barrier()
     ext = torch.cuda.ExternalStream(dn.stream_ptr(), device=dev)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(ext)
     for _ in range(args.steps):
-        st, step_k, s1, sk = step()
+        st, step_k, table, s1, sk, stt = step()
     e1.record(ext); barrier()
     t = torch.tensor([e0.elapsed_time(e1) * 1e-3 / args.steps], dtype=torch.float64, device=dev)
     if world > 1:
@@ -95,7 +108,7 @@ def main():
     pick = np.linspace(0, len(grid) - 1, min(args.zstd_pieces, len(grid))).astype(int)
     tot = []
     t_host = time.perf_counter()
-    for by, hist in (s0, s1, sk):
+    for by, hist in (s0, s1, sk, stt):
         h = hist.cpu().numpy()
         raw_b, ent_b = float(h.sum()), float(np.maximum(codec.entropy_bytes(h), 1.0).sum())
         zu = zc = 0.0
@@ -111,8 +124,10 @@ def main():
     if world > 1:
         dist.all_reduce(tt)
     if rank == 0:
-        tt = tt.cpu().numpy().reshape(3, 4)
-        names = ("noisy input", "denoised, step 1", "denoised, step %.3g (kappa %.2g)" % (step_k, args.kappa))
+        tt = tt.cpu().numpy().reshape(4, 4)
+        names = ("noisy input", "denoised, step 1", "denoised, step %.3g (kappa %.2g)" % (step_k, args.kappa),
+                 "denoised, step per 64^3 chunk (kappa %.2g, steps %.3g .. %.3g)"
+                 % (args.kappa, float(table.steps.min()), float(table.steps.max())))
         res = {
             "config": "BASELINE configs[4]: %dx%dx%d uint16, denoise + offset + quantize + chunk shuffle, %d x B200" % (D, H, W, world),
             "seconds_per_volume_device": float(t.item()), "voxels_per_s": D * H * W / float(t.item()),
